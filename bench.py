@@ -2,7 +2,7 @@
 """bench.py -- encode throughput of the fractal encoder hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--size S] [--block B] [--pattern structured|noise]
+                    [--size S] [--block B] [--pattern structured|noise] [--dump-outputs DIR]
 
 One "step" = one full encode (pool build + range x domain search + code solve) of one
 synthetic greyscale image with the whole domain pool as the search window
@@ -55,7 +55,35 @@ def parse():
     ap.add_argument("--no-lena", action="store_true", help="skip the bundled-image object (BASELINE configs[0], [1], [4])")
     ap.add_argument("--parity-ranges", type=int, default=128,
                     help="range blocks of the timed result compared with the CPU oracle after the timed loop (0: skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the codes of the last timed step to DIR/*.npy (--impl ours), so that two builds can be "
+                         "compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+DUMP_LIMIT = 64 << 20   # bytes of all arrays --dump-outputs writes
+
+
+def dump_outputs(out_dir, info, q, seed=2026):
+    """Writes what a caller of the timed encode receives: info.npy (imageInfo floats, float32) and codes.npy (the
+    writeData ints, as float64, which holds every int32 exactly).  Above DUMP_LIMIT a fixed, seeded sample of range
+    blocks is written instead, with their indices in rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"info": np.asarray(info, np.float32), "codes": np.asarray(q, np.float64)}
+    NR = info.shape[0]
+    row_bytes = sum(a.itemsize * a.shape[1] for a in arrays.values())
+    if NR * row_bytes > DUMP_LIMIT:
+        n = (DUMP_LIMIT - 4096) // (row_bytes + 8)   # 8: the float64 row index; 4096: room for the .npy headers
+        rows = np.sort(np.random.default_rng(seed).choice(NR, n, replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def peaks():
@@ -436,6 +464,9 @@ def run_ours(args):
     sampler.start()
     total_ms, kernel_ms, search_ms, pool_ms, launches = timed(step_device, args.steps, True)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        res_info, res_q = (d_info, d_q) if world == 1 else last_out
+        dump_outputs(args.dump_outputs, res_info.cpu().numpy(), res_q.cpu().numpy())
     t = handle.timings()
     engine = t.engine
     step_evals = t.search_evals  # this rank's evaluations per step
