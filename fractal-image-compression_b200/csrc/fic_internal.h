@@ -75,7 +75,7 @@ int launch_solve(const Work &w, const Geom &g, int64_t j0, int64_t j1, float *d_
 // bare tcgen05.mma loop (M = 128, N = n_cols in {128, 256}): measured dense rate of kind::i8 (f16 = 0) or
 // kind::f16 on this GPU in TOP/s (< 0 on error)
 double measure_mma_peak(int num_sms, cudaStream_t s, int reps, int f16, int n_cols, const char **err);
-double measure_mma_peak_pair(int num_sms, cudaStream_t s, int reps, int f16, uint32_t *tmem_bases, const char **err, int a_in_tmem = 0);
+double measure_mma_peak_pair(int num_sms, cudaStream_t s, int reps, int f16, uint32_t *tmem_bases, const char **err);
 // 1: kind::f16 accumulators are the exact integer covariances on this device; 0: not; < 0: CUDA error
 int umma_f16_selftest(int num_sms, cudaStream_t s, const char **err);
 bool umma_applicable(const Geom &g);
@@ -88,13 +88,14 @@ size_t umma_opB_bytes(const Geom &g, int kind);
 // device table: sweep position -> domain index (-1: padding), valid after a launch; probe only
 void umma_debug_positions(const Work &w, const Geom &g, int64_t rows, int num_sms, int kind,
                           const int32_t **d_pos_dom, int64_t *npos);
+// k0 / k1 (optional): events recorded around the search kernel.  pair: FIC_UMMA_PAIR_AUTO / _ON / _OFF; *pair_used
+// (optional) = 1 if the CTA-pair kernel ran.  dump (optional, probe / self-test): every accumulator (kov) of every
+// (operand row, sweep position) pair, row stride dump_ld; status_dev (optional, mapped host memory): the code of a
+// pipeline wait that timed out.
 int launch_search_umma(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms,
                        cudaStream_t s, const char **err, int kind, cudaEvent_t k0 = nullptr,
-                       cudaEvent_t k1 = nullptr, int pair = 0 /* FIC_UMMA_PAIR_AUTO */, int *pair_used = nullptr);
-int launch_search_umma_debug(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms,
-                             cudaStream_t s, const char **err, int kind, int32_t *dump, int64_t dump_ld,
-                             int *status_dev, int variant, uint32_t dbg = 0, cudaEvent_t k0 = nullptr,
-                             cudaEvent_t k1 = nullptr, int *pair_used = nullptr);
+                       cudaEvent_t k1 = nullptr, int pair = FIC_UMMA_PAIR_AUTO, int *pair_used = nullptr,
+                       int32_t *dump = nullptr, int64_t dump_ld = 0, int *status_dev = nullptr);
 
 // decoder
 int launch_dequant(const int32_t *d_q, float *d_code, int32_t *d_off, const Geom &g, int unquantised,

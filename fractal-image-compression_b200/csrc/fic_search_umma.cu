@@ -77,7 +77,7 @@
 //               tcgen05.ld.32x32b.x32, one hand-back (t_empty[q]); the tile's bounds come from
 //               the blob in global memory at the top of each tile.  Rare paths (flag recording,
 //               mbarrier polling) are out of line.  kind::f16, B <= 8: the four loads are software-pipelined
-//               (template parameter EPI).
+//               (epilogue loop epi_of<B, F16, PAIR>).
 // A work unit is (super-block of 512 rows) x (1/n_chunks of the domain tiles); units are
 // ordered chunk-major and a row's lower bound is carried from unit to unit (row_lb).  (RGB at B = 16:
 // 256-row super-blocks, two of the four accumulators, Cfg<16, true>.)
@@ -119,8 +119,8 @@ constexpr int kBoundBytes = kChunksPerTile * 2 * 4 + 16 + kChunksPerTile * 4;
 constexpr int kNormOff = kChunksPerTile * 2 * 4 + 16;     // offset of the norms inside the bounds area
 // Flag lists of a (row, unit): two lists (column halves of the tiles, a historical split) of 32 entries each.
 constexpr int kFlagBytes = 4 * (4 + 8 * 16);         // per (row, unit): list lengths + entries (with slack)
-__host__ __device__ constexpr int kListsOf(int) { return 2; }
-__host__ __device__ constexpr int kCapOf(int) { return 32; }
+constexpr int kFlagLists = 2;
+constexpr int kFlagCap = 32;
 constexpr float kOneMinusEps = 1.0f - 1.9073486328125e-06f;  // 1 - 2^-19 (applied to the squared score)
 
 // Operand geometry of one (block size, MMA kind) pair.  F16 = false: kind::i8, two s8 digits per
@@ -263,10 +263,10 @@ __device__ __noinline__ float flag_threshold(float lb, float tie_abs)  // rare p
 // threshold.
 // share != 0: publish a raised bound to `sh_lb` (isometry rows share one bound).
 struct RowFilter { float thresh, lbmax; int cnt; };
-__device__ __noinline__ RowFilter flag_chunk(RowFilter st, float lb, float ub, float tie_abs, int2 *list, int cap,
-                                             int chunk_id, uint32_t sh_lb, int share)
+__device__ __noinline__ RowFilter flag_chunk(RowFilter st, float lb, float ub, float tie_abs, int2 *list, int chunk_id,
+                                             uint32_t sh_lb, int share)
 {
-    if (st.cnt < cap) list[st.cnt] = make_int2(chunk_id, __float_as_int(ub));
+    if (st.cnt < kFlagCap) list[st.cnt] = make_int2(chunk_id, __float_as_int(ub));
     st.cnt++;
     if (lb > st.lbmax) {
         st.lbmax = lb;
@@ -1059,15 +1059,20 @@ constexpr uint32_t kIdescF16Pair = (1u << 4) | (0u << 7) | (0u << 10) | ((uint32
 
 // ---------------------------------------------------------------- the search kernel --
 
-// DBG (probe builds only): 1 = skip the scoring, 3 = skip the TMEM loads too, 4 = issue the MMAs of the first tile
-// of a unit only (the epilogue alone), 8 = count the cycles an epilogue warp spends in each phase (into `dump`).  DUMP: write every
-// accumulator to `dump` (the probe's exactness check).  The product runs <B, 0, false>.
-// EPI selects how an epilogue warp walks its accumulator (warp e owns lane quarter e % 4 of accumulator e / 4 in every
-// variant).  0: load a 32-column chunk, evaluate it, load the next.  2 (kind::f16): software-pipelined -- the load of
-// the next chunk is issued behind the first level of the current chunk's max tree.  3 (kind::f16): as 2, and the four
-// flag tests wait until the accumulator has been handed back.  (A fourth mapping -- every warp takes one chunk of
-// EVERY accumulator, so that the oldest accumulator is drained by four warps at once -- handed accumulators back
-// soonest and still lost on every configuration to its four waits per tile; profiles/README.md.)
+// How an epilogue warp walks its accumulator (warp e owns lane quarter e % 4 of accumulator e / 4 in every loop).
+// 0: load a 32-column chunk, evaluate it, load the next.  2 (kind::f16): software-pipelined -- the load of the next
+// chunk is issued behind the first level of the current chunk's max tree.  3 (kind::f16): as 2, and the four flag
+// tests wait until the accumulator has been handed back.  Each configuration runs the loop measured fastest for it
+// (profiles/README.md): kind::f16 B = 8 gains 1.5-5 % from the pipelined loads, B = 4 (epilogue bound) 10 % from
+// deferring the flag tests as well, and the pairs at B <= 8 (the tensor pipe at its full rate) 10 % from the earlier
+// hand-back.  (A fourth mapping -- every warp takes one chunk of EVERY accumulator, so that the oldest accumulator is
+// drained by four warps at once -- handed accumulators back soonest and still lost on every configuration to its four
+// waits per tile.)
+template <int B, bool F16, bool PAIR>
+__host__ __device__ constexpr int epi_of() { return (!F16 || B == 16) ? 0 : ((B == 4 || PAIR) ? 3 : 2); }
+
+// DUMP: write every accumulator to `dump` (the probe's and the self-test's exactness check); runs the plain loop.
+// status: where a bounded mbarrier wait that timed out leaves its code before the trap (null: nowhere).
 //
 // PAIR: the kernel runs as clusters of two CTAs (one TPC) sharing every tcgen05.mma (cta_group::2, M = 256, N = 128):
 // each CTA keeps its own super-block (its 4 x 128 accumulator rows in its own TMEM) and supplies HALF of every domain
@@ -1076,16 +1081,16 @@ constexpr uint32_t kIdescF16Pair = (1u << 4) | (0u << 7) | (0u << 10) | ((uint32
 // multicast to both CTAs' barriers; CTA 1's warp 1 relays "my half has landed" to CTA 0's full barriers and CTA 1's
 // epilogue warps hand accumulators back on CTA 0's t_empty barriers (remote mbarrier arrives).  The epilogue is
 // the same code in both CTAs.  n_sb must be even.
-template <int B, bool F16, int DBG, bool DUMP, int EPI, bool PAIR = false>
+template <int B, bool F16, bool PAIR, bool DUMP>
 __global__ void __launch_bounds__(kThreads, 1)
 k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, const int32_t *__restrict__ vRarr,
               const float *__restrict__ nRarr, int2 *__restrict__ flag_list, int32_t *__restrict__ flag_cnt, uint32_t *__restrict__ row_lb, int n_sb,
-              int n_chunks, int ntiles, int iso_shift, int64_t rows_padded, int32_t *__restrict__ dump, int64_t dump_ld, volatile int *status,
-              uint32_t lbo_bytes_a, uint32_t sbo_bytes_a, uint32_t lbo_bytes_b, uint32_t sbo_bytes_b)
+              int n_chunks, int ntiles, int iso_shift, int64_t rows_padded, int32_t *__restrict__ dump, int64_t dump_ld, volatile int *status)
 {
     using C = Cfg<B, F16>;
     using L = Lay<B, F16>;
     static_assert(!PAIR || F16 || C::KSPLIT, "CTA pairs: kind::f16, or the K-split configurations (B = 16)");
+    constexpr int EPI = DUMP ? 0 : epi_of<B, F16, PAIR>();
     // issuing warps of a pair: two for the whole-tile kernels (see below); one where a tile is 9-17 K-slices per
     // accumulator (K-split: the issuing thread is not the bottleneck there)
     constexpr int NISS = (PAIR && !C::KSPLIT) ? 2 : 1;
@@ -1218,10 +1223,7 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                 // ===================== MMA issuer of a K-split pair (CTA 0, one warp) =====================
                 uint32_t stage = 0, phase = 0, a_phase = 0, t_phase = 0;
                 const uint32_t elected = elect_one();
-                const long long clk0 = clock64();
-                unsigned long long ns0 = 0;
-                if (status) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns0));
-                const uint64_t a_desc0 = make_desc(smem_u32(sA), lbo_bytes_a, sbo_bytes_a);
+                const uint64_t a_desc0 = make_desc(smem_u32(sA), 128, L::SBO_A);
                 for (int u = u_first; u < n_units; u += u_step) {
                     int ch = u / n_sbu;
                     int t0 = (int)((int64_t)ch * ntiles / n_chunks), t1 = (int)((int64_t)(ch + 1) * ntiles / n_chunks);
@@ -1238,7 +1240,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                             if (elected) {
 #pragma unroll
                                 for (int s = 0; s < L::KS0; s++) {
-                                    if ((DBG & 4) && t != t0) continue;  // probe only: epilogue without the tensor pipe
                                     const uint64_t ad = a_desc0 + (uint64_t)((q * L::A_BLOCK_BYTES + s * 256) >> 4);
                                     if (F16) tc_mma2_f16(tmem_base + q * kTileN, ad, b0 + (uint64_t)((s * 256) >> 4), kIdescF16Pair, s > 0 ? 1u : 0u);
                                     else tc_mma2_i8(tmem_base + q * kTileN, ad, b0 + (uint64_t)((s * 256) >> 4), kIdescPair, s > 0 ? 1u : 0u);
@@ -1260,7 +1261,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                                 if (elected) {
 #pragma unroll
                                     for (int s = 0; s < C::KS_B - L::KS0; s++) {
-                                        if ((DBG & 4) && t != t0) continue;
                                         const int sa = F16 ? L::KS0 + s : s;  // kind::i8: the low digits meet the r slices again
                                         const uint64_t ad = a_desc0 + (uint64_t)((q * L::A_BLOCK_BYTES + sa * 256) >> 4);
                                         if (F16) tc_mma2_f16(tmem_base + q * kTileN, ad, b1 + (uint64_t)((s * 256) >> 4), kIdescF16Pair, 1u);
@@ -1278,16 +1278,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                     if (elected) tc_commit2(BAR_A_EMPTY, 3u);
                     __syncwarp();
                     a_phase ^= 1;
-                }
-                if (status && blockIdx.x == 0 && elected) {
-                    const long long dt = clock64() - clk0;
-                    unsigned long long ns1;
-                    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns1));
-                    status[2] = (int)(dt & 0x7fffffff);
-                    status[3] = (int)(dt >> 31);
-                    status[4] = (int)(ns1 - ns0);
-                    status[5] = 0;
-                    status[6] = 0;
                 }
             } else {
                 // ===================== relay (CTA 1 of a K-split pair) =====================
@@ -1320,38 +1310,24 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                 const int qi = warp >> 1;  // 0 or 1
                 uint32_t stage = 0, phase = 0, a_phase = 0, t_phase = 0;
                 const uint32_t elected = elect_one();
-                const long long clk0 = clock64();
-                unsigned long long ns0 = 0;
-                if (status) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns0));
-                const uint64_t a_desc0 = make_desc(smem_u32(sA), lbo_bytes_a, sbo_bytes_a);
-                const uint64_t b_desc0 = make_desc(smem_u32(sB), lbo_bytes_b, sbo_bytes_b);
-                uint32_t iw_t = 0, iw_b = 0;
-                uint32_t ts_e[2] = {0, 0}, ts_i[2] = {0, 0};
+                const uint64_t a_desc0 = make_desc(smem_u32(sA), 128, L::SBO_A);
+                const uint64_t b_desc0 = make_desc(smem_u32(sB), 128, L::SBO_B);
                 for (int u = u_first; u < n_units; u += u_step) {
                     int ch = u / n_sbu;
                     int t0 = (int)((int64_t)ch * ntiles / n_chunks), t1 = (int)((int64_t)(ch + 1) * ntiles / n_chunks);
                     mbar_wait(BAR_A_FULL, a_phase, status, 3);
                     for (int t = t0; t < t1; t++) {
-                        const uint32_t wb0 = (DBG & 8) ? (uint32_t)clock() : 0u;
                         mbar_wait(BAR_B_FULL(stage), phase, status, 4);  // both halves: this CTA's copy + the peer's relayed arrival
-                        if (DBG & 8) iw_b += (uint32_t)clock() - wb0;
                         tc_fence_after();
                         const uint64_t b_desc = b_desc0 + (uint64_t)((stage * SLOT) >> 4);
 #pragma unroll
                         for (int k = 0; k < 2; k++) {
                             const int q = qi + 2 * k;
-                            const uint32_t w0 = (DBG & 8) ? (uint32_t)clock() : 0u;
                             mbar_wait(BAR_T_EMPTY(q), ((t_phase >> k) & 1) ^ 1, status, 5);  // the epilogue warps of both CTAs
-                            if (DBG & 8) {
-                                const uint32_t now = (uint32_t)clock();
-                                iw_t += now - w0;
-                                ts_e[k] += now;
-                            }
                             tc_fence_after();
                             if (elected) {
 #pragma unroll
                                 for (int s = 0; s < C::NS; s++) {
-                                    if ((DBG & 4) && t != t0) continue;  // probe only: epilogue without the tensor pipe
                                     const uint64_t ad = a_desc0 + (uint64_t)((q * L::A_BLOCK_BYTES + C::amap(s) * 256) >> 4);
                                     tc_mma2_f16(tmem_base + q * kTileN, ad, b_desc + (uint64_t)((s * 256) >> 4), kIdescF16Pair, s > 0 ? 1u : 0u);
                                 }
@@ -1359,7 +1335,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                                 if (k == 1) tc_commit2(BAR_B_EMPTY(stage), 3u);  // this issuer's MMAs have read both CTAs' slots
                             }
                             __syncwarp();
-                            if (DBG & 8) ts_i[k] += (uint32_t)clock();
                             t_phase ^= 1u << k;
                         }
                         if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
@@ -1367,22 +1342,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                     if (elected) tc_commit2(BAR_A_EMPTY, 3u);  // this issuer's MMAs on the A super-block have completed
                     __syncwarp();
                     a_phase ^= 1;
-                }
-                if (status && blockIdx.x == 0 && elected && qi == 0) {
-                    const long long dt = clock64() - clk0;
-                    unsigned long long ns1;
-                    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns1));
-                    status[2] = (int)(dt & 0x7fffffff);
-                    status[3] = (int)(dt >> 31);
-                    status[4] = (int)(ns1 - ns0);  // the same interval in nanoseconds: the SM's real clock under load
-                    status[5] = (int)iw_t;
-                    status[6] = (int)iw_b;
-                }
-                if ((DBG & 8) && dump && blockIdx.x == 0 && elected) {
-                    for (int k = 0; k < 2; k++) {
-                        dump[32768 + qi + 2 * k] = (int32_t)ts_e[k];
-                        dump[32768 + kAccs + qi + 2 * k] = (int32_t)ts_i[k];
-                    }
                 }
             } else if (warp == 1) {
                 // ===================== relay (CTA 1 of a pair) =====================
@@ -1413,22 +1372,15 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
         // uniform registers; one elected lane issues tcgen05.mma / tcgen05.commit.
         uint32_t stage = 0, phase = 0, a_phase = 0, t_phase = 0;  // t_phase: bit q
         const uint32_t elected = elect_one();
-        const long long clk0 = clock64();  // probe only (status != nullptr): elapsed SM clocks of CTA 0's issuer
-        unsigned long long ns0 = 0;
-        if (status) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns0));
         // descriptors differ only in the 14-bit start-address field (16-byte units)
-        const uint64_t a_desc0 = make_desc(smem_u32(sA), lbo_bytes_a, sbo_bytes_a);
-        const uint64_t b_desc0 = make_desc(smem_u32(sB), lbo_bytes_b, sbo_bytes_b);
-        uint32_t iw_t = 0, iw_b = 0;  // DBG & 8: clocks the issuer spent waiting for accumulators / for domain tiles
-        uint32_t ts_e[kAccs] = {0, 0, 0, 0}, ts_i[kAccs] = {0, 0, 0, 0};  // DBG & 8: sums (mod 2^32) of the clock at "accumulator free seen" / "MMAs issued"
+        const uint64_t a_desc0 = make_desc(smem_u32(sA), 128, L::SBO_A);
+        const uint64_t b_desc0 = make_desc(smem_u32(sB), 128, L::SBO_B);
         for (int u = u_first; u < n_units; u += u_step) {
             int ch = u / n_sbu;
             int t0 = (int)((int64_t)ch * ntiles / n_chunks), t1 = (int)((int64_t)(ch + 1) * ntiles / n_chunks);
             mbar_wait(BAR_A_FULL, a_phase, status, 3);
             for (int t = t0; t < t1; t++) {
-                const uint32_t wb0 = (DBG & 8) ? (uint32_t)clock() : 0u;
                 mbar_wait(BAR_B_FULL(stage), phase, status, 4);
-                if (DBG & 8) iw_b += (uint32_t)clock() - wb0;
                 tc_fence_after();
                 // tile flag written by k_umma_pack_domains: 0 -> every low digit of the tile is zero
                 const uint32_t has_l = *(volatile const uint32_t *)(sB + stage * L::SLOT_BYTES + L::B_OP_BYTES + kChunksPerTile * 8);
@@ -1443,7 +1395,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                         if (elected) {
 #pragma unroll
                             for (int s = 0; s < L::KS0; s++) {
-                                if ((DBG & 4) && t != t0) continue;  // probe only: epilogue without the tensor pipe
                                 const uint64_t ad = a_desc0 + (uint64_t)((q * L::A_BLOCK_BYTES + s * 256) >> 4);  // A slice s (kind::i8: s = 8 is rmean)
                                 if (F16) tc_mma_f16(tmem_base + q * kTileN, ad, b0 + (uint64_t)((s * 256) >> 4), kIdescF16, s > 0 ? 1u : 0u);
                                 else tc_mma_i8(tmem_base + q * kTileN, ad, b0 + (uint64_t)((s * 256) >> 4), kIdesc, s > 0 ? 1u : 0u);
@@ -1465,7 +1416,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                             if (elected) {
 #pragma unroll
                                 for (int s = 0; s < C::KS_B - L::KS0; s++) {
-                                    if ((DBG & 4) && t != t0) continue;
                                     // kind::i8: the low digits meet the r slices again; kind::f16: the second half of K
                                     const int sa = F16 ? L::KS0 + s : s;
                                     const uint64_t ad = a_desc0 + (uint64_t)((q * L::A_BLOCK_BYTES + sa * 256) >> 4);
@@ -1490,7 +1440,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                     if (elected) {
 #pragma unroll
                         for (int s = 0; s < C::NS; s++) {
-                            if ((DBG & 4) && t != t0) continue;        // probe only: epilogue without the tensor pipe
                             if (C::is_l_slice(s) && !has_l) continue;  // sum r*l == 0 for the whole tile
                             const uint64_t ad = a_desc0 + (uint64_t)((q * L::A_BLOCK_BYTES + C::amap(s) * 256) >> 4);
                             const uint64_t bd = b_desc + (uint64_t)((s * 256) >> 4);
@@ -1509,22 +1458,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
             if (elected) tc_commit(BAR_A_EMPTY);  // every MMA that reads this A super-block has completed
             __syncwarp();
             a_phase ^= 1;
-        }
-        if (status && blockIdx.x == 0 && elected) {
-            const long long dt = clock64() - clk0;
-            unsigned long long ns1;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns1));
-            status[2] = (int)(dt & 0x7fffffff);
-            status[3] = (int)(dt >> 31);
-            status[4] = (int)(ns1 - ns0);  // the same interval in nanoseconds: the SM's real clock under load
-            status[5] = (int)iw_t;
-            status[6] = (int)iw_b;
-            if ((DBG & 8) && dump) {
-                for (int q = 0; q < kAccs; q++) {
-                    dump[32768 + q] = (int32_t)ts_e[q];
-                    dump[32768 + kAccs + q] = (int32_t)ts_i[q];
-                }
-            }
         }
     } else if (warp >= 4) {
         // ===================== epilogue =====================
@@ -1546,18 +1479,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
         // round once partial sums pass 2^24; see the chunk test below.  Warps of unused accumulators idle.
         constexpr bool SLACK = B == 16 && F16;
         const int n_units_mine = q < C::NB ? n_units : 0;
-        // DBG & 8 (probe only): per-warp cycle accounting of the epilogue phases.  tcgen05.wait::ld is a
-        // scoreboard wait, so the TMEM latency shows up at the first use of the loaded registers ("math").
-        uint32_t tk_b = 0, tk_t = 0, tk_l = 0, tk_m = 0, tk_mark = 0;
-        uint32_t ts_f = 0, ts_h = 0;  // DBG & 8: sums (mod 2^32) of the clock at "t_full seen" / "handed back"
-        const uint32_t tk_begin = (DBG & 8) ? (uint32_t)clock() : 0u;
-        auto tick = [&](uint32_t &acc) {
-            if (DBG & 8) {
-                const uint32_t now = (uint32_t)clock();
-                acc += now - tk_mark;
-                tk_mark = now;
-            }
-        };
         for (int u = u_first; u < n_units_mine; u += u_step) {
             // Units are ordered chunk-major (u = ch * n_sb + sb): the units of one super-block run in different
             // waves, so the lower bound a row reached in an earlier unit (row_lb, global memory) can seed the
@@ -1589,9 +1510,8 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                     st.thresh = flag_threshold(seed, tie_abs);
                 }
             }
-            int2 *const list0 = flag_list + (((int64_t)ch * rows_padded + row) * 2) * kCapOf(0);
+            int2 *const list0 = flag_list + (((int64_t)ch * rows_padded + row) * kFlagLists) * kFlagCap;
             int cnt0 = 0, cnt1 = 0;  // entries of the two lists (column halves) of this (row, unit)
-            if (DBG & 8) tk_mark = (uint32_t)clock();
             for (int t = t0; t < t1; t++) {
                 // (rhi, rlo) of the tile's four chunks, from the tile blob in global memory (the shared-memory ring
                 // belongs to the producer and the MMA issuer alone): a broadcast load that every warp of the CTA
@@ -1600,7 +1520,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                 const float4 bnd01 = __ldg(gb), bnd23 = __ldg(gb + 1);
                 float4 bndn = make_float4(0.0f, 0.0f, 0.0f, 0.0f);  // >= ||gD||_2 of the rows of each chunk
                 if (SLACK) bndn = __ldg(gb + 3);
-                tick(tk_b);
                 mbar_wait(BAR_T_FULL(q), tf_phase, status, 7);
                 tc_fence_after();
                 if (iso_shift) {  // adopt a better bound found by another isometry of the same range block
@@ -1610,9 +1529,7 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                         st.thresh = flag_threshold(other, tie_abs);
                     }
                 }
-                tick(tk_t);
-                if (DBG & 8) ts_f += tk_mark;
-                if constexpr ((EPI == 2 || EPI == 3) && F16 && !DUMP && !(DBG & 3)) {
+                if constexpr (EPI != 0) {
                     // Software-pipelined visit (kind::f16).  The first level of the |.| max tree reads all 32 registers
                     // of a chunk in 11 instructions; the load of the NEXT chunk is issued behind them (into the same
                     // registers) so that its TMEM latency hides behind the rest of the tree.  EPI == 3 also defers the
@@ -1629,7 +1546,7 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                         const float ub = Mc[c] * rhi;
                         if (ub > st.thresh) {  // may hold the winner or one of its float ties
                             st.cnt = c < 2 ? cnt0 : cnt1;
-                            st = flag_chunk(st, Mc[c] * rlo, ub, tie_abs, list0 + (c >> 1) * kCapOf(0), kCapOf(0), t * kChunksPerTile + c, sh_lb, iso_shift ? 1 : 0);
+                            st = flag_chunk(st, Mc[c] * rlo, ub, tie_abs, list0 + (c >> 1) * kFlagCap, t * kChunksPerTile + c, sh_lb, iso_shift ? 1 : 0);
                             if (c < 2) cnt0 = st.cnt;
                             else cnt1 = st.cnt;
                         }
@@ -1661,8 +1578,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                                 tc_fence_before();
                                 __syncwarp();
                                 if (lane == 0) hand_back();
-                                tick(tk_l);  // t_full seen -> accumulator handed back
-                                if (DBG & 8) ts_h += tk_mark;
                                 if (EPI == 3) {  // the deferred tests of the first three chunks, in sweep order
                                     asm volatile("" : "+f"(Mc[0]), "+f"(Mc[1]), "+f"(Mc[2]) : : "memory");
                                     test(0);
@@ -1673,23 +1588,18 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                         }
                     }
                     if (EPI == 3) test(kChunksPerTile - 1);
-                    tick(tk_m);  // hand-back -> end of the visit
                 } else {
 #pragma unroll
                 for (int c = 0; c < kChunksPerTile; c++) {
                     uint32_t v[32];
-                    if (!(DBG & 2)) {
-                        tmem_ld32(ta + c * 32, v);
-                        tmem_ld_wait();
-                    }
-                    tick(tk_l);
+                    tmem_ld32(ta + c * 32, v);
+                    tmem_ld_wait();
                     if (c == kChunksPerTile - 1) {
                         // last read of accumulator q for this tile: hand it back
                         tc_fence_before();
                         __syncwarp();
                         if (lane == 0) hand_back();
                     }
-                    if (DBG & 1) continue;  // probe only: measure the pipeline without the scoring
                     float M;  // max |kov| over the chunk, exact
                     if (F16) {
                         // binary32 accumulators holding exact integers.  FMNMX3 takes |.| on all three
@@ -1749,11 +1659,10 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                         // the refine step reads two lists per (row, unit), one per column half, as the layout of
                         // the earlier two-warps-per-accumulator mapping had it
                         st.cnt = c < 2 ? cnt0 : cnt1;
-                        st = flag_chunk(st, Ml * rlo, ub, tie_abs, list0 + (c >> 1) * kCapOf(0), kCapOf(0), t * kChunksPerTile + c, sh_lb, iso_shift ? 1 : 0);
+                        st = flag_chunk(st, Ml * rlo, ub, tie_abs, list0 + (c >> 1) * kFlagCap, t * kChunksPerTile + c, sh_lb, iso_shift ? 1 : 0);
                         if (c < 2) cnt0 = st.cnt;
                         else cnt1 = st.cnt;
                     }
-                    tick(tk_m);
                 }
                 }
                 tf_phase ^= 1;
@@ -1762,16 +1671,6 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
             flag_cnt[((int64_t)ch * rows_padded + row) * 2 + 1] = cnt1;
             // the row's bound after this unit: seeds its later units and lets the refine step drop stale flags
             if (st.lbmax > 0.0f) atomicMax(row_lb + ((row >> iso_shift) << iso_shift), __float_as_uint(st.lbmax));
-        }
-        if ((DBG & 8) && lane == 0 && dump) {
-            int32_t *o = dump + ((int64_t)blockIdx.x * kEpiWarps + e) * 8;
-            o[0] = (int32_t)((uint32_t)clock() - tk_begin);
-            o[1] = (int32_t)tk_b;
-            o[2] = (int32_t)tk_t;
-            o[3] = (int32_t)tk_l;
-            o[4] = (int32_t)tk_m;
-            o[5] = (int32_t)ts_f;
-            o[6] = (int32_t)ts_h;
         }
     }
 
@@ -1851,10 +1750,7 @@ __global__ void __launch_bounds__(128, 1) k_mma_peak(int iters, uint32_t seed)
 // The same loop issued by CTA pairs: tcgen05.mma.cta_group::2, M = 256 (128 rows per CTA), N = 128 (64 operand rows
 // per CTA): per MMA an SM reads 4 KB of A and 2 KB of B from its shared memory instead of 4 + 4.  out[blockIdx.x]
 // receives the CTA's TMEM base address (both CTAs of a pair must report the same one).
-// TS: the A operand comes from tensor memory (tcgen05.mma [d], [a_tmem], b_desc: 8 columns behind the accumulators)
-// instead of shared memory -- a probe of what the tensor pipe sustains under the board's power cap when an SM reads
-// only the B half-tile (2 KB per MMA) from shared memory.
-template <bool F16, bool TS = false>
+template <bool F16>
 __global__ void __launch_bounds__(128, 1) k_mma_peak_pair(int iters, uint32_t seed, uint32_t *out)
 {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -1877,7 +1773,7 @@ __global__ void __launch_bounds__(128, 1) k_mma_peak_pair(int iters, uint32_t se
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(TS ? 512u : 256u) : "memory");
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(256u) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
     }
     tc_fence_before();
@@ -1885,21 +1781,6 @@ __global__ void __launch_bounds__(128, 1) k_mma_peak_pair(int iters, uint32_t se
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     if (threadIdx.x == 0 && out) out[blockIdx.x] = tmem_base;
-    if (TS) {
-        // this warp's lane quarter of the A operand: 32 rows x 8 columns (one 32-byte K-slice per row)
-        uint32_t x = (uint32_t)threadIdx.x * 2654435761u + seed;
-        x ^= x >> 15; x *= 0x2c1b3c6du; x ^= x >> 12;
-        if (F16) x &= 0x3fff3fffu;
-        const uint32_t ta = tmem_base + ((uint32_t)(warp * 32) << 16) + 256u;
-        asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(ta), "r"(x), "r"(x ^ 0x01010101u),
-                     "r"(x ^ 0x02020202u), "r"(x ^ 0x03030303u), "r"(x ^ 0x04040404u), "r"(x ^ 0x05050505u), "r"(x ^ 0x06060606u),
-                     "r"(x ^ 0x07070707u)
-                     : "memory");
-        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-        tc_fence_before();
-        cluster_sync_all();
-        tc_fence_after();
-    }
     if (warp == 1) {
         if (rank == 0) {
             const uint32_t elected = elect_one();
@@ -1910,20 +1791,6 @@ __global__ void __launch_bounds__(128, 1) k_mma_peak_pair(int iters, uint32_t se
             if (elected) {
                 for (int i = 0; i < iters; i++) {
                     const uint32_t d = tmem_base + (uint32_t)(i & 1) * 128;
-                    if (TS) {
-                        const uint32_t acc = i >= 2 ? 1u : 0u;
-                        if (F16)
-                            asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                                         "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(d), "r"(tmem_base + 256u), "l"(bd),
-                                         "r"(idesc), "r"(acc)
-                                         : "memory");
-                        else
-                            asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                                         "tcgen05.mma.cta_group::2.kind::i8 [%0], [%1], %2, %3, p;\n\t}" ::"r"(d), "r"(tmem_base + 256u), "l"(bd),
-                                         "r"(idesc), "r"(acc)
-                                         : "memory");
-                        continue;
-                    }
                     if (F16) tc_mma2_f16(d, ad, bd, idesc, i >= 2 ? 1u : 0u);
                     else tc_mma2_i8(d, ad, bd, idesc, i >= 2 ? 1u : 0u);
                 }
@@ -1937,7 +1804,7 @@ __global__ void __launch_bounds__(128, 1) k_mma_peak_pair(int iters, uint32_t se
     cluster_sync_all();
     if (warp == 0) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TS ? 512u : 256u) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256u) : "memory");
     }
 }
 
@@ -1975,16 +1842,16 @@ __device__ __forceinline__ int refine_kov(const uint32_t *rw, int rmean, int vR,
 template <class F>
 __device__ __forceinline__ void for_each_flagged(int lane, int64_t i, int64_t rows_padded, int n_chunks, int64_t npos,
                                                  const int2 *__restrict__ flag_list, const int32_t *__restrict__ flag_cnt,
-                                                 float th, int lpu, int cap, F &&consider)
+                                                 float th, F &&consider)
 {
-    const int n_lists = lpu * n_chunks;  // (unit of the row, list of the unit): lpu = kListsOf(EPI) <= 4, n_chunks <= 8
-    const int my_cnt = lane < n_lists ? flag_cnt[((int64_t)(lane / lpu) * rows_padded + i) * lpu + (lane % lpu)] : 0;
-    const bool overflow = __any_sync(0xffffffffu, my_cnt > cap);
+    const int n_lists = kFlagLists * n_chunks;  // (unit of the row, list of the unit): n_chunks <= 8
+    const int my_cnt = lane < n_lists ? flag_cnt[((int64_t)(lane / kFlagLists) * rows_padded + i) * kFlagLists + (lane % kFlagLists)] : 0;
+    const bool overflow = __any_sync(0xffffffffu, my_cnt > kFlagCap);
     if (!overflow) {
         for (int lh = 0; lh < n_lists; lh++) {
             const int cnt = __shfl_sync(0xffffffffu, my_cnt, lh);
             if (cnt == 0) continue;
-            const int2 *lst = flag_list + (((int64_t)(lh / lpu) * rows_padded + i) * lpu + (lh % lpu)) * cap;
+            const int2 *lst = flag_list + (((int64_t)(lh / kFlagLists) * rows_padded + i) * kFlagLists + (lh % kFlagLists)) * kFlagCap;
             const int2 mine = lane < cnt ? lst[lane] : make_int2(0, 0);
             unsigned live = __ballot_sync(0xffffffffu, lane < cnt && __int_as_float(mine.y) > th);
             while (live) {
@@ -2010,7 +1877,7 @@ __global__ void __launch_bounds__(128)
 k_umma_refine(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum, const uint8_t *__restrict__ pos_raw,
               const int4 *__restrict__ pos_info,
               const int2 *__restrict__ flag_list, const int32_t *__restrict__ flag_cnt,
-              const uint32_t *__restrict__ row_lb, int n_chunks, int lpu, int cap,
+              const uint32_t *__restrict__ row_lb, int n_chunks,
               int64_t rows_padded, int64_t rows, int64_t npos, const int64_t *__restrict__ dom0_pos,
               int32_t *__restrict__ best, Geom g, int64_t j0)
 {
@@ -2072,7 +1939,7 @@ k_umma_refine(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum,
         }
     };
     if (lane == 0) consider(*dom0_pos);
-    for_each_flagged(lane, i, rows_padded, n_chunks, npos, flag_list, flag_cnt, th_row, lpu, cap, consider);
+    for_each_flagged(lane, i, rows_padded, n_chunks, npos, flag_list, flag_cnt, th_row, consider);
     for (int o = 16; o > 0; o >>= 1) {
         float e2 = __shfl_down_sync(0xffffffffu, be, o);
         int i2 = __shfl_down_sync(0xffffffffu, bi, o);
@@ -2091,7 +1958,7 @@ template <int B>
 __global__ void __launch_bounds__(128)
 k_umma_refine_iso(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum, const uint8_t *__restrict__ pos_raw,
                   const int4 *__restrict__ pos_info, const int2 *__restrict__ flag_list,
-                  const int32_t *__restrict__ flag_cnt, const uint32_t *__restrict__ row_lb, int n_chunks, int lpu, int cap,
+                  const int32_t *__restrict__ flag_cnt, const uint32_t *__restrict__ row_lb, int n_chunks,
                   int64_t rows_padded, int64_t ranges, int64_t npos,
                   const int64_t *__restrict__ dom0_pos, int32_t *__restrict__ best, Geom g, int64_t j0)
 {
@@ -2157,19 +2024,20 @@ k_umma_refine_iso(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
     int built = 0;
     bool overflow = false;
     for (int ch = 0; ch < n_chunks && !overflow; ch++) {
-        // 8 * lpu (<= 32) contiguous list lengths: operand row 8 r + k, list h of the unit at lane lpu * k + h
-        const int64_t base = ((int64_t)ch * rows_padded + r * 8) * lpu;
-        const int my_cnt = lane < 8 * lpu ? flag_cnt[base + lane] : 0;
-        if (__any_sync(0xffffffffu, my_cnt > cap)) { overflow = true; break; }
+        // 8 * kFlagLists (<= 32) contiguous list lengths: operand row 8 r + k, list h of the unit at lane kFlagLists * k + h
+        const int64_t base = ((int64_t)ch * rows_padded + r * 8) * kFlagLists;
+        const int my_cnt = lane < 8 * kFlagLists ? flag_cnt[base + lane] : 0;
+        if (__any_sync(0xffffffffu, my_cnt > kFlagCap)) { overflow = true; break; }
         for (int kiso = 0; kiso < 8; kiso++) {
             int any = 0;
-            for (int h = 0; h < lpu; h++) any |= __shfl_sync(0xffffffffu, my_cnt, lpu * kiso + h);
+            for (int h = 0; h < kFlagLists; h++) any |= __shfl_sync(0xffffffffu, my_cnt, kFlagLists * kiso + h);
             if (any == 0) continue;
             if (built != kiso) { build(kiso); built = kiso; }
-            for (int h = 0; h < lpu; h++) {
-                const int cnt = __shfl_sync(0xffffffffu, my_cnt, lpu * kiso + h);
+#pragma unroll 1  // one copy of the candidate loop
+            for (int h = 0; h < kFlagLists; h++) {
+                const int cnt = __shfl_sync(0xffffffffu, my_cnt, kFlagLists * kiso + h);
                 if (cnt == 0) continue;
-                const int2 *lst = flag_list + (base + lpu * kiso + h) * cap;
+                const int2 *lst = flag_list + (base + kFlagLists * kiso + h) * kFlagCap;
                 const int2 mine = lane < cnt ? lst[lane] : make_int2(0, 0);
                 unsigned live = __ballot_sync(0xffffffffu, lane < cnt && __int_as_float(mine.y) > th_row);  // see for_each_flagged
                 while (live) {
@@ -2201,7 +2069,7 @@ template <int B>
 __global__ void __launch_bounds__(128)
 k_umma_refine_rgb(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum, const uint8_t *__restrict__ opB,
                   const int4 *__restrict__ pos_info, const int2 *__restrict__ flag_list, const int32_t *__restrict__ flag_cnt,
-                  const uint32_t *__restrict__ row_lb, int n_chunks, int lpu, int cap,
+                  const uint32_t *__restrict__ row_lb, int n_chunks,
                   int64_t rows_padded, int64_t rows, int64_t npos, const int64_t *__restrict__ dom0_pos,
                   int32_t *__restrict__ best, Geom g, int64_t j0)
 {
@@ -2274,7 +2142,7 @@ k_umma_refine_rgb(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
         }
     };
     if (lane == 0) consider(*dom0_pos);
-    for_each_flagged(lane, i, rows_padded, n_chunks, npos, flag_list, flag_cnt, th_row, lpu, cap, consider);
+    for_each_flagged(lane, i, rows_padded, n_chunks, npos, flag_list, flag_cnt, th_row, consider);
     for (int o = 16; o > 0; o >>= 1) {
         float e2 = __shfl_down_sync(0xffffffffu, be, o);
         int i2 = __shfl_down_sync(0xffffffffu, bi, o);
@@ -2366,22 +2234,7 @@ size_t opA_bytes_t(const Geom &g, int64_t rows, int num_sms)
 }
 
 using KernelT = void (*)(const uint8_t *, const uint8_t *, const int32_t *, const float *, int2 *, int32_t *, uint32_t *, int, int,
-                         int, int, int64_t, int32_t *, int64_t, volatile int *, uint32_t, uint32_t, uint32_t, uint32_t);
-
-// dbg (probe only): 1 / 3 strip the scoring / the TMEM loads too, 4: epilogue alone, 8 / 12: phase cycle counts
-template <int B, bool F16, int EPI, bool PAIR = false>
-KernelT pick_kernel(bool dump, uint32_t dbg)
-{
-    if (dump) return k_umma_search<B, F16, 0, true, EPI, PAIR>;
-    if ((dbg & 3u) == 1) return k_umma_search<B, F16, 1, false, EPI, PAIR>;
-    if ((dbg & 3u) == 3) return k_umma_search<B, F16, 3, false, EPI, PAIR>;
-    if (dbg == 4) return k_umma_search<B, F16, 4, false, EPI, PAIR>;
-    if (dbg == 8) return k_umma_search<B, F16, 8, false, EPI, PAIR>;
-    if constexpr (!PAIR) {
-        if (dbg == 12) return k_umma_search<B, F16, 12, false, EPI>;
-    }
-    return k_umma_search<B, F16, 0, false, EPI, PAIR>;
-}
+                         int, int, int64_t, int32_t *, int64_t, volatile int *);
 
 // CTA pairs exist for the kind::f16 kernels (B = 4, 8: grey, RGB and the isometry extension; two issuing warps) and for
 // the K-split B = 16 configurations (kind::i8 grey, kind::f16 RGB; one issuing warp, each CTA loads half of either part
@@ -2430,15 +2283,9 @@ inline bool pair_launchable(KernelT kern, int smem_bytes)
     return ok;
 }
 
-// Epilogue variant each configuration runs by default (measured, profiles/README.md): kind::f16 B = 8 gains 1.5-5 %
-// from the pipelined loads, B = 4 (epilogue bound) 10 % from deferring the flag tests as well.
-template <int B, bool F16>
-constexpr int default_epi() { return (!F16 || B == 16) ? 0 : (B == 4 ? 3 : 2); }
-
 template <int B, bool F16>
 int launch_t(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, cudaStream_t s, const char **err,
-             int32_t *dump, int64_t dump_ld, int *status_dev, int variant, cudaEvent_t k0 = nullptr,
-             cudaEvent_t k1 = nullptr, uint32_t dbg = 0, int *pair_used = nullptr)
+             cudaEvent_t k0, cudaEvent_t k1, int pair_mode, int *pair_used, int32_t *dump, int64_t dump_ld, int *status_dev)
 {
     using L = Lay<B, F16>;
     if (j1 <= j0) return 0;
@@ -2482,24 +2329,13 @@ int launch_t(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, 
         k_umma_pack_ranges<B, F16><<<(unsigned)((rp + 127) / 128), 128, 0, s>>>(w.src, w.rsum, opA, vR, g, j0, j1, rp);
     }
     launches += 2;
-    // 3. the fused search
-    // Epilogue mapping (see k_umma_search): the default of this (block size, kind) pair, or the probe's choice
-    // (variant bit 1: plain, bit 3: software-pipelined, bit 4: pipelined with deferred flag tests).
-    // CTA pairs: variant bit 5 = on, bit 6 = off, neither = where measured faster (pair_default).  The pair kernel runs
-    // the deferred-test epilogue (EPI 3) unless the probe asks for EPI 2: with the tensor pipe at its full rate the
-    // earlier hand-back is worth 10 %.
-    const int epi = (variant & 2) ? 0 : ((variant & 8) ? 2 : ((variant & 16) ? 3 : default_epi<B, F16>()));
+    // 3. the fused search: CTA pairs on request (FIC_UMMA_PAIR_ON / _OFF), else where measured faster (pair_default)
     bool pair = false;
-    if constexpr (pair_capable<B, F16>())
-        pair = ((variant & 32) ? true : ((variant & 64) ? false : pair_default<B, F16>())) && dbg != 12 && num_sms >= 2;
-    KernelT kern = pick_kernel<B, F16, 0>(dump && !(dbg & 8u), dbg);
-    if (epi == 2) kern = pick_kernel<B, F16, 2>(dump && !(dbg & 8u), dbg);
-    if (epi == 3) kern = pick_kernel<B, F16, 3>(dump && !(dbg & 8u), dbg);
+    KernelT kern = dump ? k_umma_search<B, F16, false, true> : k_umma_search<B, F16, false, false>;
     if constexpr (pair_capable<B, F16>()) {
+        pair = (pair_mode == FIC_UMMA_PAIR_ON || (pair_mode != FIC_UMMA_PAIR_OFF && pair_default<B, F16>())) && num_sms >= 2;
         if (pair) {
-            KernelT pk;
-            if constexpr (F16 && B != 16) pk = (variant & 8) ? pick_kernel<B, F16, 2, true>(dump, dbg) : pick_kernel<B, F16, 3, true>(dump, dbg);
-            else pk = pick_kernel<B, F16, 0, true>(dump, dbg);  // B = 16 (kind::i8, RGB kind::f16): the plain epilogue loop
+            KernelT pk = dump ? k_umma_search<B, F16, true, true> : k_umma_search<B, F16, true, false>;
             ce = cudaFuncSetAttribute(pk, cudaFuncAttributeMaxDynamicSharedMemorySize, L::SMEM_BYTES);
             if (ce != cudaSuccess) { *err = cudaGetErrorString(ce); return -1; }
             if (pair_launchable(pk, L::SMEM_BYTES)) kern = pk;
@@ -2507,14 +2343,11 @@ int launch_t(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, 
         }
     }
     if (pair_used) *pair_used = pair ? 1 : 0;
-    if (dbg == 8 || dbg == 12) dump = w.best;  // phase cycle counts -> w.best
     ce = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::SMEM_BYTES);
     if (ce != cudaSuccess) { *err = cudaGetErrorString(ce); return -1; }
     int n_units = pair ? (p.n_sb / 2) * p.n_chunks : p.n_sb * p.n_chunks;
     const int slots = pair ? num_sms / 2 : num_sms;  // CTAs, or CTA pairs (one TPC each)
     int grid = (n_units < slots ? n_units : slots) * (pair ? 2 : 1);
-    uint32_t lbo_a = 128, sbo_a = L::SBO_A, lbo_b = 128, sbo_b = L::SBO_B;
-    if (variant & 1) { lbo_a = L::SBO_A; sbo_a = 128; lbo_b = L::SBO_B; sbo_b = 128; }  // probe only
     if (k0) cudaEventRecord(k0, s);
     cudaMemsetAsync(row_lb, 0, (size_t)rp * 4, s);
     {
@@ -2536,23 +2369,21 @@ int launch_t(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, 
         const int iso_shift = g.n_iso > 1 ? 3 : 0;
         volatile int *status_v = status_dev;
         ce = cudaLaunchKernelEx(&cfg, kern, opA_c, opB_c, vR_c, norm_c, flag_list, flag_cnt, row_lb, p.n_sb, p.n_chunks, p.ntiles, iso_shift,
-                                rp, dump, dump_ld, status_v, lbo_a, sbo_a, lbo_b, sbo_b);
+                                rp, dump, dump_ld, status_v);
         if (ce != cudaSuccess) { *err = cudaGetErrorString(ce); return -1; }
     }
     if (k1) cudaEventRecord(k1, s);
     // 4. exact refine of the flagged chunks
-    if (!(dbg & 8u)) {
-        if (rgb) {
-            if constexpr (F16)
-                k_umma_refine_rgb<B><<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(w.src, w.rsum, w.opB, pos_info, flag_list, flag_cnt,
-                                                                                row_lb, p.n_chunks, kListsOf(epi), kCapOf(epi), rp, rows, p.npos, dom0, w.best, g, j0);
-        } else if (g.n_iso > 1)
-            k_umma_refine_iso<B><<<(unsigned)((j1 - j0 + 3) / 4), 128, 0, s>>>(w.src, w.rsum, pos_raw, pos_info, flag_list, flag_cnt,
-                                                                             row_lb, p.n_chunks, kListsOf(epi), kCapOf(epi), rp, j1 - j0, p.npos, dom0, w.best, g, j0);
-        else
-            k_umma_refine<B><<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(w.src, w.rsum, pos_raw, pos_info, flag_list, flag_cnt,
-                                                                        row_lb, p.n_chunks, kListsOf(epi), kCapOf(epi), rp, rows, p.npos, dom0, w.best, g, j0);
-    }
+    if (rgb) {
+        if constexpr (F16)
+            k_umma_refine_rgb<B><<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(w.src, w.rsum, w.opB, pos_info, flag_list, flag_cnt,
+                                                                            row_lb, p.n_chunks, rp, rows, p.npos, dom0, w.best, g, j0);
+    } else if (g.n_iso > 1)
+        k_umma_refine_iso<B><<<(unsigned)((j1 - j0 + 3) / 4), 128, 0, s>>>(w.src, w.rsum, pos_raw, pos_info, flag_list, flag_cnt,
+                                                                         row_lb, p.n_chunks, rp, j1 - j0, p.npos, dom0, w.best, g, j0);
+    else
+        k_umma_refine<B><<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(w.src, w.rsum, pos_raw, pos_info, flag_list, flag_cnt,
+                                                                    row_lb, p.n_chunks, rp, rows, p.npos, dom0, w.best, g, j0);
     launches += 2;
     ce = cudaGetLastError();
     if (ce != cudaSuccess) { *err = cudaGetErrorString(ce); return -1; }
@@ -2716,7 +2547,11 @@ int umma_f16_selftest(int num_sms, cudaStream_t s, const char **err)
             launch_decimate(w.src, w.dec, *gp, s);
             launch_domain_stats(w.dec, w.dsum, w.dsq, *gp, s);
             launch_range_stats(w.src, w.rsum, *gp, s);
-            if (launch_t<8, true>(w, *gp, 0, gp->NR, num_sms, s, err, dump, dump_ld, nullptr, 0) < 0) { launched = false; break; }
+            if (launch_t<8, true>(w, *gp, 0, gp->NR, num_sms, s, err, nullptr, nullptr, FIC_UMMA_PAIR_AUTO, nullptr, dump, dump_ld,
+                                  nullptr) < 0) {
+                launched = false;
+                break;
+            }
             const int64_t total = gp->NR * p.npos;
             k_umma_selftest_check<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(
                 w.src, w.dec, w.rsum, w.dsum, (const int32_t *)(w.opB + OpBLayout<8, true>(g, p).off_posdom), dump, dump_ld,
@@ -2751,11 +2586,10 @@ int umma_debug_sort(uint32_t *d_keys, int32_t *d_vals, uint32_t *d_keys_out, int
 
 // Bare loop of the CTA-pair instruction shape (cta_group::2, M = 256, N = 128): TOP/s, best of `reps`; tmem_bases (if
 // not null) receives the TMEM base address each of the first 4 CTAs was given.
-double measure_mma_peak_pair(int num_sms, cudaStream_t s, int reps, int f16, uint32_t *tmem_bases, const char **err, int a_in_tmem)
+double measure_mma_peak_pair(int num_sms, cudaStream_t s, int reps, int f16, uint32_t *tmem_bases, const char **err)
 {
     const int smem = 200 * 1024;
-    void (*kern)(int, uint32_t, uint32_t *) = a_in_tmem ? (f16 ? k_mma_peak_pair<true, true> : k_mma_peak_pair<false, true>)
-                                                        : (f16 ? k_mma_peak_pair<true> : k_mma_peak_pair<false>);
+    void (*kern)(int, uint32_t, uint32_t *) = f16 ? k_mma_peak_pair<true> : k_mma_peak_pair<false>;
     cudaError_t ce = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (ce != cudaSuccess) { *err = cudaGetErrorString(ce); return -1.0; }
     uint32_t *d_out = nullptr;
@@ -2821,24 +2655,15 @@ size_t umma_opB_bytes(const Geom &g, int kind)
                              (OpBLayout<8, true>(g, p).total), (OpBLayout<16, true>(g, p).total));
 }
 
-// Debug entry used by tools/umma_probe: also dumps the raw accumulators (kov) of every
-// (row, sweep position) pair, and lets the probe pick the descriptor variant.
-int launch_search_umma_debug(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, cudaStream_t s,
-                             const char **err, int kind, int32_t *dump, int64_t dump_ld, int *status_dev, int variant,
-                             uint32_t dbg, cudaEvent_t k0, cudaEvent_t k1, int *pair_used)
+int launch_search_umma(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, cudaStream_t s,
+                       const char **err, int kind, cudaEvent_t k0, cudaEvent_t k1, int pair, int *pair_used,
+                       int32_t *dump, int64_t dump_ld, int *status_dev)
 {
-#define FIC_UMMA_ARGS w, g, j0, j1, num_sms, s, err, dump, dump_ld, status_dev, variant, k0, k1, dbg, pair_used
+#define FIC_UMMA_ARGS w, g, j0, j1, num_sms, s, err, k0, k1, pair, pair_used, dump, dump_ld, status_dev
     return FIC_UMMA_DISPATCH(g.B, use_f16(g, kind), (launch_t<4, false>(FIC_UMMA_ARGS)), (launch_t<8, false>(FIC_UMMA_ARGS)),
                              (launch_t<16, false>(FIC_UMMA_ARGS)), (launch_t<4, true>(FIC_UMMA_ARGS)),
                              (launch_t<8, true>(FIC_UMMA_ARGS)), (launch_t<16, true>(FIC_UMMA_ARGS)));
 #undef FIC_UMMA_ARGS
-}
-
-int launch_search_umma(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, cudaStream_t s,
-                       const char **err, int kind, cudaEvent_t k0, cudaEvent_t k1, int pair, int *pair_used)
-{
-    const int variant = pair == FIC_UMMA_PAIR_ON ? 32 : (pair == FIC_UMMA_PAIR_OFF ? 64 : 0);
-    return launch_search_umma_debug(w, g, j0, j1, num_sms, s, err, kind, nullptr, 0, nullptr, variant, 0, k0, k1, pair_used);
 }
 
 }  // namespace fic

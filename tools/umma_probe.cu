@@ -1,19 +1,20 @@
 // umma_probe -- development probe for the tcgen05 fused search (not part of the product).
 //
-//   umma_probe <mode> <B> <W> [variant] [pattern] [dbg] [kind]
-//     mode   check : dump every accumulator (kov) and compare with a CPU integer dot
-//                    product, then compare winners with the direct CUDA-core search
-//            time  : no dump; time the fused search and the direct search, compare winners
-//            peak  : bare tcgen05.mma loops (B, W ignored): tensor-pipe rate by kind and MMA shape
-//     B      4 | 8       W = H, multiple of B
-//     variant 0 = descriptor strides as designed (LBO 128, SBO KS*256), 1 = swapped
+//   umma_probe check|time <B> <W> [pattern] [kind] [pair]
+//     check : dump every accumulator (kov) and compare with a CPU integer dot
+//             product, then compare winners with the direct CUDA-core search
+//     time  : no dump; time the fused search (k0 / k1 events around k_umma_search) and the
+//             direct search, compare winners
+//     B       4 | 8 | 16   W = H, multiple of B
 //     pattern 0 = noise, 1 = structured, 2 = flat + sparse dots (tie-heavy), 3 = binary 0/255 noise,
 //             4 = binary 0/255 in 4x4 pixel cells (the largest |kov| the operands can produce)
-//     dbg     1 = no scoring math, 3 = no TMEM loads either (timing floors)
-//     kind    0 = auto, 1 = kind::i8, 2 = kind::f16
+//     kind    0 = auto, 1 = kind::i8, 2 = kind::f16 (B = 16 always runs kind::i8)
+//     pair    0 = auto, 1 = off, 2 = on (FIC_UMMA_PAIR_*)
+//   umma_probe peak : bare tcgen05.mma loops: tensor-pipe rate by kind and MMA shape
+//   umma_probe ldtm | alu | mix | chain | sort : micro-benchmarks and the radix-sort check (below)
 //
-// Runs each experiment in its own process so that a faulting variant cannot poison the
-// next one; every mbarrier wait in the kernel is bounded (trap + status code).
+// Runs each experiment in its own process so that a fault cannot poison the next one;
+// every mbarrier wait in the kernel is bounded (trap + status code).
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -553,11 +554,7 @@ int main(int argc, char **argv)
     if (argc > 1 && !strcmp(argv[1], "mix")) return run_mix();
     if (argc > 1 && !strcmp(argv[1], "chain")) return run_chain();
     if (argc > 1 && !strcmp(argv[1], "sort")) return run_sort();
-    if (argc < 4) {
-        printf("usage: umma_probe check|time B W [variant] [pattern]\n");
-        return 2;
-    }
-    if (!strcmp(argv[1], "peak")) {  // bare MMA loops: rate by kind and shape
+    if (argc > 1 && !strcmp(argv[1], "peak")) {  // bare MMA loops: rate by kind and shape
         cudaDeviceProp prop;
         CK(cudaGetDeviceProperties(&prop, 0));
         cudaStream_t s;
@@ -575,35 +572,24 @@ int main(int argc, char **argv)
             printf("peak kind::%s cta_group::2 M=256 N=128: %.1f TOP/s %s  (TMEM bases of CTAs 0-3: %x %x %x %x)\n", f16 ? "f16" : "i8", t,
                    t < 0 ? err : "", bases[0], bases[1], bases[2], bases[3]);
         }
-        // sustained (power-capped) rates, kind::f16 pairs: A from shared memory against A from tensor memory, 40 back-to-back
-        // launches each (~0.5 s), alternating twice
-        for (int round = 0; round < 2; round++)
-            for (int ts = 0; ts < 2; ts++) {
-                const char *err = "";
-                double best = 0, sum = 0;
-                for (int r = 0; r < 10; r++) {
-                    double t = measure_mma_peak_pair(prop.multiProcessorCount, s, 3, 1, nullptr, &err, ts);
-                    if (t < 0) { printf("sustained: %s\n", err); return 1; }
-                    sum += t;
-                    if (t > best) best = t;
-                }
-                printf("sustained kind::f16 cta_group::2, A from %s: mean-of-best %.1f, best %.1f TFLOP/s\n", ts ? "TMEM" : "smem", sum / 10, best);
-            }
         return 0;
+    }
+    if (argc < 4 || (strcmp(argv[1], "check") && strcmp(argv[1], "time"))) {
+        printf("usage: umma_probe check|time B W [pattern] [kind] [pair]   or   umma_probe peak|ldtm|alu|mix|chain|sort\n");
+        return 2;
     }
     bool check = !strcmp(argv[1], "check");
     int B = atoi(argv[2]), W = atoi(argv[3]);
-    int variant = argc > 4 ? atoi(argv[4]) : 0;
-    int pattern = argc > 5 ? atoi(argv[5]) : 0;
-    uint32_t dbg = argc > 6 ? (uint32_t)atoi(argv[6]) : 0;  // 1: no scoring math, 3: no TMEM loads either, 4: no slow path
-    int kind = argc > 7 ? atoi(argv[7]) : 0;
+    int pattern = argc > 4 ? atoi(argv[4]) : 0;
+    int kind = argc > 5 ? atoi(argv[5]) : 0;
+    int pair = argc > 6 ? atoi(argv[6]) : FIC_UMMA_PAIR_AUTO;
     int H = W;
     Geom g;
     const char *why = "";
     int wk = 2 * (W / B) - 3;
     if (make_geom(W, H, B, wk, 0, &g, &why)) { printf("bad geometry: %s\n", why); return 2; }
     if (!umma_applicable(g)) { printf("umma not applicable\n"); return 2; }
-    printf("probe mode=%s B=%d W=%d variant=%d pattern=%d kind=%d NR=%lld ND=%lld\n", argv[1], B, W, variant, pattern, kind,
+    printf("probe mode=%s B=%d W=%d pattern=%d kind=%d pair=%d NR=%lld ND=%lld\n", argv[1], B, W, pattern, kind, pair,
            (long long)g.NR, (long long)g.ND);
 
     cudaDeviceProp prop;
@@ -664,17 +650,17 @@ int main(int argc, char **argv)
         cudaEvent_t k0, k1;
         CK(cudaEventCreate(&k0));
         CK(cudaEventCreate(&k1));
-        int n = launch_search_umma_debug(w, g, 0, g.NR, prop.multiProcessorCount, s, &err, kind, dump, dump_ld, status_d, variant, dbg, k0, k1);
+        int pair_used = 0;
+        int n = launch_search_umma(w, g, 0, g.NR, prop.multiProcessorCount, s, &err, kind, k0, k1, pair, &pair_used, dump, dump_ld,
+                                   status_d);
         if (n < 0) { printf("launch failed: %s\n", err); return 3; }
         CK(cudaEventRecord(e1, s));
         CK(cudaStreamSynchronize(s));
         CK(cudaEventElapsedTime(&ms_umma, e0, e1));
         float ms_k = 0;
         CK(cudaEventElapsedTime(&ms_k, k0, k1));
-        const long long clk = (long long)status_h[2] | ((long long)status_h[3] << 31);
-        printf("umma search run %d: pack+search+merge %.3f ms, k_umma_search alone %.3f ms   dbg=%u status=%d   CTA 0 issuer: %lld clk in %.3f ms (%.3f GHz)\n", r,
-               ms_umma, ms_k, dbg, *status_h, clk, status_h[4] * 1e-6, status_h[4] > 0 ? clk / (double)status_h[4] : 0.0);
-        if (dbg & 8u) printf("  issuer waits: accumulators %u clk, domain tiles %u clk\n", (unsigned)status_h[5], (unsigned)status_h[6]);
+        printf("umma search run %d: pack+search+merge %.3f ms, k_umma_search alone %.3f ms   pairs=%d status=%d\n", r, ms_umma, ms_k,
+               pair_used, *status_h);
     }
     CK(cudaMemcpy(best_umma.data(), w.best, 4 * g.NR, cudaMemcpyDeviceToHost));
     double evals = (double)g.NR * (double)g.ND;
@@ -732,28 +718,6 @@ int main(int argc, char **argv)
         printf("accumulator check: %lld mismatches of %lld\n", bad, (long long)(g.NR * g.ND));
         if (bad) rc = 1;
     }
-    if (dbg & 8u) {  // per-warp cycle accounting written by the kernel into w.best
-        for (int cta = 0; cta < 2; cta++)
-            for (int e = 0; e < 16; e++) {
-                const int32_t *o = &best_umma[(size_t)(cta * 16 + e) * 8];
-                printf("cta %d epilogue warp %2d: total %9d clk  bounds+rest %5.1f%%  wait T_FULL %5.1f%%  to hand-back %5.1f%%  after %5.1f%%\n", cta, e,
-                       o[0], 100.0 * o[1] / o[0], 100.0 * o[2] / o[0], 100.0 * o[3] / o[0], 100.0 * o[4] / o[0]);
-            }
-    }
-    if (dbg & 8u) {  // hand-over chain of CTA 0 (pair kernel): average clocks between the four events of an accumulator's cycle
-        const long long tiles = (long long)(((g.ND + 127) / 128));
-        const int32_t *is = &best_umma[32768];
-        printf("CTA 0 hand-over chain (sums mod 2^32; divide by the tiles CTA 0 walked):\n");
-        for (int q = 0; q < 4; q++)
-            for (int lq = 0; lq < 4; lq++) {
-                const int32_t *o = &best_umma[(size_t)(q * 4 + lq) * 8];
-                printf("  acc %d quarter %d: sum(full seen - issued) %u  sum(handed back - full seen) %u  sum(free seen - handed back) %d  sum(issued - free seen) %u\n", q, lq,
-                       (unsigned)((uint32_t)o[5] - (uint32_t)is[4 + q]), (unsigned)((uint32_t)o[6] - (uint32_t)o[5]),
-                       (int)((uint32_t)is[q] - (uint32_t)o[6]), (unsigned)((uint32_t)is[4 + q] - (uint32_t)is[q]));
-            }
-        (void)tiles;
-    }
-    if (dbg & 15u) { printf("dbg run: winners not checked\nPROBE DONE\n"); return 0; }
     long long diff = 0, shown = 0;
     for (int64_t i = 0; i < g.NR; i++)
         if (best_direct[i] != best_umma[i]) {
