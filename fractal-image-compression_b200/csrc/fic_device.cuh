@@ -74,7 +74,24 @@ __host__ __device__ inline int iso_inverse(int k) { return k == 1 ? 3 : (k == 3 
 // Java (int)float: truncate toward zero, saturate, NaN -> 0 == cvt.rzi.s32.f32.
 __device__ __forceinline__ int j_f2i(float f) { return __float2int_rz(f); }
 
-__device__ __forceinline__ int clamp255(int v) { return v < 0 ? 0 : (v > 255 ? 255 : v); }
+// FC:72 getMittelwert: the integer mean of a block from its pixel sum, mean = sum / n.  Returns
+// sum (x - mean) = sum - n * mean (FC:671, FC:790), the exact integer in [0, n) that the reference's scores divide by.
+__device__ __forceinline__ int centred_sum(int sum, int n, int *mean)
+{
+    const int m = sum / n;
+    *mean = m;
+    return sum - n * m;
+}
+
+// RGB (FC:760-791): the three channel means m[c] of block j, from per-channel sums stored as sum[c * count + j];
+// returns the centred sums added over the channels (vR of a range block, vD of a domain).
+__device__ __forceinline__ int centred_sum_rgb(const int32_t *__restrict__ sum, int64_t count, int64_t j, int n, int m[3])
+{
+    int v = 0;
+#pragma unroll
+    for (int c = 0; c < 3; c++) v += centred_sum(sum[c * count + j], n, &m[c]);
+    return v;
+}
 
 // The reference's grey "error" of one candidate (FC:677-683), from exact integers:
 // kov = sum (r-rmean)(d-dmean), vR = sum (r-rmean), varD = sum (d-dmean)^2.
@@ -89,6 +106,38 @@ __device__ __forceinline__ float grey_error(int kov, int vR, double sqd)
     }
     r = __fmul_rn(r, r);
     return __fmul_rn(__fmul_rn(fvR, fvR), __fsub_rn(1.0f, r));
+}
+
+// One step of the reference's RGB covariance, kov += gR * gD in binary32 (FC:789), gR and gD being the channel-summed
+// centred pixels (FC:783-786).  |gR|, |gD| <= 765 are exact small integers, so their product is exact and one rounding
+// of kov + product equals the reference's multiply-then-add -- also at B = 16, where kov may pass 2^24 and round.
+__device__ __forceinline__ float rgb_kov_step(float kov, float gR, float gD) { return __fmaf_rn(gR, gD, kov); }
+
+// The reference's RGB "error" of one candidate (FC:797-803): r = kov / (vR * vD), error = vR^2 (1 - r^2), all binary32.
+// vR, vD are the channel-summed centred sums (FC:790-791): the domain's `variance` stays 0 on the RGB path.
+__device__ __forceinline__ float rgb_error(float kov, float vR, float vD)
+{
+    float r = 0.0f;
+    if (!(vR == 0.0f || vD == 0.0f)) r = __fdiv_rn(kov, __fmul_rn(vR, vD));
+    r = __fmul_rn(r, r);
+    return __fmul_rn(__fmul_rn(vR, vR), __fsub_rn(1.0f, r));
+}
+
+// Lexicographic (error, index) minimum: with the candidates visited in ascending index order, the reference's strict
+// `error < best` (FC:627, FC:710) keeps the lowest index among equal errors, and so does this order.
+__device__ __forceinline__ void argmin_merge(float &err, int &idx, float e2, int i2)
+{
+    if (e2 < err || (e2 == err && i2 < idx)) { err = e2; idx = i2; }
+}
+
+// argmin_merge over the 32 lanes of a warp; lane 0 ends with the warp's minimum.
+__device__ __forceinline__ void warp_argmin(float &err, int &idx)
+{
+    for (int o = 16; o > 0; o >>= 1) {
+        const float e2 = __shfl_down_sync(0xffffffffu, err, o);
+        const int i2 = __shfl_down_sync(0xffffffffu, idx, o);
+        argmin_merge(err, idx, e2, i2);
+    }
 }
 
 // varD = sum d^2 - 2*dmean*sum d + n*dmean^2 with dmean = floor(sum d / n) (DB:92-115).

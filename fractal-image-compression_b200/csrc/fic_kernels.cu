@@ -43,25 +43,27 @@ int launch_unpack(const int32_t *d_argb, uint8_t *d_planes, int W, int H, int C,
     return 1;
 }
 
-// planes -> ARGB (0xff alpha), grey replicates the plane (FC:404, FC:490).
+// planes -> ARGB (0xff alpha), grey replicates the plane (FC:404, FC:490).  Grid-stride over quads of pixels with
+// blockDim.x == 256.
 template <int C>
-__global__ void k_pack_argb(const uchar4 *__restrict__ planes, int4 *__restrict__ argb, int64_t quads)
+__device__ __forceinline__ void pack_argb(const uchar4 *planes, int4 *argb, int64_t quads)
 {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (; i < quads; i += stride) {
-        uchar4 r = planes[i], g = r, b = r;
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < quads; i += (int64_t)gridDim.x * 256) {
+        const uchar4 r = planes[i];
+        uchar4 g = r, b = r;
         if (C == 3) {
             g = planes[quads + i];
             b = planes[2 * quads + i];
         }
-        int4 o;
-        o.x = (int)(0xff000000u | (r.x << 16) | (g.x << 8) | b.x);
-        o.y = (int)(0xff000000u | (r.y << 16) | (g.y << 8) | b.y);
-        o.z = (int)(0xff000000u | (r.z << 16) | (g.z << 8) | b.z);
-        o.w = (int)(0xff000000u | (r.w << 16) | (g.w << 8) | b.w);
-        argb[i] = o;
+        auto px = [](uint32_t r, uint32_t g, uint32_t b) { return (int)(0xff000000u | (r << 16) | (g << 8) | b); };
+        argb[i] = make_int4(px(r.x, g.x, b.x), px(r.y, g.y, b.y), px(r.z, g.z, b.z), px(r.w, g.w, b.w));
     }
+}
+
+template <int C>
+__global__ void k_pack_argb(const uchar4 *__restrict__ planes, int4 *__restrict__ argb, int64_t quads)
+{
+    pack_argb<C>(planes, argb, quads);
 }
 
 int launch_pack_argb(const uint8_t *d_planes, int32_t *d_argb, int W, int H, int C, cudaStream_t s)
@@ -231,22 +233,12 @@ constexpr int kDirectThreads = 128;
 
 __device__ __forceinline__ void block_argmin(float &err, int &c, float *s_err, int *s_c)
 {
-    // warp level
-    for (int o = 16; o > 0; o >>= 1) {
-        float e2 = __shfl_down_sync(0xffffffffu, err, o);
-        int c2 = __shfl_down_sync(0xffffffffu, c, o);
-        if (e2 < err || (e2 == err && c2 < c)) { err = e2; c = c2; }
-    }
+    warp_argmin(err, c);
     int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (lane == 0) { s_err[warp] = err; s_c[warp] = c; }
     __syncthreads();
-    if (threadIdx.x == 0) {
-        for (int w = 1; w < kDirectThreads / 32; w++) {
-            float e2 = s_err[w];
-            int c2 = s_c[w];
-            if (e2 < err || (e2 == err && c2 < c)) { err = e2; c = c2; }
-        }
-    }
+    if (threadIdx.x == 0)
+        for (int w = 1; w < kDirectThreads / 32; w++) argmin_merge(err, c, s_err[w], s_c[w]);
 }
 
 // sum r * d over one candidate block with packed-byte dot products: kov = sum r d - rmean * sum d - dmean * vR
@@ -283,9 +275,8 @@ k_search_direct_grey(const uint8_t *__restrict__ src, const uint8_t *__restrict_
     __shared__ int s_c[kDirectThreads / 32];
     int64_t j = j0 + blockIdx.x;
     int xr = (int)(j % g.rpw), yr = (int)(j / g.rpw);
-    int rs = rsum[j];
-    int rmean = rs / n;       // FC:72
-    int vR = rs - n * rmean;  // sum (r - rmean), FC:671
+    int rmean;
+    const int vR = centred_sum(rsum[j], n, &rmean);
     for (int t = threadIdx.x; t < n / 4; t += kDirectThreads) {
         int ry = (4 * t) / B, rx = (4 * t) % B;  // 4-byte aligned: W, xr * B and rx are multiples of 4
         s_rw[t] = *(const uint32_t *)(src + (int64_t)(yr * B + ry) * g.W + xr * B + rx);
@@ -341,19 +332,12 @@ __device__ __forceinline__ RgbScore rgb_score(const float *s_gR, float vR, const
 #pragma unroll
             for (int e = 0; e < LW; e++) {
                 const float gD = (float)((int)((w[e >> 1] >> (16 * (e & 1))) & 0xffffu) - dmsum);
-                // FC:789 kov += gR * gD: the product is an exact integer (< 2^20), so the fused form rounds exactly
-                // like the reference's multiply-then-add, once, in pixel order
-                kov = __fmaf_rn(s_gR[ry * B + rx + e], gD, kov);
+                kov = rgb_kov_step(kov, s_gR[ry * B + rx + e], gD);
             }
         }
     }
-    // FC:778 + FC:791: vD = sqrt(variance) (0 on the RGB path) + sum gD, an exact small integer = sum_c (dsum_c mod n)
-    const float vD = (float)vDi;
-    float r = 0.0f;
-    if (!(vR == 0.0f || vD == 0.0f)) r = __fdiv_rn(kov, __fmul_rn(vR, vD));  // FC:797-800
-    r = __fmul_rn(r, r);
     RgbScore o;
-    o.err = __fmul_rn(__fmul_rn(vR, vR), __fsub_rn(1.0f, r));  // FC:803
+    o.err = rgb_error(kov, vR, (float)vDi);
     o.kov = kov;
     return o;
 }
@@ -365,12 +349,7 @@ __device__ __forceinline__ float rgb_range_prep(const uint8_t *src, const int32_
 {
     int xr = (int)(j % g.rpw), yr = (int)(j / g.rpw);
     int64_t plane = (int64_t)g.W * g.H;
-    int v = 0;
-    for (int c = 0; c < 3; c++) {
-        int rs = rsum[(int64_t)c * g.NR + j];
-        rm[c] = rs / g.n;
-        v += rs - g.n * rm[c];
-    }
+    const int v = centred_sum_rgb(rsum, g.NR, j, g.n, rm);
     for (int t = threadIdx.x; t < g.n; t += blockDim.x) {
         int ry = t / g.B, rx = t % g.B;
         int64_t o = (int64_t)(yr * g.B + ry) * g.W + xr * g.B + rx;
@@ -401,14 +380,9 @@ k_search_direct_rgb(const uint8_t *__restrict__ src, const uint16_t *__restrict_
         int ky = c / g.wk, kx = c - ky * g.wk;
         int gx = dx + kx, gy = dy + ky;
         int64_t idx = gx + (int64_t)gy * g.dpw;
-        int dmsum = 0, vDi = 0;
-#pragma unroll
-        for (int ch = 0; ch < 3; ch++) {
-            const int ds = dsum[ch * g.ND + idx];
-            dmsum += ds / g.n;
-            vDi += ds - g.n * (ds / g.n);
-        }
-        RgbScore sc = rgb_score<B>(s_gR, vR, dec3, g, gx, gy, dmsum, vDi);
+        int dm[3];
+        const int vDi = centred_sum_rgb(dsum, g.ND, idx, g.n, dm);
+        RgbScore sc = rgb_score<B>(s_gR, vR, dec3, g, gx, gy, dm[0] + dm[1] + dm[2], vDi);
         if (sc.err < best_err) { best_err = sc.err; best_c = c; }  // FC:710
     }
     block_argmin(best_err, best_c, s_err, s_c);
@@ -429,9 +403,8 @@ k_search_direct_grey_iso(const uint8_t *__restrict__ src, const uint8_t *__restr
     __shared__ int s_c[kDirectThreads / 32];
     int64_t j = j0 + blockIdx.x;
     int xr = (int)(j % g.rpw), yr = (int)(j / g.rpw);
-    int rs = rsum[j];
-    int rmean = rs / g.n;
-    int vR = rs - g.n * rmean;
+    int rmean;
+    const int vR = centred_sum(rsum[j], g.n, &rmean);
     for (int t = threadIdx.x; t < 8 * g.n; t += kDirectThreads) {
         int k = t / g.n, p = t % g.n;
         int ry, rx;  // the range pixel that T_k sends to domain pixel p
@@ -515,6 +488,73 @@ int launch_search_direct(const Work &w, const Geom &g, int64_t j0, int64_t j1, c
 
 
 // ------------------------------------------------------------------------------------
+// Solve + quantisation of a winning candidate, shared by the fused encode (K2f) and the code solve (K3s).
+// ------------------------------------------------------------------------------------
+// Quantisation scales of the code stream: written by FC:242-244 / FC:250-254, read back by FC:372-374 / FC:446-450.
+constexpr float kGreyAScale = 100.0f, kRgbAScale = 1000000.0f, kRgbBScale = 100000.0f;
+
+// Grey (FC:634-641): contrast a = kov / varD clamped to [-1, 1] -- 0/0 gives NaN on flat winners and NaN passes the
+// clamp -- and brightness b = rmean - a * dmean.
+__device__ __forceinline__ float2 grey_solve(int kov, int varD, int rmean, int dmean)
+{
+    float a = __fdiv_rn((float)kov, (float)varD);
+    if (a < -1.0f) a = -1.0f;
+    else if (a > 1.0f) a = 1.0f;
+    return make_float2(a, __fsub_rn((float)rmean, __fmul_rn(a, (float)dmean)));
+}
+
+// RGB (FC:718-731): one contrast for the three channels over varianzSquare, which the reference computes as
+// varianceR + varianceG + mittelWertB (FC:776, sic); one brightness per channel.  Returns {a, bR, bG, bB}.
+__device__ __forceinline__ float4 rgb_solve(float kov, const int dv[3], const int dm[3], const int rm[3])
+{
+    float a = __fdiv_rn(kov, __fadd_rn(__fadd_rn((float)dv[0], (float)dv[1]), (float)dm[2]));
+    if (a > 1.0f) a = 1.0f;
+    if (a < -1.0f) a = -1.0f;
+    return make_float4(a, __fsub_rn((float)rm[0], __fmul_rn(a, (float)dm[0])), __fsub_rn((float)rm[1], __fmul_rn(a, (float)dm[1])),
+                       __fsub_rn((float)rm[2], __fmul_rn(a, (float)dm[2])));
+}
+
+// Code of range j for window candidate c: the floats into info and the quantised ints into q (FC:242-244), either
+// optional.  iso: the isometry extension's fourth column kiso.
+__device__ __forceinline__ void write_grey_code(float *info, int32_t *q, int64_t j, int c, float2 ab, bool iso, int kiso)
+{
+    const int S = iso ? 4 : 3;
+    const float fc = (float)c;
+    if (info) {
+        info[S * j + 0] = fc;
+        info[S * j + 1] = ab.x;
+        info[S * j + 2] = ab.y;
+        if (iso) info[S * j + 3] = (float)kiso;
+    }
+    if (q) {
+        q[S * j + 0] = j_f2i(fc);
+        q[S * j + 1] = j_f2i(__fmul_rn(ab.x, kGreyAScale));
+        q[S * j + 2] = j_f2i(ab.y);
+        if (iso) q[S * j + 3] = kiso;
+    }
+}
+
+// RGB (FC:250-254): code = {c, a, bR, bG, bB}.
+__device__ __forceinline__ void write_rgb_code(float *info, int32_t *q, int64_t j, int c, float4 ab)
+{
+    const float fc = (float)c;
+    if (info) {
+        info[5 * j + 0] = fc;
+        info[5 * j + 1] = ab.x;
+        info[5 * j + 2] = ab.y;
+        info[5 * j + 3] = ab.z;
+        info[5 * j + 4] = ab.w;
+    }
+    if (q) {
+        q[5 * j + 0] = j_f2i(fc);
+        q[5 * j + 1] = j_f2i(__fmul_rn(ab.x, kRgbAScale));
+        q[5 * j + 2] = j_f2i(__fmul_rn(ab.y, kRgbBScale));
+        q[5 * j + 3] = j_f2i(__fmul_rn(ab.z, kRgbBScale));
+        q[5 * j + 4] = j_f2i(ab.w);
+    }
+}
+
+// ------------------------------------------------------------------------------------
 // K2f: fused windowed encode -- the reference's default configuration in ONE launch.
 //
 // For the windows the reference's GUI offers (widthKernel <= 16, RLEAppView.fxml:104) the whole chain
@@ -590,8 +630,7 @@ k_encode_fused(const void *__restrict__ src, float *__restrict__ info, int32_t *
     for (int c = 0; c < C; c++) {
         int rs = 0;
         for (int w = 0; w < kDirectThreads / 32; w++) rs += s_sum[c][w];
-        rm[c] = rs / n;          // FC:72
-        vR += rs - n * rm[c];    // sum (r - rmean), FC:671 / FC:790
+        vR += centred_sum(rs, n, &rm[c]);
     }
     if (C == 3) {
         for (int t = threadIdx.x; t < n; t += kDirectThreads)
@@ -628,33 +667,29 @@ k_encode_fused(const void *__restrict__ src, float *__restrict__ info, int32_t *
                 for (int ry = 0; ry < B; ry++)
 #pragma unroll
                     for (int rx = 0; rx < B; rx++) ds += p[ch * TW * TW + ry * TW + rx];
-                dmsum += ds / n;
-                vDi += ds - n * (ds / n);
+                int dm;
+                vDi += centred_sum(ds, n, &dm);
+                dmsum += dm;
             }
-            float kov = 0.0f;  // FC:775: sequential binary32 accumulation in pixel order (see rgb_score)
+            float kov = 0.0f;  // FC:775: sequential binary32 accumulation in pixel order
             for (int ry = 0; ry < B; ry++)
 #pragma unroll
                 for (int rx = 0; rx < B; rx++) {
                     const int o = ry * TW + rx;
                     const float gD = (float)((int)p[o] + (int)p[(C == 3 ? 1 : 0) * TW * TW + o] + (int)p[(C - 1) * TW * TW + o] - dmsum);
-                    kov = __fmaf_rn(s_gR[ry * B + rx], gD, kov);
+                    kov = rgb_kov_step(kov, s_gR[ry * B + rx], gD);
                 }
-            const float fvR = (float)vR, vD = (float)vDi;
-            float r = 0.0f;
-            if (!(fvR == 0.0f || vD == 0.0f)) r = __fdiv_rn(kov, __fmul_rn(fvR, vD));  // FC:797-800
-            r = __fmul_rn(r, r);
-            err = __fmul_rn(__fmul_rn(fvR, fvR), __fsub_rn(1.0f, r));  // FC:803
+            err = rgb_error(kov, (float)vR, (float)vDi);
         }
         if (err < best_err) { best_err = err; best_c = c; }  // FC:627 / FC:710
     }
     block_argmin(best_err, best_c, s_err, s_c);
     if (threadIdx.x != 0) return;
-    // ---- solve + quantise the winner (FC:634-643 / FC:718-733; FC:242-244 / FC:250-254)
+    // ---- solve + quantise the winner
     const int c = best_c;
     const int ky = c / g.wk, kx = c - ky * g.wk;
     const uint8_t *p = s_tile + (ky * step) * TW + kx * step;
-    const float fc = (float)c;
-    if (C == 1) {
+    if constexpr (C == 1) {
         int ds = 0, dsq = 0, dot = 0;
         for (int ry = 0; ry < B; ry++)
             for (int rx = 0; rx < B; rx++) {
@@ -665,15 +700,9 @@ k_encode_fused(const void *__restrict__ src, float *__restrict__ info, int32_t *
             }
         int dmean;
         const int varD = dom_var(ds, dsq, n, &dmean);
-        const int kov = dot - dmean * vR;
-        float a = __fdiv_rn((float)kov, (float)varD);  // FC:634 (0/0 -> NaN on flat winners)
-        if (a < -1.0f) a = -1.0f;                      // FC:636-639 (NaN passes through)
-        else if (a > 1.0f) a = 1.0f;
-        const float b = __fsub_rn((float)rm[0], __fmul_rn(a, (float)dmean));  // FC:641
-        if (info) { info[3 * j] = fc; info[3 * j + 1] = a; info[3 * j + 2] = b; }
-        if (q) { q[3 * j] = j_f2i(fc); q[3 * j + 1] = j_f2i(__fmul_rn(a, 100.0f)); q[3 * j + 2] = j_f2i(b); }
+        write_grey_code(info, q, j, c, grey_solve(dot - dmean * vR, varD, rm[0], dmean), false, 0);
     } else {
-        int dm[C], dv[C], dmsum = 0;
+        int dm[3], dv[3], dmsum = 0;
 #pragma unroll
         for (int ch = 0; ch < C; ch++) {
             int ds = 0, dsq = 0;
@@ -691,24 +720,9 @@ k_encode_fused(const void *__restrict__ src, float *__restrict__ info, int32_t *
             for (int rx = 0; rx < B; rx++) {
                 const int o = ry * TW + rx;
                 const float gD = (float)((int)p[o] + (int)p[(C == 3 ? 1 : 0) * TW * TW + o] + (int)p[(C - 1) * TW * TW + o] - dmsum);
-                kov = __fmaf_rn(s_gR[ry * B + rx], gD, kov);
+                kov = rgb_kov_step(kov, s_gR[ry * B + rx], gD);
             }
-        // FC:776: varianzSquare = varianceR + varianceG + mittelWertB (sic)
-        const float varSq = __fadd_rn(__fadd_rn((float)dv[0], (float)dv[C == 3 ? 1 : 0]), (float)dm[C - 1]);
-        float a = __fdiv_rn(kov, varSq);  // FC:718
-        if (a > 1.0f) a = 1.0f;           // FC:721-724
-        if (a < -1.0f) a = -1.0f;
-        const float bR = __fsub_rn((float)rm[0], __fmul_rn(a, (float)dm[0]));  // FC:727-731
-        const float bG = __fsub_rn((float)rm[C == 3 ? 1 : 0], __fmul_rn(a, (float)dm[C == 3 ? 1 : 0]));
-        const float bB = __fsub_rn((float)rm[C - 1], __fmul_rn(a, (float)dm[C - 1]));
-        if (info) { info[5 * j] = fc; info[5 * j + 1] = a; info[5 * j + 2] = bR; info[5 * j + 3] = bG; info[5 * j + 4] = bB; }
-        if (q) {
-            q[5 * j] = j_f2i(fc);
-            q[5 * j + 1] = j_f2i(__fmul_rn(a, 1000000.0f));
-            q[5 * j + 2] = j_f2i(__fmul_rn(bR, 100000.0f));
-            q[5 * j + 3] = j_f2i(__fmul_rn(bG, 100000.0f));
-            q[5 * j + 4] = j_f2i(bB);
-        }
+        write_rgb_code(info, q, j, c, rgb_solve(kov, dv, dm, rm));
     }
 }
 
@@ -740,8 +754,7 @@ int launch_encode_fused(const void *d_src, int src_is_argb, const Geom &g, int64
 }
 
 // ------------------------------------------------------------------------------------
-// K3s: code solve + quantisation for the winning candidate (FC:634-643 grey,
-// FC:718-733 RGB; quantisation FC:242-244 / FC:250-254).  One thread per range block.
+// K3s: code solve + quantisation for the winning candidate.  One thread per range block.
 // ------------------------------------------------------------------------------------
 __global__ void k_solve_grey(const uint8_t *__restrict__ src, const uint8_t *__restrict__ dec,
                              const int32_t *__restrict__ dsum, const int32_t *__restrict__ dsq,
@@ -759,8 +772,8 @@ __global__ void k_solve_grey(const uint8_t *__restrict__ src, const uint8_t *__r
     int ky = c / g.wk, kx = c - ky * g.wk;
     int gx = dx + kx, gy = dy + ky;
     int64_t idx = gx + (int64_t)gy * g.dpw;
-    int rs = rsum[j];
-    int rmean = rs / g.n, vR = rs - g.n * rmean;
+    int rmean;
+    const int vR = centred_sum(rsum[j], g.n, &rmean);
     const uint8_t *pr = src + (int64_t)(yr * g.B) * g.W + xr * g.B;
     const uint8_t *pd = dec + (int64_t)(gy * g.step) * g.sw + gx * g.step;
     int dot = 0;
@@ -772,25 +785,7 @@ __global__ void k_solve_grey(const uint8_t *__restrict__ src, const uint8_t *__r
         }
     int dmean;
     int varD = dom_var(dsum[idx], dsq[idx], g.n, &dmean);
-    int kov = dot - dmean * vR;
-    float a = __fdiv_rn((float)kov, (float)varD);  // FC:634 (0/0 -> NaN on flat winners)
-    if (a < -1.0f) a = -1.0f;                      // FC:636-639 (NaN passes through)
-    else if (a > 1.0f) a = 1.0f;
-    float b = __fsub_rn((float)rmean, __fmul_rn(a, (float)dmean));  // FC:641
-    float fc = (float)c;
-    const int S = iso ? 4 : 3;
-    if (info) {
-        info[S * j + 0] = fc;
-        info[S * j + 1] = a;
-        info[S * j + 2] = b;
-        if (iso) info[S * j + 3] = (float)kiso;
-    }
-    if (q) {
-        q[S * j + 0] = j_f2i(fc);                     // FC:242
-        q[S * j + 1] = j_f2i(__fmul_rn(a, 100.0f));   // FC:243
-        q[S * j + 2] = j_f2i(b);                      // FC:244
-        if (iso) q[S * j + 3] = kiso;
-    }
+    write_grey_code(info, q, j, c, grey_solve(dot - dmean * vR, varD, rmean, dmean), iso, kiso);
 }
 
 __global__ void k_solve_rgb(const uint8_t *__restrict__ src, const uint8_t *__restrict__ dec,
@@ -808,47 +803,21 @@ __global__ void k_solve_rgb(const uint8_t *__restrict__ src, const uint8_t *__re
     int gx = dx + kx, gy = dy + ky;
     int64_t idx = gx + (int64_t)gy * g.dpw;
     int rm[3], dm[3], dv[3];
-    for (int ch = 0; ch < 3; ch++) {
-        rm[ch] = rsum[(int64_t)ch * g.NR + j] / g.n;
-        dv[ch] = dom_var(dsum[(int64_t)ch * g.ND + idx], dsq[(int64_t)ch * g.ND + idx], g.n, &dm[ch]);
-    }
+    centred_sum_rgb(rsum, g.NR, j, g.n, rm);
+    for (int ch = 0; ch < 3; ch++) dv[ch] = dom_var(dsum[(int64_t)ch * g.ND + idx], dsq[(int64_t)ch * g.ND + idx], g.n, &dm[ch]);
+    const int dmsum = dm[0] + dm[1] + dm[2];
     int64_t planeS = (int64_t)g.W * g.H, planeD = (int64_t)g.sw * g.sh;
     const uint8_t *pr = src + (int64_t)(yr * g.B) * g.W + xr * g.B;
     const uint8_t *pd = dec + (int64_t)(gy * g.step) * g.sw + gx * g.step;
-    float dR = (float)dm[0], dG = (float)dm[1], dB = (float)dm[2];
     float kov = 0.0f;
     for (int ry = 0; ry < g.B; ry++)
         for (int rx = 0; rx < g.B; rx++) {
             int64_t os = (int64_t)ry * g.W + rx, od = (int64_t)ry * g.sw + rx;
-            float gD = __fadd_rn(__fadd_rn(__fsub_rn((float)pd[od], dR), __fsub_rn((float)pd[planeD + od], dG)),
-                                 __fsub_rn((float)pd[2 * planeD + od], dB));
-            float gR = (float)(((int)pr[os] - rm[0]) + ((int)pr[planeS + os] - rm[1]) +
-                               ((int)pr[2 * planeS + os] - rm[2]));
-            kov = __fadd_rn(kov, __fmul_rn(gR, gD));
+            const int gD = (int)pd[od] + (int)pd[planeD + od] + (int)pd[2 * planeD + od] - dmsum;
+            const int gR = ((int)pr[os] - rm[0]) + ((int)pr[planeS + os] - rm[1]) + ((int)pr[2 * planeS + os] - rm[2]);
+            kov = rgb_kov_step(kov, (float)gR, (float)gD);
         }
-    // FC:776: varianzSquare = varianceR + varianceG + mittelWertB (sic)
-    float varSq = __fadd_rn(__fadd_rn((float)dv[0], (float)dv[1]), (float)dm[2]);
-    float a = __fdiv_rn(kov, varSq);  // FC:718
-    if (a > 1.0f) a = 1.0f;           // FC:721-724
-    if (a < -1.0f) a = -1.0f;
-    float bR = __fsub_rn((float)rm[0], __fmul_rn(a, dR));  // FC:727-731
-    float bG = __fsub_rn((float)rm[1], __fmul_rn(a, dG));
-    float bB = __fsub_rn((float)rm[2], __fmul_rn(a, dB));
-    float fc = (float)c;
-    if (info) {
-        info[5 * j + 0] = fc;
-        info[5 * j + 1] = a;
-        info[5 * j + 2] = bR;
-        info[5 * j + 3] = bG;
-        info[5 * j + 4] = bB;
-    }
-    if (q) {
-        q[5 * j + 0] = j_f2i(fc);                          // FC:250
-        q[5 * j + 1] = j_f2i(__fmul_rn(a, 1000000.0f));    // FC:251
-        q[5 * j + 2] = j_f2i(__fmul_rn(bR, 100000.0f));    // FC:252
-        q[5 * j + 3] = j_f2i(__fmul_rn(bG, 100000.0f));    // FC:253
-        q[5 * j + 4] = j_f2i(bB);                          // FC:254
-    }
+    write_rgb_code(info, q, j, c, rgb_solve(kov, dv, dm, rm));
 }
 
 int launch_solve(const Work &w, const Geom &g, int64_t j0, int64_t j1, float *d_info, int32_t *d_q, cudaStream_t s)
@@ -882,14 +851,14 @@ __device__ __forceinline__ void dequant_one(int64_t j, const int32_t *__restrict
         for (int k = 0; k < S; k++) v[k] = info_in[S * j + k];
     } else if (g.C == 1) {
         v[0] = (float)q[S * j];
-        v[1] = __fdiv_rn((float)q[S * j + 1], 100.0f);
+        v[1] = __fdiv_rn((float)q[S * j + 1], kGreyAScale);
         v[2] = (float)q[S * j + 2];
         if (S == 4) v[3] = (float)(q[S * j + 3] & 7);  // isometry index (extension)
     } else {
         v[0] = (float)q[5 * j];
-        v[1] = __fdiv_rn((float)q[5 * j + 1], 1000000.0f);
-        v[2] = __fdiv_rn((float)q[5 * j + 2], 100000.0f);
-        v[3] = __fdiv_rn((float)q[5 * j + 3], 100000.0f);
+        v[1] = __fdiv_rn((float)q[5 * j + 1], kRgbAScale);
+        v[2] = __fdiv_rn((float)q[5 * j + 2], kRgbBScale);
+        v[3] = __fdiv_rn((float)q[5 * j + 3], kRgbBScale);
         v[4] = (float)q[5 * j + 4];
     }
     int dy, dx;
@@ -956,35 +925,43 @@ __device__ __forceinline__ bool sweep_done(const SweepCtl &ctl)
     return ctl.st && ((volatile const uint32_t *)ctl.st)[ST_DONE] != 0;
 }
 
-// Folds a finished sweep whose float running sum needs no replay into the state: avgError = S / (W*H) with the exact
-// integer S when S < 2^24 (every float partial sum is then exact); S >= 2^24 >= W*H means "not converged" and the
-// value is discarded (FC:416-417).  fic_api.cu only asks for this (ctl.finish) on sweeps where that argument holds.
-__device__ __forceinline__ void sweep_fold(unsigned long long *st, unsigned long long S, int it, float fwh)
+// Records sweep `it` whose float running sum of squared changes is `sum` (FC:407 / FC:493): avgError = sum / (W*H)
+// (FC:413); below 1 the decode has converged and stops with that value (FC:414), otherwise the value is kept only
+// after the last allowed sweep (FC:416-417).
+__device__ __forceinline__ void record_sweep(uint32_t *w, int it, float sum, float fwh, bool last)
 {
-    uint32_t *w = (uint32_t *)st;
-    const float sum = S < (1ull << 24) ? (float)S : 2.0f * fwh;
-    const float avg = __fdiv_rn(sum, fwh);  // FC:413
+    const float avg = __fdiv_rn(sum, fwh);
     w[ST_ITERS] = (uint32_t)(it + 1);
-    if (avg < 1.0f) {  // FC:414
+    if (avg < 1.0f) {
         w[ST_AVG] = __float_as_uint(avg);
         w[ST_DONE] = 1u;
     } else {
-        w[ST_AVG] = 0u;  // FC:416-417 (never the last sweep here)
+        w[ST_AVG] = last ? __float_as_uint(avg) : 0u;
     }
 }
 
-// Common tail of the sweep kernels: add the CTA's squared changes to st[0]; with ctl.finish the last CTA to get
-// here folds the sweep (no separate kernel, no host round trip per sweep).
-__device__ __forceinline__ void sweep_tail(const SweepCtl &ctl, unsigned long long local)
+// Sum of `local` over the CTA (blockDim.x == 256), valid in thread 0.
+__device__ __forceinline__ unsigned long long cta_sum(unsigned long long local)
 {
-    if (!ctl.st) return;
-    __shared__ unsigned long long s_part[8];  // blockDim.x == 256
+    __shared__ unsigned long long s_part[8];
     for (int o = 16; o > 0; o >>= 1) local += __shfl_down_sync(0xffffffffu, local, o);
     if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = local;
     __syncthreads();
-    if (threadIdx.x == 0) {
-        unsigned long long tot = 0;
+    unsigned long long tot = 0;
+    if (threadIdx.x == 0)
         for (int wv = 0; wv < 8; wv++) tot += s_part[wv];
+    return tot;
+}
+
+// Common tail of the sweep kernels: add the CTA's squared changes to st[0]; with ctl.finish the last CTA to get
+// here records the sweep (no separate kernel, no host round trip per sweep).  fic_api.cu only asks for that on
+// sweeps whose float running sum needs no replay: it is the exact integer S when S < 2^24 (every float partial sum
+// is then exact); S >= 2^24 >= W*H means "not converged" and the value is discarded (never the last sweep here).
+__device__ __forceinline__ void sweep_tail(const SweepCtl &ctl, unsigned long long local)
+{
+    if (!ctl.st) return;
+    const unsigned long long tot = cta_sum(local);
+    if (threadIdx.x == 0) {
         if (tot) atomicAdd(ctl.st, tot);
         if (!ctl.finish) return;
         __threadfence();
@@ -993,9 +970,19 @@ __device__ __forceinline__ void sweep_tail(const SweepCtl &ctl, unsigned long lo
             __threadfence();
             const unsigned long long S = atomicExch(ctl.st, 0ull);
             w[ST_TICKET] = 0u;
-            sweep_fold(ctl.st, S, ctl.it, ctl.fwh);
+            record_sweep(w, ctl.it, S < (1ull << 24) ? (float)S : 2.0f * ctl.fwh, ctl.fwh, false);
         }
     }
+}
+
+// A reconstructed pixel, (int)(a * domain + b) -- float multiply, then float add (FC:396 / FC:482) -- clamped to
+// [0, 255] (FC:396-402, FC:743-749).  cvt.rzi.u8.f32 does the cast and the clamp in one instruction: it truncates
+// toward zero and saturates to the destination range, NaN -> 0, like Java's cast followed by applyThreshold.
+__device__ __forceinline__ uint32_t decode_px(float a, float b, uint32_t domain)
+{
+    uint32_t r;
+    asm("cvt.rzi.u8.f32 %0, %1;" : "=r"(r) : "f"(__fadd_rn(__fmul_rn(a, (float)domain), b)));
+    return r;
 }
 
 // One Jacobi sweep of FC:386-412 / FC:463-499.  The reference snapshots the codebook
@@ -1046,12 +1033,8 @@ k_decode_sweep(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img, ui
         for (int c = 0; c < C; c++) {
             float b = cd[2 + c];
             const uint8_t *pd = dec_in + c * planeD + off;
-            int d00 = pd[o00], d10 = pd[o10], d01 = pd[o01], d11 = pd[o11];
-            // FC:396 / FC:482: (int)(a * domain + b), float multiply then float add
-            int v00 = clamp255(j_f2i(__fadd_rn(__fmul_rn(a, (float)d00), b)));
-            int v10 = clamp255(j_f2i(__fadd_rn(__fmul_rn(a, (float)d10), b)));
-            int v01 = clamp255(j_f2i(__fadd_rn(__fmul_rn(a, (float)d01), b)));
-            int v11 = clamp255(j_f2i(__fadd_rn(__fmul_rn(a, (float)d11), b)));
+            const int v00 = (int)decode_px(a, b, pd[o00]), v10 = (int)decode_px(a, b, pd[o10]);
+            const int v01 = (int)decode_px(a, b, pd[o01]), v11 = (int)decode_px(a, b, pd[o11]);
             uint8_t *pi = img + c * planeI + (int64_t)y * g.W + x;
             uchar2 o0 = *(uchar2 *)pi, o1 = *(uchar2 *)(pi + g.W);
             e[0] += (o0.x - v00) * (o0.x - v00);  // FC:407 / FC:493
@@ -1077,14 +1060,6 @@ k_decode_sweep(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img, ui
 // Vector path (W % 8 == 0): one thread owns an 8 x 2 pixel strip (four quads): 8-byte loads of the old
 // pixels, 8-byte stores of the new ones, one 4-byte store of the new decimated pixels; the 16 domain
 // bytes are gathered from the (L2-resident) decimated plane.
-// (int)(float) followed by the reference's clamp to [0, 255] (FC:396-402, FC:743-749) in one instruction: the
-// conversion truncates toward zero and saturates to the destination range, NaN -> 0, like Java's cast + applyThreshold.
-__device__ __forceinline__ uint32_t f2u8_rz_sat(float f)
-{
-    uint32_t r;
-    asm("cvt.rzi.u8.f32 %0, %1;" : "=r"(r) : "f"(f));
-    return r;
-}
 
 // FIRST: the sweep that starts from the constant-128 image (FC:360): every old pixel and every domain pixel is 128,
 // so nothing is read -- the start image and its decimated plane are never materialised (B >= 8 only).
@@ -1172,11 +1147,8 @@ k_decode_sweep_v8(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img,
                     dr0[qd] = (uint32_t)pd[0] | ((uint32_t)pd[1] << 8);
                     dr1[qd] = (uint32_t)pd[g.sw] | ((uint32_t)pd[g.sw + 1] << 8);
                 }
-                // FC:396 / FC:482: (int)(a * domain + b), float multiply then float add, then the clamp
-                const uint32_t v00 = f2u8_rz_sat(__fadd_rn(__fmul_rn(a, (float)(dr0[qd] & 0xffu)), b));
-                const uint32_t v10 = f2u8_rz_sat(__fadd_rn(__fmul_rn(a, (float)(dr0[qd] >> 8)), b));
-                const uint32_t v01 = f2u8_rz_sat(__fadd_rn(__fmul_rn(a, (float)(dr1[qd] & 0xffu)), b));
-                const uint32_t v11 = f2u8_rz_sat(__fadd_rn(__fmul_rn(a, (float)(dr1[qd] >> 8)), b));
+                const uint32_t v00 = decode_px(a, b, dr0[qd] & 0xffu), v10 = decode_px(a, b, dr0[qd] >> 8);
+                const uint32_t v01 = decode_px(a, b, dr1[qd] & 0xffu), v11 = decode_px(a, b, dr1[qd] >> 8);
                 const int sh = 16 * (qd & 1);
                 const uint32_t newq = v00 | (v10 << 8) | (v01 << 16) | (v11 << 24);
                 const uint32_t oldq = ((old0[qd >> 1] >> sh) & 0xffffu) | (((old1[qd >> 1] >> sh) & 0xffffu) << 16);
@@ -1237,12 +1209,8 @@ __host__ __device__ inline bool sweep_interleaved(const Geom &g)
 
 __device__ __forceinline__ uint32_t decode_row4(float a, float b, uint32_t dom4)
 {
-    // FC:396 / FC:482: (int)(a * domain + b), float multiply then float add, then the clamp
-    const uint32_t v0 = f2u8_rz_sat(__fadd_rn(__fmul_rn(a, (float)(dom4 & 0xffu)), b));
-    const uint32_t v1 = f2u8_rz_sat(__fadd_rn(__fmul_rn(a, (float)((dom4 >> 8) & 0xffu)), b));
-    const uint32_t v2 = f2u8_rz_sat(__fadd_rn(__fmul_rn(a, (float)((dom4 >> 16) & 0xffu)), b));
-    const uint32_t v3 = f2u8_rz_sat(__fadd_rn(__fmul_rn(a, (float)(dom4 >> 24)), b));
-    return v0 | (v1 << 8) | (v2 << 16) | (v3 << 24);
+    return decode_px(a, b, dom4 & 0xffu) | (decode_px(a, b, (dom4 >> 8) & 0xffu) << 8) |
+           (decode_px(a, b, (dom4 >> 16) & 0xffu) << 16) | (decode_px(a, b, dom4 >> 24) << 24);
 }
 
 // The sweep itself (all strips this CTA owns); returns the thread's sum of squared pixel changes.  NC: the codes and
@@ -1376,7 +1344,7 @@ k_decode_sweep_il(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img,
 // then sweep / barrier / fold (one thread decides FC:413-417) / barrier until the sweep converges, then write the ARGB
 // ints.  It takes the cases whose avgError needs no replay of the float sum: the exact total is below 2^24 and nothing
 // is carried in (the float sum IS that integer), or the total is so large that the sweep certainly did not converge
-// (skip_from, see k_replay_*) and is not the last allowed one.  Anything else -- a last sweep that has not converged, a
+// (skip_from_of) and is not the last allowed one.  Anything else -- a last sweep that has not converged, a
 // carried-in avgError on a sweep that might converge -- sets the bail word and the host repeats the decode through the
 // per-sweep kernels.
 enum { ST_BARRIER = 8, ST_BAIL = 9 };  // further 32-bit words of the state block
@@ -1400,7 +1368,6 @@ k_decode_small(const int32_t *__restrict__ q, float *__restrict__ code, int32_t 
                uint8_t *__restrict__ dec_a, uint8_t *__restrict__ dec_b, int32_t *__restrict__ argb_out, Geom g,
                unsigned long long *st, int max_iters, float carry, float fwh, unsigned long long skip_from)
 {
-    __shared__ unsigned long long s_part[8];
     uint32_t *w = (uint32_t *)st;
     uint32_t epoch = 0;
     for (int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x; j < g.NR; j += (int64_t)gridDim.x * 256)
@@ -1411,28 +1378,15 @@ k_decode_small(const int32_t *__restrict__ q, float *__restrict__ code, int32_t 
     for (int it = 0; it < max_iters; it++) {
         unsigned long long local = it == 0 ? sweep_il_body<C, B, false, true, false>(din, img, dout, code, dpos, g, nullptr)
                                            : sweep_il_body<C, B, false, false, false>(din, img, dout, code, dpos, g, nullptr);
-        for (int o = 16; o > 0; o >>= 1) local += __shfl_down_sync(0xffffffffu, local, o);
-        if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = local;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            unsigned long long tot = 0;
-            for (int wv = 0; wv < 8; wv++) tot += s_part[wv];
-            if (tot) atomicAdd(st, tot);
-        }
+        const unsigned long long tot = cta_sum(local);
+        if (threadIdx.x == 0 && tot) atomicAdd(st, tot);
         grid_barrier(w + ST_BARRIER, epoch);
         if (blockIdx.x == 0 && threadIdx.x == 0) {
             const unsigned long long S = atomicExch(st, 0ull);
             const bool last = it == max_iters - 1;
             const float c0 = it == 0 ? carry : 0.0f;
             if (c0 == 0.0f && S < (1ull << 24)) {  // the float sum is the exact integer
-                const float avg = __fdiv_rn((float)S, fwh);  // FC:413
-                w[ST_ITERS] = (uint32_t)(it + 1);
-                if (avg < 1.0f) {  // FC:414
-                    w[ST_AVG] = __float_as_uint(avg);
-                    w[ST_DONE] = 1u;
-                } else {
-                    w[ST_AVG] = last ? __float_as_uint(avg) : 0u;  // FC:416-417
-                }
+                record_sweep(w, it, (float)S, fwh, last);
             } else if (!last && c0 >= 0.0f && S >= skip_from) {  // certainly not converged; the value is discarded
                 w[ST_ITERS] = (uint32_t)(it + 1);
                 w[ST_AVG] = 0u;
@@ -1447,23 +1401,7 @@ k_decode_small(const int32_t *__restrict__ q, float *__restrict__ code, int32_t 
         if (done || it == max_iters - 1) { ok = true; break; }
         uint8_t *t = din; din = dout; dout = t;
     }
-    if (ok && argb_out) {
-        const int64_t quads = (int64_t)g.W * g.H / 4;
-        const uchar4 *planes = (const uchar4 *)img;
-        for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < quads; i += (int64_t)gridDim.x * 256) {
-            uchar4 r = planes[i], gg = r, b = r;
-            if (C == 3) {
-                gg = planes[quads + i];
-                b = planes[2 * quads + i];
-            }
-            int4 o;
-            o.x = (int)(0xff000000u | (r.x << 16) | (gg.x << 8) | b.x);
-            o.y = (int)(0xff000000u | (r.y << 16) | (gg.y << 8) | b.y);
-            o.z = (int)(0xff000000u | (r.z << 16) | (gg.z << 8) | b.z);
-            o.w = (int)(0xff000000u | (r.w << 16) | (gg.w << 8) | b.w);
-            ((int4 *)argb_out)[i] = o;
-        }
-    }
+    if (ok && argb_out) pack_argb<C>((const uchar4 *)img, (int4 *)argb_out, (int64_t)g.W * g.H / 4);
 }
 
 // The sweeps are grid-stride over exactly one wave of resident CTAs (SMs x occupancy of the kernel): a second, partly
@@ -1478,9 +1416,20 @@ static int64_t sweep_wave_ctas(K kernel)
     return (int64_t)sms * per_sm;
 }
 
+// skip_from: exact totals from which a sweep over `count` pixels certainly did not converge (only its value < W*H would
+// be kept, FC:413-417).  Every float add loses at most half an ulp, and below W*H an ulp is at most ulp(W*H): with
+// S >= W*H + count * ulp / 2 the float sum cannot end below W*H.  (~0 when no total qualifies.)
+static unsigned long long skip_from_of(float fwh, int64_t count)
+{
+    if (fwh < 1.0f) return ~0ull;
+    int ex = 0;
+    frexpf(fwh, &ex);  // fwh = m * 2^ex, 0.5 <= m < 1: ulp(fwh) = 2^(ex - 24)
+    return (unsigned long long)((double)fwh + (double)count * ldexp(1.0, ex - 25)) + 2ull;
+}
+
 // Small images: the whole decode in one cooperative launch (k_decode_small).  Returns 1 if the kernel was launched (the
 // state block then tells whether it finished or bailed), 0 if this geometry / device does not take the fused path.
-// The state block must be zero.  skip_from as in launch_sweep_finish.
+// The state block must be zero.
 template <int C, int B>
 static int launch_small_t(const int32_t *d_q, float *d_code, int32_t *d_pos, uint8_t *d_img, uint8_t *d_dec_a, uint8_t *d_dec_b,
                           int32_t *d_argb, const Geom &g, unsigned long long *d_state, int max_iters, float carry, float fwh,
@@ -1514,12 +1463,7 @@ int launch_decode_small(const int32_t *d_q, float *d_code, int32_t *d_pos, uint8
                         cudaStream_t s)
 {
     if (!sweep_interleaved(g) || (int64_t)g.W * g.H > ((int64_t)1 << 20)) return 0;
-    unsigned long long skip_from = ~0ull;
-    if (fwh >= 1.0f) {
-        int ex = 0;
-        frexpf(fwh, &ex);
-        skip_from = (unsigned long long)((double)fwh + (double)g.W * g.H * ldexp(1.0, ex - 25)) + 2ull;
-    }
+    const unsigned long long skip_from = skip_from_of(fwh, (int64_t)g.W * g.H);
     if (g.B == 8)
         return g.C == 1 ? launch_small_t<1, 8>(d_q, d_code, d_pos, d_img, d_dec_a, d_dec_b, d_argb, g, d_state, max_iters, carry, fwh, skip_from, s)
                         : launch_small_t<3, 8>(d_q, d_code, d_pos, d_img, d_dec_a, d_dec_b, d_argb, g, d_state, max_iters, carry, fwh, skip_from, s);
@@ -1642,15 +1586,8 @@ __global__ void k_sweep_finish(const int32_t *__restrict__ perr, int64_t count, 
         a = (float)S;
     }
     if (lane == 0) {
-        const float avg = __fdiv_rn(a, fwh);  // FC:413
         *st = 0ull;
-        w[ST_ITERS] = (uint32_t)(it + 1);
-        if (avg < 1.0f) {  // FC:414
-            w[ST_AVG] = __float_as_uint(avg);
-            w[ST_DONE] = 1u;
-        } else {
-            w[ST_AVG] = last ? __float_as_uint(avg) : 0u;  // FC:416-417
-        }
+        record_sweep(w, it, a, fwh, last);
     }
 }
 
@@ -1671,9 +1608,7 @@ __global__ void k_sweep_finish(const int32_t *__restrict__ perr, int64_t count, 
 constexpr int kRepChunk = 4096;                 // pixels per chunk = 256 threads x 16
 struct ReplayChunk { uint32_t sum; int32_t k; uint32_t d0, d1, e0, e1; };  // exact sum, guessed binade (0: none), transducers for binades k and k - 1
 
-// skip_from: exact totals from which a sweep certainly did not converge (only its value < W*H would be kept, FC:413-417).
-// Every float add loses at most half an ulp, and below W*H an ulp is at most ulp(W*H): with S >= W*H + count * ulp / 2
-// the float sum cannot end below W*H.  (~0 on the last allowed sweep, whose value is kept whatever it is.)
+// skip_from: see skip_from_of.
 __device__ __forceinline__ bool replay_not_needed(const unsigned long long *st, float carry, unsigned long long skip_from)
 {
     // done already; or the sweep's exact total is below 2^24 and nothing is carried in: the float sum is that integer
@@ -1923,15 +1858,8 @@ __global__ void k_replay_walk(const int32_t *__restrict__ perr, int64_t count, c
         }
     }
     if (lane == 0) {
-        const float avg = __fdiv_rn(a, fwh);  // FC:413
         *st = 0ull;
-        w[ST_ITERS] = (uint32_t)(it + 1);
-        if (avg < 1.0f) {  // FC:414
-            w[ST_AVG] = __float_as_uint(avg);
-            w[ST_DONE] = 1u;
-        } else {
-            w[ST_AVG] = last ? __float_as_uint(avg) : 0u;  // FC:416-417
-        }
+        record_sweep(w, it, a, fwh, last);
     }
 }
 
@@ -1951,13 +1879,8 @@ int launch_sweep_finish(const int32_t *d_perr, int64_t count, unsigned long long
         const int nchunks = (int)replay_chunks(count), ngroups = (int)replay_groups(count);
         ReplayGroup *gr = (ReplayGroup *)d_workspace;
         ReplayChunk *ch = (ReplayChunk *)(gr + ngroups);
-        unsigned long long skip_from = ~0ull;
-        if (!last && fwh >= 1.0f && carry >= 0.0f) {
-            int ex = 0;
-            frexpf(fwh, &ex);                                   // fwh = m * 2^ex, 0.5 <= m < 1: ulp(fwh) = 2^(ex - 24)
-            const double half_ulp = ldexp(1.0, ex - 25);
-            skip_from = (unsigned long long)((double)fwh + (double)count * half_ulp) + 2ull;
-        }
+        // the last allowed sweep keeps its value whatever it is
+        const unsigned long long skip_from = !last && carry >= 0.0f ? skip_from_of(fwh, count) : ~0ull;
         k_replay_sums<<<nchunks, 256, 0, s>>>(d_perr, count, ch, d_state, carry, skip_from);
         k_replay_scan<<<1, 1024, 0, s>>>(ch, nchunks, d_state, carry, skip_from);
         k_replay_transducers<<<nchunks, 256, 0, s>>>(d_perr, count, ch, d_state, carry, skip_from);

@@ -118,7 +118,6 @@ constexpr int kChunksPerTile = kTileN / 32;
 constexpr int kBoundBytes = kChunksPerTile * 2 * 4 + 16 + kChunksPerTile * 4;
 constexpr int kNormOff = kChunksPerTile * 2 * 4 + 16;     // offset of the norms inside the bounds area
 // Flag lists of a (row, unit): two lists (column halves of the tiles, a historical split) of 32 entries each.
-constexpr int kFlagBytes = 4 * (4 + 8 * 16);         // per (row, unit): list lengths + entries (with slack)
 constexpr int kFlagLists = 2;
 constexpr int kFlagCap = 32;
 constexpr float kOneMinusEps = 1.0f - 1.9073486328125e-06f;  // 1 - 2^-19 (applied to the squared score)
@@ -612,9 +611,8 @@ k_umma_pack_ranges(const uint8_t *__restrict__ src, const int32_t *__restrict__ 
     }
     int xr = (int)(j % g.rpw), yr = (int)(j / g.rpw);
     const uint8_t *p = src + (int64_t)(yr * B) * g.W + xr * B;
-    int rs = rsum[j];
-    int rmean = rs / n;
-    vRout[i] = rs - n * rmean;
+    int rmean;
+    vRout[i] = centred_sum(rsum[j], n, &rmean);
     constexpr int PCH = n / 16;
 #pragma unroll
     for (int c = 0; c < PCH; c++) {
@@ -679,18 +677,6 @@ k_umma_pack_ranges(const uint8_t *__restrict__ src, const int32_t *__restrict__ 
 //     ||gR|| ||gD|| >= 2^24 and 0 below; the packers store upper bounds of ||gR|| per range row and of max ||gD|| per
 //     32-domain chunk.  k_umma_refine_rgb replays the float sum in pixel order, i.e. ranks by kov_ref itself.
 
-__device__ __forceinline__ int rgb_dom_vd(const int32_t *__restrict__ dsum, int64_t ND, int64_t j, int n, int dm[3])
-{
-    int vd = 0;
-#pragma unroll
-    for (int c = 0; c < 3; c++) {
-        const int ds = dsum[(int64_t)c * ND + j];
-        dm[c] = ds / n;
-        vd += ds - n * dm[c];
-    }
-    return vd;
-}
-
 // Sort keys of the RGB pool: vD^2 (plays the role of varD), payload: the domain index.
 __global__ void k_umma_sortkeys_rgb(const int32_t *__restrict__ dsum, int n, int64_t ND, uint32_t *__restrict__ keys,
                                     int32_t *__restrict__ vals)
@@ -698,7 +684,7 @@ __global__ void k_umma_sortkeys_rgb(const int32_t *__restrict__ dsum, int n, int
     int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= ND) return;
     int dm[3];
-    const int vd = rgb_dom_vd(dsum, ND, j, n, dm);
+    const int vd = centred_sum_rgb(dsum, ND, j, n, dm);
     keys[j] = (uint32_t)(vd * vd);
     vals[j] = (int32_t)j;
 }
@@ -743,7 +729,7 @@ k_umma_pack_domains_rgb(const uint16_t *__restrict__ dec3, const int32_t *__rest
         // pixels: B = 8 reads pixel pairs (4-byte loads), B = 16 groups of four (8-byte loads)
         const uint16_t *p = dec3 + (int64_t)(gy * g.step) * g.sw + gx * g.step;
         int dm[3];
-        const int vd = rgb_dom_vd(dsum, g.ND, j, n, dm);
+        const int vd = centred_sum_rgb(dsum, g.ND, j, n, dm);
         const int dmsum = dm[0] + dm[1] + dm[2];
         uint32_t sumsq = 0;  // sum gD^2 <= 256 * 765^2 = 1.5e8: exact in u32
 #pragma unroll
@@ -830,13 +816,9 @@ k_umma_pack_ranges_rgb(const uint8_t *__restrict__ src, const int32_t *__restric
     const int xr = (int)(j % g.rpw), yr = (int)(j / g.rpw);
     const int64_t plane = (int64_t)g.W * g.H;
     const uint8_t *p = src + (int64_t)(yr * B) * g.W + xr * B;
-    int rmsum = 0, vR = 0;
-#pragma unroll
-    for (int c = 0; c < 3; c++) {
-        const int rs = rsum[(int64_t)c * g.NR + j];
-        rmsum += rs / n;
-        vR += rs - n * (rs / n);
-    }
+    int rm[3];
+    const int vR = centred_sum_rgb(rsum, g.NR, j, n, rm);
+    const int rmsum = rm[0] + rm[1] + rm[2];
     uint32_t sumsq = 0;
 #pragma unroll
     for (int c = 0; c < NCH; c++) {
@@ -1887,8 +1869,8 @@ k_umma_refine(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum,
     const int64_t i = (int64_t)blockIdx.x * 4 + warp;  // operand row == range block (the isometry extension has its own kernel)
     if (i >= rows) return;
     const int64_t j = j0 + i;
-    const int rs = rsum[j];
-    const int rmean = rs / n, vR = rs - n * rmean;
+    int rmean;
+    const int vR = centred_sum(rsum[j], n, &rmean);
     if (vR == 0) {  // FC:677-678 + FC:627: all errors are 0, the first candidate wins
         if (lane == 0) best[j] = 0;
         return;
@@ -1931,8 +1913,7 @@ k_umma_refine(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum,
             // x = |kov| / sqrt(varD) within (1 +- 2^-22): |kov| and varD < 2^24 are exact in binary32
             const float ax = varD > 0 ? fabsf((float)kov) * __frsqrt_rn((float)varD) : 0.0f;
             if (ax * (1.0f + 2.384185791015625e-07f) > th) {
-                const float err = grey_error(kov, vR, __dsqrt_rn((double)varD));
-                if (err < be || (err == be && idx < bi)) { be = err; bi = idx; }
+                argmin_merge(be, bi, grey_error(kov, vR, __dsqrt_rn((double)varD)), idx);
                 const float xlo = ax * (1.0f - 2.384185791015625e-07f);
                 if (xlo > lb) { lb = xlo; th = flag_threshold(lb, tie_abs); }
             }
@@ -1940,11 +1921,7 @@ k_umma_refine(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum,
     };
     if (lane == 0) consider(*dom0_pos);
     for_each_flagged(lane, i, rows_padded, n_chunks, npos, flag_list, flag_cnt, th_row, consider);
-    for (int o = 16; o > 0; o >>= 1) {
-        float e2 = __shfl_down_sync(0xffffffffu, be, o);
-        int i2 = __shfl_down_sync(0xffffffffu, bi, o);
-        if (e2 < be || (e2 == be && i2 < bi)) { be = e2; bi = i2; }
-    }
+    warp_argmin(be, bi);
     if (lane == 0) best[j] = bi == 0x7fffffff ? 0 : bi;
 }
 
@@ -1969,8 +1946,8 @@ k_umma_refine_iso(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
     const int64_t r = (int64_t)blockIdx.x * 4 + warp;
     if (r >= ranges) return;
     const int64_t j = j0 + r;
-    const int rs = rsum[j];
-    const int rmean = rs / n, vR = rs - n * rmean;
+    int rmean;
+    const int vR = centred_sum(rsum[j], n, &rmean);
     if (vR == 0) {  // FC:677-678 + FC:627: all errors are 0, the first candidate wins
         if (lane == 0) best[j] = 0;
         return;
@@ -2011,9 +1988,7 @@ k_umma_refine_iso(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
             const int kov = refine_kov<B>(rw, rmean, vR, pos_raw, pos, pi.z);
             const float ax = pi.y > 0 ? fabsf((float)kov) * __frsqrt_rn((float)pi.y) : 0.0f;
             if (ax * (1.0f + 2.384185791015625e-07f) > th) {
-                const float err = grey_error(kov, vR, __dsqrt_rn((double)pi.y));
-                const int c = pi.x * 8 + kiso;
-                if (err < be || (err == be && c < bi)) { be = err; bi = c; }
+                argmin_merge(be, bi, grey_error(kov, vR, __dsqrt_rn((double)pi.y)), pi.x * 8 + kiso);
                 const float xlo = ax * (1.0f - 2.384185791015625e-07f);
                 if (xlo > lb) { lb = xlo; th = flag_threshold(lb, tie_abs); }
             }
@@ -2054,11 +2029,7 @@ k_umma_refine_iso(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
             for (int64_t pos = lane; pos < npos; pos += 32) consider(pos, kiso);
         }
     }
-    for (int o = 16; o > 0; o >>= 1) {
-        float e2 = __shfl_down_sync(0xffffffffu, be, o);
-        int i2 = __shfl_down_sync(0xffffffffu, bi, o);
-        if (e2 < be || (e2 == be && i2 < bi)) { be = e2; bi = i2; }
-    }
+    warp_argmin(be, bi);
     if (lane == 0) best[j] = bi == 0x7fffffff ? 0 : bi;
 }
 
@@ -2079,13 +2050,9 @@ k_umma_refine_rgb(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
     const int64_t i = (int64_t)blockIdx.x * 4 + warp;
     if (i >= rows) return;
     const int64_t j = j0 + i;
-    int rmsum = 0, vRi = 0;
-#pragma unroll
-    for (int c = 0; c < 3; c++) {
-        const int rs = rsum[(int64_t)c * g.NR + j];
-        rmsum += rs / n;
-        vRi += rs - n * (rs / n);
-    }
+    int rm[3];
+    const int vRi = centred_sum_rgb(rsum, g.NR, j, n, rm);
+    const int rmsum = rm[0] + rm[1] + rm[2];
     if (vRi == 0) {  // FC:797 + FC:710: all errors are 0, the first candidate wins
         if (lane == 0) best[j] = 0;
         return;
@@ -2113,9 +2080,7 @@ k_umma_refine_rgb(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
         if (idx >= 0) {
             const int row = (int)(pos % kTileN);
             uint8_t *const blob = const_cast<uint8_t *>(opB) + (pos / kTileN) * L::B_TILE_BYTES;
-            // the reference's kov: sequential binary32 accumulation in pixel order (FC:781-792); every product is an
-            // exact integer, so the fused multiply-add rounds exactly like the reference's multiply-then-add -- also
-            // where partial sums pass 2^24 (B = 16) and the sum is no longer an exact integer
+            // the reference's kov: sequential binary32 accumulation in pixel order (FC:781-792)
             float kov = 0.0f;
 #pragma unroll 8
             for (int c = 0; c < n / 8; c++) {
@@ -2124,18 +2089,14 @@ k_umma_refine_rgb(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
 #pragma unroll
                 for (int e = 0; e < 4; e++) {
                     const float2 f = __half22float2(*(const __half2 *)&w[e]);
-                    kov = __fmaf_rn(gR[c * 8 + 2 * e], f.x, kov);
-                    kov = __fmaf_rn(gR[c * 8 + 2 * e + 1], f.y, kov);
+                    kov = rgb_kov_step(kov, gR[c * 8 + 2 * e], f.x);
+                    kov = rgb_kov_step(kov, gR[c * 8 + 2 * e + 1], f.y);
                 }
             }
             const float vD = (float)pi.y;
             const float ax = pi.y > 0 ? __fdiv_rn(fabsf(kov), vD) : 0.0f;  // x within (1 +- 2^-24)
             if (ax * (1.0f + 2.384185791015625e-07f) > th) {
-                float r = 0.0f;
-                if (pi.y != 0) r = __fdiv_rn(kov, __fmul_rn(vR, vD));   // FC:797-800 (vR != 0 here)
-                r = __fmul_rn(r, r);
-                const float err = __fmul_rn(__fmul_rn(vR, vR), __fsub_rn(1.0f, r));  // FC:803
-                if (err < be || (err == be && idx < bi)) { be = err; bi = idx; }
+                argmin_merge(be, bi, rgb_error(kov, vR, vD), idx);
                 const float xlo = ax * (1.0f - 2.384185791015625e-07f);
                 if (xlo > lb) { lb = xlo; th = flag_threshold(lb, tie_abs); }
             }
@@ -2143,11 +2104,7 @@ k_umma_refine_rgb(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
     };
     if (lane == 0) consider(*dom0_pos);
     for_each_flagged(lane, i, rows_padded, n_chunks, npos, flag_list, flag_cnt, th_row, consider);
-    for (int o = 16; o > 0; o >>= 1) {
-        float e2 = __shfl_down_sync(0xffffffffu, be, o);
-        int i2 = __shfl_down_sync(0xffffffffu, bi, o);
-        if (e2 < be || (e2 == be && i2 < bi)) { be = e2; bi = i2; }
-    }
+    warp_argmin(be, bi);
     if (lane == 0) best[j] = bi == 0x7fffffff ? 0 : bi;
 }
 
@@ -2224,13 +2181,28 @@ struct OpBLayout {
     }
 };
 
+// opA workspace: [A blobs][vR s32][flag_cnt][flag_list][row_lb u32][row_norm f32], per (unit, operand row) of
+// flag_cnt a header of kCntSlots list lengths (s32; the first kFlagLists are used) and of flag_list kFlagLists lists
+// of kFlagCap entries (s32 chunk id, f32 bound)
+template <int B, bool F16>
+struct OpALayout {
+    static constexpr int kCntSlots = 4;
+    size_t off_vR, off_cnt, off_list, off_lb, off_norm, total;
+    explicit OpALayout(const Plan &p)
+    {
+        off_vR = (size_t)p.n_sb * Lay<B, F16>::A_SB_BYTES;
+        off_cnt = off_vR + (size_t)p.rp * 4;
+        off_list = off_cnt + (size_t)p.rp * p.n_chunks * kCntSlots * 4;  // 8-byte aligned: the blobs are, and rp is even
+        off_lb = off_list + (size_t)p.rp * p.n_chunks * kFlagLists * kFlagCap * sizeof(int2);
+        off_norm = off_lb + (size_t)p.rp * 4;
+        total = off_norm + (size_t)p.rp * 4 + 1024;
+    }
+};
+
 template <int B, bool F16>
 size_t opA_bytes_t(const Geom &g, int64_t rows, int num_sms)
 {
-    Plan p = make_plan(g, rows, num_sms);
-    // [A blobs][vR s32][flag_cnt s32 x n_chunks x lists][flag_list (s32 id, f32 bound) x n_chunks x lists x cap][row_lb u32]
-    return (size_t)p.n_sb * Lay<B, F16>::A_SB_BYTES + (size_t)p.rp * 4 + (size_t)p.rp * p.n_chunks * kFlagBytes +
-           (size_t)p.rp * 4 /*row_lb*/ + (size_t)p.rp * 4 /*row norms (RGB, blockgroesse 16)*/ + 1024;
+    return OpALayout<B, F16>(make_plan(g, rows, num_sms)).total;
 }
 
 using KernelT = void (*)(const uint8_t *, const uint8_t *, const int32_t *, const float *, int2 *, int32_t *, uint32_t *, int, int,
@@ -2293,11 +2265,12 @@ int launch_t(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, 
     Plan p = make_plan(g, rows, num_sms);
     const int64_t rp = p.rp;
     uint8_t *opA = w.opA;
-    int32_t *vR = (int32_t *)(opA + (size_t)p.n_sb * L::A_SB_BYTES);
-    int32_t *flag_cnt = vR + rp;
-    int2 *flag_list = (int2 *)(flag_cnt + rp * p.n_chunks * 4);  // 8-byte aligned: the blobs are, and rp is even
-    uint32_t *row_lb = (uint32_t *)(flag_list + rp * p.n_chunks * 64);  // per operand row: best lower bound of max x reached by finished units
-    float *row_norm = (float *)(row_lb + rp);                            // per operand row: >= ||gR||_2 (RGB at blockgroesse 16)
+    const OpALayout<B, F16> la(p);
+    int32_t *vR = (int32_t *)(opA + la.off_vR);
+    int32_t *flag_cnt = (int32_t *)(opA + la.off_cnt);
+    int2 *flag_list = (int2 *)(opA + la.off_list);
+    uint32_t *row_lb = (uint32_t *)(opA + la.off_lb);  // per operand row: best lower bound of max x reached by finished units
+    float *row_norm = (float *)(opA + la.off_norm);    // per operand row: >= ||gR||_2 (RGB at blockgroesse 16)
     const bool rgb = g.C == 3;                        // kind::f16 only (see "RGB operands")
     if (rgb && !F16) { *err = "the RGB tensor path is kind::f16 only"; return -1; }
     OpBLayout<B, F16> lay(g, p);
@@ -2471,10 +2444,11 @@ __global__ void k_umma_selftest_check(const uint8_t *__restrict__ src, const uin
     const int B = g.B, n = g.n;
     int rmean = 0, dmean = 0, vd = 0;
     for (int c = 0; c < g.C; c++) {
-        rmean += rsum[(int64_t)c * g.NR + i] / n;
-        const int ds = dsum[(int64_t)c * g.ND + j];
-        dmean += ds / n;
-        vd += ds - n * (ds / n);
+        int rm, dm;
+        centred_sum(rsum[(int64_t)c * g.NR + i], n, &rm);
+        vd += centred_sum(dsum[(int64_t)c * g.ND + j], n, &dm);
+        rmean += rm;
+        dmean += dm;
     }
     const uint8_t *r = src + (int64_t)((i / g.rpw) * B) * g.W + (i % g.rpw) * B;
     const uint8_t *d = dec + (int64_t)((j / g.dpw) * g.step) * g.sw + (j % g.dpw) * g.step;
