@@ -95,7 +95,7 @@ struct DrainOnExit {
     ~DrainOnExit() { cudaStreamSynchronize(s); }
 };
 
-enum Slot { S_ARGB, S_SRC, S_DEC, S_DSUM, S_DSQ, S_RSUM, S_BEST, S_INFO, S_Q, S_OPA, S_OPB, S_IMG, S_DEC2, S_DCODE, S_PERR, S_ACC, S_DEC3, S_REPLAY };
+enum Slot { S_ARGB, S_SRC, S_DEC, S_DSUM, S_DSQ, S_RSUM, S_BEST, S_INFO, S_Q, S_OPA, S_OPB, S_IMG, S_DEC2, S_DCODE, S_PERR, S_STATE, S_DEC3, S_REPLAY };
 
 template <typename T>
 static int ensure(fic_handle *h, T *&p, int slot, size_t bytes)
@@ -120,6 +120,13 @@ static int ensure(fic_handle *h, T *&p, int slot, size_t bytes)
         int rc_ = ensure(h, ptr, slot, (size_t)(bytes)); \
         if (rc_) return rc_;                           \
     } while (0)
+
+// The error of a decoder entry (fic_decode.cu); out_of_pool: the message for a code outside the domain pool.
+static int decode_err(fic_handle *h, const DecodeStatus &st, const char *out_of_pool)
+{
+    if (st.rc == FIC_E_CUDA) return set_err(h, FIC_E_CUDA, "%s failed: %s (%s:%d)", st.call, cudaGetErrorString(st.cuda), st.file, st.line);
+    return st.rc ? set_err(h, st.rc, "%s", out_of_pool) : FIC_OK;
+}
 
 extern "C" {
 
@@ -181,7 +188,7 @@ void fic_destroy(fic_handle *h)
     cudaStreamSynchronize(h->stream);
     Work &w = h->w;
     void *ptrs[] = {w.argb, w.src, w.dec, w.dsum, w.dsq, w.rsum, w.best, w.info, w.q, w.opA, w.opB,
-                    w.img, w.dec2, w.dcode, w.perr, w.acc, w.avgf, w.dec3, w.replay};
+                    w.img, w.dec2, w.dcode, w.perr, w.state, w.dec3, w.replay};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (int i = 0; i < 8; i++)
@@ -581,24 +588,13 @@ int fic_debug_float_sum(fic_handle *h, const int32_t *terms, int64_t count, floa
     Work &w = h->w;
     cudaStream_t s = h->stream;
     ENSURE(w.perr, S_PERR, sizeof(int32_t) * (size_t)count);
-    ENSURE(w.acc, S_ACC, 64 * sizeof(unsigned long long));
-    const size_t replay_bytes = sweep_finish_workspace(count);
+    ENSURE(w.state, S_STATE, sizeof(DecodeState));
+    const size_t replay_bytes = decode_replay_bytes(count);
     if (replay_bytes) ENSURE(w.replay, S_REPLAY, replay_bytes);
-    unsigned long long state[8] = {0};
-    for (int64_t i = 0; i < count; i++) {
+    for (int64_t i = 0; i < count; i++)
         if (terms[i] < 0 || terms[i] > 3 * 255 * 255) return set_err(h, FIC_E_ARG, "terms must lie in [0, 3 * 255^2]");
-        state[0] += (unsigned long long)terms[i];  // what a sweep leaves in the state block: the exact total
-    }
     DrainOnExit drain(s);
-    CU(cudaMemcpyAsync(w.perr, terms, sizeof(int32_t) * (size_t)count, cudaMemcpyHostToDevice, s));
-    CU(cudaMemcpyAsync(w.acc, state, sizeof state, cudaMemcpyHostToDevice, s));
-    // "last sweep" keeps the value whatever it is; divided by 1 it is the sum itself
-    launch_sweep_finish(w.perr, count, w.acc, 0, 1, carry, 1.0f, replay_bytes ? w.replay : nullptr, s);
-    CU(cudaMemcpyAsync(h->h_acc, w.acc, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    CU(cudaGetLastError());
-    memcpy(sum, &((const uint32_t *)h->h_acc)[7], sizeof *sum);
-    return FIC_OK;
+    return decode_err(h, decode_float_sum(w, terms, count, carry, h->h_acc, sum, s), "");
 }
 
 int fic_build_pool(fic_handle *h, const int32_t *argb, int is_rgb, int W, int H, int B, uint8_t *decimated,
@@ -634,18 +630,8 @@ int fic_build_pool(fic_handle *h, const int32_t *argb, int is_rgb, int W, int H,
 // decode / collage
 // ------------------------------------------------------------------------------------
 
-// Decoder core.  Codes come from the host (`qcodes`) or from device memory (`d_qcodes`); the image goes to host ARGB
+// Decoder entries.  Codes come from the host (`qcodes`) or from device memory (`d_qcodes`); the image goes to host ARGB
 // ints (the reference's RasterImage.argb), host 8-bit planes or device 8-bit planes -- exactly one of the three.
-//
-// avgError bookkeeping (FC:407-417).  The reference adds every squared pixel change to a binary32 running sum,
-// divides by W*H after the sweep and stops below 1.  The sum is an exact integer while it stays below 2^24, so with
-// W*H <= 2^24 the integer total S decides: S < 2^24 -> the float sum equals S; otherwise the float sum is
-// >= 2^24 >= W*H and the sweep did not converge (its value is then discarded, FC:416-417).  Such sweeps are folded
-// into the device-side state by the sweep kernel's last CTA.  Sweeps whose float sum may be both inexact and kept
-// (carry-in on the first sweep, the last allowed sweep, images above 2^24 pixels) also write the per-pixel squared
-// changes in loop order and are folded by k_sweep_finish, which replays the float accumulation where it must.
-// Sweeps are enqueued eight at a time without looking at the result: once the done flag is set the remaining ones
-// return immediately, and the host reads the state once per batch instead of once per sweep.
 static int decode_core(fic_handle *h, int is_rgb, int W, int H, int B, int wk, const int32_t *qcodes, const int32_t *d_qcodes,
                        int max_iters, int32_t *argb_out, uint8_t *planes_out, uint8_t *d_planes_out, float *avg_error,
                        int *iterations)
@@ -668,110 +654,17 @@ static int decode_core(fic_handle *h, int is_rgb, int W, int H, int B, int wk, c
     if (!d_planes_out) ENSURE(w.img, S_IMG, g.C * plane);
     ENSURE(w.dec, S_DEC, (size_t)g.C * g.sw * g.sh);
     ENSURE(w.dec2, S_DEC2, (size_t)g.C * g.sw * g.sh);
-    ENSURE(w.acc, S_ACC, 64 * sizeof(unsigned long long));
+    ENSURE(w.state, S_STATE, sizeof(DecodeState));
     if (argb_out) ENSURE(w.argb, S_ARGB, sizeof(int32_t) * plane);
-    const bool big = (int64_t)W * H > ((int64_t)1 << 24);
-    const float carry = avg_error ? *avg_error : 0.0f;
-    const float fwh = (float)(W * H);  // FC:413 (float)(width*height)
     ENSURE(w.perr, S_PERR, sizeof(int32_t) * plane);  // per-pixel squared changes of the sweeps that may need a replay
-    const size_t replay_bytes = sweep_finish_workspace((int64_t)plane);
+    const size_t replay_bytes = decode_replay_bytes((int64_t)plane);
     if (replay_bytes) ENSURE(w.replay, S_REPLAY, replay_bytes);
-    uint8_t *img = d_planes_out ? d_planes_out : w.img;
     DrainOnExit drain(s);
     CU(cudaEventRecord(h->ev[0], s));
     if (!d_qcodes) CU(cudaMemcpyAsync(w.q, qcodes, sizeof(int32_t) * g.NR * S, cudaMemcpyHostToDevice, s));
-    CU(cudaMemsetAsync(w.acc, 0, 64 * sizeof(unsigned long long), s));
-    int launches = 0;
-    int32_t *doff = (int32_t *)(w.dcode + g.NR * S);
-    // B >= 8, W % 16 == 0: the sweeps keep the decimated plane row-pair interleaved (k_decode_sweep_il) and take the
-    // domain positions packed
-    const int il = decode_sweep_interleaved(g) ? 1 : 0;
-    const uint32_t *hst = (const uint32_t *)h->h_acc;  // host copy of the state block as 32-bit words: [5..7] = done, iters, avg; [9] = bail
-    // Small images (the reference's own sizes): the whole decode in ONE cooperative launch (k_decode_small) -- unless its
-    // avgError would need the float sum replayed (word 9 of the state: bail), in which case the decode is repeated below.
-    if (il && plane <= ((size_t)1 << 20) &&
-        launch_decode_small(d_qcodes ? d_qcodes : w.q, w.dcode, doff, img, w.dec, w.dec2, argb_out ? w.argb : nullptr, g, w.acc, max_iters,
-                            carry, fwh, s)) {
-        launches++;
-        CU(cudaMemcpyAsync(h->h_acc, w.acc, 5 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
-        // the output is copied without waiting for the verdict (<= 4 MB); a bailed decode overwrites it below
-        if (argb_out) CU(cudaMemcpyAsync(argb_out, w.argb, sizeof(int32_t) * plane, cudaMemcpyDeviceToHost, s));
-        else if (planes_out) CU(cudaMemcpyAsync(planes_out, img, g.C * plane, cudaMemcpyDeviceToHost, s));
-        CU(cudaEventRecord(h->ev[5], s));
-        CU(cudaStreamSynchronize(s));
-        if (h->h_acc[1]) return set_err(h, FIC_E_STREAM, "a code indexes outside the domain pool (the reference would throw ArrayIndexOutOfBounds)");
-        if (!hst[9]) {
-            CU(cudaGetLastError());
-            float ms = 0;
-            if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[5]) == cudaSuccess) h->tm.total_ms = ms;
-            h->tm.launches = launches;
-            float avg;
-            memcpy(&avg, &hst[7], sizeof avg);
-            if (avg_error) *avg_error = avg;
-            if (iterations) *iterations = (int)hst[6];
-            return FIC_OK;
-        }
-        CU(cudaMemsetAsync(w.acc, 0, 64 * sizeof(unsigned long long), s));
-    }
-    launches += launch_dequant(d_qcodes ? d_qcodes : w.q, w.dcode, doff, g, 0, nullptr, w.acc, il, s);
-    // The start image is the constant 128 (FC:360, FC:1142-1148) and so is its 2x-decimated plane, for every tap rule
-    // (FC:970-1007, FC:901-962).  For B >= 8 neither is materialised: the first sweep knows what it would read.
-    const bool implicit_start = decode_sweep_has_first(g);
-    if (!implicit_start) {
-        launches += launch_fill(img, g.C * plane, 128, s);
-        CU(cudaMemsetAsync(w.dec, 128, (size_t)g.C * g.sw * g.sh, s));
-    }
-    uint8_t *dcur = w.dec, *dnext = w.dec2;
-    // Small images: the output copy is enqueued behind every batch, so that a decode that converges within the batch
-    // (the usual case) costs one host synchronisation in all; a later batch simply copies again.
-    const bool speculative_out = !d_planes_out && plane * (argb_out ? 4 : g.C) <= ((size_t)4 << 20);
-    auto enqueue_output = [&]() -> int {
-        if (argb_out) {
-            launches += launch_pack_argb(img, w.argb, W, H, g.C, s);
-            CU(cudaMemcpyAsync(argb_out, w.argb, sizeof(int32_t) * plane, cudaMemcpyDeviceToHost, s));
-        } else if (planes_out) {
-            CU(cudaMemcpyAsync(planes_out, img, g.C * plane, cudaMemcpyDeviceToHost, s));
-        }
-        return FIC_OK;
-    };
-    int it = 0;
-    bool out_done = false;
-    while (it < max_iters) {
-        // a skipped sweep still costs a launch (~1.5 us), a second batch a host round trip (~40 us): grey decodes converge
-        // in 5-9 sweeps, the reference's RGB quantisation (FC:250-254) needs 13-22
-        const int batch = (g.C == 3 && speculative_out) ? 16 : 8;
-        const int batch_end = it + batch < max_iters ? it + batch : max_iters;
-        for (; it < batch_end; it++) {
-            const bool last = it == max_iters - 1;
-            const bool replay = big || last || (it == 0 && carry != 0.0f);
-            SweepCtl ctl = {w.acc, it, replay ? 0 : 1, fwh};
-            launches += launch_decode_sweep(dcur, img, dnext, w.dcode, doff, g, ctl, replay ? w.perr : nullptr, it == 0 && implicit_start, il, s);
-            if (replay) launches += launch_sweep_finish(w.perr, (int64_t)plane, w.acc, it, last, it == 0 ? carry : 0.0f, fwh, replay_bytes ? w.replay : nullptr, s);
-            uint8_t *t = dcur; dcur = dnext; dnext = t;
-        }
-        CU(cudaMemcpyAsync(h->h_acc, w.acc, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
-        if (speculative_out && (rc = enqueue_output())) return rc;
-        // device-resident output: the batch is the whole call (the end event must not wait for the host's state read)
-        if (speculative_out || d_planes_out) CU(cudaEventRecord(h->ev[5], s));
-        CU(cudaStreamSynchronize(s));
-        if (h->h_acc[1]) return set_err(h, FIC_E_STREAM, "a code indexes outside the domain pool (the reference would throw ArrayIndexOutOfBounds)");
-        out_done = speculative_out || d_planes_out;
-        if (hst[5]) break;  // converged (FC:414)
-    }
-    if (!out_done) {
-        if ((rc = enqueue_output())) return rc;
-        CU(cudaEventRecord(h->ev[5], s));
-        CU(cudaStreamSynchronize(s));
-    }
-    CU(cudaGetLastError());
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[5]) == cudaSuccess) h->tm.total_ms = ms;
-    h->tm.launches = launches;
-    float avg;
-    memcpy(&avg, &hst[7], sizeof avg);
-    if (avg_error) *avg_error = avg;
-    if (iterations) *iterations = (int)hst[6];
-    return FIC_OK;
+    const DecodeStatus st = decode_run(w, g, d_qcodes ? d_qcodes : w.q, d_planes_out ? d_planes_out : w.img, argb_out, planes_out,
+                                       max_iters, avg_error, iterations, h->h_acc, h->ev[0], h->ev[5], &h->tm, s);
+    return decode_err(h, st, "a code indexes outside the domain pool (the reference would throw ArrayIndexOutOfBounds)");
 }
 
 int fic_decode(fic_handle *h, int is_rgb, int W, int H, int B, int wk, const int32_t *qcodes, int max_iters,
@@ -813,25 +706,13 @@ int fic_collage(fic_handle *h, int is_rgb, const int32_t *argb, int W, int H, in
     ENSURE(w.info, S_INFO, sizeof(float) * g.NR * S);
     ENSURE(w.dcode, S_DCODE, sizeof(float) * g.NR * (S + 1));
     ENSURE(w.img, S_IMG, g.C * plane);
-    ENSURE(w.acc, S_ACC, 64 * sizeof(unsigned long long));
+    ENSURE(w.state, S_STATE, sizeof(DecodeState));
     DrainOnExit drain(s);
     CU(cudaMemcpyAsync(w.argb, argb, sizeof(int32_t) * plane, cudaMemcpyHostToDevice, s));
     CU(cudaMemcpyAsync(w.info, info, sizeof(float) * g.NR * S, cudaMemcpyHostToDevice, s));
-    CU(cudaMemsetAsync(w.acc, 0, 64 * sizeof(unsigned long long), s));
     launch_unpack(w.argb, w.src, W, H, g.C, s);
-    launch_decimate(w.src, w.dec, g, s);                       // FC:275 codebook of the source
-    int32_t *doff = (int32_t *)(w.dcode + g.NR * S);
-    launch_dequant(nullptr, w.dcode, doff, g, 1, w.info, w.acc, 0, s);  // FC:273 calculateIndices
-    launch_fill(w.img, g.C * plane, 0xa0, s);                  // RasterImage.java:19,31
-    launch_decode_sweep(w.dec, w.img, nullptr, w.dcode, doff, g, SweepCtl{nullptr, 0, 0, 0.0f}, nullptr, 0, 0, s);
-    launch_pack_argb(w.img, w.argb, W, H, g.C, s);
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(h->h_acc, w.acc, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(argb_out, w.argb, sizeof(int32_t) * plane, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(info, w.dcode, sizeof(float) * g.NR * S, cudaMemcpyDeviceToHost, s));  // FC:888 in-place
-    CU(cudaStreamSynchronize(s));
-    if (h->h_acc[1]) return set_err(h, FIC_E_STREAM, "a code indexes outside the domain pool");
-    return FIC_OK;
+    launch_decimate(w.src, w.dec, g, s);  // FC:275 codebook of the source
+    return decode_err(h, collage_run(w, g, argb_out, info, h->h_acc, s), "a code indexes outside the domain pool");
 }
 
 }  // extern "C"

@@ -148,6 +148,17 @@ __device__ __forceinline__ int dom_var(int dsum, int dsq, int n, int *dmean)
     return dsq - m * (2 * dsum - n * m);
 }
 
+// One pixel of the 2x decimation (K1b in fic_kernels.cu) from the taps p00, p10 (row y), p01, p11 (row y + 1) of source
+// column x.  Used by the pool builder and by the decoder sweeps, which decimate the image they write.
+__device__ __forceinline__ int dec_tap4(int p00, int p10, int p01, int p11, int x, int H, bool rgb)
+{
+    int fourth = (x + 1 >= H) ? 128 : (rgb ? p01 : p11);
+    return (p00 + p10 + p01 + fourth) / 4;
+}
+
+// Quantisation scales of the code stream: written by FC:242-244 / FC:250-254, read back by FC:372-374 / FC:446-450.
+constexpr float kGreyAScale = 100.0f, kRgbAScale = 1000000.0f, kRgbBScale = 100000.0f;
+
 #endif  // __CUDACC__
 
 }  // namespace fic

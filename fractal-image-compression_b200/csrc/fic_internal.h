@@ -2,6 +2,7 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
 
 #include "../../include/fic_b200.h"
@@ -28,6 +29,17 @@ __host__ __device__ inline int code_stride(const Geom &g) { return g.C == 3 ? 5 
 // reference's exceptions).
 int make_geom(int W, int H, int B, int wk, int mode, Geom *g, const char **why);
 
+// State block of a decode (device memory), shared by its kernels and read back by the host: the running sweep's exact
+// sum of squared pixel changes, a "code indexes outside the pool" flag, the ticket of the sweep's CTAs, the done flag
+// (converged, FC:414), the sweeps run, avgError's bits, and the grid barrier and bail word of the one-launch decoder.
+// 8-byte aligned for the u64 atomics.
+struct DecodeState {
+    unsigned long long sq_sum, bad_index;
+    uint32_t ticket, done, iters, avg_bits, barrier, bail;
+};
+static_assert(sizeof(DecodeState) == 40 && offsetof(DecodeState, bad_index) == 8 && offsetof(DecodeState, ticket) == 16 &&
+              offsetof(DecodeState, avg_bits) == 28 && offsetof(DecodeState, bail) == 36, "u64 words 0-1, u32 words 4-9");
+
 // Device workspace owned by a handle (grow-only).
 struct Work {
     int32_t *argb = nullptr;    // W*H staging of the caller's ARGB ints
@@ -45,10 +57,9 @@ struct Work {
     // decoder
     uint8_t *img = nullptr;     // C planes W*H: the image being reconstructed (updated in place)
     uint8_t *dec2 = nullptr;    // second decimated buffer (Jacobi ping-pong with `dec`)
-    float *avgf = nullptr;      // 1 float: running avgError for the exact replay kernel
     float *dcode = nullptr;     // [NR][3|5] dequantised codes with codebook indices, then s32 doff[NR] (domain byte offsets)
     int32_t *perr = nullptr;    // per-pixel squared change in reference loop order (exact avgError path)
-    unsigned long long *acc = nullptr;  // [64] integer accumulators / flags
+    DecodeState *state = nullptr;  // the decoder's state block
     uint16_t *dec3 = nullptr;   // RGB: R + G + B of the decimated planes (CUDA-core search)
     uint8_t *replay = nullptr;  // decoder, large images: per-chunk records of the exact avgError replay
     size_t cap[20] = {0};
@@ -56,7 +67,6 @@ struct Work {
 
 // ---- kernel launchers (each returns the number of kernels it launched) -----------
 int launch_unpack(const int32_t *d_argb, uint8_t *d_planes, int W, int H, int C, cudaStream_t s);
-int launch_pack_argb(const uint8_t *d_planes, int32_t *d_argb, int W, int H, int C, cudaStream_t s);
 int launch_decimate(const uint8_t *d_src, uint8_t *d_dec, const Geom &g, cudaStream_t s);
 int launch_domain_stats(const uint8_t *d_dec, int32_t *d_dsum, int32_t *d_dsq, const Geom &g,
                         cudaStream_t s);
@@ -97,39 +107,31 @@ int launch_search_umma(const Work &w, const Geom &g, int64_t j0, int64_t j1, int
                        cudaEvent_t k1 = nullptr, int pair = FIC_UMMA_PAIR_AUTO, int *pair_used = nullptr,
                        int32_t *dump = nullptr, int64_t dump_ld = 0, int *status_dev = nullptr);
 
-// decoder
-int launch_dequant(const int32_t *d_q, float *d_code, int32_t *d_off, const Geom &g, int unquantised,
-                   const float *d_info, unsigned long long *d_acc, int packed, cudaStream_t s);
-int launch_fill(uint8_t *d_planes, size_t bytes, int value, cudaStream_t s);
-// Control block of one decoder sweep.  st == nullptr: a plain sweep (the one-shot collage).  Otherwise st points at
-// the decoder state (fic_kernels.cu, "Decoder state block"): the sweep returns at once when the done flag is set,
-// adds its squared pixel changes to st[0] and, with finish != 0, its last CTA folds the sweep into the state
-// (avgError, iteration count, done flag; FC:413-417) so that the host need not look at every sweep.
-struct SweepCtl {
-    unsigned long long *st;
-    int it;      // sweep index (FC:381 counter)
-    int finish;  // 1: fold inside the sweep kernel -- only when the float sum needs no replay (see k_sweep_finish)
-    float fwh;   // (float)(W*H), FC:413
+// ---- decoder (fic_decode.cu) -----------------------------------------------------------------------------------------
+// Outcome of a decoder entry.  rc: FIC_OK; FIC_E_STREAM when a code indexes outside the domain pool (the reference
+// throws ArrayIndexOutOfBounds); FIC_E_CUDA when `call` (file:line) returned `cuda`.
+struct DecodeStatus {
+    int rc = FIC_OK;
+    cudaError_t cuda = cudaSuccess;
+    const char *call = nullptr, *file = nullptr;
+    int line = 0;
 };
-// first (only where decode_sweep_has_first(g)): the sweep starts from the constant-128 image (FC:360) and reads nothing
-// interleaved (only where decode_sweep_interleaved(g)): decoder loop over the row-pair interleaved decimated plane
-// (k_decode_sweep_il); d_off then holds packed positions (launch_dequant with packed = 1)
-int launch_decode_sweep(const uint8_t *d_dec_in, uint8_t *d_img, uint8_t *d_dec_out,
-                        const float *d_code, const int32_t *d_off, const Geom &g,
-                        const SweepCtl &ctl, int32_t *d_perr, int first, int interleaved, cudaStream_t s);
-bool decode_sweep_has_first(const Geom &g);
-// Small images (<= 2^20 pixels, interleaved-plane geometry): dequantisation, every sweep, the convergence rule and the
-// ARGB conversion (d_argb may be null) in ONE cooperative launch.  Returns 1 if launched: the state block (zero on
-// entry) then holds done / sweeps / avgError as after the per-sweep kernels, or word 9 != 0 = "bailed: repeat through the
-// per-sweep kernels" (a float avgError sum that would need a replay).  0: not taken (geometry, device).
-int launch_decode_small(const int32_t *d_q, float *d_code, int32_t *d_pos, uint8_t *d_img, uint8_t *d_dec_a, uint8_t *d_dec_b,
-                        int32_t *d_argb, const Geom &g, unsigned long long *d_state, int max_iters, float carry, float fwh,
-                        cudaStream_t s);
-bool decode_sweep_interleaved(const Geom &g);
-// folds a sweep whose float running sum may have to be replayed in loop order (see k_sweep_finish)
-// d_workspace: sweep_finish_workspace(count) bytes (0 for small images: one warp replays the sum literally)
-int launch_sweep_finish(const int32_t *d_perr, int64_t count, unsigned long long *d_state, int it, int last,
-                        float carry, float fwh, void *d_workspace, cudaStream_t s);
-size_t sweep_finish_workspace(int64_t count);
+
+// Iterative decode (FC:355-420) of the codes at d_q into the device planes d_img, also copied to argb_out (host ARGB) or
+// planes_out (host planes) when given.  avg_error (optional): in, the avgError the last decode left (FC:20); out, this
+// decode's.  tm: total_ms from ev0 (recorded by the caller) to end, and launches.  h_scratch: pinned, sizeof(DecodeState).
+// Workspace: dcode, dec, dec2, state, perr (W*H ints), replay (decode_replay_bytes(W*H)) and, with argb_out, argb.
+DecodeStatus decode_run(const Work &w, const Geom &g, const int32_t *d_q, uint8_t *d_img, int32_t *argb_out,
+                        uint8_t *planes_out, int max_iters, float *avg_error, int *iterations, void *h_scratch,
+                        cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, cudaStream_t s);
+// One collage step (FC:268-280): the float codes in w.info applied once to the source's codebook w.dec over an image of
+// 0xa0 pixels; the image to argb_out, the codes with codebook indices (FC:888) to info_out.  Also uses dcode, img, argb.
+DecodeStatus collage_run(const Work &w, const Geom &g, int32_t *argb_out, float *info_out, void *h_scratch, cudaStream_t s);
+// *sum = carry + terms[0] + ... + terms[count - 1] in binary32, in order, as the last sweep of a decode over `count`
+// pixels folds it (terms in [0, 3 * 255^2]).  Workspace: perr (count ints), state, replay (decode_replay_bytes(count)).
+DecodeStatus decode_float_sum(const Work &w, const int32_t *terms, int64_t count, float carry, void *h_scratch, float *sum,
+                              cudaStream_t s);
+// Device workspace of the chunked replay of a sweep over `pixels` pixels (0: the one-warp replay needs none).
+size_t decode_replay_bytes(int64_t pixels);
 
 }  // namespace fic

@@ -1,4 +1,4 @@
-"""The arithmetic behind the decoder's chunked avgError replay (DESIGN 4.5, k_replay_* in csrc/fic_kernels.cu), as a
+"""The arithmetic behind the decoder's chunked avgError replay (DESIGN 4.5, k_replay_* in csrc/fic_decode.cu), as a
 numpy model that runs without a GPU: above 2^24 a binary32 running sum a = A * u (u = ulp, 2^23 <= A < 2^24) that
 receives an integer e = m * u + r moves to A + m + c with c = [r > u/2], or the parity of A + m on a tie r == u/2
 (round to nearest even).  A run of terms therefore acts on A through its parity only -- a two-state transducer
