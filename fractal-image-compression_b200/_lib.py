@@ -35,6 +35,7 @@ ABI_SYMBOLS = [
     "fic_create_multi", "fic_destroy_multi", "fic_multi_last_error", "fic_multi_device_count", "fic_multi_handle",
     "fic_multi_set_option", "fic_multi_get_timings", "fic_multi_range_slice", "fic_multi_encode_grey",
     "fic_multi_encode_rgb", "fic_multi_encode_grey_iso", "fic_multi_encode_grey_u8", "fic_multi_encode_rgb_planes",
+    "fic_encode_batch", "fic_encode_batch_u8", "fic_decode_batch", "fic_decode_batch_u8",
 ]
 
 
@@ -84,6 +85,10 @@ def load() -> C.CDLL:
         fn.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, i64, i64, vp, vp]
     for fn in (L.fic_decode_u8, L.fic_decode_planes_dev):
         fn.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, f32p, C.POINTER(C.c_int)]
+    for fn in (L.fic_encode_batch, L.fic_encode_batch_u8):
+        fn.argtypes = [vp, C.c_int, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]
+    for fn in (L.fic_decode_batch, L.fic_decode_batch_u8):
+        fn.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, vp, vp]
     L.fic_create_multi.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(vp)]
     L.fic_destroy_multi.argtypes = [vp]
     L.fic_destroy_multi.restype = None

@@ -206,6 +206,71 @@ class Handle:
                                        C.byref(avg), C.byref(it)))
         return out, np.float32(avg.value), it.value
 
+    def encode_batch(self, argb: np.ndarray, B: int, wk: int, rgb, info: np.ndarray | None = None,
+                     q: np.ndarray | None = None):
+        """fic_encode_batch: n same-size images, int32 ARGB [n, H, W], mode rgb = False / True / FIC_MODE_GREY_ISO;
+        returns (info float32 [n, NR, S], qcodes int32 [n, NR, S]), each image's rows equal to encode() of that image."""
+        a = np.ascontiguousarray(argb, dtype=np.int32)
+        assert a.ndim == 3, "argb must be [n, H, W]"
+        n, H, W = a.shape
+        info, q = self._batch_codes(n, W, H, B, (3, 5, 4)[int(rgb)], info, q)
+        self._check(self._L.fic_encode_batch(self._h, int(rgb), _ptr(a), n, W, H, B, wk, _ptr(info), _ptr(q)))
+        return info, q
+
+    def encode_batch_u8(self, planes: np.ndarray, B: int, wk: int, rgb=None, info: np.ndarray | None = None,
+                        q: np.ndarray | None = None):
+        """fic_encode_batch_u8: uint8 [n, H, W] (grey: the red channel; rgb may be FIC_MODE_GREY_ISO) or [n, 3, H, W]
+        (RGB).  rgb=None takes the mode from the shape."""
+        a = np.ascontiguousarray(planes, dtype=np.uint8)
+        assert a.ndim in (3, 4) and (a.ndim == 3 or a.shape[1] == 3), "planes must be [n, H, W] or [n, 3, H, W]"
+        if rgb is None:
+            rgb = a.ndim == 4
+        assert (a.ndim == 4) == (int(rgb) == 1), "RGB takes [n, 3, H, W] planes, grey [n, H, W]"
+        n, H, W = a.shape[0], a.shape[-2], a.shape[-1]
+        info, q = self._batch_codes(n, W, H, B, (3, 5, 4)[int(rgb)], info, q)
+        self._check(self._L.fic_encode_batch_u8(self._h, int(rgb), _ptr(a), n, W, H, B, wk, _ptr(info), _ptr(q)))
+        return info, q
+
+    @staticmethod
+    def _batch_codes(n, W, H, B, S, info, q):
+        nr = (W // B) * (H // B) if B > 0 else 0
+        if info is None:
+            info = np.zeros((n, max(nr, 0), S), np.float32)
+        if q is None:
+            q = np.zeros((n, max(nr, 0), S), np.int32)
+        for t, dt in ((info, np.float32), (q, np.int32)):
+            assert t.dtype == dt and t.shape == (n, max(nr, 0), S) and t.flags["C_CONTIGUOUS"]
+        return info, q
+
+    def _decode_batch(self, fn, q, W, H, B, wk, rgb, avg_error, max_iters, out):
+        qq = np.ascontiguousarray(q, dtype=np.int32)
+        assert qq.ndim == 3, "q must be [n, NR, S]"
+        n = qq.shape[0]
+        avg = np.zeros(n, np.float32) if avg_error is None else np.array(avg_error, np.float32).reshape(n)
+        it = np.zeros(n, np.int32)
+        self._check(fn(self._h, int(rgb), n, W, H, B, wk, _ptr(qq), max_iters, _ptr(out), _ptr(avg), _ptr(it)))
+        return out, avg, it
+
+    def decode_batch(self, q: np.ndarray, W: int, H: int, B: int, wk: int, rgb, avg_error=None, max_iters: int = 50,
+                     out: np.ndarray | None = None):
+        """fic_decode_batch: codes [n, NR, S] -> (ARGB int32 [n, H, W], avgError float32 [n], iterations int32 [n]).
+        avg_error: each image's carry-in (the reference's never-reset static, FC:20), None for 0."""
+        n = np.shape(q)[0]
+        if out is None:
+            out = np.empty((n, H, W), np.int32)
+        assert out.dtype == np.int32 and out.shape == (n, H, W) and out.flags["C_CONTIGUOUS"]
+        return self._decode_batch(self._L.fic_decode_batch, q, W, H, B, wk, rgb, avg_error, max_iters, out)
+
+    def decode_batch_u8(self, q: np.ndarray, W: int, H: int, B: int, wk: int, rgb, avg_error=None, max_iters: int = 50,
+                        out: np.ndarray | None = None):
+        """fic_decode_batch_u8: as decode_batch with 8-bit planes, uint8 [n, H, W] (grey) or [n, 3, H, W] (RGB)."""
+        n = np.shape(q)[0]
+        shape = (n, 3, H, W) if int(rgb) == 1 else (n, H, W)
+        if out is None:
+            out = np.empty(shape, np.uint8)
+        assert out.dtype == np.uint8 and out.shape == shape and out.flags["C_CONTIGUOUS"]
+        return self._decode_batch(self._L.fic_decode_batch_u8, q, W, H, B, wk, rgb, avg_error, max_iters, out)
+
     def float_sum(self, terms: np.ndarray, carry: float = 0.0) -> np.float32:
         """fic_debug_float_sum: the reference's sequential binary32 running sum (FC:407) over integer terms, computed
         the way the decoder folds a sweep."""

@@ -309,14 +309,15 @@ static int pick_engine(fic_handle *h, const Geom &g, int64_t j0, int64_t j1, int
     return FIC_OK;
 }
 
-// Fused windowed encode straight from the caller's pixels (ARGB ints or planes).  Records events 1..4.
+// Fused windowed encode straight from the caller's pixels (ARGB ints or planes).  Records events 1..4.  n_images > 1: a
+// batch, every range of that many images back to back (launch_encode_fused).
 static int encode_fused_on_device(fic_handle *h, const Geom &g, const void *d_pixels, int is_argb, int64_t j0, int64_t j1,
-                                  float *d_info, int32_t *d_q)
+                                  float *d_info, int32_t *d_q, int n_images = 1)
 {
     cudaStream_t s = h->stream;
     // one kernel: events 1 and 4 bracket it (collect_timings reads the stages of this engine from those two alone)
     CU(cudaEventRecord(h->ev[1], s));
-    const int launches = launch_encode_fused(d_pixels, is_argb, g, j0, j1, d_info, d_q, s);
+    const int launches = launch_encode_fused(d_pixels, is_argb, g, j0, j1, d_info, d_q, s, n_images);
     CU(cudaEventRecord(h->ev[4], s));
     CU(cudaGetLastError());
     h->tm.engine = FIC_ENGINE_FUSED;
@@ -475,7 +476,153 @@ static int encode_host(fic_handle *h, int is_rgb, const void *pixels, int src_u8
     return FIC_OK;
 }
 
+// ---- batches of same-size images ----------------------------------------------------------------------------------
+
+// Input pixels one group of a batch uploads at most: the grow-only workspace does not grow with the batch.
+constexpr size_t kBatchGroupBytes = (size_t)64 << 20;
+static_assert(kDecodeBatchMax * sizeof(DecodeState) <= kStageBytes, "a decode group's state blocks come back through h_stage");
+
+// The checks every batch entry adds to make_geom's: n_images >= 1 and byte counts of the whole batch that fit.
+static int batch_geom(fic_handle *h, int mode, int n_images, int W, int H, int B, int wk, Geom *g)
+{
+    if (n_images < 1) return set_err(h, FIC_E_ARG, "n_images must be >= 1");
+    const char *why = "";
+    const int rc = make_geom(W, H, B, wk, mode, g, &why);
+    if (rc) return set_err(h, rc, "%s", why);
+    int64_t bytes;
+    if (__builtin_mul_overflow((int64_t)n_images, (int64_t)W * H * 4, &bytes) ||
+        __builtin_mul_overflow((int64_t)n_images, g->NR * code_stride(*g) * 4, &bytes))
+        return set_err(h, FIC_E_ARG, "n_images = %d images of %d x %d overflow a byte count", n_images, W, H);
+    return FIC_OK;
+}
+
+// A batch encode: the codes of n_images images back to back, [n][NR][S], each equal to a single encode of that image.
+// Where pick_engine chooses the fused encode, one launch per group covers every range of every image; otherwise each
+// image runs encode_on_device.  Groups of images go up in one copy and their codes come down in one.
+static int encode_batch_host(fic_handle *h, int mode, const void *pixels, int src_u8, int n_images, int W, int H, int B, int wk,
+                             float *info, int32_t *qcodes)
+{
+    if (!h) return FIC_E_ARG;
+    if (!pixels || (!info && !qcodes)) return set_err(h, FIC_E_ARG, "the images and at least one of info/qcodes must be non-NULL");
+    Geom g;
+    int rc = batch_geom(h, mode, n_images, W, H, B, wk, &g);
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    memset(&h->tm, 0, sizeof h->tm);
+    Work &w = h->w;
+    cudaStream_t s = h->stream;
+    int engine;
+    if ((rc = pick_engine(h, g, 0, g.NR, &engine))) return rc;
+    const bool fused = engine == FIC_ENGINE_FUSED;
+    const int S = code_stride(g);
+    const size_t plane = (size_t)W * H, image_bytes = src_u8 ? g.C * plane : sizeof(int32_t) * plane;
+    const size_t codes = (size_t)g.NR * S, table = sizeof(float) * codes;  // one image's code table (float and int32 alike)
+    const int group = (int)(kBatchGroupBytes / image_bytes < (size_t)n_images ? (kBatchGroupBytes / image_bytes > 0 ? kBatchGroupBytes / image_bytes : 1) : n_images);
+    if (src_u8) {
+        ENSURE(w.src, S_SRC, image_bytes * group);
+    } else {
+        ENSURE(w.argb, S_ARGB, image_bytes * group);
+        if (!fused) ENSURE(w.src, S_SRC, g.C * plane);  // one image's planes, unpacked before its encode
+    }
+    ENSURE(w.info, S_INFO, table * group);
+    ENSURE(w.q, S_Q, table * group);
+    DrainOnExit drain(s);
+    CU(cudaEventRecord(h->ev[0], s));
+    for (int i0 = 0; i0 < n_images; i0 += group) {
+        const int gn = n_images - i0 < group ? n_images - i0 : group;
+        void *d_pixels = src_u8 ? (void *)w.src : (void *)w.argb;
+        CU(cudaMemcpyAsync(d_pixels, (const uint8_t *)pixels + i0 * image_bytes, image_bytes * gn, cudaMemcpyHostToDevice, s));
+        if (fused) {
+            if ((rc = encode_fused_on_device(h, g, d_pixels, !src_u8, 0, g.NR, w.info, w.q, gn))) return rc;
+        } else {
+            for (int i = 0; i < gn; i++) {
+                const uint8_t *d_src = w.src + i * g.C * plane;
+                if (!src_u8) {
+                    h->tm.launches += launch_unpack(w.argb + i * plane, w.src, W, H, g.C, s);
+                    d_src = w.src;
+                }
+                if ((rc = encode_on_device(h, g, d_src, 0, g.NR, w.info + i * codes, w.q + i * codes, engine))) return rc;
+            }
+        }
+        if (info) CU(cudaMemcpyAsync(info + i0 * codes, w.info, table * gn, cudaMemcpyDeviceToHost, s));
+        if (qcodes) CU(cudaMemcpyAsync(qcodes + i0 * codes, w.q, table * gn, cudaMemcpyDeviceToHost, s));
+    }
+    CU(cudaEventRecord(h->ev[5], s));
+    CU(cudaStreamSynchronize(s));
+    CU(cudaGetLastError());
+    const int launches = h->tm.launches, used = h->tm.engine;
+    memset(&h->tm, 0, sizeof h->tm);  // the per-stage events saw the last image only: report the whole call
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[5]) == cudaSuccess) h->tm.total_ms = ms;
+    h->tm.engine = used;
+    h->tm.launches = launches;
+    h->tm.search_evals = (double)n_images * (double)g.NR * (double)g.wk * (double)g.wk * (double)g.n_iso;
+    return FIC_OK;
+}
+
+// A batch decode (decode_batch_run): every image as a single decode with its own carry-in would give it.
+static int decode_batch_host(fic_handle *h, int mode, int n_images, int W, int H, int B, int wk, const int32_t *qcodes,
+                             int max_iters, int32_t *argb_out, uint8_t *planes_out, float *avg_error, int *iterations)
+{
+    if (!h) return FIC_E_ARG;
+    if (!qcodes || (!argb_out && !planes_out)) return set_err(h, FIC_E_ARG, "codes and the output images must be non-NULL");
+    if (max_iters < 1) return set_err(h, FIC_E_ARG, "max_iters must be >= 1");
+    Geom g;
+    int rc = batch_geom(h, mode, n_images, W, H, B, wk, &g);
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    memset(&h->tm, 0, sizeof h->tm);
+    Work &w = h->w;
+    cudaStream_t s = h->stream;
+    const int S = code_stride(g);
+    const size_t plane = (size_t)W * H;
+    const int batch = decode_batch_group(g), group = batch < n_images ? batch : n_images;
+    const size_t k = group > 0 ? group : 1;  // images the one-launch workspace holds (decode_run needs one)
+    ENSURE(w.q, S_Q, sizeof(int32_t) * g.NR * S * k);
+    ENSURE(w.dcode, S_DCODE, sizeof(float) * g.NR * (S + 1) * k);
+    ENSURE(w.img, S_IMG, g.C * plane * k);
+    ENSURE(w.dec, S_DEC, (size_t)g.C * g.sw * g.sh * k);
+    ENSURE(w.dec2, S_DEC2, (size_t)g.C * g.sw * g.sh * k);
+    ENSURE(w.state, S_STATE, (sizeof(DecodeState) + sizeof(float)) * k);  // state blocks, then the carries
+    if (argb_out) ENSURE(w.argb, S_ARGB, sizeof(int32_t) * plane * k);
+    ENSURE(w.perr, S_PERR, sizeof(int32_t) * plane);
+    const size_t replay_bytes = decode_replay_bytes((int64_t)plane);
+    if (replay_bytes) ENSURE(w.replay, S_REPLAY, replay_bytes);
+    DrainOnExit drain(s);
+    CU(cudaEventRecord(h->ev[0], s));
+    int bad = -1;
+    const DecodeStatus st = decode_batch_run(w, g, n_images, group, qcodes, argb_out, planes_out, max_iters, avg_error, iterations,
+                                             h->h_stage, h->h_acc, h->ev[0], h->ev[5], &h->tm, &bad, s);
+    if (st.rc == FIC_E_STREAM)
+        return set_err(h, FIC_E_STREAM, "image %d: a code indexes outside the domain pool (the reference would throw ArrayIndexOutOfBounds)", bad);
+    return decode_err(h, st, "");
+}
+
 extern "C" {
+
+int fic_encode_batch(fic_handle *h, int mode, const int32_t *argb, int n_images, int W, int H, int B, int wk, float *info,
+                     int32_t *qcodes)
+{
+    return encode_batch_host(h, mode, argb, 0, n_images, W, H, B, wk, info, qcodes);
+}
+
+int fic_encode_batch_u8(fic_handle *h, int mode, const uint8_t *planes, int n_images, int W, int H, int B, int wk, float *info,
+                        int32_t *qcodes)
+{
+    return encode_batch_host(h, mode, planes, 1, n_images, W, H, B, wk, info, qcodes);
+}
+
+int fic_decode_batch(fic_handle *h, int mode, int n_images, int W, int H, int B, int wk, const int32_t *qcodes, int max_iters,
+                     int32_t *argb_out, float *avg_error, int *iterations)
+{
+    return decode_batch_host(h, mode, n_images, W, H, B, wk, qcodes, max_iters, argb_out, nullptr, avg_error, iterations);
+}
+
+int fic_decode_batch_u8(fic_handle *h, int mode, int n_images, int W, int H, int B, int wk, const int32_t *qcodes, int max_iters,
+                        uint8_t *planes_out, float *avg_error, int *iterations)
+{
+    return decode_batch_host(h, mode, n_images, W, H, B, wk, qcodes, max_iters, nullptr, planes_out, avg_error, iterations);
+}
 
 int fic_encode_grey(fic_handle *h, const int32_t *argb, int W, int H, int B, int wk, int64_t range_begin,
                     int64_t range_end, float *info, int32_t *qcodes)

@@ -6,6 +6,8 @@
 #include <math.h>
 #include <string.h>
 
+#include <vector>
+
 #include "fic_device.cuh"
 
 namespace fic {
@@ -411,10 +413,15 @@ __device__ __forceinline__ T sweep_ld(const T *p)
     return *p;
 }
 
+// Warp tiles of a sweep over the interleaved plane: 16 x 2 strips each (see sweep_il_body).
+__host__ __device__ inline uint32_t il_tiles(const Geom &g) { return (((uint32_t)g.W / 8u + 15u) >> 4) * ((uint32_t)g.H >> 2); }
+
+// The warp sweeps tiles wt, wt + wt_step, ... below wt_end.
 template <int C, int B, bool PERR, bool FIRST, bool NC = true>
 __device__ __forceinline__ unsigned long long sweep_il_body(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img,
                                                             uint8_t *__restrict__ dec_out, const float *__restrict__ code,
-                                                            const int32_t *__restrict__ dpos, const Geom &g, int32_t *__restrict__ perr)
+                                                            const int32_t *__restrict__ dpos, const Geom &g, int32_t *__restrict__ perr,
+                                                            uint32_t wt, uint32_t wt_end, uint32_t wt_step)
 {
     constexpr int LB = B == 8 ? 3 : 4, BM = B - 1, S = C == 1 ? 3 : 5;
     const uint32_t W = (uint32_t)g.W, sw = (uint32_t)g.sw, rpw = (uint32_t)g.rpw;
@@ -425,9 +432,9 @@ __device__ __forceinline__ unsigned long long sweep_il_body(const uint8_t *__res
     // A warp owns a tile of 16 x 2 strips: lanes 0-15 the strips of decimated row 2 tr, lanes 16-31 the same columns of
     // row 2 tr + 1 -- the two rows of one interleaved pair, so that the warp's one store of decimated pixels writes whole
     // 32-byte sectors (half-written sectors cost a read-modify-write once the planes no longer fit in L2).
-    const uint32_t tiles_x = (sw8 + 15u) >> 4, tiles = tiles_x * ((uint32_t)g.H >> 2);
+    const uint32_t tiles_x = (sw8 + 15u) >> 4;
     const uint32_t lane = threadIdx.x & 31u;
-    for (uint32_t wt = blockIdx.x * 8u + (threadIdx.x >> 5); wt < tiles; wt += gridDim.x * 8u) {
+    for (; wt < wt_end; wt += wt_step) {
         const uint32_t tr = wt / tiles_x, tx = wt - tr * tiles_x;
         const uint32_t qy = 2u * tr + (lane >> 4), s8 = 16u * tx + (lane & 15u);
         if (s8 >= sw8) continue;
@@ -522,7 +529,8 @@ k_decode_sweep_il(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img,
                   int32_t *__restrict__ perr)
 {
     if (sweep_done(ctl)) return;
-    sweep_tail(ctl, sweep_il_body<C, B, PERR, FIRST>(dec_in, img, dec_out, code, dpos, g, perr));
+    sweep_tail(ctl, sweep_il_body<C, B, PERR, FIRST>(dec_in, img, dec_out, code, dpos, g, perr, blockIdx.x * 8u + (threadIdx.x >> 5),
+                                                     il_tiles(g), gridDim.x * 8u));
 }
 
 // ---- small images: the whole decode in ONE cooperative launch ------------------------------------------------------
@@ -535,6 +543,13 @@ k_decode_sweep_il(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img,
 // (skip_from_of) and is not the last allowed one.  Anything else -- a last sweep that has not converged, a
 // carried-in avgError on a sweep that might converge -- sets the bail word and the host repeats the decode through the
 // per-sweep kernels.
+//
+// A batch of n same-size images (fic_decode_batch) runs in the same launch: one state block per image, the images'
+// buffers back to back.  A unit of work is (image, 8 consecutive warp tiles), one CTA's worth; CTAs grid-stride over
+// the units of all images, so with one image unit blockIdx.x + k gridDim.x is exactly the tiles the per-sweep kernel's
+// CTA visits.  A CTA sums its squared changes per image and adds them to that image's state when its next unit belongs
+// to another image and at the end of the sweep.  The fold decides every image on its own; an image that converged or
+// bailed is frozen (its units are skipped) while the others sweep on.
 
 __device__ __forceinline__ void grid_barrier(uint32_t *counter, uint32_t &epoch)
 {
@@ -549,45 +564,102 @@ __device__ __forceinline__ void grid_barrier(uint32_t *counter, uint32_t &epoch)
     __syncthreads();
 }
 
-template <int C, int B>
-__global__ void __launch_bounds__(256)
+// MULTI: n_img images with their carried-in avgError at `carries`; otherwise the one image of a single decode with `carry`
+// (n_img == 1 is then known at compile time, and what only a batch needs -- the flushes between images, the frozen
+// images, the fold loop -- compiles away).  The batch form asks for 4 CTAs per SM (<= 64 registers): left to itself
+// ptxas gives it 40 registers and a spill.
+template <int C, int B, bool MULTI>
+__global__ void __launch_bounds__(256, MULTI ? 4 : 0)
 k_decode_small(const int32_t *__restrict__ q, float *__restrict__ code, int32_t *__restrict__ dpos, uint8_t *__restrict__ img,
                uint8_t *__restrict__ dec_a, uint8_t *__restrict__ dec_b, int32_t *__restrict__ argb_out, Geom g,
-               DecodeState *st, int max_iters, float carry, float fwh, unsigned long long skip_from)
+               DecodeState *st, int max_iters, float carry, float fwh, unsigned long long skip_from, uint32_t n_img,
+               const float *__restrict__ carries)
 {
+    constexpr int S = C == 1 ? 3 : 5;
+    const uint32_t NR = (uint32_t)g.NR, n = MULTI ? n_img : 1u;
+    const size_t planeI = (size_t)C * g.W * g.H, planeD = (size_t)C * g.sw * g.sh;
     uint32_t epoch = 0;
-    for (int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x; j < g.NR; j += (int64_t)gridDim.x * 256)
-        dequant_one(j, q, nullptr, code, dpos, g, 0, st, 1);
+    for (uint32_t jf = blockIdx.x * 256u + threadIdx.x; jf < n * NR; jf += gridDim.x * 256u) {
+        const uint32_t im = MULTI ? jf / NR : 0u;
+        dequant_one(jf - im * NR, q + (size_t)im * NR * S, nullptr, code + (size_t)im * NR * S, dpos + (size_t)im * NR, g, 0, st + im, 1);
+    }
     grid_barrier(&st->barrier, epoch);
+    const uint32_t tiles = il_tiles(g), per_img = (tiles + 7u) / 8u, units = n * per_img, warp = threadIdx.x >> 5;
+    // unit u = im * per_img + lu, stepped by gridDim.x = dq * per_img + dr without a division per unit
+    const uint32_t im0 = MULTI ? blockIdx.x / per_img : 0u, lu0 = blockIdx.x - im0 * per_img;
+    const uint32_t dq = MULTI ? gridDim.x / per_img : 0u, dr = MULTI ? gridDim.x - dq * per_img : 0u;
     uint8_t *din = dec_a, *dout = dec_b;
-    bool ok = false;
+    uint32_t bail0 = 0;  // the first image's bail word after the last fold
     for (int it = 0; it < max_iters; it++) {
-        unsigned long long local = it == 0 ? sweep_il_body<C, B, false, true, false>(din, img, dout, code, dpos, g, nullptr)
-                                           : sweep_il_body<C, B, false, false, false>(din, img, dout, code, dpos, g, nullptr);
-        const unsigned long long tot = cta_sum(local);
-        if (threadIdx.x == 0 && tot) atomicAdd(&st->sq_sum, tot);
-        grid_barrier(&st->barrier, epoch);
-        if (blockIdx.x == 0 && threadIdx.x == 0) {
-            const unsigned long long S = atomicExch(&st->sq_sum, 0ull);
-            const bool last = it == max_iters - 1;
-            const float c0 = it == 0 ? carry : 0.0f;
-            if (c0 == 0.0f && S < (1ull << 24)) {  // the float sum is the exact integer
-                record_sweep(st, it, (float)S, fwh, last);
-            } else if (!last && c0 >= 0.0f && S >= skip_from) {  // certainly not converged; the value is discarded
-                st->iters = (uint32_t)(it + 1);
-                st->avg_bits = 0u;
-            } else {
-                st->bail = 1u;
+        unsigned long long local = 0;  // this CTA's squared changes of image `cur` so far
+        uint32_t cur = im0, im = im0, lu = lu0;
+        bool pending = false;
+        for (uint32_t u = blockIdx.x; u < units; u += gridDim.x, im += dq, lu += dr) {
+            if (MULTI && lu >= per_img) {
+                lu -= per_img;
+                im++;
             }
-            __threadfence();
+            const uint32_t t0 = 8u * (MULTI ? lu : u);
+            if (im != cur) {
+                if (pending) {
+                    const unsigned long long tot = cta_sum(local);
+                    if (threadIdx.x == 0 && tot) atomicAdd(&st[cur].sq_sum, tot);
+                    __syncthreads();  // cta_sum's shared partials are read by thread 0 before they are rewritten
+                    local = 0;
+                    pending = false;
+                }
+                cur = im;
+            }
+            // frozen (with one image the loop only runs while it sweeps)
+            if (MULTI && (state_word(st[im].done) | state_word(st[im].bail))) continue;
+            const uint32_t wt = t0 + warp, wt_end = min(tiles, t0 + 8u);
+            uint8_t *const pi = img + im * planeI, *const pin = din + im * planeD, *const pout = dout + im * planeD;
+            const float *const pc = code + (size_t)im * NR * S;
+            const int32_t *const pp = dpos + (size_t)im * NR;
+            local += it == 0 ? sweep_il_body<C, B, false, true, false>(pin, pi, pout, pc, pp, g, nullptr, wt, wt_end, 8u)
+                             : sweep_il_body<C, B, false, false, false>(pin, pi, pout, pc, pp, g, nullptr, wt, wt_end, 8u);
+            pending = true;
+        }
+        const unsigned long long tot = cta_sum(local);
+        if (threadIdx.x == 0 && tot) atomicAdd(&st[cur].sq_sum, tot);
+        grid_barrier(&st->barrier, epoch);
+        if (blockIdx.x == 0) {
+            const bool last = it == max_iters - 1;
+            bool sweeping = false;  // some image of this thread sweeps again
+            for (uint32_t i = threadIdx.x; i < n; i += 256u) {
+                DecodeState *const si = st + i;
+                // frozen images (one image is still sweeping whenever the loop runs: no state read on that path)
+                if (MULTI && (si->done | si->bail)) continue;
+                const unsigned long long sum = atomicExch(&si->sq_sum, 0ull);
+                const float c0 = it == 0 ? (MULTI ? carries[i] : carry) : 0.0f;
+                bool again;  // the image sweeps again
+                if (c0 == 0.0f && sum < (1ull << 24)) {  // the float sum is the exact integer
+                    record_sweep(si, it, (float)sum, fwh, last);
+                    again = !(__fdiv_rn((float)sum, fwh) < 1.0f);  // not converged (record_sweep's test)
+                } else if (!last && c0 >= 0.0f && sum >= skip_from) {  // certainly not converged; the value is discarded
+                    si->iters = (uint32_t)(it + 1);
+                    si->avg_bits = 0u;
+                    again = true;
+                } else {
+                    si->bail = 1u;
+                    again = false;
+                }
+                sweeping |= !last && again;
+            }
+            if (MULTI) sweeping = __syncthreads_or(sweeping);  // (one image: thread 0 folded it)
+            if (threadIdx.x == 0) {
+                st->ticket = sweeping ? 1u : 0u;
+                __threadfence();
+            }
         }
         grid_barrier(&st->barrier, epoch);
-        const uint32_t done = state_word(st->done), bail = state_word(st->bail);
-        if (bail) return;
-        if (done || it == max_iters - 1) { ok = true; break; }
+        bail0 = state_word(st->bail);  // read beside the ticket: the one image's verdict costs no extra round trip
+        if (!state_word(st->ticket)) break;
         uint8_t *t = din; din = dout; dout = t;
     }
-    if (ok && argb_out) pack_argb<C>((const uchar4 *)img, (int4 *)argb_out, (int64_t)g.W * g.H / 4);
+    if (argb_out)
+        for (uint32_t i = 0; i < n; i++)
+            if (!(i == 0 ? bail0 : state_word(st[i].bail))) pack_argb<C>((const uchar4 *)(img + i * planeI), (int4 *)(argb_out + (size_t)i * g.W * g.H), (int64_t)g.W * g.H / 4);
 }
 
 // The literal float accumulation (FC:407 / FC:493) over perr[begin, end), stopping once the sum reaches `limit` (one
@@ -1007,11 +1079,12 @@ static unsigned long long skip_from_of(float fwh, int64_t count)
     return (unsigned long long)((double)fwh + (double)count * ldexp(1.0, ex - 25)) + 2ull;
 }
 
-// The whole decode in one cooperative launch (k_decode_small; p.one_launch only).  Returns 1 if the kernel was launched
-// (the state block, zero on entry, then tells whether it finished or bailed), 0 if this device does not take it.
-template <int C, int B>
+// The whole decode of n_img images in one cooperative launch (k_decode_small; p.one_launch only).  Returns 1 if the kernel
+// was launched (the state blocks, zero on entry, then tell whether each image finished or bailed), 0 if this device does
+// not take it.  MULTI (a batch): carries, device [n_img]; otherwise the one image of a single decode, `carry`.
+template <int C, int B, bool MULTI>
 static int launch_small(const Work &w, const Geom &g, const int32_t *d_q, int32_t *d_pos, uint8_t *d_img, int32_t *d_argb,
-                        int max_iters, float carry, float fwh, cudaStream_t s)
+                        int max_iters, float carry, float fwh, cudaStream_t s, uint32_t n_img, const float *carries)
 {
     static int coop = -1, per_sm = 0, sms = 0;
     if (coop < 0) {
@@ -1019,12 +1092,11 @@ static int launch_small(const Work &w, const Geom &g, const int32_t *d_q, int32_
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_decode_small<C, B>, 256, 0) != cudaSuccess) per_sm = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_decode_small<C, B, MULTI>, 256, 0) != cudaSuccess) per_sm = 0;
         cudaGetLastError();
     }
     if (coop <= 0 || per_sm < 1) return 0;
-    const int64_t tiles = (int64_t)((g.W / 8 + 15) / 16) * (g.H / 4);
-    int64_t grid = (tiles + 7) / 8;
+    int64_t grid = (int64_t)n_img * ((il_tiles(g) + 7) / 8);  // units of 8 warp tiles
     if (grid > (int64_t)sms * per_sm) grid = (int64_t)sms * per_sm;
     Geom gg = g;
     float *code = w.dcode;
@@ -1032,8 +1104,9 @@ static int launch_small(const Work &w, const Geom &g, const int32_t *d_q, int32_
     DecodeState *st = w.state;
     unsigned long long skip_from = skip_from_of(fwh, (int64_t)g.W * g.H);
     void *args[] = {(void *)&d_q, (void *)&code, (void *)&d_pos, (void *)&d_img, (void *)&dec_a, (void *)&dec_b, (void *)&d_argb,
-                    (void *)&gg, (void *)&st, (void *)&max_iters, (void *)&carry, (void *)&fwh, (void *)&skip_from};
-    if (cudaLaunchCooperativeKernel((const void *)k_decode_small<C, B>, dim3((unsigned)grid), dim3(256), args, 0, s) != cudaSuccess) {
+                    (void *)&gg, (void *)&st, (void *)&max_iters, (void *)&carry, (void *)&fwh, (void *)&skip_from, (void *)&n_img,
+                    (void *)&carries};
+    if (cudaLaunchCooperativeKernel((const void *)k_decode_small<C, B, MULTI>, dim3((unsigned)grid), dim3(256), args, 0, s) != cudaSuccess) {
         cudaGetLastError();
         return 0;
     }
@@ -1112,8 +1185,9 @@ DecodeStatus decode_run(const Work &w, const Geom &g, const int32_t *d_q, uint8_
     bool done = false;
     // Small images (the reference's own sizes): the whole decode in ONE cooperative launch (k_decode_small) -- unless its
     // avgError would need the float sum replayed (bail), in which case the decode is repeated below.
-    const auto small = g.B == 8 ? (g.C == 1 ? launch_small<1, 8> : launch_small<3, 8>) : (g.C == 1 ? launch_small<1, 16> : launch_small<3, 16>);
-    if (p.one_launch && small(w, g, d_q, doff, img, argb_out ? w.argb : nullptr, max_iters, carry, fwh, s)) {
+    const auto small = g.B == 8 ? (g.C == 1 ? launch_small<1, 8, false> : launch_small<3, 8, false>)
+                                : (g.C == 1 ? launch_small<1, 16, false> : launch_small<3, 16, false>);
+    if (p.one_launch && small(w, g, d_q, doff, img, argb_out ? w.argb : nullptr, max_iters, carry, fwh, s, 1u, nullptr)) {
         launches++;
         DCU(cudaMemcpyAsync(h_scratch, w.state, sizeof(DecodeState), cudaMemcpyDeviceToHost, s));
         // the output is copied without waiting for the verdict (<= 4 MB); a bailed decode overwrites it below
@@ -1170,6 +1244,81 @@ DecodeStatus decode_run(const Work &w, const Geom &g, const int32_t *d_q, uint8_
     tm->launches = launches;
     if (avg_error) memcpy(avg_error, &hs->avg_bits, sizeof *avg_error);
     if (iterations) *iterations = (int)hs->iters;
+    return DecodeStatus{};
+}
+
+int decode_batch_group(const Geom &g)
+{
+    if (!decode_plan(g).one_launch) return 0;
+    // the images of one launch stay L2-resident together, the budget sweep_interleaved gives one image (so at least 1)
+    const int64_t per_image = (int64_t)g.C * ((int64_t)g.W * g.H + 2 * (int64_t)g.sw * g.sh);
+    const int64_t n = ((int64_t)48 << 20) / per_image;
+    return (int)(n < kDecodeBatchMax ? n : kDecodeBatchMax);
+}
+
+// Groups of `group` images through k_decode_small, then every image the one-launch decoder did not finish -- it bailed
+// (its avgError needs the float sum replayed), the geometry has no one-launch form (group == 0) or the device cannot
+// launch it cooperatively -- through decode_run, one image at a time: the path fic_decode takes.
+DecodeStatus decode_batch_run(const Work &w, const Geom &g, int n, int group, const int32_t *qcodes, int32_t *argb_out,
+                              uint8_t *planes_out, int max_iters, float *avg_error, int *iterations, void *h_stage,
+                              void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, int *bad_image, cudaStream_t s)
+{
+    const size_t plane = (size_t)g.W * g.H, codes = (size_t)g.NR * code_stride(g);
+    const float fwh = (float)(g.W * g.H);  // FC:413 (float)(width*height)
+    int launches = 0;
+    std::vector<char> redo((size_t)n, group == 0);
+    const auto small = g.B == 8 ? (g.C == 1 ? launch_small<1, 8, true> : launch_small<3, 8, true>)
+                                : (g.C == 1 ? launch_small<1, 16, true> : launch_small<3, 16, true>);
+    const DecodeState *hs = (const DecodeState *)h_stage;
+    for (int i0 = 0; group > 0 && i0 < n; i0 += group) {
+        const int gn = n - i0 < group ? n - i0 : group;
+        int32_t *dpos = (int32_t *)(w.dcode + (size_t)group * codes);
+        float *d_carry = (float *)(w.state + group);
+        DCU(cudaMemcpyAsync(w.q, qcodes + i0 * codes, sizeof(int32_t) * gn * codes, cudaMemcpyHostToDevice, s));
+        DCU(cudaMemsetAsync(w.state, 0, sizeof(DecodeState) * gn, s));
+        if (avg_error) DCU(cudaMemcpyAsync(d_carry, avg_error + i0, sizeof(float) * gn, cudaMemcpyHostToDevice, s));
+        else DCU(cudaMemsetAsync(d_carry, 0, sizeof(float) * gn, s));
+        if (!small(w, g, w.q, dpos, w.img, argb_out ? w.argb : nullptr, max_iters, 0.0f, fwh, s, (uint32_t)gn, d_carry)) {
+            for (int i = i0; i < n; i++) redo[i] = 1;  // no cooperative launch on this device
+            break;
+        }
+        launches++;
+        DCU(cudaMemcpyAsync(h_stage, w.state, sizeof(DecodeState) * gn, cudaMemcpyDeviceToHost, s));
+        if (argb_out) DCU(cudaMemcpyAsync(argb_out + i0 * plane, w.argb, sizeof(int32_t) * plane * gn, cudaMemcpyDeviceToHost, s));
+        else DCU(cudaMemcpyAsync(planes_out + i0 * g.C * plane, w.img, g.C * plane * gn, cudaMemcpyDeviceToHost, s));
+        DCU(cudaStreamSynchronize(s));
+        for (int i = 0; i < gn; i++) {
+            const DecodeState &x = hs[i];
+            if (x.bad_index) {
+                *bad_image = i0 + i;
+                return DecodeStatus{FIC_E_STREAM};
+            }
+            if (x.bail) {
+                redo[i0 + i] = 1;  // avg_error[i0 + i] still holds its carry
+                continue;
+            }
+            if (avg_error) memcpy(avg_error + i0 + i, &x.avg_bits, sizeof(float));
+            if (iterations) iterations[i0 + i] = (int)x.iters;
+        }
+    }
+    for (int i = 0; i < n; i++) {
+        if (!redo[i]) continue;
+        DCU(cudaMemcpyAsync(w.q, qcodes + i * codes, sizeof(int32_t) * codes, cudaMemcpyHostToDevice, s));
+        fic_timings one = {};
+        const DecodeStatus st = decode_run(w, g, w.q, w.img, argb_out ? argb_out + i * plane : nullptr,
+                                           planes_out ? planes_out + i * g.C * plane : nullptr, max_iters,
+                                           avg_error ? avg_error + i : nullptr, iterations ? iterations + i : nullptr, h_scratch, ev0,
+                                           end, &one, s);
+        if (st.rc == FIC_E_STREAM) *bad_image = i;
+        if (st.rc) return st;
+        launches += one.launches;
+    }
+    DCU(cudaEventRecord(end, s));
+    DCU(cudaStreamSynchronize(s));
+    DCU(cudaGetLastError());
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, ev0, end) == cudaSuccess) tm->total_ms = ms;
+    tm->launches = launches;
     return DecodeStatus{};
 }
 

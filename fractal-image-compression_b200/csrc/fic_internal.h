@@ -32,7 +32,8 @@ int make_geom(int W, int H, int B, int wk, int mode, Geom *g, const char **why);
 // State block of a decode (device memory), shared by its kernels and read back by the host: the running sweep's exact
 // sum of squared pixel changes, a "code indexes outside the pool" flag, the ticket of the sweep's CTAs, the done flag
 // (converged, FC:414), the sweeps run, avgError's bits, and the grid barrier and bail word of the one-launch decoder.
-// 8-byte aligned for the u64 atomics.
+// 8-byte aligned for the u64 atomics.  The one-launch decoder of a batch keeps one block per image; the first block's
+// barrier is the launch's grid barrier and its ticket the launch's "some image is still sweeping" word.
 struct DecodeState {
     unsigned long long sq_sum, bad_index;
     uint32_t ticket, done, iters, avg_bits, barrier, bail;
@@ -74,10 +75,11 @@ int launch_range_stats(const uint8_t *d_src, int32_t *d_rsum, const Geom &g, cud
 int launch_sum_planes(const uint8_t *d_dec, uint16_t *d_dec3, const Geom &g, cudaStream_t s);  // RGB only
 int launch_search_direct(const Work &w, const Geom &g, int64_t j0, int64_t j1, cudaStream_t s);
 // Fused windowed encode (widthKernel <= 16, no isometries): decimation, stats, search, solve and quantisation in one
-// launch, straight from the caller's pixels (ARGB ints or 8-bit planes); no intermediate arrays.
+// launch, straight from the caller's pixels (ARGB ints or 8-bit planes); no intermediate arrays.  n_images > 1: that
+// many images back to back at d_src, every range of each (j0 = 0, j1 = NR), codes in [n][NR] tables.
 bool fused_encode_applicable(const Geom &g);
 int launch_encode_fused(const void *d_src, int src_is_argb, const Geom &g, int64_t j0, int64_t j1, float *d_info,
-                        int32_t *d_q, cudaStream_t s);
+                        int32_t *d_q, cudaStream_t s, int n_images = 1);
 int launch_solve(const Work &w, const Geom &g, int64_t j0, int64_t j1, float *d_info, int32_t *d_q,
                  cudaStream_t s);
 
@@ -133,5 +135,19 @@ DecodeStatus decode_float_sum(const Work &w, const int32_t *terms, int64_t count
                               cudaStream_t s);
 // Device workspace of the chunked replay of a sweep over `pixels` pixels (0: the one-warp replay needs none).
 size_t decode_replay_bytes(int64_t pixels);
+
+// Batch decode (fic_decode_batch): images per cooperative launch of the one-launch decoder for geometry g, 0 when g
+// decodes image by image (decode_run).  At most kDecodeBatchMax.
+constexpr int kDecodeBatchMax = 2048;
+int decode_batch_group(const Geom &g);
+// n images, codes [n][NR][S] at host `qcodes`, the decoded images to argb_out [n][H][W] or planes_out [n][C][H][W]; avg_error
+// (optional) [n]: in, each image's carry; out, each image's avgError; iterations (optional) [n].  group =
+// decode_batch_group(g).  Workspace: q, dcode, img, dec, dec2, argb (with argb_out) for `group` images (1 if 0),
+// state for group (DecodeState + float carry), and what decode_run needs for one image.  h_stage: pinned, >= group *
+// sizeof(DecodeState); h_scratch as decode_run's.  On FIC_E_STREAM *bad_image is the lowest image whose codes index
+// outside the pool.
+DecodeStatus decode_batch_run(const Work &w, const Geom &g, int n, int group, const int32_t *qcodes, int32_t *argb_out,
+                              uint8_t *planes_out, int max_iters, float *avg_error, int *iterations, void *h_stage,
+                              void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, int *bad_image, cudaStream_t s);
 
 }  // namespace fic

@@ -536,9 +536,13 @@ __device__ __forceinline__ void fused_px(const void *__restrict__ src, int64_t p
     }
 }
 
+// A batch of same-size images (fic_encode_batch) is one launch over n * NR CTAs: the flat CTA index jf = image * NR + j
+// picks the image, whose pixels start img_stride elements (ARGB ints or bytes of its C planes) after the previous
+// image's, and the codes go to row jf of the [n][NR] code tables.
 template <int B, int C, bool ARGB>
 __global__ void __launch_bounds__(kDirectThreads)
-k_encode_fused(const void *__restrict__ src, float *__restrict__ info, int32_t *__restrict__ q, Geom g, int64_t j0)
+k_encode_fused(const void *__restrict__ src, float *__restrict__ info, int32_t *__restrict__ q, Geom g, int64_t j0,
+               size_t img_stride)
 {
     constexpr int n = B * B, step = B / 4;
     extern __shared__ __align__(16) uint8_t s_tile[];  // C planes of TW x TW decimated pixels
@@ -547,7 +551,9 @@ k_encode_fused(const void *__restrict__ src, float *__restrict__ info, int32_t *
     __shared__ int s_sum[C][kDirectThreads / 32];
     __shared__ float s_err[kDirectThreads / 32];
     __shared__ int s_c[kDirectThreads / 32];
-    const int64_t j = j0 + blockIdx.x;
+    const int64_t jf = j0 + blockIdx.x;
+    const int64_t image = jf / g.NR, j = jf - image * g.NR;
+    src = ARGB ? (const void *)((const int32_t *)src + image * img_stride) : (const void *)((const uint8_t *)src + image * img_stride);
     const int xr = (int)(j % g.rpw), yr = (int)(j / g.rpw);
     const int64_t plane = (int64_t)g.W * g.H;
     int dy, dx;
@@ -657,7 +663,7 @@ k_encode_fused(const void *__restrict__ src, float *__restrict__ info, int32_t *
             }
         int dmean;
         const int varD = dom_var(ds, dsq, n, &dmean);
-        write_grey_code(info, q, j, c, grey_solve(dot - dmean * vR, varD, rm[0], dmean), false, 0);
+        write_grey_code(info, q, jf, c, grey_solve(dot - dmean * vR, varD, rm[0], dmean), false, 0);
     } else {
         int dm[3], dv[3], dmsum = 0;
 #pragma unroll
@@ -679,23 +685,24 @@ k_encode_fused(const void *__restrict__ src, float *__restrict__ info, int32_t *
                 const float gD = (float)((int)p[o] + (int)p[(C == 3 ? 1 : 0) * TW * TW + o] + (int)p[(C - 1) * TW * TW + o] - dmsum);
                 kov = rgb_kov_step(kov, s_gR[ry * B + rx], gD);
             }
-        write_rgb_code(info, q, j, c, rgb_solve(kov, dv, dm, rm));
+        write_rgb_code(info, q, jf, c, rgb_solve(kov, dv, dm, rm));
     }
 }
 
 bool fused_encode_applicable(const Geom &g) { return g.wk <= 16 && g.n_iso == 1; }
 
 template <int C, bool ARGB>
-static int launch_fused_t(const void *d_src, const Geom &g, int64_t j0, int64_t j1, float *d_info, int32_t *d_q, cudaStream_t s)
+static int launch_fused_t(const void *d_src, const Geom &g, int64_t j0, int64_t j1, size_t img_stride, float *d_info, int32_t *d_q,
+                          cudaStream_t s)
 {
     const int step = g.B / 4, TW = (g.wk - 1) * step + g.B;
     const size_t smem = (size_t)C * TW * TW;  // <= 3 * 76 * 76 = 17 KB
     int launches = 0;
     for (int64_t at = j0; at < j1;) {
         const unsigned chunk = (unsigned)(j1 - at < (1 << 30) ? j1 - at : (1 << 30));
-        if (g.B == 4) k_encode_fused<4, C, ARGB><<<chunk, kDirectThreads, smem, s>>>(d_src, d_info, d_q, g, at);
-        else if (g.B == 8) k_encode_fused<8, C, ARGB><<<chunk, kDirectThreads, smem, s>>>(d_src, d_info, d_q, g, at);
-        else k_encode_fused<16, C, ARGB><<<chunk, kDirectThreads, smem, s>>>(d_src, d_info, d_q, g, at);
+        if (g.B == 4) k_encode_fused<4, C, ARGB><<<chunk, kDirectThreads, smem, s>>>(d_src, d_info, d_q, g, at, img_stride);
+        else if (g.B == 8) k_encode_fused<8, C, ARGB><<<chunk, kDirectThreads, smem, s>>>(d_src, d_info, d_q, g, at, img_stride);
+        else k_encode_fused<16, C, ARGB><<<chunk, kDirectThreads, smem, s>>>(d_src, d_info, d_q, g, at, img_stride);
         at += chunk;
         launches++;
     }
@@ -703,11 +710,13 @@ static int launch_fused_t(const void *d_src, const Geom &g, int64_t j0, int64_t 
 }
 
 int launch_encode_fused(const void *d_src, int src_is_argb, const Geom &g, int64_t j0, int64_t j1, float *d_info, int32_t *d_q,
-                        cudaStream_t s)
+                        cudaStream_t s, int n_images)
 {
     if (j1 <= j0) return 0;
-    if (g.C == 1) return src_is_argb ? launch_fused_t<1, true>(d_src, g, j0, j1, d_info, d_q, s) : launch_fused_t<1, false>(d_src, g, j0, j1, d_info, d_q, s);
-    return src_is_argb ? launch_fused_t<3, true>(d_src, g, j0, j1, d_info, d_q, s) : launch_fused_t<3, false>(d_src, g, j0, j1, d_info, d_q, s);
+    const size_t plane = (size_t)g.W * g.H, stride = src_is_argb ? plane : g.C * plane;
+    if (n_images > 1) j1 = n_images * g.NR;  // a batch: every range of every image, the flat range [0, n NR)
+    if (g.C == 1) return src_is_argb ? launch_fused_t<1, true>(d_src, g, j0, j1, stride, d_info, d_q, s) : launch_fused_t<1, false>(d_src, g, j0, j1, stride, d_info, d_q, s);
+    return src_is_argb ? launch_fused_t<3, true>(d_src, g, j0, j1, stride, d_info, d_q, s) : launch_fused_t<3, false>(d_src, g, j0, j1, stride, d_info, d_q, s);
 }
 
 // ------------------------------------------------------------------------------------

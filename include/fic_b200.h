@@ -189,6 +189,38 @@ int fic_decode_planes_dev(fic_handle *h, int is_rgb, int W, int H, int B, int wk
                           const int32_t *d_qcodes, int max_iters, uint8_t *d_planes_out,
                           float *avg_error, int *iterations);
 
+/* ---- batches: n_images same-size images per call ------------------------------- */
+
+/* n_images images of W x H, back to back: argb [n][H][W]; codes [n][NR][S], S = 3 / 5 / 4 by mode
+ * (FIC_MODE_GREY / FIC_MODE_RGB / FIC_MODE_GREY_ISO).  Every image's codes, decoded pixels, avgError bits and
+ * iteration count equal what the single entries give for that image alone, bit for bit.
+ *
+ * Encode: where the single encode would run the fused one-launch kernel (widthKernel <= 16, no isometries, up to 16 K
+ * range blocks per image, FIC_ENGINE_AUTO or _FUSED) the whole batch is one launch per group of images.  Every other
+ * case (forced DIRECT or UMMA, widthKernel > 16, the isometry extension, larger images) runs the single-image engine
+ * once per image inside the call: the images still go up and their codes come down in one copy per group, but
+ * there is no launch saving.  planes (the _u8 form): [n][C][H][W], C = 3 for RGB, else 1 (the red channel).
+ *
+ * Decode: where the single decode would run its one-launch decoder (blockgroesse >= 8, W % 16 == 0, no isometries, up to
+ * 2^20 pixels) a group of images decodes in one cooperative launch; every other image decodes as fic_decode would.
+ * The reference's avgError is a never-reset static (FC:20), so a chain of single decodes carries each image's value
+ * into the next image; a batch cannot reproduce that chain without running the images one after another, so it takes
+ * one carry-in per image: avg_error[i] is read on entry and written on exit, exactly like the scalar of fic_decode,
+ * and NULL means 0 for every image.  iterations: [n] or NULL.  planes_out: [n][C][H][W].
+ *
+ * FIC_E_ARG for n_images < 1, NULL images or codes, or a batch whose byte count overflows, besides the single entries'
+ * rejections; FIC_E_STREAM when some image's codes index outside the domain pool (fic_last_error names the lowest
+ * such image).  fic_get_timings then reports the whole call: total_ms, launches, engine (encode) and search_evals
+ * (n * NR * widthKernel^2 * isometries). */
+int fic_encode_batch(fic_handle *h, int mode, const int32_t *argb, int n_images, int W, int H, int B, int wk,
+                     float *info, int32_t *qcodes);
+int fic_encode_batch_u8(fic_handle *h, int mode, const uint8_t *planes, int n_images, int W, int H, int B, int wk,
+                        float *info, int32_t *qcodes);
+int fic_decode_batch(fic_handle *h, int mode, int n_images, int W, int H, int B, int wk, const int32_t *qcodes,
+                     int max_iters, int32_t *argb_out, float *avg_error, int *iterations);
+int fic_decode_batch_u8(fic_handle *h, int mode, int n_images, int W, int H, int B, int wk, const int32_t *qcodes,
+                        int max_iters, uint8_t *planes_out, float *avg_error, int *iterations);
+
 /* getBestGeneratedCollage[RGB] (FC:269-347): one decode step from the source image
  * with the unquantised codes.  Like the reference it rewrites info[.][0] in place from
  * window-local to codebook index (FC:273). */
