@@ -326,59 +326,70 @@ static int encode_fused_on_device(fic_handle *h, const Geom &g, const void *d_pi
     return FIC_OK;
 }
 
-// Pool build + search + solve on device-resident planes.  Records events 1..4.
+// The MMA kind a tcgen05 search runs with, and whether it runs at all: the first kind::f16 search of a handle verifies,
+// once, that this device's f16 tensor path accumulates the integer covariances exactly; a device that does not runs
+// kind::i8 instead.  RGB has a kind::f16 tensor path only; without an exact f16 path it stays on the CUDA-core kernel
+// (*engine becomes FIC_ENGINE_DIRECT).  (The self-test allocates and synchronises on this stream: one-time cost of the
+// first such call; fic_get_option(FIC_OPT_F16_EXACT) runs it ahead of time.)
+static int umma_kind_of(fic_handle *h, const Geom &g, int *engine, int *kind)
+{
+    *kind = h->umma_kind;
+    if (*engine != FIC_ENGINE_UMMA) return FIC_OK;
+    const bool rgb = g.C == 3;
+    const bool wants_f16 = rgb || (g.B != 16 && (*kind == FIC_UMMA_KIND_F16 || (*kind == FIC_UMMA_KIND_AUTO && umma_default_kind(g) == FIC_UMMA_KIND_F16)));
+    if (wants_f16 && h->f16_state == 0) {
+        const char *why = nullptr;
+        int ok = umma_f16_selftest(h->num_sms, h->stream, &why);
+        if (ok < 0) return set_err(h, FIC_E_CUDA, "kind::f16 self-test failed to run: %s", why ? why : "?");
+        h->f16_state = ok ? 1 : -1;
+    }
+    if (wants_f16 && h->f16_state < 0) {
+        if (rgb) *engine = FIC_ENGINE_DIRECT;
+        else *kind = FIC_UMMA_KIND_I8;
+    }
+    return FIC_OK;
+}
+
+// Pool build + search + solve on device-resident planes.  Records events 1..4.  n_images > 1 (tcgen05 engine only):
+// a group of images, planes back to back at d_src, ranges [0, NR) of each, codes in [n][NR] tables -- one launch of
+// every kernel for the whole group (launch_search_umma).
 static int encode_on_device(fic_handle *h, const Geom &g, const uint8_t *d_src, int64_t j0, int64_t j1,
-                            float *d_info, int32_t *d_q, int engine)
+                            float *d_info, int32_t *d_q, int engine, int n_images = 1)
 {
     Work &w = h->w;
     cudaStream_t s = h->stream;
     if (engine == FIC_ENGINE_FUSED) return encode_fused_on_device(h, g, d_src, 0, j0, j1, d_info, d_q);
-    ENSURE(w.dec, S_DEC, (size_t)g.C * g.sw * g.sh);
-    ENSURE(w.dsum, S_DSUM, sizeof(int32_t) * g.C * g.ND);
-    ENSURE(w.dsq, S_DSQ, sizeof(int32_t) * g.C * g.ND);
-    ENSURE(w.rsum, S_RSUM, sizeof(int32_t) * g.C * g.NR);
-    ENSURE(w.best, S_BEST, sizeof(int32_t) * g.NR);
-    if (g.C == 3) ENSURE(w.dec3, S_DEC3, sizeof(uint16_t) * (size_t)g.sw * g.sh);  // R + G + B of the decimated planes
-    int kind = h->umma_kind;
+    const size_t n = (size_t)n_images;
+    ENSURE(w.dec, S_DEC, (size_t)g.C * g.sw * g.sh * n);
+    ENSURE(w.dsum, S_DSUM, sizeof(int32_t) * g.C * g.ND * n);
+    ENSURE(w.dsq, S_DSQ, sizeof(int32_t) * g.C * g.ND * n);
+    ENSURE(w.rsum, S_RSUM, sizeof(int32_t) * g.C * g.NR * n);
+    ENSURE(w.best, S_BEST, sizeof(int32_t) * g.NR * n);
+    if (g.C == 3) ENSURE(w.dec3, S_DEC3, sizeof(uint16_t) * (size_t)g.sw * g.sh * n);  // R + G + B of the decimated planes
+    int kind, rc;
     h->pair_used = 0;
+    if ((rc = umma_kind_of(h, g, &engine, &kind))) return rc;
+    if (n_images > 1 && engine != FIC_ENGINE_UMMA) return set_err(h, FIC_E_ARG, "a group of images runs the tcgen05 search only");
     if (engine == FIC_ENGINE_UMMA) {
-        // The first kind::f16 search of a handle verifies, once, that this device's f16 tensor path
-        // accumulates the integer covariances exactly; a device that does not runs kind::i8 instead.
-        // RGB has a kind::f16 tensor path only; without an exact f16 path it stays on the CUDA-core kernel.
-        // (The self-test allocates and synchronises on this stream: one-time cost of the first such call;
-        // fic_get_option(FIC_OPT_F16_EXACT) runs it ahead of time.)
-        const bool rgb = g.C == 3;
-        const bool wants_f16 = rgb || (g.B != 16 && (kind == FIC_UMMA_KIND_F16 || (kind == FIC_UMMA_KIND_AUTO && umma_default_kind(g) == FIC_UMMA_KIND_F16)));
-        if (wants_f16 && h->f16_state == 0) {
-            const char *why = nullptr;
-            int ok = umma_f16_selftest(h->num_sms, s, &why);
-            if (ok < 0) return set_err(h, FIC_E_CUDA, "kind::f16 self-test failed to run: %s", why ? why : "?");
-            h->f16_state = ok ? 1 : -1;
-        }
-        if (wants_f16 && h->f16_state < 0) {
-            if (rgb) engine = FIC_ENGINE_DIRECT;
-            else kind = FIC_UMMA_KIND_I8;
-        }
-    }
-    if (engine == FIC_ENGINE_UMMA) {
-        ENSURE(w.opA, S_OPA, umma_opA_bytes(g, j0, j1, h->num_sms, kind));
-        ENSURE(w.opB, S_OPB, umma_opB_bytes(g, kind));
+        ENSURE(w.opA, S_OPA, umma_opA_bytes(g, j0, j1, h->num_sms, kind, n_images));
+        ENSURE(w.opB, S_OPB, umma_opB_bytes(g, kind, n_images));
     }
     Work call = w;  // per-call view: the source planes may belong to the caller
     call.src = const_cast<uint8_t *>(d_src);
     int launches = 0;
     CU(cudaEventRecord(h->ev[1], s));
-    launches += launch_decimate(d_src, w.dec, g, s);
-    launches += launch_domain_stats(w.dec, w.dsum, w.dsq, g, s);
-    launches += launch_range_stats(d_src, w.rsum, g, s);
+    launches += launch_decimate(d_src, w.dec, g, s, n_images);
+    launches += launch_domain_stats(w.dec, w.dsum, w.dsq, g, s, n_images);
+    launches += launch_range_stats(d_src, w.rsum, g, s, n_images);
     CU(cudaEventRecord(h->ev[2], s));
     CU(cudaEventRecord(h->ev[6], s));  // (the tcgen05 launcher re-records 6 / 7 around its search kernel)
     CU(cudaEventRecord(h->ev[7], s));
     if (engine == FIC_ENGINE_UMMA) {
         const char *why = nullptr;
-        int n = launch_search_umma(call, g, j0, j1, h->num_sms, s, &why, kind, h->ev[6], h->ev[7], h->umma_pair, &h->pair_used);
-        if (n < 0) return set_err(h, FIC_E_CUDA, "tcgen05 search launch failed: %s", why ? why : "?");
-        launches += n;
+        int nl = launch_search_umma(call, g, j0, j1, h->num_sms, s, &why, kind, h->ev[6], h->ev[7], h->umma_pair, &h->pair_used,
+                                    nullptr, 0, nullptr, n_images);
+        if (nl < 0) return set_err(h, FIC_E_CUDA, "tcgen05 search launch failed: %s", why ? why : "?");
+        launches += nl;
     } else {
         if (g.C == 3) launches += launch_sum_planes(w.dec, w.dec3, g, s);
         CU(cudaEventRecord(h->ev[6], s));
@@ -386,12 +397,13 @@ static int encode_on_device(fic_handle *h, const Geom &g, const uint8_t *d_src, 
         CU(cudaEventRecord(h->ev[7], s));
     }
     CU(cudaEventRecord(h->ev[3], s));
-    launches += launch_solve(call, g, j0, j1, d_info, d_q, s);
+    if (n_images > 1) launches += launch_solve(call, g, 0, g.NR * n_images, d_info, d_q, s);  // the flat range of the group
+    else launches += launch_solve(call, g, j0, j1, d_info, d_q, s);
     CU(cudaEventRecord(h->ev[4], s));
     CU(cudaGetLastError());
     h->tm.engine = engine;
     h->tm.launches += launches;
-    h->tm.search_evals = (double)(j1 - j0) * (double)g.wk * (double)g.wk * (double)g.n_iso;
+    h->tm.search_evals = (double)(j1 - j0) * (double)g.wk * (double)g.wk * (double)g.n_iso * (double)n_images;
     return FIC_OK;
 }
 
@@ -480,6 +492,18 @@ static int encode_host(fic_handle *h, int is_rgb, const void *pixels, int src_u8
 
 // Input pixels one group of a batch uploads at most: the grow-only workspace does not grow with the batch.
 constexpr size_t kBatchGroupBytes = (size_t)64 << 20;
+// A group on the tcgen05 engine also holds at most 256 images (the image index is the top digit of the pool sort's
+// keys) and at most this much operand workspace (opA + opB: packed operands, flag lists, position tables and sort
+// scratch, about 2-6 MB per image of 256^2 - 512^2 at blockgroesse 8) -- or one image, however large.
+constexpr int kBatchUmmaImages = 256;
+constexpr size_t kBatchUmmaBytes = (size_t)1 << 30;
+// AUTO on a batch of full-pool images that a single call would give to the CUDA-core search picks the tcgen05 group
+// search for groups of at least this many images.  Measured on a B200 (tools/batch_bench.py,
+// profiles/r4_batch_fullpool.json): the tensor chain costs 160-190 us per call at 128^2-256^2 plus 5-10 us per image,
+// the direct search 70-130 us per image, so the group pays from about three images on (n = 8: 2.5-4x faster per image).
+// Where the single call runs the fused one-launch kernel (full pools of at most 16 x 16 domains, e.g. 64^2 at B = 8)
+// that kernel stays faster at every batch size (0.6 against 1.0 us per image at n = 256), so AUTO keeps it.
+constexpr int kBatchUmmaMinImages = 4;
 static_assert(kDecodeBatchMax * sizeof(DecodeState) <= kStageBytes, "a decode group's state blocks come back through h_stage");
 
 // The checks every batch entry adds to make_geom's: n_images >= 1 and byte counts of the whole batch that fit.
@@ -496,9 +520,31 @@ static int batch_geom(fic_handle *h, int mode, int n_images, int W, int H, int B
     return FIC_OK;
 }
 
+// Images per tcgen05 group of a batch (see kBatchUmmaImages / kBatchUmmaBytes), at most `limit`.
+static int umma_group_size(fic_handle *h, const Geom &g, int kind, int limit)
+{
+    int n = limit < kBatchUmmaImages ? limit : kBatchUmmaImages;
+    auto bytes = [&](int k) { return umma_opA_bytes(g, 0, g.NR, h->num_sms, kind, k) + umma_opB_bytes(g, kind, k); };
+    for (size_t b; n > 1 && (b = bytes(n)) > kBatchUmmaBytes;) n = (int)((double)n * kBatchUmmaBytes / b);
+    return n > 1 ? n : 1;
+}
+
+// Per-stage times of the last encode_on_device (events 1..4, 6, 7) added to the call's.
+static void add_stage_times(fic_handle *h, fic_timings *acc)
+{
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, h->ev[1], h->ev[2]) == cudaSuccess) acc->pool_ms += ms;
+    if (cudaEventElapsedTime(&ms, h->ev[2], h->ev[3]) == cudaSuccess) acc->search_ms += ms;
+    if (cudaEventElapsedTime(&ms, h->ev[6], h->ev[7]) == cudaSuccess) acc->kernel_ms += ms;
+    if (cudaEventElapsedTime(&ms, h->ev[3], h->ev[4]) == cudaSuccess) acc->solve_ms += ms;
+}
+
 // A batch encode: the codes of n_images images back to back, [n][NR][S], each equal to a single encode of that image.
-// Where pick_engine chooses the fused encode, one launch per group covers every range of every image; otherwise each
-// image runs encode_on_device.  Groups of images go up in one copy and their codes come down in one.
+// Where pick_engine chooses the fused encode, one launch per group covers every range of every image; on the tcgen05
+// engine (full-pool windows: forced, AUTO where the single call runs it, or AUTO instead of the CUDA-core search for
+// groups of kBatchUmmaMinImages and more) every group is one
+// block-diagonal search -- one launch of each pool, sort, pack, search, refine and solve kernel; otherwise each image
+// runs encode_on_device.  Groups of images go up in one copy and their codes come down in one.
 static int encode_batch_host(fic_handle *h, int mode, const void *pixels, int src_u8, int n_images, int W, int H, int B, int wk,
                              float *info, int32_t *qcodes)
 {
@@ -513,27 +559,49 @@ static int encode_batch_host(fic_handle *h, int mode, const void *pixels, int sr
     cudaStream_t s = h->stream;
     int engine;
     if ((rc = pick_engine(h, g, 0, g.NR, &engine))) return rc;
-    const bool fused = engine == FIC_ENGINE_FUSED;
     const int S = code_stride(g);
     const size_t plane = (size_t)W * H, image_bytes = src_u8 ? g.C * plane : sizeof(int32_t) * plane;
     const size_t codes = (size_t)g.NR * S, table = sizeof(float) * codes;  // one image's code table (float and int32 alike)
-    const int group = (int)(kBatchGroupBytes / image_bytes < (size_t)n_images ? (kBatchGroupBytes / image_bytes > 0 ? kBatchGroupBytes / image_bytes : 1) : n_images);
+    int group = (int)(kBatchGroupBytes / image_bytes < (size_t)n_images ? (kBatchGroupBytes / image_bytes > 0 ? kBatchGroupBytes / image_bytes : 1) : n_images);
+    // AUTO: the tcgen05 group search instead of the CUDA-core search for groups of enough images, else the single
+    // call's engine
+    int want = h->engine_opt == FIC_ENGINE_AUTO && engine == FIC_ENGINE_DIRECT && umma_applicable(g) ? FIC_ENGINE_UMMA : engine, kind = 0;
+    if ((rc = umma_kind_of(h, g, &want, &kind))) return rc;
+    if (want == FIC_ENGINE_UMMA) {
+        const int ug = umma_group_size(h, g, kind, group);
+        if (engine == FIC_ENGINE_UMMA || ug >= kBatchUmmaMinImages) {
+            engine = FIC_ENGINE_UMMA;
+            group = ug;
+        }
+    } else if (engine == FIC_ENGINE_UMMA) {
+        engine = want;  // RGB on a device without an exact kind::f16 path: the CUDA-core search, image by image
+    }
+    const bool fused = engine == FIC_ENGINE_FUSED, grouped = engine == FIC_ENGINE_UMMA;
     if (src_u8) {
         ENSURE(w.src, S_SRC, image_bytes * group);
     } else {
         ENSURE(w.argb, S_ARGB, image_bytes * group);
-        if (!fused) ENSURE(w.src, S_SRC, g.C * plane);  // one image's planes, unpacked before its encode
+        if (!fused) ENSURE(w.src, S_SRC, g.C * plane * (grouped ? group : 1));  // planes unpacked before the encode
     }
     ENSURE(w.info, S_INFO, table * group);
     ENSURE(w.q, S_Q, table * group);
     DrainOnExit drain(s);
+    fic_timings stages;  // the tcgen05 engine: per-stage times summed over the groups
+    memset(&stages, 0, sizeof stages);
     CU(cudaEventRecord(h->ev[0], s));
     for (int i0 = 0; i0 < n_images; i0 += group) {
         const int gn = n_images - i0 < group ? n_images - i0 : group;
         void *d_pixels = src_u8 ? (void *)w.src : (void *)w.argb;
+        if (grouped && i0 > 0) {  // the previous group's stage events, before this group records them again
+            CU(cudaStreamSynchronize(s));
+            add_stage_times(h, &stages);
+        }
         CU(cudaMemcpyAsync(d_pixels, (const uint8_t *)pixels + i0 * image_bytes, image_bytes * gn, cudaMemcpyHostToDevice, s));
         if (fused) {
             if ((rc = encode_fused_on_device(h, g, d_pixels, !src_u8, 0, g.NR, w.info, w.q, gn))) return rc;
+        } else if (grouped) {
+            if (!src_u8) h->tm.launches += launch_unpack(w.argb, w.src, W, H, g.C, s, gn);
+            if ((rc = encode_on_device(h, g, w.src, 0, g.NR, w.info, w.q, engine, gn))) return rc;
         } else {
             for (int i = 0; i < gn; i++) {
                 const uint8_t *d_src = w.src + i * g.C * plane;
@@ -550,8 +618,15 @@ static int encode_batch_host(fic_handle *h, int mode, const void *pixels, int sr
     CU(cudaEventRecord(h->ev[5], s));
     CU(cudaStreamSynchronize(s));
     CU(cudaGetLastError());
+    if (grouped) add_stage_times(h, &stages);
     const int launches = h->tm.launches, used = h->tm.engine;
-    memset(&h->tm, 0, sizeof h->tm);  // the per-stage events saw the last image only: report the whole call
+    memset(&h->tm, 0, sizeof h->tm);  // the per-stage events saw the last image or group only: report the whole call
+    if (grouped) {
+        h->tm.pool_ms = stages.pool_ms;
+        h->tm.search_ms = stages.search_ms;
+        h->tm.kernel_ms = stages.kernel_ms;
+        h->tm.solve_ms = stages.solve_ms;
+    }
     float ms = 0;
     if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[5]) == cudaSuccess) h->tm.total_ms = ms;
     h->tm.engine = used;

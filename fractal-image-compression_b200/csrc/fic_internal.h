@@ -67,12 +67,14 @@ struct Work {
 };
 
 // ---- kernel launchers (each returns the number of kernels it launched) -----------
-int launch_unpack(const int32_t *d_argb, uint8_t *d_planes, int W, int H, int C, cudaStream_t s);
-int launch_decimate(const uint8_t *d_src, uint8_t *d_dec, const Geom &g, cudaStream_t s);
+// The pool builders take n_images same-size images back to back, one launch for all: ARGB [n][H][W] -> planes
+// [n][C][H][W] -> decimated planes [n][C][sh][sw], dsum / dsq [n][C][ND], rsum [n][C][NR], dec3 [n][sh][sw].
+int launch_unpack(const int32_t *d_argb, uint8_t *d_planes, int W, int H, int C, cudaStream_t s, int n_images = 1);
+int launch_decimate(const uint8_t *d_src, uint8_t *d_dec, const Geom &g, cudaStream_t s, int n_images = 1);
 int launch_domain_stats(const uint8_t *d_dec, int32_t *d_dsum, int32_t *d_dsq, const Geom &g,
-                        cudaStream_t s);
-int launch_range_stats(const uint8_t *d_src, int32_t *d_rsum, const Geom &g, cudaStream_t s);
-int launch_sum_planes(const uint8_t *d_dec, uint16_t *d_dec3, const Geom &g, cudaStream_t s);  // RGB only
+                        cudaStream_t s, int n_images = 1);
+int launch_range_stats(const uint8_t *d_src, int32_t *d_rsum, const Geom &g, cudaStream_t s, int n_images = 1);
+int launch_sum_planes(const uint8_t *d_dec, uint16_t *d_dec3, const Geom &g, cudaStream_t s, int n_images = 1);  // RGB only
 int launch_search_direct(const Work &w, const Geom &g, int64_t j0, int64_t j1, cudaStream_t s);
 // Fused windowed encode (widthKernel <= 16, no isometries): decimation, stats, search, solve and quantisation in one
 // launch, straight from the caller's pixels (ARGB ints or 8-bit planes); no intermediate arrays.  n_images > 1: that
@@ -80,6 +82,8 @@ int launch_search_direct(const Work &w, const Geom &g, int64_t j0, int64_t j1, c
 bool fused_encode_applicable(const Geom &g);
 int launch_encode_fused(const void *d_src, int src_is_argb, const Geom &g, int64_t j0, int64_t j1, float *d_info,
                         int32_t *d_q, cudaStream_t s, int n_images = 1);
+// Solve of ranges [j0, j1); a group of images (after the pool builders and launch_search_umma with n_images) passes
+// the flat range [0, n * NR): best, info and q are [n][NR] tables.
 int launch_solve(const Work &w, const Geom &g, int64_t j0, int64_t j1, float *d_info, int32_t *d_q,
                  cudaStream_t s);
 
@@ -95,19 +99,22 @@ bool umma_applicable(const Geom &g);
 int umma_debug_sort(uint32_t *d_keys, int32_t *d_vals, uint32_t *d_keys_out, int32_t *d_vals_out, int64_t n, cudaStream_t s);
 // `kind`: FIC_UMMA_KIND_AUTO / _I8 / _F16 (B = 16 always runs kind::i8); umma_default_kind = what AUTO picks
 int umma_default_kind(const Geom &g);
-size_t umma_opA_bytes(const Geom &g, int64_t j0, int64_t j1, int num_sms, int kind);
-size_t umma_opB_bytes(const Geom &g, int kind);
+size_t umma_opA_bytes(const Geom &g, int64_t j0, int64_t j1, int num_sms, int kind, int n_images = 1);
+size_t umma_opB_bytes(const Geom &g, int kind, int n_images = 1);
 // device table: sweep position -> domain index (-1: padding), valid after a launch; probe only
 void umma_debug_positions(const Work &w, const Geom &g, int64_t rows, int num_sms, int kind,
                           const int32_t **d_pos_dom, int64_t *npos);
 // k0 / k1 (optional): events recorded around the search kernel.  pair: FIC_UMMA_PAIR_AUTO / _ON / _OFF; *pair_used
 // (optional) = 1 if the CTA-pair kernel ran.  dump (optional, probe / self-test): every accumulator (kov) of every
 // (operand row, sweep position) pair, row stride dump_ld; status_dev (optional, mapped host memory): the code of a
-// pipeline wait that timed out.
+// pipeline wait that timed out.  n_images (1 to 256): a group of same-size images searched as one block-diagonal
+// problem -- ranges [j0, j1) of every image, each against its own pool, in one pool sort, one pack of either operand,
+// one search kernel and one refine; workspace (w.src, w.dec, w.dsum, w.dsq, w.rsum, w.dec3) holds the group back to
+// back as the pool builders write it, w.best is [n][NR], opA / opB are sized with the same n_images.
 int launch_search_umma(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms,
                        cudaStream_t s, const char **err, int kind, cudaEvent_t k0 = nullptr,
                        cudaEvent_t k1 = nullptr, int pair = FIC_UMMA_PAIR_AUTO, int *pair_used = nullptr,
-                       int32_t *dump = nullptr, int64_t dump_ld = 0, int *status_dev = nullptr);
+                       int32_t *dump = nullptr, int64_t dump_ld = 0, int *status_dev = nullptr, int n_images = 1);
 
 // ---- decoder (fic_decode.cu) -----------------------------------------------------------------------------------------
 // Outcome of a decoder entry.  rc: FIC_OK; FIC_E_STREAM when a code indexes outside the domain pool (the reference

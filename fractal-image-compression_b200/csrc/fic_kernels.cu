@@ -15,6 +15,8 @@ namespace fic {
 // K1a: ARGB int32 -> 8-bit planes.  Grey keeps the red channel only (FC:596, FC:977).
 // 16-byte loads, 4-byte stores per plane.
 // ------------------------------------------------------------------------------------
+// Several images: quads runs over all of them; image i's planes start 3 * plane_quads quads after image i - 1's (grey:
+// the one plane of each image directly follows the previous one, so the flat index needs no image).
 template <int C>
 __global__ void k_unpack(const int4 *__restrict__ argb, uchar4 *__restrict__ planes, int64_t quads,
                          int64_t plane_quads)
@@ -23,24 +25,27 @@ __global__ void k_unpack(const int4 *__restrict__ argb, uchar4 *__restrict__ pla
     int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (; i < quads; i += stride) {
         int4 p = __ldg(argb + i);
-        planes[i] = make_uchar4((p.x >> 16) & 0xff, (p.y >> 16) & 0xff, (p.z >> 16) & 0xff, (p.w >> 16) & 0xff);
-        if (C == 3) {
-            planes[plane_quads + i] =
+        if (C == 1) {
+            planes[i] = make_uchar4((p.x >> 16) & 0xff, (p.y >> 16) & 0xff, (p.z >> 16) & 0xff, (p.w >> 16) & 0xff);
+        } else {
+            const int64_t image = i >= plane_quads ? i / plane_quads : 0, o = i + 2 * image * plane_quads;  // quad of image's R plane
+            planes[o] = make_uchar4((p.x >> 16) & 0xff, (p.y >> 16) & 0xff, (p.z >> 16) & 0xff, (p.w >> 16) & 0xff);
+            planes[plane_quads + o] =
                 make_uchar4((p.x >> 8) & 0xff, (p.y >> 8) & 0xff, (p.z >> 8) & 0xff, (p.w >> 8) & 0xff);
-            planes[2 * plane_quads + i] = make_uchar4(p.x & 0xff, p.y & 0xff, p.z & 0xff, p.w & 0xff);
+            planes[2 * plane_quads + o] = make_uchar4(p.x & 0xff, p.y & 0xff, p.z & 0xff, p.w & 0xff);
         }
     }
 }
 
-int launch_unpack(const int32_t *d_argb, uint8_t *d_planes, int W, int H, int C, cudaStream_t s)
+int launch_unpack(const int32_t *d_argb, uint8_t *d_planes, int W, int H, int C, cudaStream_t s, int n_images)
 {
-    int64_t quads = (int64_t)W * H / 4;  // W % 4 == 0 is guaranteed by make_geom
+    int64_t quads = (int64_t)W * H / 4 * n_images;  // W % 4 == 0 is guaranteed by make_geom
     int blocks = (int)((quads + 255) / 256 < 148 * 16 ? (quads + 255) / 256 : 148 * 16);
     if (blocks < 1) blocks = 1;
     if (C == 1)
         k_unpack<1><<<blocks, 256, 0, s>>>((const int4 *)d_argb, (uchar4 *)d_planes, quads, quads);
     else
-        k_unpack<3><<<blocks, 256, 0, s>>>((const int4 *)d_argb, (uchar4 *)d_planes, quads, quads);
+        k_unpack<3><<<blocks, 256, 0, s>>>((const int4 *)d_argb, (uchar4 *)d_planes, quads, quads / n_images);
     return 1;
 }
 
@@ -50,16 +55,16 @@ int launch_unpack(const int32_t *d_argb, uint8_t *d_planes, int W, int H, int C,
 //   (x, y+1)).  With W, H even the only live border branch is the reference's
 //   `x + 1 >= image.height` test (FC:993, FC:940), which substitutes 128 for the fourth
 //   tap on landscape images; it is reproduced here.
-// One thread makes 2 output pixels from two 4-byte loads; stores are 2 bytes.
+// One thread makes 2 output pixels from two 4-byte loads; stores are 2 bytes.  `planes` = C * images: the planes of a
+// group of images follow each other in source and output alike.
 // ------------------------------------------------------------------------------------
-__global__ void k_decimate(const uint8_t *__restrict__ src, uint8_t *__restrict__ dec, int W, int H, int C)
+__global__ void k_decimate(const uint8_t *__restrict__ src, uint8_t *__restrict__ dec, int W, int H, int planes, bool rgb)
 {
     int sw = W / 2, sh = H / 2;
     int64_t pairs_per_plane = (int64_t)(sw / 2) * sh;
-    int64_t total = pairs_per_plane * C;
+    int64_t total = pairs_per_plane * planes;
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    bool rgb = C == 3;
     for (; i < total; i += stride) {
         int c = (int)(i / pairs_per_plane);
         int64_t k = i - c * pairs_per_plane;
@@ -76,13 +81,12 @@ __global__ void k_decimate(const uint8_t *__restrict__ src, uint8_t *__restrict_
 }
 
 // Vector path (W % 16 == 0): one thread makes 8 output pixels from two 16-byte loads, one 8-byte store.
-__global__ void k_decimate_v8(const uint8_t *__restrict__ src, uint8_t *__restrict__ dec, int W, int H, int C)
+__global__ void k_decimate_v8(const uint8_t *__restrict__ src, uint8_t *__restrict__ dec, int W, int H, int planes, bool rgb)
 {
     const int sw = W / 2, sh = H / 2;
     const int64_t oct_per_plane = (int64_t)(sw / 8) * sh;
-    const int64_t total = oct_per_plane * C;
+    const int64_t total = oct_per_plane * planes;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    const bool rgb = C == 3;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
         const int c = (int)(i / oct_per_plane);
         const int64_t k = i - c * oct_per_plane;
@@ -103,19 +107,20 @@ __global__ void k_decimate_v8(const uint8_t *__restrict__ src, uint8_t *__restri
     }
 }
 
-int launch_decimate(const uint8_t *d_src, uint8_t *d_dec, const Geom &g, cudaStream_t s)
+int launch_decimate(const uint8_t *d_src, uint8_t *d_dec, const Geom &g, cudaStream_t s, int n_images)
 {
+    const int planes = g.C * n_images;
     if (g.W % 16 == 0) {
-        int64_t total = (int64_t)(g.sw / 8) * g.sh * g.C;
+        int64_t total = (int64_t)(g.sw / 8) * g.sh * planes;
         int blocks = (int)((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
         if (blocks < 1) blocks = 1;
-        k_decimate_v8<<<blocks, 256, 0, s>>>(d_src, d_dec, g.W, g.H, g.C);
+        k_decimate_v8<<<blocks, 256, 0, s>>>(d_src, d_dec, g.W, g.H, planes, g.C == 3);
         return 1;
     }
-    int64_t total = (int64_t)(g.sw / 2) * g.sh * g.C;
+    int64_t total = (int64_t)(g.sw / 2) * g.sh * planes;
     int blocks = (int)((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
     if (blocks < 1) blocks = 1;
-    k_decimate<<<blocks, 256, 0, s>>>(d_src, d_dec, g.W, g.H, g.C);
+    k_decimate<<<blocks, 256, 0, s>>>(d_src, d_dec, g.W, g.H, planes, g.C == 3);
     return 1;
 }
 
@@ -125,9 +130,9 @@ int launch_decimate(const uint8_t *d_src, uint8_t *d_dec, const Geom &g, cudaStr
 // exact in s32; mean and variance follow from them (dom_var()).
 // ------------------------------------------------------------------------------------
 __global__ void k_domain_stats(const uint8_t *__restrict__ dec, int32_t *__restrict__ dsum,
-                               int32_t *__restrict__ dsq, Geom g)
+                               int32_t *__restrict__ dsq, Geom g, int planes)  // planes = C * images
 {
-    int64_t total = g.ND * g.C;
+    int64_t total = g.ND * planes;
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
     int c = (int)(i / g.ND);
@@ -147,17 +152,17 @@ __global__ void k_domain_stats(const uint8_t *__restrict__ dec, int32_t *__restr
     dsq[i] = s2;
 }
 
-int launch_domain_stats(const uint8_t *d_dec, int32_t *d_dsum, int32_t *d_dsq, const Geom &g, cudaStream_t s)
+int launch_domain_stats(const uint8_t *d_dec, int32_t *d_dsum, int32_t *d_dsq, const Geom &g, cudaStream_t s, int n_images)
 {
-    int64_t total = g.ND * g.C;
-    k_domain_stats<<<(unsigned)((total + 127) / 128), 128, 0, s>>>(d_dec, d_dsum, d_dsq, g);
+    int64_t total = g.ND * g.C * n_images;
+    k_domain_stats<<<(unsigned)((total + 127) / 128), 128, 0, s>>>(d_dec, d_dsum, d_dsq, g, g.C * n_images);
     return 1;
 }
 
 // K1d: per-range pixel sums (FC:67-73 getMittelwert of FC:588-602 getRangeblock).
-__global__ void k_range_stats(const uint8_t *__restrict__ src, int32_t *__restrict__ rsum, Geom g)
+__global__ void k_range_stats(const uint8_t *__restrict__ src, int32_t *__restrict__ rsum, Geom g, int planes)  // C * images
 {
-    int64_t total = g.NR * g.C;
+    int64_t total = g.NR * planes;
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
     int c = (int)(i / g.NR);
@@ -175,10 +180,10 @@ __global__ void k_range_stats(const uint8_t *__restrict__ src, int32_t *__restri
     rsum[i] = s1;
 }
 
-int launch_range_stats(const uint8_t *d_src, int32_t *d_rsum, const Geom &g, cudaStream_t s)
+int launch_range_stats(const uint8_t *d_src, int32_t *d_rsum, const Geom &g, cudaStream_t s, int n_images)
 {
-    int64_t total = g.NR * g.C;
-    k_range_stats<<<(unsigned)((total + 127) / 128), 128, 0, s>>>(d_src, d_rsum, g);
+    int64_t total = g.NR * g.C * n_images;
+    k_range_stats<<<(unsigned)((total + 127) / 128), 128, 0, s>>>(d_src, d_rsum, g, g.C * n_images);
     return 1;
 }
 
@@ -404,17 +409,20 @@ k_search_direct_grey_iso(const uint8_t *__restrict__ src, const uint8_t *__restr
     if (threadIdx.x == 0) best[j] = best_c;
 }
 
-// RGB: dec3 = R + G + B of the decimated planes (what k_search_direct_rgb reads instead of three planes).
-__global__ void k_sum_planes(const uint8_t *__restrict__ dec, uint16_t *__restrict__ dec3, int64_t count)
+// RGB: dec3 = R + G + B of the decimated planes (what k_search_direct_rgb reads instead of three planes); `total`
+// pixels of images of `count` pixels each.
+__global__ void k_sum_planes(const uint8_t *__restrict__ dec, uint16_t *__restrict__ dec3, int64_t count, int64_t total)
 {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < count) dec3[i] = (uint16_t)((int)dec[i] + (int)dec[count + i] + (int)dec[2 * count + i]);
+    if (i >= total) return;
+    const uint8_t *d = dec + 2 * (i >= count ? i / count : 0) * count + i;  // pixel i % count of its image's R plane
+    dec3[i] = (uint16_t)((int)d[0] + (int)d[count] + (int)d[2 * count]);
 }
 
-int launch_sum_planes(const uint8_t *d_dec, uint16_t *d_dec3, const Geom &g, cudaStream_t s)
+int launch_sum_planes(const uint8_t *d_dec, uint16_t *d_dec3, const Geom &g, cudaStream_t s, int n_images)
 {
-    const int64_t count = (int64_t)g.sw * g.sh;
-    k_sum_planes<<<(unsigned)((count + 255) / 256), 256, 0, s>>>(d_dec, d_dec3, count);
+    const int64_t count = (int64_t)g.sw * g.sh, total = count * n_images;
+    k_sum_planes<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(d_dec, d_dec3, count, total);
     return 1;
 }
 
@@ -720,15 +728,26 @@ int launch_encode_fused(const void *d_src, int src_is_argb, const Geom &g, int64
 }
 
 // ------------------------------------------------------------------------------------
-// K3s: code solve + quantisation for the winning candidate.  One thread per range block.
+// K3s: code solve + quantisation for the winning candidate.  One thread per range block.  A group of images passes
+// the flat range [0, n NR): flat row jf = image * NR + j reads that image's planes and stats (as the pool builders lay
+// them out) and writes row jf of best / info / q.
 // ------------------------------------------------------------------------------------
 __global__ void k_solve_grey(const uint8_t *__restrict__ src, const uint8_t *__restrict__ dec,
                              const int32_t *__restrict__ dsum, const int32_t *__restrict__ dsq,
                              const int32_t *__restrict__ rsum, const int32_t *__restrict__ best,
                              float *__restrict__ info, int32_t *__restrict__ q, Geom g, int64_t j0, int64_t j1)
 {
-    int64_t j = j0 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= j1) return;
+    const int64_t jf = j0 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (jf >= j1) return;
+    const int64_t image = jf >= g.NR ? jf / g.NR : 0, j = jf - image * g.NR;  // (a single image divides nothing)
+    src += image * g.W * g.H;
+    dec += image * g.sw * g.sh;
+    dsum += image * g.ND;
+    dsq += image * g.ND;
+    rsum += image * g.NR;
+    best += image * g.NR;
+    info = info ? info + image * g.NR * code_stride(g) : info;
+    q = q ? q + image * g.NR * code_stride(g) : q;
     int xr = (int)(j % g.rpw), yr = (int)(j / g.rpw);
     const bool iso = g.n_iso > 1;  // extension: best = c * 8 + isometry
     int c = iso ? best[j] >> 3 : best[j];
@@ -759,8 +778,17 @@ __global__ void k_solve_rgb(const uint8_t *__restrict__ src, const uint8_t *__re
                             const int32_t *__restrict__ rsum, const int32_t *__restrict__ best,
                             float *__restrict__ info, int32_t *__restrict__ q, Geom g, int64_t j0, int64_t j1)
 {
-    int64_t j = j0 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= j1) return;
+    const int64_t jf = j0 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;  // see k_solve_grey
+    if (jf >= j1) return;
+    const int64_t image = jf >= g.NR ? jf / g.NR : 0, j = jf - image * g.NR;
+    src += image * 3 * g.W * g.H;
+    dec += image * 3 * g.sw * g.sh;
+    dsum += image * 3 * g.ND;
+    dsq += image * 3 * g.ND;
+    rsum += image * 3 * g.NR;
+    best += image * g.NR;
+    info = info ? info + image * g.NR * 5 : info;
+    q = q ? q + image * g.NR * 5 : q;
     int xr = (int)(j % g.rpw), yr = (int)(j / g.rpw);
     int c = best[j];
     int dy, dx;

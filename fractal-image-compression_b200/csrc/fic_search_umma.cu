@@ -286,14 +286,16 @@ __host__ __device__ __forceinline__ int64_t sweep_to_sorted(int64_t pos, uint32_
     return (int64_t)(((chunk * (uint64_t)mult) % (uint64_t)nch) * 32 + ((uint64_t)pos & 31));
 }
 
-// Sort keys: varD of every domain (DB:106-115), payload: the domain index.
+// Sort keys: varD of every domain (DB:106-115), payload: the domain index.  A group of n_img images ([n_img][ND]
+// stats) keys domain j of image i as i << 24 | varD and carries the group-global index i * ND + j: a stable sort on
+// four digits leaves every image's domains contiguous and in the order a single image's three-digit sort gives them.
 __global__ void k_umma_sortkeys(const int32_t *__restrict__ dsum, const int32_t *__restrict__ dsq, int n,
-                                int64_t ND, uint32_t *__restrict__ keys, int32_t *__restrict__ vals)
+                                int64_t ND, int64_t count, uint32_t *__restrict__ keys, int32_t *__restrict__ vals)
 {
     int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= ND) return;
+    if (j >= count) return;
     int dmean;
-    keys[j] = (uint32_t)dom_var(dsum[j], dsq[j], n, &dmean);
+    keys[j] = (uint32_t)(j >= ND ? j / ND : 0) << 24 | (uint32_t)dom_var(dsum[j], dsq[j], n, &dmean);
     vals[j] = (int32_t)j;
 }
 
@@ -402,25 +404,27 @@ __global__ void __launch_bounds__(256) k_sort_scatter(const uint32_t *__restrict
     }
 }
 
-// Sorts n pairs (keys0, vals0) by the low 24 bits of the key; the result is in (keys1, vals1).  `hist` holds
-// 256 * (ceil(n / kSortSub) + 1) counters (the table and the 256 row totals).  Returns the number of launches.
+// Sorts n pairs (keys0, vals0) by the low 8 * passes bits of the key; the result is in (keys1, vals1) for an odd
+// number of passes, in (keys0, vals0) for an even one.  `hist` holds 256 * (ceil(n / kSortSub) + 1) counters (the
+// table and the 256 row totals).  Returns the number of launches.
 inline size_t sort_hist_bytes(int64_t n) { return (size_t)256 * (size_t)((n + kSortSub - 1) / kSortSub + 1) * 4; }
 
-inline int launch_sort_pairs(uint32_t *keys0, int32_t *vals0, uint32_t *keys1, int32_t *vals1, uint32_t *hist, int64_t n, cudaStream_t s)
+inline int launch_sort_pairs(uint32_t *keys0, int32_t *vals0, uint32_t *keys1, int32_t *vals1, uint32_t *hist, int64_t n,
+                             int passes, cudaStream_t s)
 {
     const int64_t nwarps = (n + kSortSub - 1) / kSortSub;
     const unsigned blocks = (unsigned)((nwarps + 7) / 8);
     uint32_t *totals = hist + 256 * nwarps;
     uint32_t *kin = keys0, *kout = keys1;
     int32_t *vin = vals0, *vout = vals1;
-    for (int pass = 0; pass < 3; pass++) {
+    for (int pass = 0; pass < passes; pass++) {
         k_sort_hist<<<blocks, 256, 0, s>>>(kin, n, 8 * pass, nwarps, hist);
         k_sort_scan_rows<<<256, 256, 0, s>>>(hist, nwarps, totals);
         k_sort_scatter<<<blocks, 256, 0, s>>>(kin, vin, kout, vout, n, 8 * pass, nwarps, hist, totals);
         uint32_t *tk = kin; kin = kout; kout = tk;
         int32_t *tv = vin; vin = vout; vout = tv;
     }
-    return 9;  // three passes: the sorted pairs ended up in (keys1, vals1)
+    return 3 * passes;
 }
 
 // ---------------------------------------------------------------- operand packing ----
@@ -428,6 +432,14 @@ inline int launch_sort_pairs(uint32_t *keys0, int32_t *vals0, uint32_t *keys1, i
 __device__ __forceinline__ uint32_t pack4(int a, int b, int c, int d)
 {
     return (uint32_t)(a & 0xff) | ((uint32_t)(b & 0xff) << 8) | ((uint32_t)(c & 0xff) << 16) | ((uint32_t)(d & 0xff) << 24);
+}
+
+// A group of images keeps one OpBLayout region per image, `stride` bytes apart: a pointer into image 0's region, moved
+// to image i's.
+template <class T>
+__host__ __device__ __forceinline__ T *image_region(T *p, int64_t image, size_t stride)
+{
+    return (T *)((uint8_t *)const_cast<void *>((const void *)p) + (size_t)image * stride);
 }
 
 // Raw domain pixels for the refine step: per 32-position chunk, 16-byte piece c of position p sits at
@@ -448,18 +460,30 @@ __device__ __forceinline__ uint32_t pack_h2(int lo, int hi)
 // One thread per sweep position (a warp = one 32-position chunk): centre the domain by its
 // integer mean, write the tile-blob row (kind::i8: two s8 digits + the -alpha columns; kind::f16:
 // binary16), the position tables and the raw pixels used by the refine step, and the chunk's scale
-// bounds.
+// bounds.  A group of images: the grid covers npos positions per image (a block = one tile, inside one image); image i
+// reads its planes / stats / slice of the group's sort and writes its own OpBLayout region, opb_stride bytes on.
 template <int B, bool F16>
 __global__ void __launch_bounds__(128)
 k_umma_pack_domains(const uint8_t *__restrict__ dec, const int32_t *__restrict__ dsum,
                     const int32_t *__restrict__ dsq, const int32_t *__restrict__ perm, uint8_t *__restrict__ opB,
                     int32_t *__restrict__ pos_dom, int4 *__restrict__ pos_info,
                     uint8_t *__restrict__ pos_raw, int64_t *__restrict__ dom0_pos,
-                    Geom g, int64_t ntiles, uint32_t mult)
+                    Geom g, int64_t ntiles, uint32_t mult, int64_t npos, size_t opb_stride)
 {
     using L = Lay<B, F16>;
     constexpr int n = Cfg<B, F16>::n;
-    const int64_t pos = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t p0 = (int64_t)blockIdx.x * blockDim.x;  // (a single image divides nothing)
+    const int64_t image = p0 >= npos ? p0 / npos : 0;
+    const int64_t pos = p0 + threadIdx.x - image * npos;
+    dec += image * g.sw * g.sh;
+    dsum += image * g.ND;
+    dsq += image * g.ND;
+    perm += image * g.ND;
+    opB = image_region(opB, image, opb_stride);
+    pos_dom = image_region(pos_dom, image, opb_stride);
+    pos_info = image_region(pos_info, image, opb_stride);
+    pos_raw = image_region(pos_raw, image, opb_stride);
+    dom0_pos = image_region(dom0_pos, image, opb_stride);
     const int64_t tile = pos / kTileN;
     const int row = (int)(pos % kTileN);
     const int64_t sp = sweep_to_sorted(pos, mult, ntiles * kChunksPerTile);
@@ -480,7 +504,7 @@ k_umma_pack_domains(const uint8_t *__restrict__ dec, const int32_t *__restrict__
         pos_dom[pos] = -1;
         pos_info[pos] = make_int4(-1, 0, 0, 0);
     } else {
-        const int64_t j = perm[sp];
+        const int64_t j = perm[sp] - image * g.ND;  // the sort carries group-global indices
         const int gx = (int)(j % g.dpw), gy = (int)(j / g.dpw);
         const uint8_t *p = dec + (int64_t)(gy * g.step) * g.sw + gx * g.step;
         int dmean;
@@ -586,23 +610,27 @@ k_umma_pack_domains(const uint8_t *__restrict__ dec, const int32_t *__restrict__
 // columns; kind::f16: pixels centred by the integer mean, as binary16.  With the isometry extension
 // (g.n_iso = 8) a range block owns 8 adjacent rows: row v = (j - j0) * 8 + k holds the block permuted so that
 // its dot product with an unpermuted domain block is kov(r, T_k d) -- column p carries the range pixel that
-// T_k maps onto domain pixel p.  Means and sums do not depend on k.
+// T_k maps onto domain pixel p.  Means and sums do not depend on k.  A group of images: image i owns the rows_padded
+// operand rows (whole super-blocks) from i * rows_padded on, and reads its own planes and range sums.
 template <int B, bool F16>
 __global__ void __launch_bounds__(128)
 k_umma_pack_ranges(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum, uint8_t *__restrict__ opA,
-                   int32_t *__restrict__ vRout, Geom g, int64_t j0, int64_t j1, int64_t rows_padded)
+                   int32_t *__restrict__ vRout, Geom g, int64_t j0, int64_t j1, int64_t rows_padded, int n_img)
 {
     using L = Lay<B, F16>;
     constexpr int n = Cfg<B, F16>::n;
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= rows_padded) return;
+    if (i >= rows_padded * n_img) return;
     int64_t sb = i / L::ROWS_SB;
     int rr = (int)(i % L::ROWS_SB);
     int blk = rr / kBlockM, row = rr % kBlockM;
     uint8_t *rowp = opA + sb * L::A_SB_BYTES + blk * L::A_BLOCK_BYTES + (row >> 3) * L::SBO_A + (row & 7) * 16;
     constexpr int NCH = Cfg<B, F16>::KS_A * 2;
-    const int64_t j = j0 + i / g.n_iso;
-    const int kiso = (int)(i % g.n_iso);
+    const int64_t image = i >= rows_padded ? i / rows_padded : 0, il = i - image * rows_padded;
+    src += image * g.W * g.H;
+    rsum += image * g.NR;
+    const int64_t j = j0 + il / g.n_iso;
+    const int kiso = (int)(il % g.n_iso);
     if (j >= j1) {
 #pragma unroll
         for (int c = 0; c < NCH; c++) *(uint4 *)(rowp + c * 128) = make_uint4(0, 0, 0, 0);
@@ -677,15 +705,17 @@ k_umma_pack_ranges(const uint8_t *__restrict__ src, const int32_t *__restrict__ 
 //     ||gR|| ||gD|| >= 2^24 and 0 below; the packers store upper bounds of ||gR|| per range row and of max ||gD|| per
 //     32-domain chunk.  k_umma_refine_rgb replays the float sum in pixel order, i.e. ranks by kov_ref itself.
 
-// Sort keys of the RGB pool: vD^2 (plays the role of varD), payload: the domain index.
-__global__ void k_umma_sortkeys_rgb(const int32_t *__restrict__ dsum, int n, int64_t ND, uint32_t *__restrict__ keys,
+// Sort keys of the RGB pool: vD^2 (plays the role of varD), payload: the domain index (a group of images: see
+// k_umma_sortkeys; the stats are [n_img][3][ND]).
+__global__ void k_umma_sortkeys_rgb(const int32_t *__restrict__ dsum, int n, int64_t ND, int64_t count, uint32_t *__restrict__ keys,
                                     int32_t *__restrict__ vals)
 {
     int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= ND) return;
+    if (j >= count) return;
+    const int64_t image = j >= ND ? j / ND : 0;
     int dm[3];
-    const int vd = centred_sum_rgb(dsum, ND, j, n, dm);
-    keys[j] = (uint32_t)(vd * vd);
+    const int vd = centred_sum_rgb(dsum + image * 3 * ND, ND, j - image * ND, n, dm);
+    keys[j] = (uint32_t)image << 24 | (uint32_t)(vd * vd);
     vals[j] = (int32_t)j;
 }
 
@@ -706,11 +736,21 @@ template <int B>
 __global__ void __launch_bounds__(128)
 k_umma_pack_domains_rgb(const uint16_t *__restrict__ dec3, const int32_t *__restrict__ dsum,
                         const int32_t *__restrict__ perm, uint8_t *__restrict__ opB, int32_t *__restrict__ pos_dom,
-                        int4 *__restrict__ pos_info, int64_t *__restrict__ dom0_pos, Geom g, int64_t ntiles, uint32_t mult)
+                        int4 *__restrict__ pos_info, int64_t *__restrict__ dom0_pos, Geom g, int64_t ntiles, uint32_t mult,
+                        int64_t npos, size_t opb_stride)
 {
     using L = Lay<B, true>;
     constexpr int n = B * B;
-    const int64_t pos = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t p0 = (int64_t)blockIdx.x * blockDim.x;  // see k_umma_pack_domains
+    const int64_t image = p0 >= npos ? p0 / npos : 0;
+    const int64_t pos = p0 + threadIdx.x - image * npos;
+    dec3 += image * g.sw * g.sh;
+    dsum += image * 3 * g.ND;
+    perm += image * g.ND;
+    opB = image_region(opB, image, opb_stride);
+    pos_dom = image_region(pos_dom, image, opb_stride);
+    pos_info = image_region(pos_info, image, opb_stride);
+    dom0_pos = image_region(dom0_pos, image, opb_stride);
     const int64_t tile = pos / kTileN;
     const int row = (int)(pos % kTileN);
     const int64_t sp = sweep_to_sorted(pos, mult, ntiles * kChunksPerTile);
@@ -723,7 +763,7 @@ k_umma_pack_domains_rgb(const uint16_t *__restrict__ dec3, const int32_t *__rest
         pos_dom[pos] = -1;
         pos_info[pos] = make_int4(-1, 0, 0, 0);
     } else {
-        const int64_t j = perm[sp];
+        const int64_t j = perm[sp] - image * g.ND;
         const int gx = (int)(j % g.dpw), gy = (int)(j / g.dpw);
         // dec3 = R + G + B of the decimated planes (k_sum_planes); a block row starts at a multiple of B / 4
         // pixels: B = 8 reads pixel pairs (4-byte loads), B = 16 groups of four (8-byte loads)
@@ -794,18 +834,22 @@ k_umma_pack_domains_rgb(const uint16_t *__restrict__ dec3, const int32_t *__rest
 template <int B>
 __global__ void __launch_bounds__(128)
 k_umma_pack_ranges_rgb(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum, uint8_t *__restrict__ opA,
-                       int32_t *__restrict__ vRout, float *__restrict__ nRout, Geom g, int64_t j0, int64_t j1, int64_t rows_padded)
+                       int32_t *__restrict__ vRout, float *__restrict__ nRout, Geom g, int64_t j0, int64_t j1, int64_t rows_padded,
+                       int n_img)
 {
     using L = Lay<B, true>;
     constexpr int n = B * B;
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= rows_padded) return;
+    if (i >= rows_padded * n_img) return;
     int64_t sb = i / L::ROWS_SB;
     int rr = (int)(i % L::ROWS_SB);
     int blk = rr / kBlockM, row = rr % kBlockM;
     uint8_t *rowp = opA + sb * L::A_SB_BYTES + blk * L::A_BLOCK_BYTES + (row >> 3) * L::SBO_A + (row & 7) * 16;
     constexpr int NCH = n / 8;
-    const int64_t j = j0 + i;
+    const int64_t image = i >= rows_padded ? i / rows_padded : 0;  // see k_umma_pack_ranges
+    src += image * 3 * g.W * g.H;
+    rsum += image * 3 * g.NR;
+    const int64_t j = j0 + (i - image * rows_padded);
     if (j >= j1) {
 #pragma unroll
         for (int c = 0; c < NCH; c++) *(uint4 *)(rowp + c * 128) = make_uint4(0, 0, 0, 0);
@@ -1063,11 +1107,17 @@ __host__ __device__ constexpr int epi_of() { return (!F16 || B == 16) ? 0 : ((B 
 // multicast to both CTAs' barriers; CTA 1's warp 1 relays "my half has landed" to CTA 0's full barriers and CTA 1's
 // epilogue warps hand accumulators back on CTA 0's t_empty barriers (remote mbarrier arrives).  The epilogue is
 // the same code in both CTAs.  n_sb must be even.
-template <int B, bool F16, bool PAIR, bool DUMP>
+//
+// GROUP: a group of images (block-diagonal search): super-block sb belongs to image sb / n_sb_img, whose domain tiles
+// start opb_stride bytes after the previous image's; n_sb_img is even, so a CTA pair never straddles two images.  Only
+// the unit's opB base depends on the image -- ntiles is per image, and row-indexed arrays use the group-global row.
+// A single image runs the GROUP = false instantiation, whose code does not see the image arithmetic at all.
+template <int B, bool F16, bool PAIR, bool DUMP, bool GROUP = false>
 __global__ void __launch_bounds__(kThreads, 1)
 k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, const int32_t *__restrict__ vRarr,
               const float *__restrict__ nRarr, int2 *__restrict__ flag_list, int32_t *__restrict__ flag_cnt, uint32_t *__restrict__ row_lb, int n_sb,
-              int n_chunks, int ntiles, int iso_shift, int64_t rows_padded, int32_t *__restrict__ dump, int64_t dump_ld, volatile int *status)
+              int n_chunks, int ntiles, int iso_shift, int64_t rows_padded, int32_t *__restrict__ dump, int64_t dump_ld, volatile int *status,
+              int n_sb_img, int64_t opb_stride)
 {
     using C = Cfg<B, F16>;
     using L = Lay<B, F16>;
@@ -1143,11 +1193,12 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
             for (int u = u_first; u < n_units; u += u_step) {
                 int sb = PAIR ? 2 * (u % n_sbu) + (int)rank : u % n_sbu, ch = u / n_sbu;  // chunk-major: see the epilogue (bounds carried between units)
                 int t0 = (int)((int64_t)ch * ntiles / n_chunks), t1 = (int)((int64_t)(ch + 1) * ntiles / n_chunks);
+                const uint8_t *const opB_img = GROUP ? opB + (int64_t)(sb / n_sb_img) * opb_stride : opB;
                 mbar_wait(BAR_A_EMPTY, a_phase ^ 1, status, 1);
                 mbar_expect_tx(BAR_A_FULL, L::A_SB_BYTES);
                 bulk_g2s(smem_u32(sA), opA + (int64_t)sb * L::A_SB_BYTES, L::A_SB_BYTES, BAR_A_FULL);
                 for (int t = t0; t < t1; t++) {
-                    const uint8_t *blob = opB + (int64_t)t * L::B_TILE_BYTES;
+                    const uint8_t *blob = opB_img + (int64_t)t * L::B_TILE_BYTES;
                     if (C::KSPLIT && PAIR) {
                         // this CTA's half (operand rows 64 * rank ..) of part P0, then of part P1 unless its digits are all zero
                         const uint32_t has_l = __ldg((const uint32_t *)(blob + L::B_OP_BYTES + kChunksPerTile * 8));
@@ -1467,6 +1518,7 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
             // later ones -- any earlier bound is a valid bound, a missed one only costs extra flags.
             int sb = PAIR ? 2 * (u % n_sbu) + (int)rank : u % n_sbu, ch = u / n_sbu;
             int t0 = (int)((int64_t)ch * ntiles / n_chunks), t1 = (int)((int64_t)(ch + 1) * ntiles / n_chunks);
+            const uint8_t *const opB_img = GROUP ? opB + (int64_t)(sb / n_sb_img) * opb_stride : opB;
             // Running filter state of this thread's row (see the file header).  vR == 0: every candidate
             // scores error 0 and the first one wins (FC:677-678, FC:627) -> never flag.
             const int64_t row = (int64_t)sb * L::ROWS_SB + q * kBlockM + lq * 32 + lane;
@@ -1498,7 +1550,7 @@ k_umma_search(const uint8_t *__restrict__ opA, const uint8_t *__restrict__ opB, 
                 // (rhi, rlo) of the tile's four chunks, from the tile blob in global memory (the shared-memory ring
                 // belongs to the producer and the MMA issuer alone): a broadcast load that every warp of the CTA
                 // repeats, so it is an L1 hit for all but the first; its latency hides behind the t_full wait.
-                const float4 *gb = (const float4 *)(opB + (int64_t)t * L::B_TILE_BYTES + L::B_OP_BYTES);
+                const float4 *gb = (const float4 *)(opB_img + (int64_t)t * L::B_TILE_BYTES + L::B_OP_BYTES);
                 const float4 bnd01 = __ldg(gb), bnd23 = __ldg(gb + 1);
                 float4 bndn = make_float4(0.0f, 0.0f, 0.0f, 0.0f);  // >= ||gD||_2 of the rows of each chunk
                 if (SLACK) bndn = __ldg(gb + 3);
@@ -1854,6 +1906,8 @@ __device__ __forceinline__ void for_each_flagged(int lane, int64_t i, int64_t ro
 // Each lane runs the search kernel's filter once more on its own candidates (x bounded from the exact
 // integer kov and a correctly rounded binary32 1/sqrt(varD)), so the reference's double-precision
 // expression (FC:677-683) is only evaluated for candidates that can still win or tie.
+// A group of n_img images: warp w refines row w % rows of image w / rows -- operand row image * rp_img + that row of the
+// group, that image's planes, range sums, OpBLayout region (opb_stride bytes per image) and rows of `best`.
 template <int B>
 __global__ void __launch_bounds__(128)
 k_umma_refine(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum, const uint8_t *__restrict__ pos_raw,
@@ -1861,14 +1915,22 @@ k_umma_refine(const uint8_t *__restrict__ src, const int32_t *__restrict__ rsum,
               const int2 *__restrict__ flag_list, const int32_t *__restrict__ flag_cnt,
               const uint32_t *__restrict__ row_lb, int n_chunks,
               int64_t rows_padded, int64_t rows, int64_t npos, const int64_t *__restrict__ dom0_pos,
-              int32_t *__restrict__ best, Geom g, int64_t j0)
+              int32_t *__restrict__ best, Geom g, int64_t j0, int n_img, int64_t rp_img, size_t opb_stride)
 {
     constexpr int n = B * B;
     constexpr int NW = n / 4;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t i = (int64_t)blockIdx.x * 4 + warp;  // operand row == range block (the isometry extension has its own kernel)
-    if (i >= rows) return;
-    const int64_t j = j0 + i;
+    const int64_t w = (int64_t)blockIdx.x * 4 + warp;
+    if (w >= rows * n_img) return;
+    const int64_t image = w >= rows ? w / rows : 0, il = w - image * rows;
+    const int64_t i = image * rp_img + il;  // operand row == range block (the isometry extension has its own kernel)
+    const int64_t j = j0 + il;
+    src += image * g.W * g.H;
+    rsum += image * g.NR;
+    best += image * g.NR;
+    pos_raw = image_region(pos_raw, image, opb_stride);
+    pos_info = image_region(pos_info, image, opb_stride);
+    dom0_pos = image_region(dom0_pos, image, opb_stride);
     int rmean;
     const int vR = centred_sum(rsum[j], n, &rmean);
     if (vR == 0) {  // FC:677-678 + FC:627: all errors are 0, the first candidate wins
@@ -1937,15 +1999,24 @@ k_umma_refine_iso(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
                   const int4 *__restrict__ pos_info, const int2 *__restrict__ flag_list,
                   const int32_t *__restrict__ flag_cnt, const uint32_t *__restrict__ row_lb, int n_chunks,
                   int64_t rows_padded, int64_t ranges, int64_t npos,
-                  const int64_t *__restrict__ dom0_pos, int32_t *__restrict__ best, Geom g, int64_t j0)
+                  const int64_t *__restrict__ dom0_pos, int32_t *__restrict__ best, Geom g, int64_t j0, int n_img, int64_t rp_img,
+                  size_t opb_stride)
 {
     constexpr int n = B * B;
     constexpr int NW = n / 4;
     __shared__ uint8_t s_blk[4][n];  // the range block of each of the block's 4 warps, raster order
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t r = (int64_t)blockIdx.x * 4 + warp;
-    if (r >= ranges) return;
+    const int64_t w = (int64_t)blockIdx.x * 4 + warp;  // a group of images: see k_umma_refine
+    if (w >= ranges * n_img) return;
+    const int64_t image = w >= ranges ? w / ranges : 0, r = w - image * ranges;
+    const int64_t i0 = image * rp_img + r * 8;  // the block's first operand row in the group
     const int64_t j = j0 + r;
+    src += image * g.W * g.H;
+    rsum += image * g.NR;
+    best += image * g.NR;
+    pos_raw = image_region(pos_raw, image, opb_stride);
+    pos_info = image_region(pos_info, image, opb_stride);
+    dom0_pos = image_region(dom0_pos, image, opb_stride);
     int rmean;
     const int vR = centred_sum(rsum[j], n, &rmean);
     if (vR == 0) {  // FC:677-678 + FC:627: all errors are 0, the first candidate wins
@@ -1980,7 +2051,7 @@ k_umma_refine_iso(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
     const float tie_abs = (float)(vR * vR) * 4.76837158203125e-07f;  // vR^2 * 2^-21
     // lane-local bound / threshold, shared by the 8 isometries (they compete for one winner), seeded with the bound
     // the search kernel reached for this range block (its 8 operand rows publish into the first one's slot)
-    float lb = __uint_as_float(row_lb[r * 8]), th = lb > 0.0f ? flag_threshold(lb, tie_abs) : -1.0f;
+    float lb = __uint_as_float(row_lb[i0]), th = lb > 0.0f ? flag_threshold(lb, tie_abs) : -1.0f;
     const float th_row = th;
     auto consider = [&](int64_t pos, int kiso) {
         const int4 pi = __ldg(pos_info + pos);  // {domain index (-1: padding), varD, sum d, -}
@@ -2000,7 +2071,7 @@ k_umma_refine_iso(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
     bool overflow = false;
     for (int ch = 0; ch < n_chunks && !overflow; ch++) {
         // 8 * kFlagLists (<= 32) contiguous list lengths: operand row 8 r + k, list h of the unit at lane kFlagLists * k + h
-        const int64_t base = ((int64_t)ch * rows_padded + r * 8) * kFlagLists;
+        const int64_t base = ((int64_t)ch * rows_padded + i0) * kFlagLists;
         const int my_cnt = lane < 8 * kFlagLists ? flag_cnt[base + lane] : 0;
         if (__any_sync(0xffffffffu, my_cnt > kFlagCap)) { overflow = true; break; }
         for (int kiso = 0; kiso < 8; kiso++) {
@@ -2042,14 +2113,22 @@ k_umma_refine_rgb(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
                   const int4 *__restrict__ pos_info, const int2 *__restrict__ flag_list, const int32_t *__restrict__ flag_cnt,
                   const uint32_t *__restrict__ row_lb, int n_chunks,
                   int64_t rows_padded, int64_t rows, int64_t npos, const int64_t *__restrict__ dom0_pos,
-                  int32_t *__restrict__ best, Geom g, int64_t j0)
+                  int32_t *__restrict__ best, Geom g, int64_t j0, int n_img, int64_t rp_img, size_t opb_stride)
 {
     using L = Lay<B, true>;
     constexpr int n = B * B;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t i = (int64_t)blockIdx.x * 4 + warp;
-    if (i >= rows) return;
-    const int64_t j = j0 + i;
+    const int64_t w = (int64_t)blockIdx.x * 4 + warp;  // a group of images: see k_umma_refine
+    if (w >= rows * n_img) return;
+    const int64_t image = w >= rows ? w / rows : 0, il = w - image * rows;
+    const int64_t i = image * rp_img + il;
+    const int64_t j = j0 + il;
+    src += image * 3 * g.W * g.H;
+    rsum += image * 3 * g.NR;
+    best += image * g.NR;
+    opB = image_region(opB, image, opb_stride);
+    pos_info = image_region(pos_info, image, opb_stride);
+    dom0_pos = image_region(dom0_pos, image, opb_stride);
     int rm[3];
     const int vRi = centred_sum_rgb(rsum, g.NR, j, n, rm);
     const int rmsum = rm[0] + rm[1] + rm[2];
@@ -2113,9 +2192,12 @@ k_umma_refine_rgb(const uint8_t *__restrict__ src, const int32_t *__restrict__ r
 inline int64_t pad_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
 inline uint64_t gcd_u64(uint64_t a, uint64_t b) { while (b) { uint64_t t = a % b; a = b; b = t; } return a; }
 
+// A group of n_img images: every image's operand rows are padded on their own (rp_img, n_sb_img), the group's rows
+// follow each other (rp, n_sb); the domain sweep (ntiles, npos, mult) is per image.
 struct Plan {
-    int64_t rp;     // rows padded to whole super-blocks
-    int n_sb, ntiles, n_chunks;
+    int64_t rp;     // rows padded to whole super-blocks (the whole group)
+    int64_t rp_img; // ... per image
+    int n_img, n_sb, n_sb_img, ntiles, n_chunks;
     uint32_t mult;  // sweep-order multiplier (see sweep_to_sorted)
     int64_t npos;   // ntiles * 128 sweep positions
 };
@@ -2128,14 +2210,17 @@ struct Plan {
 // k_umma_search, whole-GPU nanoseconds per flagged chunk of k_umma_refine) -- only their ratio matters.
 inline int rows_per_sb(const Geom &g) { return (g.C == 3 && g.B == 16 ? 2 : kAccs) * kBlockM; }  // Cfg<...>::NB * 128
 
-inline Plan make_plan(const Geom &g, int64_t rows, int num_sms)
+inline Plan make_plan(const Geom &g, int64_t rows, int num_sms, int n_img = 1)
 {
     Plan p;
     const int rows_sb = rows_per_sb(g);
-    // an even number of 512-row super-blocks: CTA pairs (k_umma_search<..., PAIR>) take two at a time; padding rows
-    // are zero operands with vR = 0 (never flagged)
-    p.rp = pad_up(rows, 2 * rows_sb);
-    p.n_sb = (int)(p.rp / rows_sb);
+    // an even number of 512-row super-blocks per image: CTA pairs (k_umma_search<..., PAIR>) take two at a time and
+    // never straddle two images; padding rows are zero operands with vR = 0 (never flagged)
+    p.n_img = n_img;
+    p.rp_img = pad_up(rows, 2 * rows_sb);
+    p.rp = p.rp_img * n_img;
+    p.n_sb_img = (int)(p.rp_img / rows_sb);
+    p.n_sb = p.n_sb_img * n_img;
     p.ntiles = (int)((g.ND + kTileN - 1) / kTileN);
     p.npos = (int64_t)p.ntiles * kTileN;
     p.n_chunks = 1;
@@ -2147,7 +2232,7 @@ inline Plan make_plan(const Geom &g, int64_t rows, int num_sms)
         const int64_t waves = (units + num_sms - 1) / num_sms;
         const double tiles_per_unit = (double)((p.ntiles + c - 1) / c);
         const double flags_per_row = 2.0 * (log(2.0 * tiles_per_unit) + 0.58) + 2.0 * (c - 1) * 1.5;
-        const double cost = (double)waves * tiles_per_unit * tile_s + (double)rows * flags_per_row * flag_s;
+        const double cost = (double)waves * tiles_per_unit * tile_s + (double)rows * n_img * flags_per_row * flag_s;
         if (c == 1 || cost < best_cost * 0.98) { best_cost = cost; p.n_chunks = c; }
     }
     const uint64_t nch = (uint64_t)p.ntiles * kChunksPerTile;
@@ -2157,11 +2242,11 @@ inline Plan make_plan(const Geom &g, int64_t rows, int num_sms)
     return p;
 }
 
-// opB workspace: [tile blobs][pos_dom s32][pos_info int4][pos_raw u8 x n][dom0 pos s64]
-//                [sort: keys x2, vals x2, digit histograms]
+// opB workspace: per image [tile blobs][pos_dom s32][pos_info int4][pos_raw u8 x n][dom0 pos s64], `stride` bytes
+// per image (the offsets are image 0's), then [sort of the group's domains: keys x2, vals x2, digit histograms]
 template <int B, bool F16>
 struct OpBLayout {
-    size_t off_posdom, off_posinfo, off_posraw, off_dom0, off_keys0, off_keys1, off_vals0, off_vals1, off_temp,
+    size_t off_posdom, off_posinfo, off_posraw, off_dom0, stride, off_keys0, off_keys1, off_vals0, off_vals1, off_temp,
         temp_bytes, total;
     OpBLayout(const Geom &g, const Plan &p)
     {
@@ -2171,11 +2256,14 @@ struct OpBLayout {
         off_posinfo = take((size_t)p.npos * 16);
         off_posraw = take((size_t)p.npos * (B * B));
         off_dom0 = take(16);  // s64 sweep position of domain 0
-        off_keys0 = take((size_t)g.ND * 4);
-        off_keys1 = take((size_t)g.ND * 4);
-        off_vals0 = take((size_t)g.ND * 4);
-        off_vals1 = take((size_t)g.ND * 4);
-        temp_bytes = sort_hist_bytes(g.ND);
+        stride = (o + 255) & ~(size_t)255;
+        o = stride * p.n_img;
+        const int64_t nd = g.ND * p.n_img;
+        off_keys0 = take((size_t)nd * 4);
+        off_keys1 = take((size_t)nd * 4);
+        off_vals0 = take((size_t)nd * 4);
+        off_vals1 = take((size_t)nd * 4);
+        temp_bytes = sort_hist_bytes(nd);
         off_temp = take(temp_bytes + 256);
         total = o + 256;
     }
@@ -2200,13 +2288,13 @@ struct OpALayout {
 };
 
 template <int B, bool F16>
-size_t opA_bytes_t(const Geom &g, int64_t rows, int num_sms)
+size_t opA_bytes_t(const Geom &g, int64_t rows, int num_sms, int n_img = 1)
 {
-    return OpALayout<B, F16>(make_plan(g, rows, num_sms)).total;
+    return OpALayout<B, F16>(make_plan(g, rows, num_sms, n_img)).total;
 }
 
 using KernelT = void (*)(const uint8_t *, const uint8_t *, const int32_t *, const float *, int2 *, int32_t *, uint32_t *, int, int,
-                         int, int, int64_t, int32_t *, int64_t, volatile int *);
+                         int, int, int64_t, int32_t *, int64_t, volatile int *, int, int64_t);
 
 // CTA pairs exist for the kind::f16 kernels (B = 4, 8: grey, RGB and the isometry extension; two issuing warps) and for
 // the K-split B = 16 configurations (kind::i8 grey, kind::f16 RGB; one issuing warp, each CTA loads half of either part
@@ -2255,14 +2343,16 @@ inline bool pair_launchable(KernelT kern, int smem_bytes)
     return ok;
 }
 
+// n_img > 1: a group of images, every range of each (see launch_search_umma).
 template <int B, bool F16>
 int launch_t(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, cudaStream_t s, const char **err,
-             cudaEvent_t k0, cudaEvent_t k1, int pair_mode, int *pair_used, int32_t *dump, int64_t dump_ld, int *status_dev)
+             cudaEvent_t k0, cudaEvent_t k1, int pair_mode, int *pair_used, int32_t *dump, int64_t dump_ld, int *status_dev,
+             int n_img)
 {
     using L = Lay<B, F16>;
     if (j1 <= j0) return 0;
-    const int64_t rows = (j1 - j0) * g.n_iso;  // operand rows: one per (range, isometry)
-    Plan p = make_plan(g, rows, num_sms);
+    const int64_t rows = (j1 - j0) * g.n_iso;  // operand rows of an image: one per (range, isometry)
+    Plan p = make_plan(g, rows, num_sms, n_img);
     const int64_t rp = p.rp;
     uint8_t *opA = w.opA;
     const OpALayout<B, F16> la(p);
@@ -2280,35 +2370,42 @@ int launch_t(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, 
     int64_t *dom0 = (int64_t *)(w.opB + lay.off_dom0);
     int launches = 0;
     cudaError_t ce;
-    // 1. domains by increasing varD
+    // 1. domains by increasing varD (a group: by image, then varD -- the image index is a fourth key digit, so a group
+    // holds at most 256 images)
     uint32_t *keys0 = (uint32_t *)(w.opB + lay.off_keys0), *keys1 = (uint32_t *)(w.opB + lay.off_keys1);
     int32_t *vals0 = (int32_t *)(w.opB + lay.off_vals0), *vals1 = (int32_t *)(w.opB + lay.off_vals1);
-    if (rgb) k_umma_sortkeys_rgb<<<(unsigned)((g.ND + 255) / 256), 256, 0, s>>>(w.dsum, g.n, g.ND, keys0, vals0);
-    else k_umma_sortkeys<<<(unsigned)((g.ND + 255) / 256), 256, 0, s>>>(w.dsum, w.dsq, g.n, g.ND, keys0, vals0);
-    launches += 1 + launch_sort_pairs(keys0, vals0, keys1, vals1, (uint32_t *)(w.opB + lay.off_temp), g.ND, s);
-    const int32_t *perm = vals1;  // domains by increasing key
+    if (n_img < 1 || n_img > 256) { *err = "a tcgen05 group holds 1 to 256 images"; return -1; }
+    const int64_t nd = g.ND * n_img;
+    if (rgb) k_umma_sortkeys_rgb<<<(unsigned)((nd + 255) / 256), 256, 0, s>>>(w.dsum, g.n, g.ND, nd, keys0, vals0);
+    else k_umma_sortkeys<<<(unsigned)((nd + 255) / 256), 256, 0, s>>>(w.dsum, w.dsq, g.n, g.ND, nd, keys0, vals0);
+    const int passes = n_img > 1 ? 4 : 3;
+    launches += 1 + launch_sort_pairs(keys0, vals0, keys1, vals1, (uint32_t *)(w.opB + lay.off_temp), nd, passes, s);
+    const int32_t *perm = passes & 1 ? vals1 : vals0;  // domains by increasing key
     // 2. operand blobs
     if constexpr (F16) {
         if (rgb) {
-            launches += launch_sum_planes(w.dec, w.dec3, g, s);
-            k_umma_pack_domains_rgb<B><<<(unsigned)((p.npos + 127) / 128), 128, 0, s>>>(
-                w.dec3, w.dsum, perm, w.opB, pos_dom, pos_info, dom0, g, p.ntiles, p.mult);
-            k_umma_pack_ranges_rgb<B><<<(unsigned)((rp + 127) / 128), 128, 0, s>>>(w.src, w.rsum, opA, vR, B == 16 ? row_norm : nullptr, g, j0, j1, rp);
+            launches += launch_sum_planes(w.dec, w.dec3, g, s, n_img);
+            k_umma_pack_domains_rgb<B><<<(unsigned)((p.npos * n_img + 127) / 128), 128, 0, s>>>(
+                w.dec3, w.dsum, perm, w.opB, pos_dom, pos_info, dom0, g, p.ntiles, p.mult, p.npos, lay.stride);
+            k_umma_pack_ranges_rgb<B><<<(unsigned)((rp + 127) / 128), 128, 0, s>>>(w.src, w.rsum, opA, vR, B == 16 ? row_norm : nullptr, g, j0, j1,
+                                                                                p.rp_img, n_img);
         }
     }
     if (!rgb) {
-        k_umma_pack_domains<B, F16><<<(unsigned)((p.npos + 127) / 128), 128, 0, s>>>(
-            w.dec, w.dsum, w.dsq, perm, w.opB, pos_dom, pos_info, pos_raw, dom0, g, p.ntiles, p.mult);
-        k_umma_pack_ranges<B, F16><<<(unsigned)((rp + 127) / 128), 128, 0, s>>>(w.src, w.rsum, opA, vR, g, j0, j1, rp);
+        k_umma_pack_domains<B, F16><<<(unsigned)((p.npos * n_img + 127) / 128), 128, 0, s>>>(
+            w.dec, w.dsum, w.dsq, perm, w.opB, pos_dom, pos_info, pos_raw, dom0, g, p.ntiles, p.mult, p.npos, lay.stride);
+        k_umma_pack_ranges<B, F16><<<(unsigned)((rp + 127) / 128), 128, 0, s>>>(w.src, w.rsum, opA, vR, g, j0, j1, p.rp_img, n_img);
     }
     launches += 2;
     // 3. the fused search: CTA pairs on request (FIC_UMMA_PAIR_ON / _OFF), else where measured faster (pair_default)
     bool pair = false;
-    KernelT kern = dump ? k_umma_search<B, F16, false, true> : k_umma_search<B, F16, false, false>;
+    const bool group = n_img > 1;
+    if (dump && group) { *err = "the accumulator dump takes one image"; return -1; }
+    KernelT kern = dump ? k_umma_search<B, F16, false, true> : group ? k_umma_search<B, F16, false, false, true> : k_umma_search<B, F16, false, false>;
     if constexpr (pair_capable<B, F16>()) {
         pair = (pair_mode == FIC_UMMA_PAIR_ON || (pair_mode != FIC_UMMA_PAIR_OFF && pair_default<B, F16>())) && num_sms >= 2;
         if (pair) {
-            KernelT pk = dump ? k_umma_search<B, F16, true, true> : k_umma_search<B, F16, true, false>;
+            KernelT pk = dump ? k_umma_search<B, F16, true, true> : group ? k_umma_search<B, F16, true, false, true> : k_umma_search<B, F16, true, false>;
             ce = cudaFuncSetAttribute(pk, cudaFuncAttributeMaxDynamicSharedMemorySize, L::SMEM_BYTES);
             if (ce != cudaSuccess) { *err = cudaGetErrorString(ce); return -1; }
             if (pair_launchable(pk, L::SMEM_BYTES)) kern = pk;
@@ -2342,21 +2439,24 @@ int launch_t(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, 
         const int iso_shift = g.n_iso > 1 ? 3 : 0;
         volatile int *status_v = status_dev;
         ce = cudaLaunchKernelEx(&cfg, kern, opA_c, opB_c, vR_c, norm_c, flag_list, flag_cnt, row_lb, p.n_sb, p.n_chunks, p.ntiles, iso_shift,
-                                rp, dump, dump_ld, status_v);
+                                rp, dump, dump_ld, status_v, p.n_sb_img, (int64_t)lay.stride);
         if (ce != cudaSuccess) { *err = cudaGetErrorString(ce); return -1; }
     }
     if (k1) cudaEventRecord(k1, s);
     // 4. exact refine of the flagged chunks
     if (rgb) {
         if constexpr (F16)
-            k_umma_refine_rgb<B><<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(w.src, w.rsum, w.opB, pos_info, flag_list, flag_cnt,
-                                                                            row_lb, p.n_chunks, rp, rows, p.npos, dom0, w.best, g, j0);
+            k_umma_refine_rgb<B><<<(unsigned)((rows * n_img + 3) / 4), 128, 0, s>>>(
+                w.src, w.rsum, w.opB, pos_info, flag_list, flag_cnt, row_lb, p.n_chunks, rp, rows, p.npos, dom0, w.best, g, j0, n_img,
+                p.rp_img, lay.stride);
     } else if (g.n_iso > 1)
-        k_umma_refine_iso<B><<<(unsigned)((j1 - j0 + 3) / 4), 128, 0, s>>>(w.src, w.rsum, pos_raw, pos_info, flag_list, flag_cnt,
-                                                                         row_lb, p.n_chunks, rp, j1 - j0, p.npos, dom0, w.best, g, j0);
+        k_umma_refine_iso<B><<<(unsigned)(((j1 - j0) * n_img + 3) / 4), 128, 0, s>>>(
+            w.src, w.rsum, pos_raw, pos_info, flag_list, flag_cnt, row_lb, p.n_chunks, rp, j1 - j0, p.npos, dom0, w.best, g, j0, n_img,
+            p.rp_img, lay.stride);
     else
-        k_umma_refine<B><<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(w.src, w.rsum, pos_raw, pos_info, flag_list, flag_cnt,
-                                                                    row_lb, p.n_chunks, rp, rows, p.npos, dom0, w.best, g, j0);
+        k_umma_refine<B><<<(unsigned)((rows * n_img + 3) / 4), 128, 0, s>>>(w.src, w.rsum, pos_raw, pos_info, flag_list, flag_cnt,
+                                                                            row_lb, p.n_chunks, rp, rows, p.npos, dom0, w.best, g, j0,
+                                                                            n_img, p.rp_img, lay.stride);
     launches += 2;
     ce = cudaGetLastError();
     if (ce != cudaSuccess) { *err = cudaGetErrorString(ce); return -1; }
@@ -2522,7 +2622,7 @@ int umma_f16_selftest(int num_sms, cudaStream_t s, const char **err)
             launch_domain_stats(w.dec, w.dsum, w.dsq, *gp, s);
             launch_range_stats(w.src, w.rsum, *gp, s);
             if (launch_t<8, true>(w, *gp, 0, gp->NR, num_sms, s, err, nullptr, nullptr, FIC_UMMA_PAIR_AUTO, nullptr, dump, dump_ld,
-                                  nullptr) < 0) {
+                                  nullptr, 1) < 0) {
                 launched = false;
                 break;
             }
@@ -2552,7 +2652,7 @@ int umma_debug_sort(uint32_t *d_keys, int32_t *d_vals, uint32_t *d_keys_out, int
     uint32_t *hist = nullptr;
     cudaError_t ce = cudaMalloc((void **)&hist, sort_hist_bytes(n) + 256);
     if (ce != cudaSuccess) return (int)ce;
-    launch_sort_pairs(d_keys, d_vals, d_keys_out, d_vals_out, hist, n, s);
+    launch_sort_pairs(d_keys, d_vals, d_keys_out, d_vals_out, hist, n, 3, s);
     ce = cudaStreamSynchronize(s);
     cudaFree(hist);
     return (int)ce;
@@ -2612,18 +2712,18 @@ bool umma_applicable(const Geom &g)
     return g.B == 4 || g.B == 8 || g.B == 16;
 }
 
-size_t umma_opA_bytes(const Geom &g, int64_t j0, int64_t j1, int num_sms, int kind)
+size_t umma_opA_bytes(const Geom &g, int64_t j0, int64_t j1, int num_sms, int kind, int n_images)
 {
     const int64_t rows = (j1 - j0) * g.n_iso;  // operand rows: one per (range, isometry)
-    return FIC_UMMA_DISPATCH(g.B, use_f16(g, kind), (opA_bytes_t<4, false>(g, rows, num_sms)),
-                             (opA_bytes_t<8, false>(g, rows, num_sms)), (opA_bytes_t<16, false>(g, rows, num_sms)),
-                             (opA_bytes_t<4, true>(g, rows, num_sms)), (opA_bytes_t<8, true>(g, rows, num_sms)),
-                             (opA_bytes_t<16, true>(g, rows, num_sms)));
+    return FIC_UMMA_DISPATCH(g.B, use_f16(g, kind), (opA_bytes_t<4, false>(g, rows, num_sms, n_images)),
+                             (opA_bytes_t<8, false>(g, rows, num_sms, n_images)), (opA_bytes_t<16, false>(g, rows, num_sms, n_images)),
+                             (opA_bytes_t<4, true>(g, rows, num_sms, n_images)), (opA_bytes_t<8, true>(g, rows, num_sms, n_images)),
+                             (opA_bytes_t<16, true>(g, rows, num_sms, n_images)));
 }
 
-size_t umma_opB_bytes(const Geom &g, int kind)
+size_t umma_opB_bytes(const Geom &g, int kind, int n_images)
 {
-    Plan p = make_plan(g, rows_per_sb(g), 148);  // the opB layout depends on the pool only
+    Plan p = make_plan(g, rows_per_sb(g), 148, n_images);  // the opB layout depends on the pool and the image count only
     return FIC_UMMA_DISPATCH(g.B, use_f16(g, kind), (OpBLayout<4, false>(g, p).total), (OpBLayout<8, false>(g, p).total),
                              (OpBLayout<16, false>(g, p).total), (OpBLayout<4, true>(g, p).total),
                              (OpBLayout<8, true>(g, p).total), (OpBLayout<16, true>(g, p).total));
@@ -2631,9 +2731,9 @@ size_t umma_opB_bytes(const Geom &g, int kind)
 
 int launch_search_umma(const Work &w, const Geom &g, int64_t j0, int64_t j1, int num_sms, cudaStream_t s,
                        const char **err, int kind, cudaEvent_t k0, cudaEvent_t k1, int pair, int *pair_used,
-                       int32_t *dump, int64_t dump_ld, int *status_dev)
+                       int32_t *dump, int64_t dump_ld, int *status_dev, int n_images)
 {
-#define FIC_UMMA_ARGS w, g, j0, j1, num_sms, s, err, k0, k1, pair, pair_used, dump, dump_ld, status_dev
+#define FIC_UMMA_ARGS w, g, j0, j1, num_sms, s, err, k0, k1, pair, pair_used, dump, dump_ld, status_dev, n_images
     return FIC_UMMA_DISPATCH(g.B, use_f16(g, kind), (launch_t<4, false>(FIC_UMMA_ARGS)), (launch_t<8, false>(FIC_UMMA_ARGS)),
                              (launch_t<16, false>(FIC_UMMA_ARGS)), (launch_t<4, true>(FIC_UMMA_ARGS)),
                              (launch_t<8, true>(FIC_UMMA_ARGS)), (launch_t<16, true>(FIC_UMMA_ARGS)));

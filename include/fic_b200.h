@@ -196,9 +196,14 @@ int fic_decode_planes_dev(fic_handle *h, int is_rgb, int W, int H, int B, int wk
  * iteration count equal what the single entries give for that image alone, bit for bit.
  *
  * Encode: where the single encode would run the fused one-launch kernel (widthKernel <= 16, no isometries, up to 16 K
- * range blocks per image, FIC_ENGINE_AUTO or _FUSED) the whole batch is one launch per group of images.  Every other
- * case (forced DIRECT or UMMA, widthKernel > 16, the isometry extension, larger images) runs the single-image engine
- * once per image inside the call: the images still go up and their codes come down in one copy per group, but
+ * range blocks per image, FIC_ENGINE_AUTO or _FUSED) the whole batch is one launch per group of images.  With the full
+ * domain pool (widthKernel == domain blocks per width == per height; RGB without isometries) a group of images is ONE
+ * tcgen05 tensor-core search: one pool build, sort, operand pack, search kernel, refine and solve for the whole group.
+ * FIC_ENGINE_UMMA always runs it; FIC_ENGINE_AUTO runs it where the single encode would, and instead of the CUDA-core
+ * search for groups of 4 images or more (full pools of up to 16 x 16 domains keep the fused kernel, which is faster
+ * there).  A tensor-core group holds at most 256 images and about 1 GB of operand workspace.  Every other case (forced
+ * DIRECT, windows between 17 and the full pool, the isometry extension below the full pool) runs the single-image
+ * engine once per image inside the call: the images still go up and their codes come down in one copy per group, but
  * there is no launch saving.  planes (the _u8 form): [n][C][H][W], C = 3 for RGB, else 1 (the red channel).
  *
  * Decode: where the single decode would run its one-launch decoder (blockgroesse >= 8, W % 16 == 0, no isometries, up to
@@ -211,7 +216,8 @@ int fic_decode_planes_dev(fic_handle *h, int is_rgb, int W, int H, int B, int wk
  * FIC_E_ARG for n_images < 1, NULL images or codes, or a batch whose byte count overflows, besides the single entries'
  * rejections; FIC_E_STREAM when some image's codes index outside the domain pool (fic_last_error names the lowest
  * such image).  fic_get_timings then reports the whole call: total_ms, launches, engine (encode) and search_evals
- * (n * NR * widthKernel^2 * isometries). */
+ * (n * NR * widthKernel^2 * isometries); on the tensor-core engine also pool_ms, search_ms, kernel_ms and solve_ms,
+ * summed over the groups. */
 int fic_encode_batch(fic_handle *h, int mode, const int32_t *argb, int n_images, int W, int H, int B, int wk,
                      float *info, int32_t *qcodes);
 int fic_encode_batch_u8(fic_handle *h, int mode, const uint8_t *planes, int n_images, int W, int H, int B, int wk,

@@ -6,6 +6,8 @@ single calls, on images of the reference's own sizes, with every batch output ch
 Host buffers are page-locked with fic_pin_host_buffer.  For each configuration and batch size n it records, per image:
 device time (the library's events, fic_get_timings total_ms, summed over the loop's calls) and host time (a clock
 around the synchronised call), for the ARGB and the 8-bit forms; the median of --reps repetitions after one warm-up.
+Full-pool rows (widthKernel = domain blocks per side) also time the 8-bit batch with the engine forced to the tcgen05
+group search and to the CUDA-core search, and record the engine AUTO ran: the data behind AUTO's batch rule.
 Writes OUT_DIR/batch_bench.json and exits 1 if any batch output differs from the single-call loop.
 """
 import argparse
@@ -27,6 +29,14 @@ CONFIGS = [  # name, W, H, B, wk, rgb
     ("RGB 256^2 B=8 wk=2", 256, 256, 8, 2, True),
     ("grey 64^2 B=8 wk=2", 64, 64, 8, 2, False),
     ("grey 256^2 B=8 wk=16", 256, 256, 8, 16, False),
+    # the full domain pool (the best-quality encode): AUTO runs groups of 4 or more images as tcgen05 group searches
+    # instead of the CUDA-core search; the last row is a pool small enough for the fused kernel, which AUTO keeps
+    ("grey 256^2 B=8 wk=61 (full pool)", 256, 256, 8, 61, False),
+    ("grey 256^2 B=16 wk=29 (full pool)", 256, 256, 16, 29, False),
+    ("grey 128^2 B=4 wk=61 (full pool)", 128, 128, 4, 61, False),
+    ("RGB 256^2 B=8 wk=61 (full pool)", 256, 256, 8, 61, True),
+    ("grey 512^2 B=8 wk=125 (full pool)", 512, 512, 8, 125, False),
+    ("grey 64^2 B=8 wk=13 (full pool, fused)", 64, 64, 8, 13, False),
 ]
 
 
@@ -146,10 +156,22 @@ def run_config(h, name, W, H, B, wk, rgb, sizes, reps, seed0):
             bad = {}
             for form, fb, fl in (("argb", enc_batch, enc_loop), ("u8", enc_batch_u8, enc_loop_u8)):
                 r[f"encode_{form}_batch_dev_ms"], r[f"encode_{form}_batch_host_ms"] = timed(h, fb, reps)
+                if form == "argb":
+                    r["encode_batch_engine"] = h.timings().engine
                 r[f"encode_{form}_loop_dev_ms"], r[f"encode_{form}_loop_host_ms"] = timed(h, fl, reps)
                 nan_b, nan_l = np.isnan(info), np.isnan(info1)
                 bad[f"encode_{form}"] = int(((bits(info) != bits(info1)) & ~(nan_b & nan_l)).any(axis=(1, 2)).sum()
                                             + (q != q1).any(axis=(1, 2)).sum())
+            if wk == 2 * (W // B) - 3 and wk == 2 * (H // B) - 3:
+                for eng, label in ((fic.FIC_ENGINE_UMMA, "umma"), (fic.FIC_ENGINE_DIRECT, "direct")):
+                    h.set_engine(eng)
+                    try:
+                        r[f"encode_u8_batch_{label}_dev_ms"], r[f"encode_u8_batch_{label}_host_ms"] = timed(h, enc_batch_u8, reps)
+                    finally:
+                        h.set_engine(fic.FIC_ENGINE_AUTO)
+                    nan_b, nan_l = np.isnan(info), np.isnan(info1)
+                    bad[f"encode_u8_{label}"] = int(((bits(info) != bits(info1)) & ~(nan_b & nan_l)).any(axis=(1, 2)).sum()
+                                                    + (q != q1).any(axis=(1, 2)).sum())
             for form, fb, fl, ob, ol in (("argb", dec_batch, dec_loop, img, img1), ("u8", dec_batch_u8, dec_loop_u8, pl, pl1)):
                 r[f"decode_{form}_batch_dev_ms"], r[f"decode_{form}_batch_host_ms"] = timed(h, fb, reps)
                 r[f"decode_{form}_loop_dev_ms"], r[f"decode_{form}_loop_host_ms"] = timed(h, fl, reps)
@@ -168,6 +190,8 @@ def run_config(h, name, W, H, B, wk, rgb, sizes, reps, seed0):
                   f"  | dec batch {r['decode_argb_batch_dev_us_per_image']:7.2f} / {r['decode_argb_batch_host_us_per_image']:7.2f}"
                   f"  loop {r['decode_argb_loop_dev_us_per_image']:7.2f} / {r['decode_argb_loop_host_us_per_image']:7.2f}"
                   f"  | u8 enc {r['encode_u8_batch_dev_us_per_image']:7.2f} / {r['encode_u8_loop_dev_us_per_image']:7.2f}"
+                  + (f" (umma {r['encode_u8_batch_umma_dev_us_per_image']:7.2f} direct {r['encode_u8_batch_direct_dev_us_per_image']:7.2f})"
+                     if "encode_u8_batch_umma_dev_ms" in r else "") +
                   f"  dec {r['decode_u8_batch_dev_us_per_image']:7.2f} / {r['decode_u8_loop_dev_us_per_image']:7.2f}"
                   f"  mismatches {sum(bad.values())}", flush=True)
         finally:
