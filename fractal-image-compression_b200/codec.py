@@ -302,6 +302,33 @@ class Handle:
                                                   C.c_void_p(d_planes_out), C.byref(avg), C.byref(it)))
         return np.float32(avg.value), it.value
 
+    def encode_quadtree(self, plane: np.ndarray, b_max: int, b_min: int, wk: int, max_mse: float) -> bytes:
+        """fic_encode_quadtree (FIC_MODE_GREY_QT extension): the grey plane (uint8 [H, W]) on a quadtree of block sizes
+        b_max .. b_min, split where a block's collage error exceeds max_mse per pixel; wk == 0: every level's whole
+        pool.  Returns the stream."""
+        a = np.ascontiguousarray(plane, dtype=np.uint8)
+        H, W = a.shape
+        cap = self._L.fic_quadtree_stream_bound(W, H, b_max, b_min)
+        buf = np.empty(max(cap, 1), np.uint8)
+        n = C.c_size_t(0)
+        self._check(self._L.fic_encode_quadtree(self._h, _ptr(a), W, H, b_max, b_min, wk, float(max_mse), _ptr(buf), cap,
+                                                C.byref(n)))
+        return buf[:n.value].tobytes()
+
+    def decode_quadtree(self, stream: bytes, max_iters: int = 50, out: np.ndarray | None = None):
+        """fic_decode_quadtree: returns (plane uint8 [H, W], avgError float32, iterations)."""
+        W, H = struct.unpack(">2i", stream[4:12]) if len(stream) >= 32 else (0, 0)
+        if not (0 < W <= 32768 and 0 < H <= 32768):
+            W = H = 0  # the library rejects the stream
+        if out is None:
+            out = np.empty((H, W), np.uint8)
+        assert out.dtype == np.uint8 and out.shape == (H, W) and out.flags["C_CONTIGUOUS"]
+        buf = np.frombuffer(stream, np.uint8)
+        avg = C.c_float(0.0)
+        it = C.c_int(0)
+        self._check(self._L.fic_decode_quadtree(self._h, _ptr(buf), len(buf), max_iters, _ptr(out), C.byref(avg), C.byref(it)))
+        return out, np.float32(avg.value), it.value
+
     def collage(self, argb: np.ndarray, info: np.ndarray, B: int, wk: int, rgb: bool):
         """fic_collage; `info` is rewritten in place (window-local -> codebook index, FC:273)."""
         a = np.ascontiguousarray(argb, dtype=np.int32)
@@ -455,6 +482,18 @@ def stream_read(stream: bytes):
     if rc:
         raise FicError(rc, "malformed .run stream")
     return (rgb if rgb == _lib.FIC_MODE_GREY_ISO else bool(rgb)), W, H, B, wk, q
+
+
+def quadtree_stream_info(stream: bytes):
+    """fic_quadtree_stream_info: (W, H, b_max, b_min, wk, n_leaves) of a checked quadtree stream."""
+    L = _lib.load()
+    buf = np.frombuffer(stream, np.uint8)
+    v = [C.c_int() for _ in range(5)]
+    n = C.c_int64()
+    rc = L.fic_quadtree_stream_info(_ptr(buf), len(buf), *[C.byref(x) for x in v], C.byref(n))
+    if rc:
+        raise FicError(rc, "malformed quadtree stream")
+    return tuple(x.value for x in v) + (n.value,)
 
 
 class FractalCompression:

@@ -8,6 +8,7 @@
 #include <string.h>
 
 #include <new>
+#include <vector>
 
 #include "fic_device.cuh"
 
@@ -95,7 +96,8 @@ struct DrainOnExit {
     ~DrainOnExit() { cudaStreamSynchronize(s); }
 };
 
-enum Slot { S_ARGB, S_SRC, S_DEC, S_DSUM, S_DSQ, S_RSUM, S_BEST, S_INFO, S_Q, S_OPA, S_OPB, S_IMG, S_DEC2, S_DCODE, S_PERR, S_STATE, S_DEC3, S_REPLAY };
+enum Slot { S_ARGB, S_SRC, S_DEC, S_DSUM, S_DSQ, S_RSUM, S_BEST, S_INFO, S_Q, S_OPA, S_OPB, S_IMG, S_DEC2, S_DCODE, S_PERR, S_STATE, S_DEC3, S_REPLAY, S_QT_STREAM, S_QT_CODES,
+            S_QT_ERR, S_QT_LEAF, S_QT_MAP };
 
 template <typename T>
 static int ensure(fic_handle *h, T *&p, int slot, size_t bytes)
@@ -188,7 +190,8 @@ void fic_destroy(fic_handle *h)
     cudaStreamSynchronize(h->stream);
     Work &w = h->w;
     void *ptrs[] = {w.argb, w.src, w.dec, w.dsum, w.dsq, w.rsum, w.best, w.info, w.q, w.opA, w.opB,
-                    w.img, w.dec2, w.dcode, w.perr, w.state, w.dec3, w.replay};
+                    w.img, w.dec2, w.dcode, w.perr, w.state, w.dec3, w.replay, w.qt_stream, w.qt_codes, w.qt_err,
+                    w.qt_leaf, w.qt_map};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (int i = 0; i < 8; i++)
@@ -1306,6 +1309,130 @@ int fic_stream_read_codes(const uint8_t *stream, size_t nbytes, int32_t *qcodes)
     size_t n = (fic_stream_size(rgb, W, H, B) - 20) / 4;
     for (size_t i = 0; i < n; i++) qcodes[i] = get_be32(stream + off + 4 * i);
     return FIC_OK;
+}
+
+// ---- quadtree extension (FIC_MODE_GREY_QT) ---------------------------------------------------------------------------
+
+size_t fic_quadtree_stream_bound(int W, int H, int b_max, int b_min)
+{
+    if (b_max <= 0 || b_min <= 0 || W <= 0 || H <= 0) return 0;
+    const size_t top = (size_t)(W / b_max) * (size_t)(H / b_max);
+    return kQtHeaderBytes + ((top + 3) & ~(size_t)3) + 12 * (size_t)(W / b_min) * (size_t)(H / b_min);
+}
+
+// One upload, then every level's ordinary grey encode (the engine fic_encode_grey_u8 would pick, into that level's code
+// table), one decimation of the source for the collage errors, and the stream body built on the device
+// (launch_qt_stream); the body comes down in one copy once the leaf count is known.
+int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b_max, int b_min, int wk, double max_mse,
+                        uint8_t *stream, size_t capacity, size_t *stream_bytes)
+{
+    if (!h) return FIC_E_ARG;
+    if (!plane || !stream_bytes) return set_err(h, FIC_E_ARG, "plane and stream_bytes must be non-NULL");
+    if (max_mse != max_mse) return set_err(h, FIC_E_ARG, "max_mse is NaN");
+    QtGeom q;
+    const char *why = "";
+    int rc = qt_geom(W, H, b_max, b_min, wk, &q, &why);
+    if (rc) return set_err(h, rc, "%s", why);
+    CU(cudaSetDevice(h->device));
+    memset(&h->tm, 0, sizeof h->tm);
+    Work &w = h->w;
+    cudaStream_t s = h->stream;
+    const Geom &fine = q.g[q.nl - 1];
+    ENSURE(w.src, S_SRC, (size_t)W * H);
+    ENSURE(w.dec, S_DEC, (size_t)fine.sw * fine.sh);
+    ENSURE(w.info, S_INFO, sizeof(float) * 3 * fine.NR);
+    ENSURE(w.qt_codes, S_QT_CODES, sizeof(int32_t) * 3 * q.codes);
+    ENSURE(w.qt_err, S_QT_ERR, sizeof(uint32_t) * qt_err_words(q));
+    ENSURE(w.qt_stream, S_QT_STREAM, fic_quadtree_stream_bound(W, H, b_max, b_min) - kQtHeaderBytes);
+    DrainOnExit drain(s);
+    CU(cudaEventRecord(h->ev[0], s));
+    CU(cudaMemcpyAsync(w.src, plane, (size_t)W * H, cudaMemcpyHostToDevice, s));
+    fic_timings acc = {};
+    for (int L = 0; L < q.nl; L++) {
+        const Geom &g = q.g[L];
+        int engine;
+        if ((rc = pick_engine(h, g, 0, g.NR, &engine))) return rc;
+        h->tm.launches = 0;
+        if ((rc = encode_on_device(h, g, w.src, 0, g.NR, w.info, w.qt_codes + 3 * q.first[L], engine))) return rc;
+        CU(cudaEventSynchronize(h->ev[4]));
+        float ms = 0;
+        if (h->tm.engine == FIC_ENGINE_FUSED) {  // one kernel between events 1 and 4
+            if (cudaEventElapsedTime(&ms, h->ev[1], h->ev[4]) == cudaSuccess) { acc.search_ms += ms; acc.kernel_ms += ms; }
+        } else {
+            add_stage_times(h, &acc);
+        }
+        acc.launches += h->tm.launches;
+        acc.search_evals += h->tm.search_evals;
+        acc.engine = h->tm.engine;
+    }
+    acc.launches += launch_decimate(w.src, w.dec, fine, s);  // the fused engine leaves no decimated plane behind
+    acc.launches += launch_qt_stream(w, q, max_mse, s);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(h->h_acc, w.qt_err, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    const int64_t leaves = *(const uint32_t *)h->h_acc;
+    const size_t need = kQtHeaderBytes + (size_t)q.flag_bytes + 12 * (size_t)leaves;
+    *stream_bytes = need;
+    if (!stream || capacity < need) return set_err(h, FIC_E_ARG, "the stream needs %zu bytes, capacity is %zu", need, capacity);
+    const int32_t hd[8] = {FIC_MODE_GREY_QT, W, H, 0, wk, b_max, b_min, (int32_t)leaves};
+    for (int k = 0; k < 8; k++) put_be32(stream + 4 * k, hd[k]);
+    CU(cudaMemcpyAsync(stream + kQtHeaderBytes, w.qt_stream, need - kQtHeaderBytes, cudaMemcpyDeviceToHost, s));
+    CU(cudaEventRecord(h->ev[5], s));
+    CU(cudaStreamSynchronize(s));
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[5]) == cudaSuccess) acc.total_ms = ms;
+    h->tm = acc;
+    return FIC_OK;
+}
+
+int fic_quadtree_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *H, int *b_max, int *b_min, int *wk,
+                             int64_t *n_leaves)
+{
+    QtGeom q;
+    const char *why = "";
+    int rc = qt_parse(stream, nbytes, &q, nullptr, true, &why);
+    if (rc) return rc;
+    if (W) *W = q.g[0].W;
+    if (H) *H = q.g[0].H;
+    if (b_max) *b_max = q.g[0].B;
+    if (b_min) *b_min = q.g[q.nl - 1].B;
+    if (wk) *wk = q.wk;
+    if (n_leaves) *n_leaves = q.leaves;
+    return FIC_OK;
+}
+
+int fic_decode_quadtree(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *plane_out,
+                        float *avg_error, int *iterations)
+{
+    if (!h) return FIC_E_ARG;
+    if (!stream || !plane_out) return set_err(h, FIC_E_ARG, "stream and plane_out must be non-NULL");
+    if (max_iters < 1) return set_err(h, FIC_E_ARG, "max_iters must be >= 1");
+    QtGeom q;
+    const char *why = "";
+    int rc = qt_parse(stream, nbytes, &q, nullptr, false, &why);
+    if (rc) return set_err(h, rc, "%s", why);
+    std::vector<int32_t> base((size_t)q.g[0].NR);  // first leaf of every top block (the first pass gave their count)
+    qt_parse(stream, nbytes, &q, base.data(), false, &why);
+    CU(cudaSetDevice(h->device));
+    memset(&h->tm, 0, sizeof h->tm);
+    Work &w = h->w;
+    cudaStream_t s = h->stream;
+    const Geom &g = q.g[0];
+    const size_t plane = (size_t)g.W * g.H, bmin = (size_t)q.g[q.nl - 1].B;
+    const size_t cells = plane / (bmin * bmin), used = kQtHeaderBytes + (size_t)q.flag_bytes + 12 * (size_t)q.leaves;
+    ENSURE(w.img, S_IMG, plane);
+    ENSURE(w.dec, S_DEC, (size_t)g.sw * g.sh);
+    ENSURE(w.dec2, S_DEC2, (size_t)g.sw * g.sh);
+    ENSURE(w.state, S_STATE, sizeof(DecodeState));
+    ENSURE(w.qt_stream, S_QT_STREAM, used - kQtHeaderBytes);
+    ENSURE(w.qt_leaf, S_QT_LEAF, sizeof(int4) * q.leaves);
+    ENSURE(w.qt_map, S_QT_MAP, sizeof(int32_t) * (cells + base.size()));
+    DrainOnExit drain(s);
+    CU(cudaEventRecord(h->ev[0], s));
+    CU(cudaMemcpyAsync(w.qt_stream, stream + kQtHeaderBytes, used - kQtHeaderBytes, cudaMemcpyHostToDevice, s));
+    CU(cudaMemcpyAsync(w.qt_map + cells, base.data(), sizeof(int32_t) * base.size(), cudaMemcpyHostToDevice, s));
+    const DecodeStatus st = decode_quadtree_run(w, q, max_iters, plane_out, avg_error, iterations, h->h_acc, h->ev[0], h->ev[5], &h->tm, s);
+    return decode_err(h, st, "a leaf indexes outside its level's domain pool");
 }
 
 }  // extern "C"

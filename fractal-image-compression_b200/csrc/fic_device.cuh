@@ -6,6 +6,7 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 
 #include "fic_internal.h"
@@ -49,6 +50,74 @@ __host__ __device__ inline void range_window(const Geom &g, int64_t j, int *dy, 
     window_origin(i, g.dpw, g.dph, g.wk, dy, dx);
 }
 
+// Java (int)float: truncate toward zero, saturate, NaN -> 0 (== cvt.rzi.s32.f32 on the device).
+__host__ __device__ __forceinline__ int j_f2i(float f)
+{
+#ifdef __CUDA_ARCH__
+    return __float2int_rz(f);
+#else
+    if (f != f) return 0;
+    if (f >= 2147483648.0f) return INT32_MAX;
+    if (f <= -2147483648.0f) return INT32_MIN;
+    return (int)f;
+#endif
+}
+
+// FC:853-893 calculateIndices for range block j: the window-local index c of its code -> codebook index, with Java's
+// float division and float remainder (FC:882-886); -1 when it falls outside the pool (the reference would throw).
+__host__ __device__ inline int64_t code_pool_index(const Geom &g, int64_t j, float c)
+{
+    int dy, dx;
+    range_window(g, j, &dy, &dx);
+    const float fwk = (float)g.wk;
+    const int yd = j_f2i(c / fwk), xd = j_f2i(fmodf(c, fwk));
+    const int64_t r = (int64_t)xd + dx + (int64_t)(yd + dy) * g.dpw;
+    return r < 0 || r >= g.ND ? -1 : r;
+}
+
+// ---- quadtree extension: the tree of one top block ----
+// Range index at level L + 1 of child k (0 TL, 1 TR, 2 BL, 3 BR) of range j at level L.
+__host__ __device__ inline int64_t qt_child(const QtGeom &q, int L, int64_t j, int k)
+{
+    const int64_t y = 2 * (j / q.g[L].rpw) + (k >> 1), x = 2 * (j % q.g[L].rpw) + (k & 1);
+    return y * q.g[L + 1].rpw + x;
+}
+
+// A flag byte may set bit 0 (the top block is split) when there is a level below, and bit 1 + k (child k is split)
+// only when bit 0 is set and there are two levels below.
+__host__ __device__ inline bool qt_flags_legal(const QtGeom &q, uint32_t f)
+{
+    const uint32_t allowed = q.nl == 1 ? 0u : (q.nl == 2 || !(f & 1u) ? 1u : 0x1fu);
+    return (f & ~allowed) == 0;
+}
+
+__host__ __device__ inline int qt_leaf_count(uint32_t f)
+{
+    if (!(f & 1u)) return 1;
+    int n = 0;
+    for (int k = 0; k < 4; k++) n += (f >> (1 + k)) & 1u ? 4 : 1;
+    return n;
+}
+
+// Calls visit(level, range index) for every leaf of top block t in stream order: depth first, children in raster order.
+#pragma nv_exec_check_disable
+template <class V>
+__host__ __device__ inline void qt_visit_leaves(const QtGeom &q, int64_t t, uint32_t f, V &&visit)
+{
+    if (!(f & 1u)) {
+        visit(0, t);
+        return;
+    }
+    for (int k = 0; k < 4; k++) {
+        const int64_t c = qt_child(q, 0, t, k);
+        if (!((f >> (1 + k)) & 1u)) {
+            visit(1, c);
+            continue;
+        }
+        for (int k2 = 0; k2 < 4; k2++) visit(2, qt_child(q, 1, c, k2));
+    }
+}
+
 // Isometry extension (not in the reference): T_k maps range pixel (ry, rx) of a B x B block to the domain
 // pixel (sy, sx) it is compared with / reconstructed from.  0 identity, 1-3 rotations, 4 mirror x, 5 mirror y,
 // 6 transpose, 7 anti-transpose.
@@ -70,9 +139,6 @@ __host__ __device__ inline void iso_map(int k, int B, int ry, int rx, int *sy, i
 __host__ __device__ inline int iso_inverse(int k) { return k == 1 ? 3 : (k == 3 ? 1 : k); }
 
 #ifdef __CUDACC__
-
-// Java (int)float: truncate toward zero, saturate, NaN -> 0 == cvt.rzi.s32.f32.
-__device__ __forceinline__ int j_f2i(float f) { return __float2int_rz(f); }
 
 // FC:72 getMittelwert: the integer mean of a block from its pixel sum, mean = sum / n.  Returns
 // sum (x - mean) = sum - n * mean (FC:671, FC:790), the exact integer in [0, n) that the reference's scores divide by.
@@ -154,6 +220,16 @@ __device__ __forceinline__ int dec_tap4(int p00, int p10, int p01, int p11, int 
 {
     int fourth = (x + 1 >= H) ? 128 : (rgb ? p01 : p11);
     return (p00 + p10 + p01 + fourth) / 4;
+}
+
+// A reconstructed pixel, (int)(a * domain + b) -- float multiply, then float add (FC:396 / FC:482) -- clamped to
+// [0, 255] (FC:396-402, FC:743-749).  cvt.rzi.u8.f32 does the cast and the clamp in one instruction: it truncates
+// toward zero and saturates to the destination range, NaN -> 0, like Java's cast followed by applyThreshold.
+__device__ __forceinline__ uint32_t decode_px(float a, float b, uint32_t domain)
+{
+    uint32_t r;
+    asm("cvt.rzi.u8.f32 %0, %1;" : "=r"(r) : "f"(__fadd_rn(__fmul_rn(a, (float)domain), b)));
+    return r;
 }
 
 // Quantisation scales of the code stream: written by FC:242-244 / FC:250-254, read back by FC:372-374 / FC:446-450.

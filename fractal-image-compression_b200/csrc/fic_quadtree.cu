@@ -1,0 +1,183 @@
+// fic_quadtree.cu -- the quadtree extension (FIC_MODE_GREY_QT, not in the reference): the stream's geometry and parser,
+// and the kernels that turn every level's codes into the stream body on the device -- the collage error of each range
+// block, the split flags of each top block, the leaf scan and the big-endian leaf scatter.  The per-level encodes are
+// the library's ordinary grey encodes (fic_api.cu); the decoder sweep lives with the other sweeps in fic_decode.cu.
+#include <string.h>
+
+#include "fic_device.cuh"
+
+namespace fic {
+
+// ---- host: geometry and parser -----------------------------------------------------------------------------------------
+
+int qt_geom(int W, int H, int b_max, int b_min, int wk, QtGeom *q, const char **why)
+{
+    if (!(b_max == 8 || b_max == 16)) { *why = "b_max must be 8 or 16"; return FIC_E_ARG; }
+    if (!(b_min == 4 || b_min == 8 || b_min == 16) || b_min > b_max) { *why = "b_min must be 4, 8 or 16 and at most b_max"; return FIC_E_ARG; }
+    if (W <= 0 || H <= 0 || W % b_max || H % b_max) { *why = "width and height must be positive multiples of b_max"; return FIC_E_ARG; }
+    if (wk < 0 || (wk == 0 && W != H)) { *why = "widthKernel must be >= 1, or 0 (every level's whole pool) on a square image"; return FIC_E_ARG; }
+    memset(q, 0, sizeof *q);
+    q->wk = wk;
+    for (int B = b_max; B >= b_min; B /= 2) {
+        const int L = q->nl++;
+        const int wk_l = wk ? wk : 2 * (W / B) - 3;  // the whole pool: domain blocks per width (== per height)
+        const int rc = make_geom(W, H, B, wk_l, FIC_MODE_GREY, &q->g[L], why);
+        if (rc) return rc;
+        q->first[L] = q->codes;
+        q->codes += q->g[L].NR;
+    }
+    q->flag_bytes = (q->g[0].NR + 3) & ~(int64_t)3;
+    return FIC_OK;
+}
+
+static int32_t be32(const uint8_t *p)
+{
+    return (int32_t)(((uint32_t)p[0] << 24) | ((uint32_t)p[1] << 16) | ((uint32_t)p[2] << 8) | (uint32_t)p[3]);
+}
+
+int qt_parse(const uint8_t *s, size_t nbytes, QtGeom *q, int32_t *base, bool check_leaves, const char **why)
+{
+    if (!s || nbytes < kQtHeaderBytes) { *why = "stream shorter than its 32-byte header"; return FIC_E_STREAM; }
+    int32_t hd[8];
+    for (int k = 0; k < 8; k++) hd[k] = be32(s + 4 * k);
+    if (hd[0] != FIC_MODE_GREY_QT || hd[3] != 0) { *why = "not a quadtree stream (header 3, W, H, 0, ...)"; return FIC_E_STREAM; }
+    if (qt_geom(hd[1], hd[2], hd[5], hd[6], hd[4], q, why)) return FIC_E_STREAM;
+    const int64_t ntop = q->g[0].NR;
+    if ((uint64_t)(nbytes - kQtHeaderBytes) < (uint64_t)q->flag_bytes) { *why = "stream truncated inside its split flags"; return FIC_E_STREAM; }
+    const uint8_t *flags = s + kQtHeaderBytes;
+    int64_t leaves = 0;
+    for (int64_t t = 0; t < ntop; t++) {
+        if (!qt_flags_legal(*q, flags[t])) { *why = "a split flag is set where no split is possible"; return FIC_E_STREAM; }
+        if (base) base[t] = (int32_t)leaves;
+        leaves += qt_leaf_count(flags[t]);
+    }
+    if (hd[7] != leaves) { *why = "n_leaves disagrees with the split flags"; return FIC_E_STREAM; }
+    q->leaves = leaves;
+    if ((uint64_t)(nbytes - kQtHeaderBytes - q->flag_bytes) / 12 < (uint64_t)leaves) { *why = "stream truncated inside its leaves"; return FIC_E_STREAM; }
+    if (check_leaves) {
+        const uint8_t *p = flags + q->flag_bytes;
+        bool ok = true;
+        for (int64_t t = 0; t < ntop && ok; t++)
+            qt_visit_leaves(*q, t, flags[t], [&](int L, int64_t j) {
+                ok = ok && code_pool_index(q->g[L], j, (float)be32(p)) >= 0;
+                p += 12;
+            });
+        if (!ok) { *why = "a leaf indexes outside its level's domain pool"; return FIC_E_STREAM; }
+    }
+    return FIC_OK;
+}
+
+// ---- device: collage error, split flags, leaf scatter --------------------------------------------------------------------
+
+// qt_err layout: [0] leaf total, then the per-top-block in-warp prefixes (flag_bytes words), the per-warp totals, then the
+// collage errors of every level (level-major, QtGeom::first).
+static int64_t qt_warps(const QtGeom &q) { return (q.flag_bytes + 31) / 32; }
+static int64_t qt_err_at(const QtGeom &q) { return 1 + q.flag_bytes + qt_warps(q); }
+size_t qt_err_words(const QtGeom &q) { return (size_t)(qt_err_at(q) + q.codes); }
+
+// E(j) = sum over range block j of (decode_px(a, b, d) - s)^2: the code dequantised as the decoder does (FC:372-374), the
+// domain pixels d read from the source's decimated plane at the code's codebook index (FC:853-893).  B threads per range
+// block, one row each (B divides 32: a block's rows share a warp and reduce with shuffles).
+__global__ void __launch_bounds__(256) k_qt_collage_sse(const uint8_t *__restrict__ src, const uint8_t *__restrict__ dec,
+                                                        const int32_t *__restrict__ q, uint32_t *__restrict__ err, Geom g)
+{
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int B = g.B;
+    const int64_t j = t / B;
+    const int ry = (int)(t - j * B);
+    uint32_t e = 0;
+    if (j < g.NR) {
+        const int32_t *c = q + 3 * j;
+        const float a = __fdiv_rn((float)c[1], kGreyAScale), b = (float)c[2];
+        int64_t idx = code_pool_index(g, j, (float)c[0]);
+        if (idx < 0) idx = 0;  // an encoder's code is always inside the pool
+        const int x = (int)(j % g.rpw) * B, y = (int)(j / g.rpw) * B;
+        const uint8_t *d = dec + (int64_t)((int)(idx / g.dpw) * g.step + ry) * g.sw + (int)(idx % g.dpw) * g.step;
+        const uint8_t *s = src + (int64_t)(y + ry) * g.W + x;
+        for (int rx = 0; rx < B; rx++) {
+            const int v = (int)decode_px(a, b, d[rx]) - (int)s[rx];
+            e += (uint32_t)(v * v);
+        }
+    }
+    for (int o = B / 2; o > 0; o >>= 1) e += __shfl_down_sync(0xffffffffu, e, o, B);
+    if (j < g.NR && ry == 0) err[j] = e;
+}
+
+struct QtSplit {
+    QtGeom q;
+    const uint32_t *err;  // level-major collage errors
+    double max_mse;
+};
+
+// A block above b_min is split iff (double)E > max_mse * (double)(B * B).
+__device__ __forceinline__ bool qt_split(const QtSplit &p, int L, int64_t j)
+{
+    return L < p.q.nl - 1 && (double)p.err[p.q.first[L] + j] > __dmul_rn(p.max_mse, (double)p.q.g[L].n);
+}
+
+// One thread per top block (and per padding byte of the flags): its flag byte into the stream, its leaf count's
+// exclusive prefix within the warp to pre[t], the warp's total to wsum[warp].
+__global__ void __launch_bounds__(256) k_qt_decide(QtSplit p, uint8_t *__restrict__ flags, uint32_t *__restrict__ pre,
+                                                   uint32_t *__restrict__ wsum)
+{
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    uint32_t f = 0, n = 0;
+    if (t < p.q.g[0].NR) {
+        if (qt_split(p, 0, t)) {
+            f = 1;
+            for (int k = 0; k < 4; k++)
+                if (qt_split(p, 1, qt_child(p.q, 0, t, k))) f |= 2u << k;
+        }
+        n = (uint32_t)qt_leaf_count(f);
+    }
+    uint32_t incl = n;
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += v;
+    }
+    if (t < p.q.flag_bytes) {
+        flags[t] = (uint8_t)f;
+        pre[t] = incl - n;
+        if (lane == 31 || t == p.q.flag_bytes - 1) wsum[t >> 5] = incl;
+    }
+}
+
+__device__ __forceinline__ uint32_t bswap32(int32_t v) { return __byte_perm((uint32_t)v, 0u, 0x0123); }
+
+// One thread per top block: its leaves' codes, big endian (DataOutputStream.writeInt), at their place in the stream.
+__global__ void __launch_bounds__(256) k_qt_scatter(QtGeom q, const int32_t *__restrict__ codes, const uint8_t *__restrict__ flags,
+                                                    const uint32_t *__restrict__ pre, const uint32_t *__restrict__ wsum,
+                                                    uint32_t *__restrict__ leaves)
+{
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= q.g[0].NR) return;
+    uint32_t *o = leaves + 3 * (int64_t)(wsum[t >> 5] + pre[t]);
+    qt_visit_leaves(q, t, flags[t], [&](int L, int64_t j) {
+        const int32_t *c = codes + 3 * (q.first[L] + j);
+        o[0] = bswap32(c[0]);
+        o[1] = bswap32(c[1]);
+        o[2] = bswap32(c[2]);
+        o += 3;
+    });
+}
+
+int launch_qt_stream(const Work &w, const QtGeom &q, double max_mse, cudaStream_t s)
+{
+    uint32_t *total = w.qt_err, *pre = w.qt_err + 1, *wsum = pre + q.flag_bytes, *err = w.qt_err + qt_err_at(q);
+    int launches = 0;
+    for (int L = 0; L < q.nl; L++) {
+        const Geom &g = q.g[L];
+        const int64_t threads = g.NR * g.B;
+        k_qt_collage_sse<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(w.src, w.dec, w.qt_codes + 3 * q.first[L], err + q.first[L], g);
+        launches++;
+    }
+    const QtSplit p = {q, err, max_mse};
+    k_qt_decide<<<(unsigned)((q.flag_bytes + 255) / 256), 256, 0, s>>>(p, w.qt_stream, pre, wsum);
+    launches += 1 + launch_scan_u32(wsum, qt_warps(q), total, s);
+    k_qt_scatter<<<(unsigned)((q.g[0].NR + 255) / 256), 256, 0, s>>>(q, w.qt_codes, w.qt_stream, pre, wsum,
+                                                                       (uint32_t *)(w.qt_stream + q.flag_bytes));
+    return launches + 1;
+}
+
+}  // namespace fic

@@ -2645,6 +2645,12 @@ int umma_f16_selftest(int num_sms, cudaStream_t s, const char **err)
     return result;
 }
 
+int launch_scan_u32(uint32_t *d, int64_t n, uint32_t *total, cudaStream_t s)
+{
+    k_sort_scan_rows<<<1, 256, 0, s>>>(d, n, total);
+    return 1;
+}
+
 // Probe / test entry of the in-tree radix sort: sorts n device pairs by the low 24 key bits (stable); the result is
 // written to (d_keys_out, d_vals_out).  Allocates its own histogram scratch.  0 or a CUDA error code.
 int umma_debug_sort(uint32_t *d_keys, int32_t *d_vals, uint32_t *d_keys_out, int32_t *d_vals_out, int64_t n, cudaStream_t s)

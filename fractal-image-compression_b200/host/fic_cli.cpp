@@ -3,6 +3,9 @@
 //   fic_cli encode in.pgm|in.ppm out.run [blockgroesse] [widthKernel]   (binary P5 / P6)
 //   fic_cli decode in.run out.pgm|out.ppm
 //   fic_cli roundtrip in.pgm|in.ppm [blockgroesse] [widthKernel]        (prints "MSE <avgError>" like the GUI label)
+//   fic_cli qtroundtrip in.pgm b_max b_min widthKernel max_mse            (quadtree extension, grey: stream size, bits
+//                                                                          per pixel, iterations, avgError, PSNR)
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -77,7 +80,34 @@ int main(int argc, char **argv)
             printf("MSE %.9g (%d iterations)\n", FractalCompression::getAvgError(), FractalCompression::lastIterations);
             return 0;
         }
-        fprintf(stderr, "usage: fic_cli encode in.pnm out.run [B] [wk] [iso] | decode in.run out.pnm | roundtrip in.pnm [B] [wk] [iso]\n");
+        if (argc >= 7 && !strcmp(argv[1], "qtroundtrip")) {
+            const RasterImage img = read_pnm(argv[2]);
+            const int W = img.width, H = img.height, b_max = atoi(argv[3]), b_min = atoi(argv[4]), wk = atoi(argv[5]);
+            std::vector<uint8_t> plane((size_t)W * H), out((size_t)W * H);
+            for (size_t i = 0; i < plane.size(); i++) plane[i] = (uint8_t)((img.argb[i] >> 16) & 0xff);  // the red channel
+            std::vector<uint8_t> stream(fic_quadtree_stream_bound(W, H, b_max, b_min) + 1);
+            fic_handle *h = nullptr;
+            size_t n = 0;
+            float avg = 0;
+            int iters = 0;
+            int rc = fic_create(0, &h);
+            if (!rc) rc = fic_encode_quadtree(h, plane.data(), W, H, b_max, b_min, wk, atof(argv[6]), stream.data(), stream.size(), &n);
+            if (!rc) rc = fic_decode_quadtree(h, stream.data(), n, 50, out.data(), &avg, &iters);
+            if (rc) {
+                fprintf(stderr, "fic_cli: error %d: %s\n", rc, fic_last_error(h));
+                fic_destroy(h);
+                return 1;
+            }
+            fic_destroy(h);
+            double se = 0;
+            for (size_t i = 0; i < plane.size(); i++) se += ((double)plane[i] - out[i]) * ((double)plane[i] - out[i]);
+            const double mse = se / (double)plane.size();
+            printf("bytes %zu bpp %.4f iterations %d MSE %.9g PSNR %.3f dB\n", n, 8.0 * n / plane.size(), iters, avg,
+                   mse > 0 ? 10.0 * std::log10(255.0 * 255.0 / mse) : INFINITY);
+            return 0;
+        }
+        fprintf(stderr, "usage: fic_cli encode in.pnm out.run [B] [wk] [iso] | decode in.run out.pnm | roundtrip in.pnm [B] [wk] [iso]"
+                        " | qtroundtrip in.pgm b_max b_min wk max_mse\n");
         return 2;
     } catch (const std::exception &e) {
         fprintf(stderr, "fic_cli: %s\n", e.what());

@@ -56,6 +56,7 @@ extern "C" {
 #define FIC_MODE_GREY 0     /* {c, a, b} per range                       */
 #define FIC_MODE_RGB 1      /* {c, a, bR, bG, bB} per range              */
 #define FIC_MODE_GREY_ISO 2 /* {c, a, b, k} per range; k = isometry 0..7 */
+#define FIC_MODE_GREY_QT 3  /* quadtree of block sizes (EXTENSION, grey only): see fic_encode_quadtree below */
 
 /* Search engine selection (fic_set_option(FIC_OPT_ENGINE, ...)). */
 #define FIC_ENGINE_AUTO 0   /* tcgen05 search when the window is the whole pool; the fused one-launch encode for the
@@ -232,6 +233,43 @@ int fic_decode_batch_u8(fic_handle *h, int mode, int n_images, int W, int H, int
  * window-local to codebook index (FC:273). */
 int fic_collage(fic_handle *h, int is_rgb, const int32_t *argb, int W, int H, int B, int wk,
                 float *info, int32_t *argb_out);
+
+/* ---- quadtree extension (FIC_MODE_GREY_QT): block sizes chosen per region by collage error ---------------------- */
+
+/* EXTENSION the reference cannot read.  Levels b_max, b_max/2, ..., b_min (b_max in {8, 16}, b_min in {4, 8, 16},
+ * b_min <= b_max); level L's codes are exactly what fic_encode_grey_u8(plane, W, H, B_L, wk_L) returns on this handle
+ * with its options, wk_L = wk, or (wk == 0, square images only) that level's whole domain pool.  The collage error of
+ * range block j at level L is E = sum (decode_px(a, b, d) - s)^2 over its B_L^2 source pixels s, with the code dequantised
+ * as the decoder does (a = qa / 100f, b = qb), d the source's decimated plane at the code's domain block, and decode_px the
+ * decoder's float multiply, float add, truncation and clamp.  A block above b_min is split into its four children iff
+ * (double)E > max_mse * (double)(B_L^2): +inf never splits, a negative value always does; NaN is rejected.
+ *
+ * Stream, big-endian int32 like writeData: header 3, W, H, 0, wk, b_max, b_min, n_leaves (the 0 sits where the reference
+ * reads blockgroesse, so that neither it nor fic_stream_read_header can take the stream for an RGB one); one split-flag
+ * byte per top-level (b_max) block in raster order, padded with zeros to a multiple of 4 (bit 0: the block is split; bit
+ * 1 + k: its child k is split, k = 0 TL, 1 TR, 2 BL, 3 BR); then 12 bytes per leaf, {c, qa, qb} as writeData writes that
+ * range's code at its level, top blocks in raster order, each subtree depth first with children in raster order.  Size:
+ * 32 + pad4(NR_top) + 12 * n_leaves <= fic_quadtree_stream_bound.
+ *
+ * Pixels in: a W*H 8-bit plane (the red channel of the grey image).  W and H must be multiples of b_max and every level
+ * must pass fic_geometry's checks (FIC_E_ARG).  If `capacity` is smaller than the stream, FIC_E_ARG with the size needed
+ * in *stream_bytes.  fic_get_timings: pool / search / kernel / solve times and search_evals summed over the levels,
+ * launches, total_ms of the whole call, and the finest level's engine. */
+size_t fic_quadtree_stream_bound(int W, int H, int b_max, int b_min);
+int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b_max, int b_min, int wk, double max_mse,
+                        uint8_t *stream, size_t capacity, size_t *stream_bytes);
+/* Parses and checks a quadtree stream (host only): FIC_E_STREAM when it is truncated, sets a split bit that cannot be
+ * meaningful, has an n_leaves that disagrees with its flags, or a leaf indexes outside its level's domain pool.  Any
+ * output may be NULL. */
+int fic_quadtree_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *H, int *b_max, int *b_min, int *wk,
+                             int64_t *n_leaves);
+/* Decodes a quadtree stream into a W*H plane: starts from the constant-128 image; each sweep decimates the last image and
+ * lets every leaf write decode_px(a, b, .) from its level's domain block; avgError = (float)S / (float)(W*H) of the exact
+ * sum S of squared pixel changes.  Stops when avgError < 1 or after max_iters sweeps; *avg_error and *iterations (either
+ * may be NULL) receive the last sweep's value and the sweep count.  No carry-in.  FIC_E_STREAM as
+ * fic_quadtree_stream_info. */
+int fic_decode_quadtree(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *plane_out,
+                        float *avg_error, int *iterations);
 
 /* ---- multi-GPU: the same encode over several GPUs of one node (SURVEY 8b, 8e) --- */
 
