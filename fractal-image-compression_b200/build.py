@@ -22,7 +22,7 @@ LIB = os.path.join(LIBDIR, "libfic_b200.so")
 PROBE = os.path.join(LIBDIR, "umma_probe")
 CLI = os.path.join(LIBDIR, "fic_cli")
 
-SOURCES = ["fic_kernels.cu", "fic_decode.cu", "fic_search_umma.cu", "fic_quadtree.cu", "fic_api.cu"]
+SOURCES = ["fic_kernels.cu", "fic_decode.cu", "fic_search_umma.cu", "fic_quadtree.cu", "fic_encode.cu", "fic_api.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

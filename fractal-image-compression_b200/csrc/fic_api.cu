@@ -48,19 +48,14 @@ int fic::make_geom(int W, int H, int B, int wk, int mode, Geom *g, const char **
 // ------------------------------------------------------------------------------------
 struct fic_handle {
     int device = 0;
-    int num_sms = 0;
     cudaStream_t own_stream = nullptr;
     cudaStream_t stream = nullptr;
-    cudaEvent_t ev[8] = {nullptr};
+    cudaEvent_t call_begin = nullptr, call_end = nullptr;  // bracket a whole call (total_ms of encodes and decodes)
     Work w;
-    int engine_opt = FIC_ENGINE_AUTO;
-    int umma_kind = FIC_UMMA_KIND_AUTO;
-    int umma_pair = FIC_UMMA_PAIR_AUTO;  // FIC_OPT_UMMA_PAIR
-    int pair_used = 0;                   // did the last tcgen05 search run the CTA-pair kernel
-    int f16_state = 0;  // kind::f16 self-test: 0 not run yet, 1 exact, -1 not exact on this device (use kind::i8)
+    Encoder enc;
     fic_timings tm;
     char err[512];
-    bool tm_pending_dev = false;
+    bool tm_pending_dev = false;  // fic_encode_planes_dev: tm's stage times are read once its run has completed
     // pinned scratch for small device->host reads
     unsigned long long *h_acc = nullptr;
     // pinned staging for small code tables: one device->host copy instead of two (info and qcodes are adjacent on the
@@ -96,38 +91,34 @@ struct DrainOnExit {
     ~DrainOnExit() { cudaStreamSynchronize(s); }
 };
 
-enum Slot { S_ARGB, S_SRC, S_DEC, S_DSUM, S_DSQ, S_RSUM, S_BEST, S_INFO, S_Q, S_OPA, S_OPB, S_IMG, S_DEC2, S_DCODE, S_PERR, S_STATE, S_DEC3, S_REPLAY, S_QT_STREAM, S_QT_CODES,
-            S_QT_ERR, S_QT_LEAF, S_QT_MAP };
-
-template <typename T>
-static int ensure(fic_handle *h, T *&p, int slot, size_t bytes)
+Status fic::fail(int rc, const char *fmt, ...)
 {
-    if (bytes == 0) bytes = 16;
-    if (h->w.cap[slot] >= bytes && p) return FIC_OK;
-    if (p) cudaFree(p);
-    p = nullptr;
-    h->w.cap[slot] = 0;
-    size_t want = (bytes + 255) & ~(size_t)255;
-    cudaError_t e = cudaMalloc((void **)&p, want);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return set_err(h, FIC_E_NOMEM, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
-    }
-    h->w.cap[slot] = want;
-    return FIC_OK;
+    Status st(rc);
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(st.msg, sizeof st.msg, fmt, ap);
+    va_end(ap);
+    return st;
 }
 
-#define ENSURE(ptr, slot, bytes)                       \
-    do {                                               \
-        int rc_ = ensure(h, ptr, slot, (size_t)(bytes)); \
-        if (rc_) return rc_;                           \
+// The handle's error for the Status of an encoder or decoder entry; out_of_pool: the message of a decoder's FIC_E_STREAM
+// (a code outside the domain pool), which the decoder leaves to its caller.
+static int status_err(fic_handle *h, const Status &st, const char *out_of_pool = "")
+{
+    return st.rc ? set_err(h, st.rc, "%s", st.msg[0] ? st.msg : out_of_pool) : FIC_OK;
+}
+
+#define ENSURE(ptr, slot, bytes)                                             \
+    do {                                                                     \
+        int rc_ = status_err(h, ensure(h->w, ptr, slot, (size_t)(bytes))); \
+        if (rc_) return rc_;                                                 \
     } while (0)
 
-// The error of a decoder entry (fic_decode.cu); out_of_pool: the message for a code outside the domain pool.
-static int decode_err(fic_handle *h, const DecodeStatus &st, const char *out_of_pool)
+// Every timed entry starts from zeroed timings; a pending read of fic_encode_planes_dev's stage times is dropped.
+static void reset_timings(fic_handle *h)
 {
-    if (st.rc == FIC_E_CUDA) return set_err(h, FIC_E_CUDA, "%s failed: %s (%s:%d)", st.call, cudaGetErrorString(st.cuda), st.file, st.line);
-    return st.rc ? set_err(h, st.rc, "%s", out_of_pool) : FIC_OK;
+    memset(&h->tm, 0, sizeof h->tm);
+    h->tm_pending_dev = false;
 }
 
 extern "C" {
@@ -164,14 +155,17 @@ int fic_create(int device, fic_handle **out)
         delete h;
         return FIC_E_CUDA;
     }
-    h->num_sms = prop.multiProcessorCount;
+    h->enc.num_sms = prop.multiProcessorCount;
     if ((e = cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking)) != cudaSuccess) {
         set_err(nullptr, FIC_E_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
         delete h;
         return FIC_E_CUDA;
     }
     h->stream = h->own_stream;
-    for (int i = 0; i < 8 && e == cudaSuccess; i++) e = cudaEventCreate(&h->ev[i]);
+    e = cudaEventCreate(&h->call_begin);
+    if (e == cudaSuccess) e = cudaEventCreate(&h->call_end);
+    for (cudaEvent_t &ev : h->enc.ev)
+        if (e == cudaSuccess) e = cudaEventCreate(&ev);
     if (e == cudaSuccess) e = cudaHostAlloc((void **)&h->h_acc, 64 * sizeof(unsigned long long), cudaHostAllocDefault);
     if (e == cudaSuccess) e = cudaHostAlloc((void **)&h->h_stage, kStageBytes, cudaHostAllocDefault);
     if (e != cudaSuccess) {
@@ -194,8 +188,10 @@ void fic_destroy(fic_handle *h)
                     w.qt_leaf, w.qt_map};
     for (void *p : ptrs)
         if (p) cudaFree(p);
-    for (int i = 0; i < 8; i++)
-        if (h->ev[i]) cudaEventDestroy(h->ev[i]);
+    for (cudaEvent_t ev : {h->call_begin, h->call_end})
+        if (ev) cudaEventDestroy(ev);
+    for (cudaEvent_t ev : h->enc.ev)
+        if (ev) cudaEventDestroy(ev);
     if (h->h_acc) cudaFreeHost(h->h_acc);
     if (h->h_stage) cudaFreeHost(h->h_stage);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
@@ -208,15 +204,15 @@ int fic_set_option(fic_handle *h, int option, int value)
 {
     if (!h) return FIC_E_ARG;
     if (option == FIC_OPT_ENGINE && value >= FIC_ENGINE_AUTO && value <= FIC_ENGINE_FUSED) {
-        h->engine_opt = value;
+        h->enc.engine_opt = value;
         return FIC_OK;
     }
     if (option == FIC_OPT_UMMA_KIND && value >= FIC_UMMA_KIND_AUTO && value <= FIC_UMMA_KIND_F16) {
-        h->umma_kind = value;
+        h->enc.umma_kind = value;
         return FIC_OK;
     }
     if (option == FIC_OPT_UMMA_PAIR && value >= FIC_UMMA_PAIR_AUTO && value <= FIC_UMMA_PAIR_ON) {
-        h->umma_pair = value;
+        h->enc.umma_pair = value;
         return FIC_OK;
     }
     return set_err(h, FIC_E_ARG, "unknown option %d / value %d", option, value);
@@ -225,19 +221,16 @@ int fic_set_option(fic_handle *h, int option, int value)
 int fic_get_option(fic_handle *h, int option, int *value)
 {
     if (!h || !value) return FIC_E_ARG;
-    if (option == FIC_OPT_ENGINE) { *value = h->engine_opt; return FIC_OK; }
-    if (option == FIC_OPT_UMMA_KIND) { *value = h->umma_kind; return FIC_OK; }
-    if (option == FIC_OPT_UMMA_PAIR) { *value = h->umma_pair; return FIC_OK; }
-    if (option == FIC_OPT_UMMA_PAIR_USED) { *value = h->pair_used; return FIC_OK; }
+    if (option == FIC_OPT_ENGINE) { *value = h->enc.engine_opt; return FIC_OK; }
+    if (option == FIC_OPT_UMMA_KIND) { *value = h->enc.umma_kind; return FIC_OK; }
+    if (option == FIC_OPT_UMMA_PAIR) { *value = h->enc.umma_pair; return FIC_OK; }
+    if (option == FIC_OPT_UMMA_PAIR_USED) { *value = h->enc.pair_used; return FIC_OK; }
     if (option == FIC_OPT_F16_EXACT) {
-        if (h->f16_state == 0) {
+        if (h->enc.f16_state == 0) {
             CU(cudaSetDevice(h->device));
-            const char *why = nullptr;
-            int ok = umma_f16_selftest(h->num_sms, h->stream, &why);
-            if (ok < 0) return set_err(h, FIC_E_CUDA, "kind::f16 self-test failed to run: %s", why ? why : "?");
-            h->f16_state = ok ? 1 : -1;
+            if (int rc = status_err(h, f16_selftest(h->enc, h->stream))) return rc;
         }
-        *value = h->f16_state > 0;
+        *value = h->enc.f16_state > 0;
         return FIC_OK;
     }
     return set_err(h, FIC_E_ARG, "unknown option %d", option);
@@ -250,17 +243,13 @@ int fic_set_stream(fic_handle *h, void *cuda_stream)
     return FIC_OK;
 }
 
-static void collect_timings(fic_handle *h, bool with_copies);
-
 int fic_get_timings(const fic_handle *h, fic_timings *out)
 {
     if (!h || !out) return FIC_E_ARG;
     fic_handle *hm = const_cast<fic_handle *>(h);
-    if (hm->tm_pending_dev) {  // asynchronous device entry: events are final once the stream has drained
-        if (cudaEventQuery(hm->ev[4]) == cudaSuccess) {
-            collect_timings(hm, false);
-            hm->tm_pending_dev = false;
-        }
+    if (hm->tm_pending_dev && run_done(hm->enc)) {  // asynchronous device entry: events are final once the run has completed
+        read_stages(hm->enc, &hm->tm, nullptr, nullptr);
+        hm->tm_pending_dev = false;
     }
     *out = h->tm;
     return FIC_OK;
@@ -290,146 +279,6 @@ int fic_sync(fic_handle *h)
 // encode
 // ------------------------------------------------------------------------------------
 
-// Which search engine a call runs (FIC_OPT_ENGINE): the tcgen05 search for whole-pool windows with enough work to
-// fill the GPU, else the fused one-launch encode for the reference's GUI windows (widthKernel <= 16), else the
-// multi-kernel direct path.
-static int pick_engine(fic_handle *h, const Geom &g, int64_t j0, int64_t j1, int *engine)
-{
-    *engine = FIC_ENGINE_DIRECT;
-    if (h->engine_opt == FIC_ENGINE_UMMA) {
-        if (!umma_applicable(g))
-            return set_err(h, FIC_E_ARG, "tcgen05 search needs widthKernel == domain blocks per width == per height (and no isometries for RGB)");
-        *engine = FIC_ENGINE_UMMA;
-    } else if (h->engine_opt == FIC_ENGINE_FUSED) {
-        if (!fused_encode_applicable(g)) return set_err(h, FIC_E_ARG, "the fused encode needs widthKernel <= 16 and no isometries");
-        *engine = FIC_ENGINE_FUSED;
-    } else if (h->engine_opt == FIC_ENGINE_AUTO) {
-        // the fused kernel spends one CTA per range block and wins where launches dominate (<= 16 K range blocks,
-        // 1.8 ms against 0.45 ms for the multi-kernel path at 4096^2, widthKernel 2: measured, profiles/README.md)
-        if (umma_applicable(g) && (j1 - j0) * g.ND >= (int64_t)1 << 22) *engine = FIC_ENGINE_UMMA;
-        else if (fused_encode_applicable(g) && g.NR <= 16384) *engine = FIC_ENGINE_FUSED;
-    }
-    return FIC_OK;
-}
-
-// Fused windowed encode straight from the caller's pixels (ARGB ints or planes).  Records events 1..4.  n_images > 1: a
-// batch, every range of that many images back to back (launch_encode_fused).
-static int encode_fused_on_device(fic_handle *h, const Geom &g, const void *d_pixels, int is_argb, int64_t j0, int64_t j1,
-                                  float *d_info, int32_t *d_q, int n_images = 1)
-{
-    cudaStream_t s = h->stream;
-    // one kernel: events 1 and 4 bracket it (collect_timings reads the stages of this engine from those two alone)
-    CU(cudaEventRecord(h->ev[1], s));
-    const int launches = launch_encode_fused(d_pixels, is_argb, g, j0, j1, d_info, d_q, s, n_images);
-    CU(cudaEventRecord(h->ev[4], s));
-    CU(cudaGetLastError());
-    h->tm.engine = FIC_ENGINE_FUSED;
-    h->tm.launches += launches;
-    h->tm.search_evals = (double)(j1 - j0) * (double)g.wk * (double)g.wk;
-    return FIC_OK;
-}
-
-// The MMA kind a tcgen05 search runs with, and whether it runs at all: the first kind::f16 search of a handle verifies,
-// once, that this device's f16 tensor path accumulates the integer covariances exactly; a device that does not runs
-// kind::i8 instead.  RGB has a kind::f16 tensor path only; without an exact f16 path it stays on the CUDA-core kernel
-// (*engine becomes FIC_ENGINE_DIRECT).  (The self-test allocates and synchronises on this stream: one-time cost of the
-// first such call; fic_get_option(FIC_OPT_F16_EXACT) runs it ahead of time.)
-static int umma_kind_of(fic_handle *h, const Geom &g, int *engine, int *kind)
-{
-    *kind = h->umma_kind;
-    if (*engine != FIC_ENGINE_UMMA) return FIC_OK;
-    const bool rgb = g.C == 3;
-    const bool wants_f16 = rgb || (g.B != 16 && (*kind == FIC_UMMA_KIND_F16 || (*kind == FIC_UMMA_KIND_AUTO && umma_default_kind(g) == FIC_UMMA_KIND_F16)));
-    if (wants_f16 && h->f16_state == 0) {
-        const char *why = nullptr;
-        int ok = umma_f16_selftest(h->num_sms, h->stream, &why);
-        if (ok < 0) return set_err(h, FIC_E_CUDA, "kind::f16 self-test failed to run: %s", why ? why : "?");
-        h->f16_state = ok ? 1 : -1;
-    }
-    if (wants_f16 && h->f16_state < 0) {
-        if (rgb) *engine = FIC_ENGINE_DIRECT;
-        else *kind = FIC_UMMA_KIND_I8;
-    }
-    return FIC_OK;
-}
-
-// Pool build + search + solve on device-resident planes.  Records events 1..4.  n_images > 1 (tcgen05 engine only):
-// a group of images, planes back to back at d_src, ranges [0, NR) of each, codes in [n][NR] tables -- one launch of
-// every kernel for the whole group (launch_search_umma).
-static int encode_on_device(fic_handle *h, const Geom &g, const uint8_t *d_src, int64_t j0, int64_t j1,
-                            float *d_info, int32_t *d_q, int engine, int n_images = 1)
-{
-    Work &w = h->w;
-    cudaStream_t s = h->stream;
-    if (engine == FIC_ENGINE_FUSED) return encode_fused_on_device(h, g, d_src, 0, j0, j1, d_info, d_q);
-    const size_t n = (size_t)n_images;
-    ENSURE(w.dec, S_DEC, (size_t)g.C * g.sw * g.sh * n);
-    ENSURE(w.dsum, S_DSUM, sizeof(int32_t) * g.C * g.ND * n);
-    ENSURE(w.dsq, S_DSQ, sizeof(int32_t) * g.C * g.ND * n);
-    ENSURE(w.rsum, S_RSUM, sizeof(int32_t) * g.C * g.NR * n);
-    ENSURE(w.best, S_BEST, sizeof(int32_t) * g.NR * n);
-    if (g.C == 3) ENSURE(w.dec3, S_DEC3, sizeof(uint16_t) * (size_t)g.sw * g.sh * n);  // R + G + B of the decimated planes
-    int kind, rc;
-    h->pair_used = 0;
-    if ((rc = umma_kind_of(h, g, &engine, &kind))) return rc;
-    if (n_images > 1 && engine != FIC_ENGINE_UMMA) return set_err(h, FIC_E_ARG, "a group of images runs the tcgen05 search only");
-    if (engine == FIC_ENGINE_UMMA) {
-        ENSURE(w.opA, S_OPA, umma_opA_bytes(g, j0, j1, h->num_sms, kind, n_images));
-        ENSURE(w.opB, S_OPB, umma_opB_bytes(g, kind, n_images));
-    }
-    Work call = w;  // per-call view: the source planes may belong to the caller
-    call.src = const_cast<uint8_t *>(d_src);
-    int launches = 0;
-    CU(cudaEventRecord(h->ev[1], s));
-    launches += launch_decimate(d_src, w.dec, g, s, n_images);
-    launches += launch_domain_stats(w.dec, w.dsum, w.dsq, g, s, n_images);
-    launches += launch_range_stats(d_src, w.rsum, g, s, n_images);
-    CU(cudaEventRecord(h->ev[2], s));
-    CU(cudaEventRecord(h->ev[6], s));  // (the tcgen05 launcher re-records 6 / 7 around its search kernel)
-    CU(cudaEventRecord(h->ev[7], s));
-    if (engine == FIC_ENGINE_UMMA) {
-        const char *why = nullptr;
-        int nl = launch_search_umma(call, g, j0, j1, h->num_sms, s, &why, kind, h->ev[6], h->ev[7], h->umma_pair, &h->pair_used,
-                                    nullptr, 0, nullptr, n_images);
-        if (nl < 0) return set_err(h, FIC_E_CUDA, "tcgen05 search launch failed: %s", why ? why : "?");
-        launches += nl;
-    } else {
-        if (g.C == 3) launches += launch_sum_planes(w.dec, w.dec3, g, s);
-        CU(cudaEventRecord(h->ev[6], s));
-        launches += launch_search_direct(call, g, j0, j1, s);
-        CU(cudaEventRecord(h->ev[7], s));
-    }
-    CU(cudaEventRecord(h->ev[3], s));
-    if (n_images > 1) launches += launch_solve(call, g, 0, g.NR * n_images, d_info, d_q, s);  // the flat range of the group
-    else launches += launch_solve(call, g, j0, j1, d_info, d_q, s);
-    CU(cudaEventRecord(h->ev[4], s));
-    CU(cudaGetLastError());
-    h->tm.engine = engine;
-    h->tm.launches += launches;
-    h->tm.search_evals = (double)(j1 - j0) * (double)g.wk * (double)g.wk * (double)g.n_iso * (double)n_images;
-    return FIC_OK;
-}
-
-static void collect_timings(fic_handle *h, bool with_copies)
-{
-    float ms = 0;
-    if (h->tm.engine == FIC_ENGINE_FUSED) {  // a single kernel between events 1 and 4
-        if (with_copies && cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]) == cudaSuccess) h->tm.h2d_ms = ms;
-        if (cudaEventElapsedTime(&ms, h->ev[1], h->ev[4]) == cudaSuccess) h->tm.search_ms = h->tm.kernel_ms = ms;
-        if (with_copies && cudaEventElapsedTime(&ms, h->ev[4], h->ev[5]) == cudaSuccess) h->tm.d2h_ms = ms;
-        if (cudaEventElapsedTime(&ms, h->ev[with_copies ? 0 : 1], h->ev[with_copies ? 5 : 4]) == cudaSuccess) h->tm.total_ms = ms;
-        return;
-    }
-    if (with_copies && cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]) == cudaSuccess) h->tm.h2d_ms = ms;
-    if (cudaEventElapsedTime(&ms, h->ev[1], h->ev[2]) == cudaSuccess) h->tm.pool_ms = ms;
-    if (cudaEventElapsedTime(&ms, h->ev[2], h->ev[3]) == cudaSuccess) h->tm.search_ms = ms;
-    if (cudaEventElapsedTime(&ms, h->ev[6], h->ev[7]) == cudaSuccess) h->tm.kernel_ms = ms;
-    if (cudaEventElapsedTime(&ms, h->ev[3], h->ev[4]) == cudaSuccess) h->tm.solve_ms = ms;
-    if (with_copies && cudaEventElapsedTime(&ms, h->ev[4], h->ev[5]) == cudaSuccess) h->tm.d2h_ms = ms;
-    if (cudaEventElapsedTime(&ms, h->ev[with_copies ? 0 : 1], h->ev[with_copies ? 5 : 4]) == cudaSuccess)
-        h->tm.total_ms = ms;
-}
-
 // `pixels` is the reference's int32 ARGB array (src_u8 == 0: FC:109 / FC:171 hand over RasterImage.argb) or 8-bit
 // planes (src_u8 == 1: grey W*H bytes = the red channel, RGB 3*W*H bytes R, G, B) -- a quarter of the upload.
 static int encode_host(fic_handle *h, int is_rgb, const void *pixels, int src_u8, int W, int H, int B, int wk, int64_t j0,
@@ -443,15 +292,14 @@ static int encode_host(fic_handle *h, int is_rgb, const void *pixels, int src_u8
     if (rc) return set_err(h, rc, "%s", why);
     if (j0 < 0 || j1 > g.NR || j0 > j1) return set_err(h, FIC_E_ARG, "range interval [%lld,%lld) outside [0,%lld]", (long long)j0, (long long)j1, (long long)g.NR);
     CU(cudaSetDevice(h->device));
-    memset(&h->tm, 0, sizeof h->tm);
+    reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
     int S = code_stride(g);
-    int engine;
-    if ((rc = pick_engine(h, g, j0, j1, &engine))) return rc;
-    const bool fused_argb = engine == FIC_ENGINE_FUSED && !src_u8;  // the fused kernel reads the ARGB ints itself
-    if (!src_u8) ENSURE(w.argb, S_ARGB, sizeof(int32_t) * (size_t)W * H);
-    if (!fused_argb) ENSURE(w.src, S_SRC, (size_t)g.C * W * H);
+    EncodePlan plan;
+    if ((rc = status_err(h, plan_encode(h->enc, g, j0, j1, 1, !src_u8, s, &plan)))) return rc;
+    if (src_u8) ENSURE(w.src, S_SRC, (size_t)g.C * W * H);
+    else ENSURE(w.argb, S_ARGB, sizeof(int32_t) * (size_t)W * H);
     const size_t table = sizeof(float) * (size_t)g.NR * S;  // bytes of one code table (float and int32 entries alike)
     const bool staged = info && qcodes && 2 * table <= kStageBytes;  // small tables: one copy through pinned staging
     if (staged) {
@@ -463,16 +311,11 @@ static int encode_host(fic_handle *h, int is_rgb, const void *pixels, int src_u8
     float *const d_info = w.info;
     int32_t *const d_q = staged ? (int32_t *)((uint8_t *)w.info + table) : w.q;
     DrainOnExit drain(s);
-    CU(cudaEventRecord(h->ev[0], s));
-    if (src_u8) {
-        CU(cudaMemcpyAsync(w.src, pixels, (size_t)g.C * W * H, cudaMemcpyHostToDevice, s));
-    } else {
-        CU(cudaMemcpyAsync(w.argb, pixels, sizeof(int32_t) * (size_t)W * H, cudaMemcpyHostToDevice, s));
-        if (!fused_argb) h->tm.launches += launch_unpack(w.argb, w.src, W, H, g.C, s);
-    }
-    rc = fused_argb ? encode_fused_on_device(h, g, w.argb, 1, j0, j1, d_info, d_q)
-                    : encode_on_device(h, g, w.src, j0, j1, d_info, d_q, engine);
-    if (rc) return rc;
+    CU(cudaEventRecord(h->call_begin, s));
+    if (src_u8) CU(cudaMemcpyAsync(w.src, pixels, (size_t)g.C * W * H, cudaMemcpyHostToDevice, s));
+    else CU(cudaMemcpyAsync(w.argb, pixels, sizeof(int32_t) * (size_t)W * H, cudaMemcpyHostToDevice, s));
+    const void *d_pixels = src_u8 ? (const void *)w.src : (const void *)w.argb;
+    if ((rc = status_err(h, run_encode(h->enc, w, g, plan, d_pixels, !src_u8, j0, j1, 1, d_info, d_q, &h->tm, s)))) return rc;
     if (j1 > j0) {
         if (staged) {
             CU(cudaMemcpyAsync(h->h_stage, d_info, 2 * table, cudaMemcpyDeviceToHost, s));
@@ -481,32 +324,18 @@ static int encode_host(fic_handle *h, int is_rgb, const void *pixels, int src_u8
             if (qcodes) CU(cudaMemcpyAsync(qcodes + j0 * S, d_q + j0 * S, sizeof(int32_t) * (j1 - j0) * S, cudaMemcpyDeviceToHost, s));
         }
     }
-    CU(cudaEventRecord(h->ev[5], s));
+    CU(cudaEventRecord(h->call_end, s));
     CU(cudaStreamSynchronize(s));
     if (staged && j1 > j0) {
         memcpy(info + j0 * S, h->h_stage + sizeof(float) * j0 * S, sizeof(float) * (j1 - j0) * S);
         memcpy(qcodes + j0 * S, h->h_stage + table + sizeof(int32_t) * j0 * S, sizeof(int32_t) * (j1 - j0) * S);
     }
-    collect_timings(h, true);
+    read_stages(h->enc, &h->tm, h->call_begin, h->call_end);
     return FIC_OK;
 }
 
 // ---- batches of same-size images ----------------------------------------------------------------------------------
 
-// Input pixels one group of a batch uploads at most: the grow-only workspace does not grow with the batch.
-constexpr size_t kBatchGroupBytes = (size_t)64 << 20;
-// A group on the tcgen05 engine also holds at most 256 images (the image index is the top digit of the pool sort's
-// keys) and at most this much operand workspace (opA + opB: packed operands, flag lists, position tables and sort
-// scratch, about 2-6 MB per image of 256^2 - 512^2 at blockgroesse 8) -- or one image, however large.
-constexpr int kBatchUmmaImages = 256;
-constexpr size_t kBatchUmmaBytes = (size_t)1 << 30;
-// AUTO on a batch of full-pool images that a single call would give to the CUDA-core search picks the tcgen05 group
-// search for groups of at least this many images.  Measured on a B200 (tools/batch_bench.py,
-// profiles/r4_batch_fullpool.json): the tensor chain costs 160-190 us per call at 128^2-256^2 plus 5-10 us per image,
-// the direct search 70-130 us per image, so the group pays from about three images on (n = 8: 2.5-4x faster per image).
-// Where the single call runs the fused one-launch kernel (full pools of at most 16 x 16 domains, e.g. 64^2 at B = 8)
-// that kernel stays faster at every batch size (0.6 against 1.0 us per image at n = 256), so AUTO keeps it.
-constexpr int kBatchUmmaMinImages = 4;
 static_assert(kDecodeBatchMax * sizeof(DecodeState) <= kStageBytes, "a decode group's state blocks come back through h_stage");
 
 // The checks every batch entry adds to make_geom's: n_images >= 1 and byte counts of the whole batch that fit.
@@ -523,31 +352,11 @@ static int batch_geom(fic_handle *h, int mode, int n_images, int W, int H, int B
     return FIC_OK;
 }
 
-// Images per tcgen05 group of a batch (see kBatchUmmaImages / kBatchUmmaBytes), at most `limit`.
-static int umma_group_size(fic_handle *h, const Geom &g, int kind, int limit)
-{
-    int n = limit < kBatchUmmaImages ? limit : kBatchUmmaImages;
-    auto bytes = [&](int k) { return umma_opA_bytes(g, 0, g.NR, h->num_sms, kind, k) + umma_opB_bytes(g, kind, k); };
-    for (size_t b; n > 1 && (b = bytes(n)) > kBatchUmmaBytes;) n = (int)((double)n * kBatchUmmaBytes / b);
-    return n > 1 ? n : 1;
-}
-
-// Per-stage times of the last encode_on_device (events 1..4, 6, 7) added to the call's.
-static void add_stage_times(fic_handle *h, fic_timings *acc)
-{
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, h->ev[1], h->ev[2]) == cudaSuccess) acc->pool_ms += ms;
-    if (cudaEventElapsedTime(&ms, h->ev[2], h->ev[3]) == cudaSuccess) acc->search_ms += ms;
-    if (cudaEventElapsedTime(&ms, h->ev[6], h->ev[7]) == cudaSuccess) acc->kernel_ms += ms;
-    if (cudaEventElapsedTime(&ms, h->ev[3], h->ev[4]) == cudaSuccess) acc->solve_ms += ms;
-}
-
 // A batch encode: the codes of n_images images back to back, [n][NR][S], each equal to a single encode of that image.
-// Where pick_engine chooses the fused encode, one launch per group covers every range of every image; on the tcgen05
-// engine (full-pool windows: forced, AUTO where the single call runs it, or AUTO instead of the CUDA-core search for
-// groups of kBatchUmmaMinImages and more) every group is one
-// block-diagonal search -- one launch of each pool, sort, pack, search, refine and solve kernel; otherwise each image
-// runs encode_on_device.  Groups of images go up in one copy and their codes come down in one.
+// The plan (plan_encode) splits the batch into groups of images that go up in one copy and whose codes come down in one.
+// The fused engine covers every range of a group's images in one launch; the tcgen05 engine searches a group as one
+// block-diagonal problem -- one launch of each pool, sort, pack, search, refine and solve kernel; the direct engine runs
+// the group image by image.
 static int encode_batch_host(fic_handle *h, int mode, const void *pixels, int src_u8, int n_images, int W, int H, int B, int wk,
                              float *info, int32_t *qcodes)
 {
@@ -557,84 +366,45 @@ static int encode_batch_host(fic_handle *h, int mode, const void *pixels, int sr
     int rc = batch_geom(h, mode, n_images, W, H, B, wk, &g);
     if (rc) return rc;
     CU(cudaSetDevice(h->device));
-    memset(&h->tm, 0, sizeof h->tm);
+    reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
-    int engine;
-    if ((rc = pick_engine(h, g, 0, g.NR, &engine))) return rc;
-    const int S = code_stride(g);
+    EncodePlan plan;
+    if ((rc = status_err(h, plan_encode(h->enc, g, 0, g.NR, n_images, !src_u8, s, &plan)))) return rc;
+    const int S = code_stride(g), group = plan.group;
     const size_t plane = (size_t)W * H, image_bytes = src_u8 ? g.C * plane : sizeof(int32_t) * plane;
     const size_t codes = (size_t)g.NR * S, table = sizeof(float) * codes;  // one image's code table (float and int32 alike)
-    int group = (int)(kBatchGroupBytes / image_bytes < (size_t)n_images ? (kBatchGroupBytes / image_bytes > 0 ? kBatchGroupBytes / image_bytes : 1) : n_images);
-    // AUTO: the tcgen05 group search instead of the CUDA-core search for groups of enough images, else the single
-    // call's engine
-    int want = h->engine_opt == FIC_ENGINE_AUTO && engine == FIC_ENGINE_DIRECT && umma_applicable(g) ? FIC_ENGINE_UMMA : engine, kind = 0;
-    if ((rc = umma_kind_of(h, g, &want, &kind))) return rc;
-    if (want == FIC_ENGINE_UMMA) {
-        const int ug = umma_group_size(h, g, kind, group);
-        if (engine == FIC_ENGINE_UMMA || ug >= kBatchUmmaMinImages) {
-            engine = FIC_ENGINE_UMMA;
-            group = ug;
-        }
-    } else if (engine == FIC_ENGINE_UMMA) {
-        engine = want;  // RGB on a device without an exact kind::f16 path: the CUDA-core search, image by image
-    }
-    const bool fused = engine == FIC_ENGINE_FUSED, grouped = engine == FIC_ENGINE_UMMA;
-    if (src_u8) {
-        ENSURE(w.src, S_SRC, image_bytes * group);
-    } else {
-        ENSURE(w.argb, S_ARGB, image_bytes * group);
-        if (!fused) ENSURE(w.src, S_SRC, g.C * plane * (grouped ? group : 1));  // planes unpacked before the encode
-    }
+    if (src_u8) ENSURE(w.src, S_SRC, image_bytes * group);
+    else ENSURE(w.argb, S_ARGB, image_bytes * group);
     ENSURE(w.info, S_INFO, table * group);
     ENSURE(w.q, S_Q, table * group);
+    const uint8_t *d_pixels = src_u8 ? w.src : (const uint8_t *)w.argb;
+    const bool grouped = plan.engine == FIC_ENGINE_UMMA;
     DrainOnExit drain(s);
-    fic_timings stages;  // the tcgen05 engine: per-stage times summed over the groups
-    memset(&stages, 0, sizeof stages);
-    CU(cudaEventRecord(h->ev[0], s));
+    CU(cudaEventRecord(h->call_begin, s));
     for (int i0 = 0; i0 < n_images; i0 += group) {
         const int gn = n_images - i0 < group ? n_images - i0 : group;
-        void *d_pixels = src_u8 ? (void *)w.src : (void *)w.argb;
         if (grouped && i0 > 0) {  // the previous group's stage events, before this group records them again
             CU(cudaStreamSynchronize(s));
-            add_stage_times(h, &stages);
+            read_stages(h->enc, &h->tm, nullptr, nullptr);
         }
-        CU(cudaMemcpyAsync(d_pixels, (const uint8_t *)pixels + i0 * image_bytes, image_bytes * gn, cudaMemcpyHostToDevice, s));
-        if (fused) {
-            if ((rc = encode_fused_on_device(h, g, d_pixels, !src_u8, 0, g.NR, w.info, w.q, gn))) return rc;
-        } else if (grouped) {
-            if (!src_u8) h->tm.launches += launch_unpack(w.argb, w.src, W, H, g.C, s, gn);
-            if ((rc = encode_on_device(h, g, w.src, 0, g.NR, w.info, w.q, engine, gn))) return rc;
-        } else {
-            for (int i = 0; i < gn; i++) {
-                const uint8_t *d_src = w.src + i * g.C * plane;
-                if (!src_u8) {
-                    h->tm.launches += launch_unpack(w.argb + i * plane, w.src, W, H, g.C, s);
-                    d_src = w.src;
-                }
-                if ((rc = encode_on_device(h, g, d_src, 0, g.NR, w.info + i * codes, w.q + i * codes, engine))) return rc;
-            }
+        CU(cudaMemcpyAsync((void *)d_pixels, (const uint8_t *)pixels + i0 * image_bytes, image_bytes * gn, cudaMemcpyHostToDevice, s));
+        const int per_run = plan.engine == FIC_ENGINE_DIRECT ? 1 : gn;
+        for (int i = 0; i < gn; i += per_run) {
+            rc = status_err(h, run_encode(h->enc, w, g, plan, d_pixels + i * image_bytes, !src_u8, 0, g.NR, per_run,
+                                          w.info + i * codes, w.q + i * codes, &h->tm, s));
+            if (rc) return rc;
         }
         if (info) CU(cudaMemcpyAsync(info + i0 * codes, w.info, table * gn, cudaMemcpyDeviceToHost, s));
         if (qcodes) CU(cudaMemcpyAsync(qcodes + i0 * codes, w.q, table * gn, cudaMemcpyDeviceToHost, s));
     }
-    CU(cudaEventRecord(h->ev[5], s));
+    CU(cudaEventRecord(h->call_end, s));
     CU(cudaStreamSynchronize(s));
     CU(cudaGetLastError());
-    if (grouped) add_stage_times(h, &stages);
-    const int launches = h->tm.launches, used = h->tm.engine;
-    memset(&h->tm, 0, sizeof h->tm);  // the per-stage events saw the last image or group only: report the whole call
-    if (grouped) {
-        h->tm.pool_ms = stages.pool_ms;
-        h->tm.search_ms = stages.search_ms;
-        h->tm.kernel_ms = stages.kernel_ms;
-        h->tm.solve_ms = stages.solve_ms;
-    }
+    if (grouped) read_stages(h->enc, &h->tm, nullptr, nullptr);
+    // the per-stage times are the tcgen05 groups' sums (0 on the other engines); total_ms is the whole call
     float ms = 0;
-    if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[5]) == cudaSuccess) h->tm.total_ms = ms;
-    h->tm.engine = used;
-    h->tm.launches = launches;
-    h->tm.search_evals = (double)n_images * (double)g.NR * (double)g.wk * (double)g.wk * (double)g.n_iso;
+    h->tm.total_ms = cudaEventElapsedTime(&ms, h->call_begin, h->call_end) == cudaSuccess ? ms : 0.0f;
     return FIC_OK;
 }
 
@@ -649,7 +419,7 @@ static int decode_batch_host(fic_handle *h, int mode, int n_images, int W, int H
     int rc = batch_geom(h, mode, n_images, W, H, B, wk, &g);
     if (rc) return rc;
     CU(cudaSetDevice(h->device));
-    memset(&h->tm, 0, sizeof h->tm);
+    reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
     const int S = code_stride(g);
@@ -667,13 +437,13 @@ static int decode_batch_host(fic_handle *h, int mode, int n_images, int W, int H
     const size_t replay_bytes = decode_replay_bytes((int64_t)plane);
     if (replay_bytes) ENSURE(w.replay, S_REPLAY, replay_bytes);
     DrainOnExit drain(s);
-    CU(cudaEventRecord(h->ev[0], s));
+    CU(cudaEventRecord(h->call_begin, s));
     int bad = -1;
-    const DecodeStatus st = decode_batch_run(w, g, n_images, group, qcodes, argb_out, planes_out, max_iters, avg_error, iterations,
-                                             h->h_stage, h->h_acc, h->ev[0], h->ev[5], &h->tm, &bad, s);
+    const Status st = decode_batch_run(w, g, n_images, group, qcodes, argb_out, planes_out, max_iters, avg_error, iterations,
+                                             h->h_stage, h->h_acc, h->call_begin, h->call_end, &h->tm, &bad, s);
     if (st.rc == FIC_E_STREAM)
         return set_err(h, FIC_E_STREAM, "image %d: a code indexes outside the domain pool (the reference would throw ArrayIndexOutOfBounds)", bad);
-    return decode_err(h, st, "");
+    return status_err(h, st);
 }
 
 extern "C" {
@@ -744,12 +514,11 @@ int fic_encode_planes_dev(fic_handle *h, const uint8_t *d_planes, int is_rgb, in
     if (rc) return set_err(h, rc, "%s", why);
     if (range_begin < 0 || range_end > g.NR || range_begin > range_end) return set_err(h, FIC_E_ARG, "range interval outside [0,NR]");
     CU(cudaSetDevice(h->device));
-    // Timings of the previous asynchronous call are final once its events completed.
-    memset(&h->tm, 0, sizeof h->tm);
-    int engine;
-    if ((rc = pick_engine(h, g, range_begin, range_end, &engine))) return rc;
-    rc = encode_on_device(h, g, d_planes, range_begin, range_end, d_info, d_qcodes, engine);
-    h->tm_pending_dev = rc == FIC_OK;
+    reset_timings(h);
+    EncodePlan plan;
+    if ((rc = status_err(h, plan_encode(h->enc, g, range_begin, range_end, 1, false, h->stream, &plan)))) return rc;
+    rc = status_err(h, run_encode(h->enc, h->w, g, plan, d_planes, false, range_begin, range_end, 1, d_info, d_qcodes, &h->tm, h->stream));
+    h->tm_pending_dev = rc == FIC_OK;  // fic_get_timings reads the stage times once the run has completed
     return rc;
 }
 
@@ -787,7 +556,7 @@ int fic_measure_mma_peak(fic_handle *h, int kind, int n_cols, double *tops)
         return FIC_E_ARG;
     CU(cudaSetDevice(h->device));
     const char *why = nullptr;
-    double v = measure_mma_peak(h->num_sms, h->stream, 3, kind == FIC_UMMA_KIND_F16, n_cols, &why);
+    double v = measure_mma_peak(h->enc.num_sms, h->stream, 3, kind == FIC_UMMA_KIND_F16, n_cols, &why);
     if (v < 0) return set_err(h, FIC_E_CUDA, "tensor peak measurement failed: %s", why ? why : "?");
     *tops = v;
     return FIC_OK;
@@ -800,7 +569,7 @@ int fic_measure_mma_peak_pair(fic_handle *h, int kind, double *tops)
     if (!h || !tops || (kind != FIC_UMMA_KIND_I8 && kind != FIC_UMMA_KIND_F16)) return FIC_E_ARG;
     CU(cudaSetDevice(h->device));
     const char *why = nullptr;
-    double v = measure_mma_peak_pair(h->num_sms, h->stream, 3, kind == FIC_UMMA_KIND_F16, nullptr, &why);
+    double v = measure_mma_peak_pair(h->enc.num_sms, h->stream, 3, kind == FIC_UMMA_KIND_F16, nullptr, &why);
     if (v < 0) return set_err(h, FIC_E_CUDA, "tensor peak measurement (CTA pairs) failed: %s", why ? why : "?");
     *tops = v;
     return FIC_OK;
@@ -819,7 +588,7 @@ int fic_debug_float_sum(fic_handle *h, const int32_t *terms, int64_t count, floa
     for (int64_t i = 0; i < count; i++)
         if (terms[i] < 0 || terms[i] > 3 * 255 * 255) return set_err(h, FIC_E_ARG, "terms must lie in [0, 3 * 255^2]");
     DrainOnExit drain(s);
-    return decode_err(h, decode_float_sum(w, terms, count, carry, h->h_acc, sum, s), "");
+    return status_err(h, decode_float_sum(w, terms, count, carry, h->h_acc, sum, s));
 }
 
 int fic_build_pool(fic_handle *h, const int32_t *argb, int is_rgb, int W, int H, int B, uint8_t *decimated,
@@ -869,7 +638,7 @@ static int decode_core(fic_handle *h, int is_rgb, int W, int H, int B, int wk, c
     int rc = make_geom(W, H, B, wk, is_rgb, &g, &why);
     if (rc) return set_err(h, rc, "%s", why);
     CU(cudaSetDevice(h->device));
-    memset(&h->tm, 0, sizeof h->tm);
+    reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
     int S = code_stride(g);
@@ -885,11 +654,11 @@ static int decode_core(fic_handle *h, int is_rgb, int W, int H, int B, int wk, c
     const size_t replay_bytes = decode_replay_bytes((int64_t)plane);
     if (replay_bytes) ENSURE(w.replay, S_REPLAY, replay_bytes);
     DrainOnExit drain(s);
-    CU(cudaEventRecord(h->ev[0], s));
+    CU(cudaEventRecord(h->call_begin, s));
     if (!d_qcodes) CU(cudaMemcpyAsync(w.q, qcodes, sizeof(int32_t) * g.NR * S, cudaMemcpyHostToDevice, s));
-    const DecodeStatus st = decode_run(w, g, d_qcodes ? d_qcodes : w.q, d_planes_out ? d_planes_out : w.img, argb_out, planes_out,
-                                       max_iters, avg_error, iterations, h->h_acc, h->ev[0], h->ev[5], &h->tm, s);
-    return decode_err(h, st, "a code indexes outside the domain pool (the reference would throw ArrayIndexOutOfBounds)");
+    const Status st = decode_run(w, g, d_qcodes ? d_qcodes : w.q, d_planes_out ? d_planes_out : w.img, argb_out, planes_out,
+                                       max_iters, avg_error, iterations, h->h_acc, h->call_begin, h->call_end, &h->tm, s);
+    return status_err(h, st, "a code indexes outside the domain pool (the reference would throw ArrayIndexOutOfBounds)");
 }
 
 int fic_decode(fic_handle *h, int is_rgb, int W, int H, int B, int wk, const int32_t *qcodes, int max_iters,
@@ -937,7 +706,7 @@ int fic_collage(fic_handle *h, int is_rgb, const int32_t *argb, int W, int H, in
     CU(cudaMemcpyAsync(w.info, info, sizeof(float) * g.NR * S, cudaMemcpyHostToDevice, s));
     launch_unpack(w.argb, w.src, W, H, g.C, s);
     launch_decimate(w.src, w.dec, g, s);  // FC:275 codebook of the source
-    return decode_err(h, collage_run(w, g, argb_out, info, h->h_acc, s), "a code indexes outside the domain pool");
+    return status_err(h, collage_run(w, g, argb_out, info, h->h_acc, s), "a code indexes outside the domain pool");
 }
 
 }  // extern "C"
@@ -1059,16 +828,18 @@ static int multi_encode(fic_multi *m, int mode, const void *pixels, int src_u8, 
     for (int r = 0; r < m->n; r++) {
         fic_handle *h = m->h[r];
         MCU(cudaSetDevice(m->devices[r]));
-        memset(&h->tm, 0, sizeof h->tm);
-        if (r == 0 && !src_u8 && (rc = ensure(h, h->w.argb, S_ARGB, sizeof(int32_t) * (size_t)W * H))) return merr(m, rc, "%s", h->err);
-        if ((rc = ensure(h, h->w.src, S_SRC, plane_bytes)) || (rc = ensure(h, h->w.info, S_INFO, sizeof(float) * g.NR * S)) ||
-            (rc = ensure(h, h->w.q, S_Q, sizeof(int32_t) * g.NR * S)))
+        reset_timings(h);
+        if (r == 0 && !src_u8 && (rc = status_err(h, ensure(h->w, h->w.argb, S_ARGB, sizeof(int32_t) * (size_t)W * H))))
+            return merr(m, rc, "%s", h->err);
+        if ((rc = status_err(h, ensure(h->w, h->w.src, S_SRC, plane_bytes))) ||
+            (rc = status_err(h, ensure(h->w, h->w.info, S_INFO, sizeof(float) * g.NR * S))) ||
+            (rc = status_err(h, ensure(h->w, h->w.q, S_Q, sizeof(int32_t) * g.NR * S))))
             return merr(m, rc, "%s", h->err);
     }
     // one upload, to the first device
     fic_handle *h0 = m->h[0];
     MCU(cudaSetDevice(m->devices[0]));
-    MCU(cudaEventRecord(h0->ev[0], h0->stream));
+    MCU(cudaEventRecord(h0->call_begin, h0->stream));
     if (src_u8) {
         MCU(cudaMemcpyAsync(h0->w.src, pixels, plane_bytes, cudaMemcpyHostToDevice, h0->stream));
     } else {
@@ -1093,9 +864,11 @@ static int multi_encode(fic_multi *m, int mode, const void *pixels, int src_u8, 
     for (int r = 0; r < m->n; r++) {
         fic_handle *h = m->h[r];
         MCU(cudaSetDevice(m->devices[r]));
-        int engine;
-        rc = pick_engine(h, g, m->j0[r], m->j1[r], &engine);
-        if (!rc) rc = encode_on_device(h, g, h->w.src, m->j0[r], m->j1[r], h->w.info, h->w.q, engine);
+        EncodePlan plan;
+        rc = status_err(h, plan_encode(h->enc, g, m->j0[r], m->j1[r], 1, false, h->stream, &plan));
+        if (!rc)
+            rc = status_err(h, run_encode(h->enc, h->w, g, plan, h->w.src, false, m->j0[r], m->j1[r], 1, h->w.info, h->w.q,
+                                          &h->tm, h->stream));
         if (rc) {
             for (int q = 0; q < m->n; q++) { cudaSetDevice(m->devices[q]); cudaStreamSynchronize(m->h[q]->stream); }
             return merr(m, rc, "device %d: %s", m->devices[r], h->err);
@@ -1105,19 +878,15 @@ static int multi_encode(fic_multi *m, int mode, const void *pixels, int src_u8, 
             if (info) MCU(cudaMemcpyAsync(info + a * S, h->w.info + a * S, sizeof(float) * (b - a) * S, cudaMemcpyDeviceToHost, h->stream));
             if (qcodes) MCU(cudaMemcpyAsync(qcodes + a * S, h->w.q + a * S, sizeof(int32_t) * (b - a) * S, cudaMemcpyDeviceToHost, h->stream));
         }
-        MCU(cudaEventRecord(h->ev[5], h->stream));
+        MCU(cudaEventRecord(h->call_end, h->stream));
     }
     memset(&m->tm, 0, sizeof m->tm);
     for (int r = 0; r < m->n; r++) {
         fic_handle *h = m->h[r];
         MCU(cudaSetDevice(m->devices[r]));
         MCU(cudaStreamSynchronize(h->stream));
-        collect_timings(h, r == 0);
-        if (r != 0) {  // ev[0] is recorded on the first device only: this device's time runs from its pool build
-            float ms = 0;
-            if (cudaEventElapsedTime(&ms, h->ev[1], h->ev[5]) == cudaSuccess) h->tm.total_ms = ms;
-            if (cudaEventElapsedTime(&ms, h->ev[4], h->ev[5]) == cudaSuccess) h->tm.d2h_ms = ms;
-        }
+        // the call's start event is recorded on the first device only: the other devices' times run from their pool build
+        read_stages(h->enc, &h->tm, r == 0 ? h->call_begin : nullptr, h->call_end);
         // the handle's view of the call: the slowest device per stage
         const fic_timings &t = h->tm;
         m->tm.h2d_ms = fmaxf(m->tm.h2d_ms, t.h2d_ms);
@@ -1334,7 +1103,7 @@ int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b
     int rc = qt_geom(W, H, b_max, b_min, wk, &q, &why);
     if (rc) return set_err(h, rc, "%s", why);
     CU(cudaSetDevice(h->device));
-    memset(&h->tm, 0, sizeof h->tm);
+    reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
     const Geom &fine = q.g[q.nl - 1];
@@ -1345,28 +1114,19 @@ int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b
     ENSURE(w.qt_err, S_QT_ERR, sizeof(uint32_t) * qt_err_words(q));
     ENSURE(w.qt_stream, S_QT_STREAM, fic_quadtree_stream_bound(W, H, b_max, b_min) - kQtHeaderBytes);
     DrainOnExit drain(s);
-    CU(cudaEventRecord(h->ev[0], s));
+    CU(cudaEventRecord(h->call_begin, s));
     CU(cudaMemcpyAsync(w.src, plane, (size_t)W * H, cudaMemcpyHostToDevice, s));
-    fic_timings acc = {};
     for (int L = 0; L < q.nl; L++) {
         const Geom &g = q.g[L];
-        int engine;
-        if ((rc = pick_engine(h, g, 0, g.NR, &engine))) return rc;
-        h->tm.launches = 0;
-        if ((rc = encode_on_device(h, g, w.src, 0, g.NR, w.info, w.qt_codes + 3 * q.first[L], engine))) return rc;
-        CU(cudaEventSynchronize(h->ev[4]));
-        float ms = 0;
-        if (h->tm.engine == FIC_ENGINE_FUSED) {  // one kernel between events 1 and 4
-            if (cudaEventElapsedTime(&ms, h->ev[1], h->ev[4]) == cudaSuccess) { acc.search_ms += ms; acc.kernel_ms += ms; }
-        } else {
-            add_stage_times(h, &acc);
-        }
-        acc.launches += h->tm.launches;
-        acc.search_evals += h->tm.search_evals;
-        acc.engine = h->tm.engine;
+        EncodePlan plan;
+        if ((rc = status_err(h, plan_encode(h->enc, g, 0, g.NR, 1, false, s, &plan)))) return rc;
+        if ((rc = status_err(h, run_encode(h->enc, w, g, plan, w.src, false, 0, g.NR, 1, w.info, w.qt_codes + 3 * q.first[L], &h->tm, s))))
+            return rc;
+        CU(cudaStreamSynchronize(s));  // the level's stage events, before the next level records them again
+        read_stages(h->enc, &h->tm, nullptr, nullptr);
     }
-    acc.launches += launch_decimate(w.src, w.dec, fine, s);  // the fused engine leaves no decimated plane behind
-    acc.launches += launch_qt_stream(w, q, max_mse, s);
+    h->tm.launches += launch_decimate(w.src, w.dec, fine, s);  // the fused engine leaves no decimated plane behind
+    h->tm.launches += launch_qt_stream(w, q, max_mse, s);
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(h->h_acc, w.qt_err, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
@@ -1377,11 +1137,10 @@ int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b
     const int32_t hd[8] = {FIC_MODE_GREY_QT, W, H, 0, wk, b_max, b_min, (int32_t)leaves};
     for (int k = 0; k < 8; k++) put_be32(stream + 4 * k, hd[k]);
     CU(cudaMemcpyAsync(stream + kQtHeaderBytes, w.qt_stream, need - kQtHeaderBytes, cudaMemcpyDeviceToHost, s));
-    CU(cudaEventRecord(h->ev[5], s));
+    CU(cudaEventRecord(h->call_end, s));
     CU(cudaStreamSynchronize(s));
     float ms = 0;
-    if (cudaEventElapsedTime(&ms, h->ev[0], h->ev[5]) == cudaSuccess) acc.total_ms = ms;
-    h->tm = acc;
+    h->tm.total_ms = cudaEventElapsedTime(&ms, h->call_begin, h->call_end) == cudaSuccess ? ms : 0.0f;  // the whole call
     return FIC_OK;
 }
 
@@ -1414,7 +1173,7 @@ int fic_decode_quadtree(fic_handle *h, const uint8_t *stream, size_t nbytes, int
     std::vector<int32_t> base((size_t)q.g[0].NR);  // first leaf of every top block (the first pass gave their count)
     qt_parse(stream, nbytes, &q, base.data(), false, &why);
     CU(cudaSetDevice(h->device));
-    memset(&h->tm, 0, sizeof h->tm);
+    reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
     const Geom &g = q.g[0];
@@ -1428,11 +1187,11 @@ int fic_decode_quadtree(fic_handle *h, const uint8_t *stream, size_t nbytes, int
     ENSURE(w.qt_leaf, S_QT_LEAF, sizeof(int4) * q.leaves);
     ENSURE(w.qt_map, S_QT_MAP, sizeof(int32_t) * (cells + base.size()));
     DrainOnExit drain(s);
-    CU(cudaEventRecord(h->ev[0], s));
+    CU(cudaEventRecord(h->call_begin, s));
     CU(cudaMemcpyAsync(w.qt_stream, stream + kQtHeaderBytes, used - kQtHeaderBytes, cudaMemcpyHostToDevice, s));
     CU(cudaMemcpyAsync(w.qt_map + cells, base.data(), sizeof(int32_t) * base.size(), cudaMemcpyHostToDevice, s));
-    const DecodeStatus st = decode_quadtree_run(w, q, max_iters, plane_out, avg_error, iterations, h->h_acc, h->ev[0], h->ev[5], &h->tm, s);
-    return decode_err(h, st, "a leaf indexes outside its level's domain pool");
+    const Status st = decode_quadtree_run(w, q, max_iters, plane_out, avg_error, iterations, h->h_acc, h->call_begin, h->call_end, &h->tm, s);
+    return status_err(h, st, "a leaf indexes outside its level's domain pool");
 }
 
 }  // extern "C"

@@ -1072,7 +1072,7 @@ k_decode_sweep_qt(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img,
 // ---- host side ------------------------------------------------------------------------------------------------------
 
 #define DCU(call) \
-    do { const cudaError_t e_ = (call); if (e_ != cudaSuccess) return DecodeStatus{FIC_E_CUDA, e_, #call, __FILE__, __LINE__}; } while (0)
+    do { const cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(FIC_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); } while (0)
 
 // Which kernels a decode of geometry g runs, decided once per call.
 enum class SweepFamily { IL, V8, QUAD };  // k_decode_sweep_il, k_decode_sweep_v8, k_decode_sweep
@@ -1245,10 +1245,10 @@ static int launch_sweep_finish(const Work &w, int64_t count, int it, bool last, 
 }
 
 // Waits for the stream, then reads the state block that was copied to h_state before.
-static DecodeStatus sync_state(const DecodeState *h_state, cudaStream_t s)
+static Status sync_state(const DecodeState *h_state, cudaStream_t s)
 {
     DCU(cudaStreamSynchronize(s));
-    return DecodeStatus{h_state->bad_index ? FIC_E_STREAM : FIC_OK};
+    return Status(h_state->bad_index ? FIC_E_STREAM : FIC_OK);
 }
 
 // avgError bookkeeping (FC:407-417).  The reference adds every squared pixel change to a binary32 running sum,
@@ -1260,7 +1260,7 @@ static DecodeStatus sync_state(const DecodeState *h_state, cudaStream_t s)
 // changes in loop order and are folded by k_sweep_finish or the chunked replay, which replay the float accumulation
 // where they must.  Sweeps are enqueued eight at a time without looking at the result: once the done flag is set the
 // remaining ones return immediately, and the host reads the state once per batch instead of once per sweep.
-DecodeStatus decode_run(const Work &w, const Geom &g, const int32_t *d_q, uint8_t *img, int32_t *argb_out, uint8_t *planes_out,
+Status decode_run(const Work &w, const Geom &g, const int32_t *d_q, uint8_t *img, int32_t *argb_out, uint8_t *planes_out,
                         int max_iters, float *avg_error, int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end,
                         fic_timings *tm, cudaStream_t s)
 {
@@ -1272,15 +1272,15 @@ DecodeStatus decode_run(const Work &w, const Geom &g, const int32_t *d_q, uint8_
     const float fwh = (float)(g.W * g.H);  // FC:413 (float)(width*height)
     int32_t *doff = (int32_t *)(w.dcode + g.NR * code_stride(g));
     int launches = 0;
-    DecodeStatus st;
-    auto enqueue_output = [&]() -> DecodeStatus {
+    Status st;
+    auto enqueue_output = [&]() -> Status {
         if (argb_out) {
             launches += launch_pack_argb(img, w.argb, g, s);
             DCU(cudaMemcpyAsync(argb_out, w.argb, sizeof(int32_t) * plane, cudaMemcpyDeviceToHost, s));
         } else if (planes_out) {
             DCU(cudaMemcpyAsync(planes_out, img, g.C * plane, cudaMemcpyDeviceToHost, s));
         }
-        return DecodeStatus{};
+        return Status();
     };
     DCU(cudaMemsetAsync(w.state, 0, sizeof(DecodeState), s));
     bool done = false;
@@ -1345,7 +1345,7 @@ DecodeStatus decode_run(const Work &w, const Geom &g, const int32_t *d_q, uint8_
     tm->launches = launches;
     if (avg_error) memcpy(avg_error, &hs->avg_bits, sizeof *avg_error);
     if (iterations) *iterations = (int)hs->iters;
-    return DecodeStatus{};
+    return Status();
 }
 
 int decode_batch_group(const Geom &g)
@@ -1360,7 +1360,7 @@ int decode_batch_group(const Geom &g)
 // Groups of `group` images through k_decode_small, then every image the one-launch decoder did not finish -- it bailed
 // (its avgError needs the float sum replayed), the geometry has no one-launch form (group == 0) or the device cannot
 // launch it cooperatively -- through decode_run, one image at a time: the path fic_decode takes.
-DecodeStatus decode_batch_run(const Work &w, const Geom &g, int n, int group, const int32_t *qcodes, int32_t *argb_out,
+Status decode_batch_run(const Work &w, const Geom &g, int n, int group, const int32_t *qcodes, int32_t *argb_out,
                               uint8_t *planes_out, int max_iters, float *avg_error, int *iterations, void *h_stage,
                               void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, int *bad_image, cudaStream_t s)
 {
@@ -1392,7 +1392,7 @@ DecodeStatus decode_batch_run(const Work &w, const Geom &g, int n, int group, co
             const DecodeState &x = hs[i];
             if (x.bad_index) {
                 *bad_image = i0 + i;
-                return DecodeStatus{FIC_E_STREAM};
+                return Status(FIC_E_STREAM);
             }
             if (x.bail) {
                 redo[i0 + i] = 1;  // avg_error[i0 + i] still holds its carry
@@ -1406,7 +1406,7 @@ DecodeStatus decode_batch_run(const Work &w, const Geom &g, int n, int group, co
         if (!redo[i]) continue;
         DCU(cudaMemcpyAsync(w.q, qcodes + i * codes, sizeof(int32_t) * codes, cudaMemcpyHostToDevice, s));
         fic_timings one = {};
-        const DecodeStatus st = decode_run(w, g, w.q, w.img, argb_out ? argb_out + i * plane : nullptr,
+        const Status st = decode_run(w, g, w.q, w.img, argb_out ? argb_out + i * plane : nullptr,
                                            planes_out ? planes_out + i * g.C * plane : nullptr, max_iters,
                                            avg_error ? avg_error + i : nullptr, iterations ? iterations + i : nullptr, h_scratch, ev0,
                                            end, &one, s);
@@ -1420,10 +1420,10 @@ DecodeStatus decode_batch_run(const Work &w, const Geom &g, int n, int group, co
     float ms = 0;
     if (cudaEventElapsedTime(&ms, ev0, end) == cudaSuccess) tm->total_ms = ms;
     tm->launches = launches;
-    return DecodeStatus{};
+    return Status();
 }
 
-DecodeStatus collage_run(const Work &w, const Geom &g, int32_t *argb_out, float *info_out, void *h_scratch, cudaStream_t s)
+Status collage_run(const Work &w, const Geom &g, int32_t *argb_out, float *info_out, void *h_scratch, cudaStream_t s)
 {
     const Plan p = plain_plan(g);  // the source's codebook is the plain decimated plane of the pool builder
     const size_t plane = (size_t)g.W * g.H;
@@ -1441,7 +1441,7 @@ DecodeStatus collage_run(const Work &w, const Geom &g, int32_t *argb_out, float 
     return sync_state((const DecodeState *)h_scratch, s);
 }
 
-DecodeStatus decode_float_sum(const Work &w, const int32_t *terms, int64_t count, float carry, void *h_scratch, float *sum,
+Status decode_float_sum(const Work &w, const int32_t *terms, int64_t count, float carry, void *h_scratch, float *sum,
                               cudaStream_t s)
 {
     DecodeState state = {};
@@ -1454,7 +1454,7 @@ DecodeStatus decode_float_sum(const Work &w, const int32_t *terms, int64_t count
     DCU(cudaStreamSynchronize(s));
     DCU(cudaGetLastError());
     memcpy(sum, &((const DecodeState *)h_scratch)->avg_bits, sizeof *sum);
-    return DecodeStatus{};
+    return Status();
 }
 
 template <bool FIRST>
@@ -1465,7 +1465,7 @@ static void launch_sweep_qt(int64_t need, bool quad, cudaStream_t s, const uint8
     else launch_wave<k_decode_sweep_qt<FIRST, false>>(need, s, dec_in, img, dec_out, leaf, map, g, lcell, ctl, last);
 }
 
-DecodeStatus decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
+Status decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
                                  int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, cudaStream_t s)
 {
     const Geom &g = q.g[0];
@@ -1475,7 +1475,7 @@ DecodeStatus decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, 
     const int lcell = __builtin_ctz((unsigned)q.g[q.nl - 1].B);
     const int32_t *base = w.qt_map + (plane >> (2 * lcell));
     int launches = 0;
-    DecodeStatus st;
+    Status st;
     DCU(cudaMemsetAsync(w.state, 0, sizeof(DecodeState), s));
     k_qt_dequant<<<(unsigned)((g.NR + 127) / 128), 128, 0, s>>>(q, w.qt_stream, base, w.qt_leaf, w.qt_map, lcell, w.state);
     launches++;
@@ -1511,7 +1511,7 @@ DecodeStatus decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, 
     tm->launches = launches;
     if (avg_error) memcpy(avg_error, &hs->avg_bits, sizeof *avg_error);
     if (iterations) *iterations = (int)hs->iters;
-    return DecodeStatus{};
+    return Status();
 }
 
 }  // namespace fic

@@ -9,6 +9,17 @@
 
 namespace fic {
 
+// Outcome of an encoder (fic_encode.cu) or decoder (fic_decode.cu) entry.  rc: FIC_OK or a FIC_E_* code; msg: the
+// message for fic_last_error, or "" where the caller words it (a decoder's FIC_E_STREAM: a code indexes outside the
+// domain pool).
+struct Status {
+    int rc;
+    char msg[512];
+    explicit Status(int code = FIC_OK) : rc(code) { msg[0] = 0; }
+};
+// A Status with code rc and a printf-style message (fic_api.cu).
+Status fail(int rc, const char *fmt, ...) __attribute__((format(printf, 2, 3)));
+
 // Block / pool geometry of one encode or decode call (FC:111-116, FC:1019-1022).
 struct Geom {
     int W, H, B, n;       // image size, block size, n = B*B
@@ -72,6 +83,28 @@ struct Work {
     size_t cap[24] = {0};
 };
 
+enum Slot { S_ARGB, S_SRC, S_DEC, S_DSUM, S_DSQ, S_RSUM, S_BEST, S_INFO, S_Q, S_OPA, S_OPB, S_IMG, S_DEC2, S_DCODE, S_PERR, S_STATE, S_DEC3, S_REPLAY, S_QT_STREAM, S_QT_CODES,
+            S_QT_ERR, S_QT_LEAF, S_QT_MAP };
+
+// Grows workspace buffer p (its capacity is w.cap[slot]) to at least `bytes`; never shrinks it.
+template <typename T>
+Status ensure(Work &w, T *&p, int slot, size_t bytes)
+{
+    if (bytes == 0) bytes = 16;
+    if (w.cap[slot] >= bytes && p) return Status();
+    if (p) cudaFree(p);
+    p = nullptr;
+    w.cap[slot] = 0;
+    size_t want = (bytes + 255) & ~(size_t)255;
+    cudaError_t e = cudaMalloc((void **)&p, want);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(FIC_E_NOMEM, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
+    }
+    w.cap[slot] = want;
+    return Status();
+}
+
 // ---- kernel launchers (each returns the number of kernels it launched) -----------
 // The pool builders take n_images same-size images back to back, one launch for all: ARGB [n][H][W] -> planes
 // [n][C][H][W] -> decimated planes [n][C][sh][sw], dsum / dsq [n][C][ND], rsum [n][C][NR], dec3 [n][sh][sw].
@@ -122,29 +155,62 @@ int launch_search_umma(const Work &w, const Geom &g, int64_t j0, int64_t j1, int
                        cudaEvent_t k1 = nullptr, int pair = FIC_UMMA_PAIR_AUTO, int *pair_used = nullptr,
                        int32_t *dump = nullptr, int64_t dump_ld = 0, int *status_dev = nullptr, int n_images = 1);
 
-// ---- decoder (fic_decode.cu) -----------------------------------------------------------------------------------------
-// Outcome of a decoder entry.  rc: FIC_OK; FIC_E_STREAM when a code indexes outside the domain pool (the reference
-// throws ArrayIndexOutOfBounds); FIC_E_CUDA when `call` (file:line) returned `cuda`.
-struct DecodeStatus {
-    int rc = FIC_OK;
-    cudaError_t cuda = cudaSuccess;
-    const char *call = nullptr, *file = nullptr;
-    int line = 0;
+// ---- encoder host side (fic_encode.cu) --------------------------------------------------------------------------------
+// Per-handle encoder state: the options that choose an engine, what the last tcgen05 search did, and the events a run
+// records around its stages (created and destroyed with the handle).
+struct Encoder {
+    int engine_opt = FIC_ENGINE_AUTO;    // FIC_OPT_ENGINE
+    int umma_kind = FIC_UMMA_KIND_AUTO;  // FIC_OPT_UMMA_KIND
+    int umma_pair = FIC_UMMA_PAIR_AUTO;  // FIC_OPT_UMMA_PAIR
+    int pair_used = 0;                   // did the last tcgen05 search run the CTA-pair kernel
+    int f16_state = 0;  // kind::f16 self-test: 0 not run yet, 1 exact, -1 not exact on this device (use kind::i8)
+    int num_sms = 0;
+    int run_engine = FIC_ENGINE_DIRECT;  // engine of the last run: which of the stage events it recorded
+    cudaEvent_t ev[6] = {nullptr};
 };
+
+// What an encode call runs: the engine (FIC_ENGINE_DIRECT / _UMMA / _FUSED), the tcgen05 instruction kind, and the most
+// images one run takes (1 unless a batch).
+struct EncodePlan {
+    int engine, kind, group;
+};
+
+// The plan for ranges [j0, j1) of n_images images of geometry g whose pixels arrive as ARGB ints (argb) or 8-bit planes;
+// n_images = 1 is a single image or range slice, more is a batch (j0 = 0, j1 = NR).  FIC_E_ARG when the forced engine
+// does not apply.  Runs the kind::f16 self-test on stream s the first time a plan would use kind::f16.
+Status plan_encode(Encoder &e, const Geom &g, int64_t j0, int64_t j1, int n_images, bool argb, cudaStream_t s,
+                   EncodePlan *plan);
+// Runs plan p on device-resident pixels (ARGB ints or 8-bit planes, n_images <= p.group images back to back): ranges
+// [j0, j1) of one image, or every range of a group (codes in [n][NR] tables).  Sizes its workspace in w, records the stage
+// events, and adds engine, launches and search_evals to *tm.
+Status run_encode(Encoder &e, Work &w, const Geom &g, const EncodePlan &p, const void *d_pixels, bool argb, int64_t j0,
+                  int64_t j1, int n_images, float *d_info, int32_t *d_q, fic_timings *tm, cudaStream_t s);
+// Whether the last run's events have completed.
+bool run_done(const Encoder &e);
+// Adds the last run's stage times (its events must have completed) to pool_ms, search_ms, kernel_ms and solve_ms of
+// *acc, and sets total_ms = begin -> end.  begin: the call's start event (then h2d_ms = begin -> the run's start), or null
+// for the run's start; end: the call's end event (then d2h_ms = the run's end -> end), or null for the run's end.
+void read_stages(const Encoder &e, fic_timings *acc, cudaEvent_t begin, cudaEvent_t end);
+// The kind::f16 self-test of the handle's device, run once per handle (Encoder::f16_state); FIC_E_CUDA if it cannot run.
+Status f16_selftest(Encoder &e, cudaStream_t s);
+
+// ---- decoder (fic_decode.cu) -----------------------------------------------------------------------------------------
+// Decoder entries return FIC_E_STREAM with no message when a code indexes outside the domain pool (the reference throws
+// ArrayIndexOutOfBounds).
 
 // Iterative decode (FC:355-420) of the codes at d_q into the device planes d_img, also copied to argb_out (host ARGB) or
 // planes_out (host planes) when given.  avg_error (optional): in, the avgError the last decode left (FC:20); out, this
 // decode's.  tm: total_ms from ev0 (recorded by the caller) to end, and launches.  h_scratch: pinned, sizeof(DecodeState).
 // Workspace: dcode, dec, dec2, state, perr (W*H ints), replay (decode_replay_bytes(W*H)) and, with argb_out, argb.
-DecodeStatus decode_run(const Work &w, const Geom &g, const int32_t *d_q, uint8_t *d_img, int32_t *argb_out,
+Status decode_run(const Work &w, const Geom &g, const int32_t *d_q, uint8_t *d_img, int32_t *argb_out,
                         uint8_t *planes_out, int max_iters, float *avg_error, int *iterations, void *h_scratch,
                         cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, cudaStream_t s);
 // One collage step (FC:268-280): the float codes in w.info applied once to the source's codebook w.dec over an image of
 // 0xa0 pixels; the image to argb_out, the codes with codebook indices (FC:888) to info_out.  Also uses dcode, img, argb.
-DecodeStatus collage_run(const Work &w, const Geom &g, int32_t *argb_out, float *info_out, void *h_scratch, cudaStream_t s);
+Status collage_run(const Work &w, const Geom &g, int32_t *argb_out, float *info_out, void *h_scratch, cudaStream_t s);
 // *sum = carry + terms[0] + ... + terms[count - 1] in binary32, in order, as the last sweep of a decode over `count`
 // pixels folds it (terms in [0, 3 * 255^2]).  Workspace: perr (count ints), state, replay (decode_replay_bytes(count)).
-DecodeStatus decode_float_sum(const Work &w, const int32_t *terms, int64_t count, float carry, void *h_scratch, float *sum,
+Status decode_float_sum(const Work &w, const int32_t *terms, int64_t count, float carry, void *h_scratch, float *sum,
                               cudaStream_t s);
 // Device workspace of the chunked replay of a sweep over `pixels` pixels (0: the one-warp replay needs none).
 size_t decode_replay_bytes(int64_t pixels);
@@ -159,7 +225,7 @@ int decode_batch_group(const Geom &g);
 // state for group (DecodeState + float carry), and what decode_run needs for one image.  h_stage: pinned, >= group *
 // sizeof(DecodeState); h_scratch as decode_run's.  On FIC_E_STREAM *bad_image is the lowest image whose codes index
 // outside the pool.
-DecodeStatus decode_batch_run(const Work &w, const Geom &g, int n, int group, const int32_t *qcodes, int32_t *argb_out,
+Status decode_batch_run(const Work &w, const Geom &g, int n, int group, const int32_t *qcodes, int32_t *argb_out,
                               uint8_t *planes_out, int max_iters, float *avg_error, int *iterations, void *h_stage,
                               void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, int *bad_image, cudaStream_t s);
 
@@ -192,7 +258,7 @@ int launch_qt_stream(const Work &w, const QtGeom &q, double max_mse, cudaStream_
 // Iterative decode of the stream in w.qt_stream (the first-leaf table in w.qt_map after the cell map) into w.img, copied to
 // planes_out.  avgError = (float)S / (float)(W*H) of the exact sum S of squared changes; stops below 1 or after
 // max_iters sweeps.  Workspace: img, dec, dec2, state, qt_leaf (q.leaves), qt_map.
-DecodeStatus decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
+Status decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
                                  int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm,
                                  cudaStream_t s);
 // Exclusive prefix sums of n counters in place (one block, the radix sort's row scan); *total = their sum.

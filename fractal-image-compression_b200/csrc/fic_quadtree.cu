@@ -1,7 +1,7 @@
 // fic_quadtree.cu -- the quadtree extension (FIC_MODE_GREY_QT, not in the reference): the stream's geometry and parser,
 // and the kernels that turn every level's codes into the stream body on the device -- the collage error of each range
 // block, the split flags of each top block, the leaf scan and the big-endian leaf scatter.  The per-level encodes are
-// the library's ordinary grey encodes (fic_api.cu); the decoder sweep lives with the other sweeps in fic_decode.cu.
+// the library's ordinary grey encodes (fic_encode.cu); the decoder sweep lives with the other sweeps in fic_decode.cu.
 #include <string.h>
 
 #include "fic_device.cuh"
