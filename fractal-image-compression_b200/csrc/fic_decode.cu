@@ -53,7 +53,8 @@ __device__ __forceinline__ void dequant_one(int64_t j, const int32_t *__restrict
         v[0] = (float)q[S * j];
         v[1] = __fdiv_rn((float)q[S * j + 1], kGreyAScale);
         v[2] = (float)q[S * j + 2];
-        if (S == 4) v[3] = (float)(q[S * j + 3] & 7);  // isometry index (extension)
+        // isometry index (extension): read through float like every other stream field, the sweep takes j_f2i(v[3]) & 7
+        if (S == 4) v[3] = (float)q[S * j + 3];
     } else {
         v[0] = (float)q[5 * j];
         v[1] = __fdiv_rn((float)q[5 * j + 1], kRgbAScale);

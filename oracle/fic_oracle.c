@@ -698,7 +698,12 @@ static int sweep(int32_t *img, int W, int H, int B, int is_rgb, const float *d, 
 /* FC:547-553 decode -> FC:356-421 decodeGreyScale / FC:430-508 decodeRGB. */
 int fic_oracle_decode(const uint8_t *s, size_t nbytes, int32_t *out, float *avg_error, int *iters)
 {
-    if (nbytes < 20) return -1;
+    return fic_oracle_decode_iters(s, nbytes, 50, out, avg_error, iters);
+}
+
+int fic_oracle_decode_iters(const uint8_t *s, size_t nbytes, int max_iters, int32_t *out, float *avg_error, int *iters)
+{
+    if (nbytes < 20 || max_iters < 1) return -1;
     int is_rgb = get_be32(s) == 2 ? 2 : (get_be32(s) != 0); /* 2: isometry extension stream */
     int W = get_be32(s + 4), H = get_be32(s + 8), B = get_be32(s + 12), wk = get_be32(s + 16);
     int rc = check_args(W, H, B, wk);
@@ -734,13 +739,13 @@ int fic_oracle_decode(const uint8_t *s, size_t nbytes, int32_t *out, float *avg_
     float avg = avg_error ? *avg_error : 0;
     int counter;
     int done = 0;
-    for (counter = 0; counter < 50; counter++) {
+    for (counter = 0; counter < max_iters; counter++) {
         rc = sweep(out, W, H, B, is_rgb, d, stride, 0, NULL, &avg);
         if (rc) { free(d); return rc; }
         done = counter + 1;
         avg = avg / (float)(W * H);
         if (avg < 1) break;
-        if (counter != 49) avg = 0;
+        if (counter != max_iters - 1) avg = 0;
     }
     if (avg_error) *avg_error = avg;
     if (iters) *iters = done;

@@ -71,9 +71,14 @@ size_t fic_oracle_write_data(int is_rgb, int W, int H, int B, int wk, const floa
 
 /* decode (FC:547-553, FC:356-421, FC:430-508).  avg_error is the reference's static
  * FractalCompression.avgError: read on entry (it is never reset between decodes)
- * and written on exit.  iters receives the number of sweeps executed. */
+ * and written on exit.  iters receives the number of sweeps executed.
+ * fic_oracle_decode_iters: the same loop with the limit max_iters (>= 1) in place of the
+ * reference's 50 (FC:381), as fic_decode's max_iters; an unconverged value is kept after
+ * the last allowed sweep (FC:416-417). */
 int fic_oracle_decode(const uint8_t *stream, size_t nbytes, int32_t *argb_out,
                       float *avg_error, int *iters);
+int fic_oracle_decode_iters(const uint8_t *stream, size_t nbytes, int max_iters,
+                            int32_t *argb_out, float *avg_error, int *iters);
 
 /* getBestGeneratedCollage[RGB] (FC:269-347): one decode step from the source image
  * with the unquantised codes.  Like the reference it rewrites info[.][0] in place

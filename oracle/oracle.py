@@ -51,6 +51,8 @@ def lib() -> C.CDLL:
         L.fic_oracle_write_data.restype = C.c_size_t
         L.fic_oracle_decode.argtypes = [u8p, C.c_size_t, i32p, f32p, C.POINTER(C.c_int)]
         L.fic_oracle_decode.restype = C.c_int
+        L.fic_oracle_decode_iters.argtypes = [u8p, C.c_size_t, C.c_int, i32p, f32p, C.POINTER(C.c_int)]
+        L.fic_oracle_decode_iters.restype = C.c_int
         L.fic_oracle_collage.argtypes = [i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, f32p, i32p]
         L.fic_oracle_collage.restype = C.c_int
         L.fic_oracle_is_grey.argtypes = [i32p, C.c_int, C.c_int]
@@ -151,8 +153,8 @@ def write_data(info: np.ndarray, W: int, H: int, B: int, wk: int, rgb: bool = Fa
     return buf.tobytes()
 
 
-def decode(stream: bytes, avg_error_in: float = 0.0):
-    """Returns (argb[H, W] int32, avgError float32, iterations)."""
+def decode(stream: bytes, avg_error_in: float = 0.0, max_iters: int = 50):
+    """Returns (argb[H, W] int32, avgError float32, iterations); max_iters replaces the reference's limit of 50."""
     import struct
 
     _, W, H, _, _ = struct.unpack(">5i", stream[:20])
@@ -160,7 +162,8 @@ def decode(stream: bytes, avg_error_in: float = 0.0):
     out = np.empty((H, W), np.int32)
     avg = C.c_float(avg_error_in)
     it = C.c_int(0)
-    rc = lib().fic_oracle_decode(_p(buf, C.c_uint8), len(buf), _p(out, C.c_int32), C.byref(avg), C.byref(it))
+    rc = lib().fic_oracle_decode_iters(_p(buf, C.c_uint8), len(buf), max_iters, _p(out, C.c_int32), C.byref(avg),
+                                       C.byref(it))
     if rc:
         raise ValueError(f"oracle decode failed (rc={rc})")
     return out, np.float32(avg.value), it.value
