@@ -5,12 +5,12 @@ reference's codec interface plus the torch.distributed plumbing for multi-GPU en
 """
 from . import _lib, synth
 from ._lib import (FIC_ENGINE_AUTO, FIC_ENGINE_DIRECT, FIC_ENGINE_FUSED, FIC_ENGINE_UMMA, FIC_UMMA_KIND_AUTO, FIC_UMMA_KIND_F16,
-                   FIC_UMMA_KIND_I8, FIC_UMMA_PAIR_AUTO, FIC_UMMA_PAIR_OFF, FIC_UMMA_PAIR_ON, FIC_MODE_GREY, FIC_MODE_RGB, FIC_MODE_GREY_ISO, FIC_MODE_GREY_QT, ABI_SYMBOLS, LIB_PATH, FicError, Timings)
+                   FIC_UMMA_KIND_I8, FIC_UMMA_PAIR_AUTO, FIC_UMMA_PAIR_OFF, FIC_UMMA_PAIR_ON, FIC_MODE_GREY, FIC_MODE_RGB, FIC_MODE_GREY_ISO, FIC_MODE_GREY_QT, FIC_MODE_RGB_QT, ABI_SYMBOLS, LIB_PATH, FicError, Timings)
 from .codec import ByteSink, FractalCompression, Handle, MultiHandle, RasterImage, quadtree_stream_info, stream_read, stream_write
 
 __all__ = [
     "ABI_SYMBOLS", "ByteSink", "FIC_ENGINE_AUTO", "FIC_ENGINE_DIRECT", "FIC_ENGINE_FUSED", "FIC_ENGINE_UMMA", "FIC_MODE_GREY", "FIC_MODE_GREY_ISO",
-    "FIC_MODE_GREY_QT", "FIC_MODE_RGB", "FIC_UMMA_KIND_AUTO",
+    "FIC_MODE_GREY_QT", "FIC_MODE_RGB", "FIC_MODE_RGB_QT", "FIC_UMMA_KIND_AUTO",
     "FIC_UMMA_KIND_F16", "FIC_UMMA_KIND_I8", "FIC_UMMA_PAIR_AUTO", "FIC_UMMA_PAIR_OFF", "FIC_UMMA_PAIR_ON", "FicError",
     "FractalCompression", "Handle", "LIB_PATH", "MultiHandle", "RasterImage", "Timings", "quadtree_stream_info", "stream_read", "stream_write", "synth",
 ]

@@ -16,7 +16,7 @@ FIC_OK = 0
 FIC_E_ARG, FIC_E_CUDA, FIC_E_NOMEM, FIC_E_STREAM, FIC_E_INTERNAL = -1, -2, -3, -4, -5
 FIC_ENGINE_AUTO, FIC_ENGINE_DIRECT, FIC_ENGINE_UMMA, FIC_ENGINE_FUSED = 0, 1, 2, 3
 FIC_UMMA_KIND_AUTO, FIC_UMMA_KIND_I8, FIC_UMMA_KIND_F16 = 0, 1, 2
-FIC_MODE_GREY, FIC_MODE_RGB, FIC_MODE_GREY_ISO, FIC_MODE_GREY_QT = 0, 1, 2, 3
+FIC_MODE_GREY, FIC_MODE_RGB, FIC_MODE_GREY_ISO, FIC_MODE_GREY_QT, FIC_MODE_RGB_QT = 0, 1, 2, 3, 4
 FIC_OPT_ENGINE = 1
 FIC_OPT_UMMA_KIND = 2
 FIC_OPT_F16_EXACT = 3
@@ -37,6 +37,7 @@ ABI_SYMBOLS = [
     "fic_multi_encode_rgb", "fic_multi_encode_grey_iso", "fic_multi_encode_grey_u8", "fic_multi_encode_rgb_planes",
     "fic_encode_batch", "fic_encode_batch_u8", "fic_decode_batch", "fic_decode_batch_u8",
     "fic_quadtree_stream_bound", "fic_encode_quadtree", "fic_quadtree_stream_info", "fic_decode_quadtree",
+    "fic_quadtree_rgb_stream_bound", "fic_encode_quadtree_rgb", "fic_quadtree_rgb_stream_info", "fic_decode_quadtree_rgb",
 ]
 
 
@@ -121,15 +122,20 @@ def load() -> C.CDLL:
     L.fic_stream_write.argtypes = [C.c_int] * 5 + [vp, vp, C.c_size_t]
     L.fic_stream_read_header.argtypes = [vp, C.c_size_t] + [C.POINTER(C.c_int)] * 5 + [C.POINTER(C.c_size_t)]
     L.fic_stream_read_codes.argtypes = [vp, C.c_size_t, vp]
-    L.fic_quadtree_stream_bound.argtypes = [C.c_int] * 4
-    L.fic_quadtree_stream_bound.restype = C.c_size_t
-    L.fic_encode_quadtree.argtypes = [vp, vp] + [C.c_int] * 5 + [C.c_double, vp, C.c_size_t, C.POINTER(C.c_size_t)]
-    L.fic_quadtree_stream_info.argtypes = [vp, C.c_size_t] + [C.POINTER(C.c_int)] * 5 + [C.POINTER(i64)]
-    L.fic_decode_quadtree.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, f32p, C.POINTER(C.c_int)]
+    for fn in (L.fic_quadtree_stream_bound, L.fic_quadtree_rgb_stream_bound):
+        fn.argtypes = [C.c_int] * 4
+        fn.restype = C.c_size_t
+    for fn in (L.fic_encode_quadtree, L.fic_encode_quadtree_rgb):
+        fn.argtypes = [vp, vp] + [C.c_int] * 5 + [C.c_double, vp, C.c_size_t, C.POINTER(C.c_size_t)]
+    for fn in (L.fic_quadtree_stream_info, L.fic_quadtree_rgb_stream_info):
+        fn.argtypes = [vp, C.c_size_t] + [C.POINTER(C.c_int)] * 5 + [C.POINTER(i64)]
+    for fn in (L.fic_decode_quadtree, L.fic_decode_quadtree_rgb):
+        fn.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, f32p, C.POINTER(C.c_int)]
     for name in ABI_SYMBOLS:
         fn = getattr(L, name)
         if fn.restype is C.c_int and name not in ("fic_version", "fic_last_error", "fic_stream_size", "fic_multi_last_error",
-                                                   "fic_multi_handle", "fic_quadtree_stream_bound"):
+                                                   "fic_multi_handle", "fic_quadtree_stream_bound",
+                                                   "fic_quadtree_rgb_stream_bound"):
             fn.restype = C.c_int
     _lib = L
     return L

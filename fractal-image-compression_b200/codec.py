@@ -302,31 +302,39 @@ class Handle:
                                                   C.c_void_p(d_planes_out), C.byref(avg), C.byref(it)))
         return np.float32(avg.value), it.value
 
-    def encode_quadtree(self, plane: np.ndarray, b_max: int, b_min: int, wk: int, max_mse: float) -> bytes:
-        """fic_encode_quadtree (FIC_MODE_GREY_QT extension): the grey plane (uint8 [H, W]) on a quadtree of block sizes
-        b_max .. b_min, split where a block's collage error exceeds max_mse per pixel; wk == 0: every level's whole
-        pool.  Returns the stream."""
-        a = np.ascontiguousarray(plane, dtype=np.uint8)
-        H, W = a.shape
-        cap = self._L.fic_quadtree_stream_bound(W, H, b_max, b_min)
+    def encode_quadtree(self, planes: np.ndarray, b_max: int, b_min: int, wk: int, max_mse: float) -> bytes:
+        """fic_encode_quadtree (FIC_MODE_GREY_QT extension) on a grey plane (uint8 [H, W]), or fic_encode_quadtree_rgb
+        (FIC_MODE_RGB_QT) on RGB planes (uint8 [3, H, W]): the image on a quadtree of block sizes b_max .. b_min, split
+        where a block's collage error exceeds max_mse per pixel and channel; wk == 0: every level's whole pool.  Returns
+        the stream."""
+        a = np.ascontiguousarray(planes, dtype=np.uint8)
+        rgb = a.ndim == 3
+        assert not rgb or a.shape[0] == 3
+        H, W = a.shape[-2:]
+        bound, fn = ((self._L.fic_quadtree_rgb_stream_bound, self._L.fic_encode_quadtree_rgb) if rgb else
+                     (self._L.fic_quadtree_stream_bound, self._L.fic_encode_quadtree))
+        cap = bound(W, H, b_max, b_min)
         buf = np.empty(max(cap, 1), np.uint8)
         n = C.c_size_t(0)
-        self._check(self._L.fic_encode_quadtree(self._h, _ptr(a), W, H, b_max, b_min, wk, float(max_mse), _ptr(buf), cap,
-                                                C.byref(n)))
+        self._check(fn(self._h, _ptr(a), W, H, b_max, b_min, wk, float(max_mse), _ptr(buf), cap, C.byref(n)))
         return buf[:n.value].tobytes()
 
     def decode_quadtree(self, stream: bytes, max_iters: int = 50, out: np.ndarray | None = None):
-        """fic_decode_quadtree: returns (plane uint8 [H, W], avgError float32, iterations)."""
+        """fic_decode_quadtree: returns (plane uint8 [H, W], avgError float32, iterations); a stream whose first int is
+        FIC_MODE_RGB_QT goes to fic_decode_quadtree_rgb and returns planes uint8 [3, H, W]."""
         W, H = struct.unpack(">2i", stream[4:12]) if len(stream) >= 32 else (0, 0)
         if not (0 < W <= 32768 and 0 < H <= 32768):
             W = H = 0  # the library rejects the stream
+        rgb = _is_rgb_quadtree(stream)
+        shape = (3, H, W) if rgb else (H, W)
         if out is None:
-            out = np.empty((H, W), np.uint8)
-        assert out.dtype == np.uint8 and out.shape == (H, W) and out.flags["C_CONTIGUOUS"]
+            out = np.empty(shape, np.uint8)
+        assert out.dtype == np.uint8 and out.shape == shape and out.flags["C_CONTIGUOUS"]
         buf = np.frombuffer(stream, np.uint8)
         avg = C.c_float(0.0)
         it = C.c_int(0)
-        self._check(self._L.fic_decode_quadtree(self._h, _ptr(buf), len(buf), max_iters, _ptr(out), C.byref(avg), C.byref(it)))
+        fn = self._L.fic_decode_quadtree_rgb if rgb else self._L.fic_decode_quadtree
+        self._check(fn(self._h, _ptr(buf), len(buf), max_iters, _ptr(out), C.byref(avg), C.byref(it)))
         return out, np.float32(avg.value), it.value
 
     def collage(self, argb: np.ndarray, info: np.ndarray, B: int, wk: int, rgb: bool):
@@ -484,13 +492,19 @@ def stream_read(stream: bytes):
     return (rgb if rgb == _lib.FIC_MODE_GREY_ISO else bool(rgb)), W, H, B, wk, q
 
 
+def _is_rgb_quadtree(stream: bytes) -> bool:
+    return len(stream) >= 4 and struct.unpack(">i", stream[:4])[0] == _lib.FIC_MODE_RGB_QT
+
+
 def quadtree_stream_info(stream: bytes):
-    """fic_quadtree_stream_info: (W, H, b_max, b_min, wk, n_leaves) of a checked quadtree stream."""
+    """fic_quadtree_stream_info (or fic_quadtree_rgb_stream_info for a stream whose first int is FIC_MODE_RGB_QT):
+    (W, H, b_max, b_min, wk, n_leaves) of a checked quadtree stream."""
     L = _lib.load()
     buf = np.frombuffer(stream, np.uint8)
     v = [C.c_int() for _ in range(5)]
     n = C.c_int64()
-    rc = L.fic_quadtree_stream_info(_ptr(buf), len(buf), *[C.byref(x) for x in v], C.byref(n))
+    fn = L.fic_quadtree_rgb_stream_info if _is_rgb_quadtree(stream) else L.fic_quadtree_stream_info
+    rc = fn(_ptr(buf), len(buf), *[C.byref(x) for x in v], C.byref(n))
     if rc:
         raise FicError(rc, "malformed quadtree stream")
     return tuple(x.value for x in v) + (n.value,)

@@ -1080,47 +1080,43 @@ int fic_stream_read_codes(const uint8_t *stream, size_t nbytes, int32_t *qcodes)
     return FIC_OK;
 }
 
-// ---- quadtree extension (FIC_MODE_GREY_QT) ---------------------------------------------------------------------------
+// ---- quadtree extension (FIC_MODE_GREY_QT, FIC_MODE_RGB_QT) ---------------------------------------------------------
+// One body per entry for both modes: the mode decides the channel count (the level encodes, the planes in and out) and,
+// inside qt_geom / qt_parse, the header value and the leaf size.
 
-size_t fic_quadtree_stream_bound(int W, int H, int b_max, int b_min)
-{
-    if (b_max <= 0 || b_min <= 0 || W <= 0 || H <= 0) return 0;
-    const size_t top = (size_t)(W / b_max) * (size_t)(H / b_max);
-    return kQtHeaderBytes + ((top + 3) & ~(size_t)3) + 12 * (size_t)(W / b_min) * (size_t)(H / b_min);
-}
-
-// One upload, then every level's ordinary grey encode (the engine fic_encode_grey_u8 would pick, into that level's code
-// table), one decimation of the source for the collage errors, and the stream body built on the device
-// (launch_qt_stream); the body comes down in one copy once the leaf count is known.
-int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b_max, int b_min, int wk, double max_mse,
-                        uint8_t *stream, size_t capacity, size_t *stream_bytes)
+// One upload, then every level's ordinary grey or RGB encode (the engine fic_encode_grey_u8 / fic_encode_rgb_planes would
+// pick, into that level's code table), one decimation of the source for the collage errors, and the stream body built on
+// the device (launch_qt_stream); the body comes down in one copy once the leaf count is known.
+static int encode_quadtree(fic_handle *h, int mode, const uint8_t *planes, int W, int H, int b_max, int b_min, int wk,
+                           double max_mse, uint8_t *stream, size_t capacity, size_t *stream_bytes)
 {
     if (!h) return FIC_E_ARG;
-    if (!plane || !stream_bytes) return set_err(h, FIC_E_ARG, "plane and stream_bytes must be non-NULL");
+    if (!planes || !stream_bytes) return set_err(h, FIC_E_ARG, "%s and stream_bytes must be non-NULL", mode == FIC_MODE_RGB_QT ? "planes" : "plane");
     if (max_mse != max_mse) return set_err(h, FIC_E_ARG, "max_mse is NaN");
     QtGeom q;
     const char *why = "";
-    int rc = qt_geom(W, H, b_max, b_min, wk, &q, &why);
+    int rc = qt_geom(mode, W, H, b_max, b_min, wk, &q, &why);
     if (rc) return set_err(h, rc, "%s", why);
     CU(cudaSetDevice(h->device));
     reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
     const Geom &fine = q.g[q.nl - 1];
-    ENSURE(w.src, S_SRC, (size_t)W * H);
-    ENSURE(w.dec, S_DEC, (size_t)fine.sw * fine.sh);
-    ENSURE(w.info, S_INFO, sizeof(float) * 3 * fine.NR);
-    ENSURE(w.qt_codes, S_QT_CODES, sizeof(int32_t) * 3 * q.codes);
+    const size_t C = (size_t)fine.C, S = (size_t)code_stride(fine);
+    ENSURE(w.src, S_SRC, C * W * H);
+    ENSURE(w.dec, S_DEC, C * fine.sw * fine.sh);
+    ENSURE(w.info, S_INFO, sizeof(float) * S * fine.NR);
+    ENSURE(w.qt_codes, S_QT_CODES, sizeof(int32_t) * S * q.codes);
     ENSURE(w.qt_err, S_QT_ERR, sizeof(uint32_t) * qt_err_words(q));
-    ENSURE(w.qt_stream, S_QT_STREAM, fic_quadtree_stream_bound(W, H, b_max, b_min) - kQtHeaderBytes);
+    ENSURE(w.qt_stream, S_QT_STREAM, qt_stream_bound(mode, W, H, b_max, b_min) - kQtHeaderBytes);
     DrainOnExit drain(s);
     CU(cudaEventRecord(h->call_begin, s));
-    CU(cudaMemcpyAsync(w.src, plane, (size_t)W * H, cudaMemcpyHostToDevice, s));
+    CU(cudaMemcpyAsync(w.src, planes, C * W * H, cudaMemcpyHostToDevice, s));
     for (int L = 0; L < q.nl; L++) {
         const Geom &g = q.g[L];
         EncodePlan plan;
         if ((rc = status_err(h, plan_encode(h->enc, g, 0, g.NR, 1, false, s, &plan)))) return rc;
-        if ((rc = status_err(h, run_encode(h->enc, w, g, plan, w.src, false, 0, g.NR, 1, w.info, w.qt_codes + 3 * q.first[L], &h->tm, s))))
+        if ((rc = status_err(h, run_encode(h->enc, w, g, plan, w.src, false, 0, g.NR, 1, w.info, w.qt_codes + S * q.first[L], &h->tm, s))))
             return rc;
         CU(cudaStreamSynchronize(s));  // the level's stage events, before the next level records them again
         read_stages(h->enc, &h->tm, nullptr, nullptr);
@@ -1131,10 +1127,10 @@ int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b
     CU(cudaMemcpyAsync(h->h_acc, w.qt_err, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     const int64_t leaves = *(const uint32_t *)h->h_acc;
-    const size_t need = kQtHeaderBytes + (size_t)q.flag_bytes + 12 * (size_t)leaves;
+    const size_t need = kQtHeaderBytes + (size_t)q.flag_bytes + qt_leaf_bytes(q) * (size_t)leaves;
     *stream_bytes = need;
     if (!stream || capacity < need) return set_err(h, FIC_E_ARG, "the stream needs %zu bytes, capacity is %zu", need, capacity);
-    const int32_t hd[8] = {FIC_MODE_GREY_QT, W, H, 0, wk, b_max, b_min, (int32_t)leaves};
+    const int32_t hd[8] = {mode, W, H, 0, wk, b_max, b_min, (int32_t)leaves};
     for (int k = 0; k < 8; k++) put_be32(stream + 4 * k, hd[k]);
     CU(cudaMemcpyAsync(stream + kQtHeaderBytes, w.qt_stream, need - kQtHeaderBytes, cudaMemcpyDeviceToHost, s));
     CU(cudaEventRecord(h->call_end, s));
@@ -1144,12 +1140,12 @@ int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b
     return FIC_OK;
 }
 
-int fic_quadtree_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *H, int *b_max, int *b_min, int *wk,
-                             int64_t *n_leaves)
+static int quadtree_stream_info(int mode, const uint8_t *stream, size_t nbytes, int *W, int *H, int *b_max, int *b_min,
+                                int *wk, int64_t *n_leaves)
 {
     QtGeom q;
     const char *why = "";
-    int rc = qt_parse(stream, nbytes, &q, nullptr, true, &why);
+    int rc = qt_parse(mode, stream, nbytes, &q, nullptr, true, &why);
     if (rc) return rc;
     if (W) *W = q.g[0].W;
     if (H) *H = q.g[0].H;
@@ -1160,38 +1156,78 @@ int fic_quadtree_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *
     return FIC_OK;
 }
 
-int fic_decode_quadtree(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *plane_out,
-                        float *avg_error, int *iterations)
+static int decode_quadtree(fic_handle *h, int mode, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *planes_out,
+                           float *avg_error, int *iterations)
 {
     if (!h) return FIC_E_ARG;
-    if (!stream || !plane_out) return set_err(h, FIC_E_ARG, "stream and plane_out must be non-NULL");
+    if (!stream || !planes_out) return set_err(h, FIC_E_ARG, "stream and %s must be non-NULL", mode == FIC_MODE_RGB_QT ? "planes_out" : "plane_out");
     if (max_iters < 1) return set_err(h, FIC_E_ARG, "max_iters must be >= 1");
     QtGeom q;
     const char *why = "";
-    int rc = qt_parse(stream, nbytes, &q, nullptr, false, &why);
+    int rc = qt_parse(mode, stream, nbytes, &q, nullptr, false, &why);
     if (rc) return set_err(h, rc, "%s", why);
     std::vector<int32_t> base((size_t)q.g[0].NR);  // first leaf of every top block (the first pass gave their count)
-    qt_parse(stream, nbytes, &q, base.data(), false, &why);
+    qt_parse(mode, stream, nbytes, &q, base.data(), false, &why);
     CU(cudaSetDevice(h->device));
     reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
     const Geom &g = q.g[0];
-    const size_t plane = (size_t)g.W * g.H, bmin = (size_t)q.g[q.nl - 1].B;
-    const size_t cells = plane / (bmin * bmin), used = kQtHeaderBytes + (size_t)q.flag_bytes + 12 * (size_t)q.leaves;
-    ENSURE(w.img, S_IMG, plane);
-    ENSURE(w.dec, S_DEC, (size_t)g.sw * g.sh);
-    ENSURE(w.dec2, S_DEC2, (size_t)g.sw * g.sh);
+    const size_t C = (size_t)g.C, plane = (size_t)g.W * g.H, bmin = (size_t)q.g[q.nl - 1].B;
+    const size_t cells = plane / (bmin * bmin), used = kQtHeaderBytes + (size_t)q.flag_bytes + qt_leaf_bytes(q) * (size_t)q.leaves;
+    ENSURE(w.img, S_IMG, C * plane);
+    ENSURE(w.dec, S_DEC, C * g.sw * g.sh);
+    ENSURE(w.dec2, S_DEC2, C * g.sw * g.sh);
     ENSURE(w.state, S_STATE, sizeof(DecodeState));
     ENSURE(w.qt_stream, S_QT_STREAM, used - kQtHeaderBytes);
-    ENSURE(w.qt_leaf, S_QT_LEAF, sizeof(int4) * q.leaves);
+    ENSURE(w.qt_leaf, S_QT_LEAF, sizeof(int4) * (C == 3 ? 2 : 1) * q.leaves);  // k_qt_dequant's records
     ENSURE(w.qt_map, S_QT_MAP, sizeof(int32_t) * (cells + base.size()));
     DrainOnExit drain(s);
     CU(cudaEventRecord(h->call_begin, s));
     CU(cudaMemcpyAsync(w.qt_stream, stream + kQtHeaderBytes, used - kQtHeaderBytes, cudaMemcpyHostToDevice, s));
     CU(cudaMemcpyAsync(w.qt_map + cells, base.data(), sizeof(int32_t) * base.size(), cudaMemcpyHostToDevice, s));
-    const Status st = decode_quadtree_run(w, q, max_iters, plane_out, avg_error, iterations, h->h_acc, h->call_begin, h->call_end, &h->tm, s);
+    const Status st = decode_quadtree_run(w, q, max_iters, planes_out, avg_error, iterations, h->h_acc, h->call_begin, h->call_end, &h->tm, s);
     return status_err(h, st, "a leaf indexes outside its level's domain pool");
+}
+
+size_t fic_quadtree_stream_bound(int W, int H, int b_max, int b_min) { return qt_stream_bound(FIC_MODE_GREY_QT, W, H, b_max, b_min); }
+
+int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b_max, int b_min, int wk, double max_mse,
+                        uint8_t *stream, size_t capacity, size_t *stream_bytes)
+{
+    return encode_quadtree(h, FIC_MODE_GREY_QT, plane, W, H, b_max, b_min, wk, max_mse, stream, capacity, stream_bytes);
+}
+
+int fic_quadtree_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *H, int *b_max, int *b_min, int *wk,
+                             int64_t *n_leaves)
+{
+    return quadtree_stream_info(FIC_MODE_GREY_QT, stream, nbytes, W, H, b_max, b_min, wk, n_leaves);
+}
+
+int fic_decode_quadtree(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *plane_out,
+                        float *avg_error, int *iterations)
+{
+    return decode_quadtree(h, FIC_MODE_GREY_QT, stream, nbytes, max_iters, plane_out, avg_error, iterations);
+}
+
+size_t fic_quadtree_rgb_stream_bound(int W, int H, int b_max, int b_min) { return qt_stream_bound(FIC_MODE_RGB_QT, W, H, b_max, b_min); }
+
+int fic_encode_quadtree_rgb(fic_handle *h, const uint8_t *planes, int W, int H, int b_max, int b_min, int wk,
+                            double max_mse, uint8_t *stream, size_t capacity, size_t *stream_bytes)
+{
+    return encode_quadtree(h, FIC_MODE_RGB_QT, planes, W, H, b_max, b_min, wk, max_mse, stream, capacity, stream_bytes);
+}
+
+int fic_quadtree_rgb_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *H, int *b_max, int *b_min, int *wk,
+                                 int64_t *n_leaves)
+{
+    return quadtree_stream_info(FIC_MODE_RGB_QT, stream, nbytes, W, H, b_max, b_min, wk, n_leaves);
+}
+
+int fic_decode_quadtree_rgb(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *planes_out,
+                            float *avg_error, int *iterations)
+{
+    return decode_quadtree(h, FIC_MODE_RGB_QT, stream, nbytes, max_iters, planes_out, avg_error, iterations);
 }
 
 }  // extern "C"

@@ -954,11 +954,13 @@ __global__ void k_replay_walk(const int32_t *__restrict__ perr, int64_t count, c
     }
 }
 
-// ---- quadtree extension (FIC_MODE_GREY_QT) --------------------------------------------------------------------------
+// ---- quadtree extension (FIC_MODE_GREY_QT, FIC_MODE_RGB_QT) ----------------------------------------------------------
 
 // One thread per top block: its leaves (stream at `stream`, leaves from flag_bytes on, big endian) dequantised with their
-// level's Geom as k_dequant does -- leaf[i] = {a, b, byte offset of the domain block in the decimated plane, log2 B_L} --
-// and every b_min x b_min cell of a leaf pointed at it in map (cw = W / b_min cells per row).
+// level's Geom as k_dequant does -- grey leaf[i] = {a, b, byte offset of the domain block in a decimated plane,
+// log2 B_L}; RGB leaf[2i] = {a, bR, bG, bB}, leaf[2i + 1] = {byte offset, log2 B_L, 0, 0} -- and every b_min x b_min cell
+// of a leaf pointed at it in map (cw = W / b_min cells per row).
+template <int C>
 __global__ void k_qt_dequant(QtGeom q, const uint8_t *__restrict__ stream, const int32_t *__restrict__ base,
                              int4 *__restrict__ leaf, int32_t *__restrict__ map, int lcell, DecodeState *st)
 {
@@ -968,16 +970,23 @@ __global__ void k_qt_dequant(QtGeom q, const uint8_t *__restrict__ stream, const
     int32_t i = base[t];
     qt_visit_leaves(q, t, stream[t], [&](int L, int64_t j) {
         const Geom &g = q.g[L];
-        const uint8_t *p = stream + q.flag_bytes + 12 * (int64_t)i;
+        const uint8_t *p = stream + q.flag_bytes + (C == 1 ? 12 : 20) * (int64_t)i;
         auto be = [](const uint8_t *b) { return (int32_t)(((uint32_t)b[0] << 24) | ((uint32_t)b[1] << 16) | ((uint32_t)b[2] << 8) | b[3]); };
         int64_t idx = code_pool_index(g, j, (float)be(p));
         if (idx < 0) {
             atomicOr(&st->bad_index, 1ull);
             idx = 0;
         }
-        const float a = __fdiv_rn((float)be(p + 4), kGreyAScale), b = (float)be(p + 8);
+        const float a = __fdiv_rn((float)be(p + 4), C == 1 ? kGreyAScale : kRgbAScale);
+        const float b = C == 1 ? (float)be(p + 8) : __fdiv_rn((float)be(p + 8), kRgbBScale);
         const int doff = (int)(idx / g.dpw) * g.step * g.sw + (int)(idx % g.dpw) * g.step;
-        leaf[i] = make_int4(__float_as_int(a), __float_as_int(b), doff, __ffs(g.B) - 1);
+        if (C == 1) {
+            leaf[i] = make_int4(__float_as_int(a), __float_as_int(b), doff, __ffs(g.B) - 1);
+        } else {  // {a, bR, bG, bB}: FC:446-450, blue is not scaled
+            const float bg = __fdiv_rn((float)be(p + 12), kRgbBScale), bb = (float)be(p + 16);
+            leaf[2 * (int64_t)i] = make_int4(__float_as_int(a), __float_as_int(b), __float_as_int(bg), __float_as_int(bb));
+            leaf[2 * (int64_t)i + 1] = make_int4(doff, __ffs(g.B) - 1, 0, 0);
+        }
         const int c0 = (int)(j % g.rpw) * (g.B >> lcell), r0 = (int)(j / g.rpw) * (g.B >> lcell);
         for (int r = 0; r < (g.B >> lcell); r++)
             for (int c = 0; c < (g.B >> lcell); c++) map[(int64_t)(r0 + r) * cw + c0 + c] = i;
@@ -985,77 +994,95 @@ __global__ void k_qt_dequant(QtGeom q, const uint8_t *__restrict__ stream, const
     });
 }
 
-// One quadtree sweep: k_decode_sweep_v8's 8 x 2 pixel strips (grey), each pixel from the leaf that covers it -- read
-// through the leaf map at b_min granularity: one leaf per strip for b_min >= 8, one per quad for b_min = 4 (QUAD) -- at
-// its own block size.  FIRST: the sweep from the constant-128 image reads neither image nor plane.  Every sweep folds
-// itself: the last CTA turns the exact total S into avgError = (float)S / (float)(W*H), which needs no replay because
-// the rule is stated on the exact sum.
-template <bool FIRST, bool QUAD>
+// One quadtree sweep: k_decode_sweep_v8's 8 x 2 pixel strips over each of the C planes, each pixel from the leaf that
+// covers it -- read through the leaf map at b_min granularity: one leaf per strip for b_min >= 8, one per quad for
+// b_min = 4 (QUAD); one lookup serves every channel -- at its own block size.  FIRST: the sweep from the constant-128
+// image reads neither image nor plane.  Every sweep folds itself: the last CTA turns the exact total S (over pixels and
+// channels) into avgError = (float)S / (float)(W*H), which needs no replay because the rule is stated on the exact sum.
+template <int C, bool FIRST, bool QUAD>
 __global__ void __launch_bounds__(256)
 k_decode_sweep_qt(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img, uint8_t *__restrict__ dec_out,
                   const int4 *__restrict__ leaf, const int32_t *__restrict__ map, Geom g, int lcell, SweepCtl ctl, int last)
 {
     if (sweep_done(ctl)) return;
+    constexpr int LS = C == 1 ? 1 : 2;  // int4 records per leaf (k_qt_dequant)
     const uint32_t usw8 = (uint32_t)(g.W / 8), nstrips = usw8 * (uint32_t)(g.H / 2);
     const int cw = g.W >> lcell;
+    const int64_t planeI = (int64_t)g.W * g.H, planeD = (int64_t)g.sw * g.sh;
     unsigned long long local = 0;
     for (uint32_t t = blockIdx.x * blockDim.x + threadIdx.x; t < nstrips; t += gridDim.x * blockDim.x) {
         const uint32_t uqy = t / usw8;
         const int qy = (int)uqy, s8 = (int)(t - uqy * usw8);
         const int y = 2 * qy, x0 = 8 * s8;
         const int32_t *mrow = map + (int64_t)(y >> lcell) * cw;
-        uint8_t *pi = img + (int64_t)y * g.W + x0;
-        uint2 o0 = make_uint2(0x80808080u, 0x80808080u), o1 = o0;
-        if (!FIRST) {
-            o0 = *(const uint2 *)pi;
-            o1 = *(const uint2 *)(pi + g.W);
-        }
-        const uint32_t old0[2] = {o0.x, o0.y}, old1[2] = {o1.x, o1.y};
-        uint32_t n0[2] = {0, 0}, n1[2] = {0, 0}, nd = 0;
-        uint32_t dr0[4], dr1[4];  // domain bytes of the four quads: row ry (low 16 bits hold 2 pixels) and ry + 1
-        int4 lf = make_int4(0, 0, 0, 0);
-        if (!QUAD) {
-            lf = __ldg(leaf + __ldg(mrow + (x0 >> lcell)));
-            const int bm = (1 << lf.w) - 1;
+        // the leaf of the strip (!QUAD) or of each quad (QUAD): grey {a, b, doff, log2 B}; RGB {a, bR, bG, bB} in lf and
+        // {doff, log2 B} in lp
+        int4 lf[QUAD ? 4 : 1], lp[QUAD ? 4 : 1];
 #pragma unroll
-            for (int qd = 0; qd < 4; qd++) dr0[qd] = dr1[qd] = 0x8080u;
-            if (!FIRST) {  // 2-byte aligned: the domain grid stride B_L / 4 and the row length W / 2 are even for B_L >= 8
-                const uint16_t *pd = (const uint16_t *)(dec_in + lf.z + (y & bm) * g.sw + (x0 & bm));
+        for (int c = 0; c < C; c++) {
+            uint8_t *pi = img + c * planeI + (int64_t)y * g.W + x0;
+            const uint8_t *din = dec_in + c * planeD;
+            uint2 o0 = make_uint2(0x80808080u, 0x80808080u), o1 = o0;
+            if (!FIRST) {
+                o0 = *(const uint2 *)pi;
+                o1 = *(const uint2 *)(pi + g.W);
+            }
+            const uint32_t old0[2] = {o0.x, o0.y}, old1[2] = {o1.x, o1.y};
+            uint32_t n0[2] = {0, 0}, n1[2] = {0, 0}, nd = 0;
+            uint32_t dr0[4], dr1[4];  // domain bytes of the four quads: row ry (low 16 bits hold 2 pixels) and ry + 1
+            if (!QUAD) {
+                if (c == 0) {
+                    const int i = __ldg(mrow + (x0 >> lcell));
+                    lf[0] = __ldg(leaf + LS * i);
+                    lp[0] = C == 1 ? make_int4(lf[0].z, lf[0].w, 0, 0) : __ldg(leaf + LS * i + 1);
+                }
+                const int bm = (1 << lp[0].y) - 1;
 #pragma unroll
-                for (int qd = 0; qd < 4; qd++) {
-                    dr0[qd] = __ldg(pd + qd);
-                    dr1[qd] = __ldg(pd + g.sw / 2 + qd);
+                for (int qd = 0; qd < 4; qd++) dr0[qd] = dr1[qd] = 0x8080u;
+                if (!FIRST) {  // 2-byte aligned: the domain grid stride B_L / 4 and the row length W / 2 are even for B_L >= 8
+                    const uint16_t *pd = (const uint16_t *)(din + lp[0].x + (y & bm) * g.sw + (x0 & bm));
+#pragma unroll
+                    for (int qd = 0; qd < 4; qd++) {
+                        dr0[qd] = __ldg(pd + qd);
+                        dr1[qd] = __ldg(pd + g.sw / 2 + qd);
+                    }
                 }
             }
-        }
 #pragma unroll
-        for (int qd = 0; qd < 4; qd++) {
-            const int x = x0 + 2 * qd;
-            if (QUAD) {
-                lf = __ldg(leaf + __ldg(mrow + (x >> lcell)));
-                dr0[qd] = dr1[qd] = 0x8080u;
-                if (!FIRST) {
-                    const int bm = (1 << lf.w) - 1;
-                    const uint8_t *pd = dec_in + lf.z + (y & bm) * g.sw + (x & bm);
-                    dr0[qd] = (uint32_t)__ldg(pd) | ((uint32_t)__ldg(pd + 1) << 8);
-                    dr1[qd] = (uint32_t)__ldg(pd + g.sw) | ((uint32_t)__ldg(pd + g.sw + 1) << 8);
+            for (int qd = 0; qd < 4; qd++) {
+                const int x = x0 + 2 * qd;
+                const int k = QUAD ? qd : 0;
+                if (QUAD) {
+                    if (c == 0) {
+                        const int i = __ldg(mrow + (x >> lcell));
+                        lf[k] = __ldg(leaf + LS * i);
+                        lp[k] = C == 1 ? make_int4(lf[k].z, lf[k].w, 0, 0) : __ldg(leaf + LS * i + 1);
+                    }
+                    dr0[qd] = dr1[qd] = 0x8080u;
+                    if (!FIRST) {
+                        const int bm = (1 << lp[k].y) - 1;
+                        const uint8_t *pd = din + lp[k].x + (y & bm) * g.sw + (x & bm);
+                        dr0[qd] = (uint32_t)__ldg(pd) | ((uint32_t)__ldg(pd + 1) << 8);
+                        dr1[qd] = (uint32_t)__ldg(pd + g.sw) | ((uint32_t)__ldg(pd + g.sw + 1) << 8);
+                    }
                 }
+                const float a = __int_as_float(lf[k].x);
+                const float b = __int_as_float(c == 0 ? lf[k].y : (c == 1 ? lf[k].z : lf[k].w));
+                const uint32_t v00 = decode_px(a, b, dr0[qd] & 0xffu), v10 = decode_px(a, b, dr0[qd] >> 8);
+                const uint32_t v01 = decode_px(a, b, dr1[qd] & 0xffu), v11 = decode_px(a, b, dr1[qd] >> 8);
+                const int sh = 16 * (qd & 1);
+                const uint32_t newq = v00 | (v10 << 8) | (v01 << 16) | (v11 << 24);
+                const uint32_t oldq = ((old0[qd >> 1] >> sh) & 0xffffu) | (((old1[qd >> 1] >> sh) & 0xffffu) << 16);
+                const uint32_t ad = __vabsdiffu4(oldq, newq);
+                local += (unsigned long long)__dp4a(ad, ad, 0u);
+                n0[qd >> 1] |= (newq & 0xffffu) << sh;
+                n1[qd >> 1] |= (newq >> 16) << sh;
+                nd |= (uint32_t)dec_tap4((int)v00, (int)v10, (int)v01, (int)v11, x, g.H, C == 3) << (8 * qd);
             }
-            const float a = __int_as_float(lf.x), b = __int_as_float(lf.y);
-            const uint32_t v00 = decode_px(a, b, dr0[qd] & 0xffu), v10 = decode_px(a, b, dr0[qd] >> 8);
-            const uint32_t v01 = decode_px(a, b, dr1[qd] & 0xffu), v11 = decode_px(a, b, dr1[qd] >> 8);
-            const int sh = 16 * (qd & 1);
-            const uint32_t newq = v00 | (v10 << 8) | (v01 << 16) | (v11 << 24);
-            const uint32_t oldq = ((old0[qd >> 1] >> sh) & 0xffffu) | (((old1[qd >> 1] >> sh) & 0xffffu) << 16);
-            const uint32_t ad = __vabsdiffu4(oldq, newq);
-            local += (unsigned long long)__dp4a(ad, ad, 0u);
-            n0[qd >> 1] |= (newq & 0xffffu) << sh;
-            n1[qd >> 1] |= (newq >> 16) << sh;
-            nd |= (uint32_t)dec_tap4((int)v00, (int)v10, (int)v01, (int)v11, x, g.H, false) << (8 * qd);
+            *(uint2 *)pi = make_uint2(n0[0], n0[1]);
+            *(uint2 *)(pi + g.W) = make_uint2(n1[0], n1[1]);
+            *(uint32_t *)(dec_out + c * planeD + (int64_t)qy * g.sw + 4 * s8) = nd;
         }
-        *(uint2 *)pi = make_uint2(n0[0], n0[1]);
-        *(uint2 *)(pi + g.W) = make_uint2(n1[0], n1[1]);
-        *(uint32_t *)(dec_out + (int64_t)qy * g.sw + 4 * s8) = nd;
     }
     const unsigned long long tot = cta_sum(local);
     if (threadIdx.x == 0) {
@@ -1458,16 +1485,17 @@ Status decode_float_sum(const Work &w, const int32_t *terms, int64_t count, floa
     return Status();
 }
 
-template <bool FIRST>
+template <int C, bool FIRST>
 static void launch_sweep_qt(int64_t need, bool quad, cudaStream_t s, const uint8_t *dec_in, uint8_t *img, uint8_t *dec_out,
                             const int4 *leaf, const int32_t *map, Geom g, int lcell, SweepCtl ctl, int last)
 {
-    if (quad) launch_wave<k_decode_sweep_qt<FIRST, true>>(need, s, dec_in, img, dec_out, leaf, map, g, lcell, ctl, last);
-    else launch_wave<k_decode_sweep_qt<FIRST, false>>(need, s, dec_in, img, dec_out, leaf, map, g, lcell, ctl, last);
+    if (quad) launch_wave<k_decode_sweep_qt<C, FIRST, true>>(need, s, dec_in, img, dec_out, leaf, map, g, lcell, ctl, last);
+    else launch_wave<k_decode_sweep_qt<C, FIRST, false>>(need, s, dec_in, img, dec_out, leaf, map, g, lcell, ctl, last);
 }
 
-Status decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
-                                 int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, cudaStream_t s)
+template <int C>
+static Status decode_quadtree_c(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
+                                int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, cudaStream_t s)
 {
     const Geom &g = q.g[0];
     const DecodeState *hs = (const DecodeState *)h_scratch;
@@ -1478,31 +1506,33 @@ Status decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_
     int launches = 0;
     Status st;
     DCU(cudaMemsetAsync(w.state, 0, sizeof(DecodeState), s));
-    k_qt_dequant<<<(unsigned)((g.NR + 127) / 128), 128, 0, s>>>(q, w.qt_stream, base, w.qt_leaf, w.qt_map, lcell, w.state);
+    k_qt_dequant<C><<<(unsigned)((g.NR + 127) / 128), 128, 0, s>>>(q, w.qt_stream, base, w.qt_leaf, w.qt_map, lcell, w.state);
     launches++;
     const int64_t need = ((int64_t)(g.W / 8) * (g.H / 2) + 255) / 256;
-    const bool speculative_out = plane <= ((size_t)4 << 20);  // as decode_run: copy behind every batch of sweeps
+    const bool speculative_out = C * plane <= ((size_t)4 << 20);  // as decode_run: copy behind every batch of sweeps
+    // as decode_run: RGB decodes need more sweeps than grey (13-22 against 5-9 in the fixed decoder)
+    const int batch = (C == 3 && speculative_out) ? 16 : 8;
     uint8_t *dcur = w.dec, *dnext = w.dec2;
     int it = 0;
     while (it < max_iters) {
-        const int batch_end = it + 8 < max_iters ? it + 8 : max_iters;
+        const int batch_end = it + batch < max_iters ? it + batch : max_iters;
         for (; it < batch_end; it++) {
             const SweepCtl ctl = {w.state, it, 1, fwh};
             const int last = it == max_iters - 1;
-            (it == 0 ? launch_sweep_qt<true> : launch_sweep_qt<false>)(need, lcell == 2, s, dcur, w.img, dnext, w.qt_leaf, w.qt_map, g, lcell, ctl, last);
+            (it == 0 ? launch_sweep_qt<C, true> : launch_sweep_qt<C, false>)(need, lcell == 2, s, dcur, w.img, dnext, w.qt_leaf, w.qt_map, g, lcell, ctl, last);
             launches++;
             uint8_t *t = dcur; dcur = dnext; dnext = t;
         }
         DCU(cudaMemcpyAsync(h_scratch, w.state, sizeof(DecodeState), cudaMemcpyDeviceToHost, s));
         if (speculative_out) {
-            DCU(cudaMemcpyAsync(planes_out, w.img, plane, cudaMemcpyDeviceToHost, s));
+            DCU(cudaMemcpyAsync(planes_out, w.img, C * plane, cudaMemcpyDeviceToHost, s));
             DCU(cudaEventRecord(end, s));
         }
         if ((st = sync_state(hs, s)).rc) return st;
         if (hs->done) break;
     }
     if (!speculative_out) {
-        DCU(cudaMemcpyAsync(planes_out, w.img, plane, cudaMemcpyDeviceToHost, s));
+        DCU(cudaMemcpyAsync(planes_out, w.img, C * plane, cudaMemcpyDeviceToHost, s));
         DCU(cudaEventRecord(end, s));
         DCU(cudaStreamSynchronize(s));
     }
@@ -1513,6 +1543,13 @@ Status decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_
     if (avg_error) memcpy(avg_error, &hs->avg_bits, sizeof *avg_error);
     if (iterations) *iterations = (int)hs->iters;
     return Status();
+}
+
+Status decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
+                                 int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, cudaStream_t s)
+{
+    return (q.g[0].C == 3 ? decode_quadtree_c<3> : decode_quadtree_c<1>)(w, q, max_iters, planes_out, avg_error, iterations,
+                                                                         h_scratch, ev0, end, tm, s);
 }
 
 }  // namespace fic

@@ -76,9 +76,10 @@ struct Work {
     uint8_t *replay = nullptr;  // decoder, large images: per-chunk records of the exact avgError replay
     // quadtree extension (fic_quadtree.cu)
     uint8_t *qt_stream = nullptr;  // stream body: encode, written by k_qt_decide / k_qt_scatter; decode, the caller's stream
-    int32_t *qt_codes = nullptr;   // encode: every level's quantised codes [NR_L][3], level after level (QtGeom::first)
+    int32_t *qt_codes = nullptr;   // encode: every level's quantised codes [NR_L][3|5], level after level (QtGeom::first)
     uint32_t *qt_err = nullptr;    // encode: leaf total, per-top-block leaf prefixes, per-warp totals, collage errors
-    int4 *qt_leaf = nullptr;       // decode: {a, b, domain byte offset, log2 blockgroesse} per leaf
+    int4 *qt_leaf = nullptr;       // decode, per leaf: grey {a, b, domain byte offset, log2 blockgroesse}; RGB two records,
+                                   // {a, bR, bG, bB} and {domain byte offset, log2 blockgroesse, 0, 0}
     int32_t *qt_map = nullptr;     // decode: leaf of every b_min x b_min cell, then the first leaf of every top block
     size_t cap[24] = {0};
 };
@@ -229,10 +230,10 @@ Status decode_batch_run(const Work &w, const Geom &g, int n, int group, const in
                               uint8_t *planes_out, int max_iters, float *avg_error, int *iterations, void *h_stage,
                               void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, int *bad_image, cudaStream_t s);
 
-// ---- quadtree extension (FIC_MODE_GREY_QT; fic_quadtree.cu) -----------------------------------------------------------
-// Levels L = 0 .. nl - 1 of blockgroesse b_max >> L over one grey image, each with its own Geom (widthKernel wk, or the
-// level's whole pool when wk == 0).  Top blocks are the level-0 range blocks; every per-level table is level-major with
-// level L starting at first[L].
+// ---- quadtree extension (FIC_MODE_GREY_QT, FIC_MODE_RGB_QT; fic_quadtree.cu) ----------------------------------------
+// Levels L = 0 .. nl - 1 of blockgroesse b_max >> L over one grey or RGB image, each with its own Geom (widthKernel wk,
+// or the level's whole pool when wk == 0); the Geoms carry the channel count (Geom::C: 1 grey, 3 RGB).  Top blocks are
+// the level-0 range blocks; every per-level table is level-major with level L starting at first[L].
 constexpr int kQtMaxLevels = 3;
 struct QtGeom {
     int nl;
@@ -244,20 +245,26 @@ struct QtGeom {
     int64_t leaves;              // n_leaves (decode: from the header)
 };
 constexpr size_t kQtHeaderBytes = 32;
-// FIC_E_ARG (with *why) unless b_max in {8, 16}, b_min in {4, 8, 16}, b_min <= b_max, wk >= 0 (0: W == H) and every
-// level passes make_geom.
-int qt_geom(int W, int H, int b_max, int b_min, int wk, QtGeom *q, const char **why);
-// Header, flags and size of a stream (FIC_E_STREAM with *why otherwise); base (optional, NR_top entries): the first leaf
-// of every top block.  check_leaves: also every leaf's domain index against its level's pool.
-int qt_parse(const uint8_t *stream, size_t nbytes, QtGeom *q, int32_t *base, bool check_leaves, const char **why);
+// mode: FIC_MODE_GREY_QT or FIC_MODE_RGB_QT.  FIC_E_ARG (with *why) unless b_max in {8, 16}, b_min in {4, 8, 16},
+// b_min <= b_max, wk >= 0 (0: W == H) and every level passes make_geom.
+int qt_geom(int mode, int W, int H, int b_max, int b_min, int wk, QtGeom *q, const char **why);
+// Bytes per leaf in the stream: 12 ({c, qa, qb}) grey, 20 ({c, qa, qbR, qbG, qbB}) RGB.
+size_t qt_leaf_bytes(const QtGeom &q);
+// Largest stream of the mode and geometry (every block split to b_min); 0 for non-positive arguments.
+size_t qt_stream_bound(int mode, int W, int H, int b_max, int b_min);
+// Header (its first int must be `mode`), flags and size of a stream (FIC_E_STREAM with *why otherwise); base (optional,
+// NR_top entries): the first leaf of every top block.  check_leaves: also every leaf's domain index against its level's
+// pool.
+int qt_parse(int mode, const uint8_t *stream, size_t nbytes, QtGeom *q, int32_t *base, bool check_leaves, const char **why);
 // Words of Work::qt_err an encode needs.
 size_t qt_err_words(const QtGeom &q);
-// After every level's codes are in w.qt_codes and the source's decimated plane in w.dec: collage errors, split flags,
+// After every level's codes are in w.qt_codes and the source's decimated planes in w.dec: collage errors, split flags,
 // leaf scan and leaf scatter into w.qt_stream (flags at 0, leaves at flag_bytes); the leaf count lands in w.qt_err[0].
 int launch_qt_stream(const Work &w, const QtGeom &q, double max_mse, cudaStream_t s);
-// Iterative decode of the stream in w.qt_stream (the first-leaf table in w.qt_map after the cell map) into w.img, copied to
-// planes_out.  avgError = (float)S / (float)(W*H) of the exact sum S of squared changes; stops below 1 or after
-// max_iters sweeps.  Workspace: img, dec, dec2, state, qt_leaf (q.leaves), qt_map.
+// Iterative decode of the stream in w.qt_stream (the first-leaf table in w.qt_map after the cell map) into w.img (C planes),
+// copied to planes_out.  avgError = (float)S / (float)(W*H) of the exact sum S of squared changes over pixels and
+// channels; stops below 1 or after max_iters sweeps.  Workspace: img, dec, dec2 (C planes each), state, qt_leaf
+// (q.leaves records, two int4 each for RGB), qt_map.
 Status decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
                                  int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm,
                                  cudaStream_t s);

@@ -5,6 +5,7 @@
 //   fic_cli roundtrip in.pgm|in.ppm [blockgroesse] [widthKernel]        (prints "MSE <avgError>" like the GUI label)
 //   fic_cli qtroundtrip in.pgm b_max b_min widthKernel max_mse            (quadtree extension, grey: stream size, bits
 //                                                                          per pixel, iterations, avgError, PSNR)
+//   fic_cli qtroundtrip_rgb in.ppm b_max b_min widthKernel max_mse        (the same, RGB: PSNR over the 3*W*H samples)
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -49,6 +50,37 @@ static void write_pnm(const char *path, const RasterImage &img)
     }
 }
 
+// Quadtree round trip on the GPU: grey (the red channel, fic_encode_quadtree) or RGB (three planes,
+// fic_encode_quadtree_rgb).  Prints the stream size, bits per pixel, iterations, avgError and the PSNR over every sample.
+static int qt_roundtrip(const RasterImage &img, bool rgb, int b_max, int b_min, int wk, double max_mse)
+{
+    const int W = img.width, H = img.height, C = rgb ? 3 : 1;
+    const size_t plane_px = (size_t)W * H;
+    std::vector<uint8_t> planes(C * plane_px), out(C * plane_px);
+    for (int c = 0; c < C; c++)  // R, G, B planes; grey: the red channel
+        for (size_t i = 0; i < plane_px; i++) planes[c * plane_px + i] = (uint8_t)((img.argb[i] >> (16 - 8 * c)) & 0xff);
+    std::vector<uint8_t> stream((rgb ? fic_quadtree_rgb_stream_bound : fic_quadtree_stream_bound)(W, H, b_max, b_min) + 1);
+    fic_handle *h = nullptr;
+    size_t n = 0;
+    float avg = 0;
+    int iters = 0;
+    int rc = fic_create(0, &h);
+    if (!rc) rc = (rgb ? fic_encode_quadtree_rgb : fic_encode_quadtree)(h, planes.data(), W, H, b_max, b_min, wk, max_mse, stream.data(), stream.size(), &n);
+    if (!rc) rc = (rgb ? fic_decode_quadtree_rgb : fic_decode_quadtree)(h, stream.data(), n, 50, out.data(), &avg, &iters);
+    if (rc) {
+        fprintf(stderr, "fic_cli: error %d: %s\n", rc, fic_last_error(h));
+        fic_destroy(h);
+        return 1;
+    }
+    fic_destroy(h);
+    double se = 0;
+    for (size_t i = 0; i < planes.size(); i++) se += ((double)planes[i] - out[i]) * ((double)planes[i] - out[i]);
+    const double mse = se / (double)planes.size();
+    printf("bytes %zu bpp %.4f iterations %d MSE %.9g PSNR %.3f dB\n", n, 8.0 * n / plane_px, iters, avg,
+           mse > 0 ? 10.0 * std::log10(255.0 * 255.0 / mse) : INFINITY);
+    return 0;
+}
+
 int main(int argc, char **argv)
 {
     // a trailing "iso" selects the isometry extension for encode / roundtrip
@@ -80,34 +112,11 @@ int main(int argc, char **argv)
             printf("MSE %.9g (%d iterations)\n", FractalCompression::getAvgError(), FractalCompression::lastIterations);
             return 0;
         }
-        if (argc >= 7 && !strcmp(argv[1], "qtroundtrip")) {
-            const RasterImage img = read_pnm(argv[2]);
-            const int W = img.width, H = img.height, b_max = atoi(argv[3]), b_min = atoi(argv[4]), wk = atoi(argv[5]);
-            std::vector<uint8_t> plane((size_t)W * H), out((size_t)W * H);
-            for (size_t i = 0; i < plane.size(); i++) plane[i] = (uint8_t)((img.argb[i] >> 16) & 0xff);  // the red channel
-            std::vector<uint8_t> stream(fic_quadtree_stream_bound(W, H, b_max, b_min) + 1);
-            fic_handle *h = nullptr;
-            size_t n = 0;
-            float avg = 0;
-            int iters = 0;
-            int rc = fic_create(0, &h);
-            if (!rc) rc = fic_encode_quadtree(h, plane.data(), W, H, b_max, b_min, wk, atof(argv[6]), stream.data(), stream.size(), &n);
-            if (!rc) rc = fic_decode_quadtree(h, stream.data(), n, 50, out.data(), &avg, &iters);
-            if (rc) {
-                fprintf(stderr, "fic_cli: error %d: %s\n", rc, fic_last_error(h));
-                fic_destroy(h);
-                return 1;
-            }
-            fic_destroy(h);
-            double se = 0;
-            for (size_t i = 0; i < plane.size(); i++) se += ((double)plane[i] - out[i]) * ((double)plane[i] - out[i]);
-            const double mse = se / (double)plane.size();
-            printf("bytes %zu bpp %.4f iterations %d MSE %.9g PSNR %.3f dB\n", n, 8.0 * n / plane.size(), iters, avg,
-                   mse > 0 ? 10.0 * std::log10(255.0 * 255.0 / mse) : INFINITY);
-            return 0;
-        }
+        if (argc >= 7 && (!strcmp(argv[1], "qtroundtrip") || !strcmp(argv[1], "qtroundtrip_rgb")))
+            return qt_roundtrip(read_pnm(argv[2]), !strcmp(argv[1], "qtroundtrip_rgb"), atoi(argv[3]), atoi(argv[4]),
+                                atoi(argv[5]), atof(argv[6]));
         fprintf(stderr, "usage: fic_cli encode in.pnm out.run [B] [wk] [iso] | decode in.run out.pnm | roundtrip in.pnm [B] [wk] [iso]"
-                        " | qtroundtrip in.pgm b_max b_min wk max_mse\n");
+                        " | qtroundtrip in.pgm b_max b_min wk max_mse | qtroundtrip_rgb in.ppm b_max b_min wk max_mse\n");
         return 2;
     } catch (const std::exception &e) {
         fprintf(stderr, "fic_cli: %s\n", e.what());

@@ -56,7 +56,8 @@ extern "C" {
 #define FIC_MODE_GREY 0     /* {c, a, b} per range                       */
 #define FIC_MODE_RGB 1      /* {c, a, bR, bG, bB} per range              */
 #define FIC_MODE_GREY_ISO 2 /* {c, a, b, k} per range; k = isometry 0..7 */
-#define FIC_MODE_GREY_QT 3  /* quadtree of block sizes (EXTENSION, grey only): see fic_encode_quadtree below */
+#define FIC_MODE_GREY_QT 3  /* quadtree of block sizes (EXTENSION, grey): see fic_encode_quadtree below */
+#define FIC_MODE_RGB_QT 4   /* quadtree of block sizes (EXTENSION, RGB): see fic_encode_quadtree_rgb below */
 
 /* Search engine selection (fic_set_option(FIC_OPT_ENGINE, ...)). */
 #define FIC_ENGINE_AUTO 0   /* tcgen05 search when the window is the whole pool; the fused one-launch encode for the
@@ -234,7 +235,7 @@ int fic_decode_batch_u8(fic_handle *h, int mode, int n_images, int W, int H, int
 int fic_collage(fic_handle *h, int is_rgb, const int32_t *argb, int W, int H, int B, int wk,
                 float *info, int32_t *argb_out);
 
-/* ---- quadtree extension (FIC_MODE_GREY_QT): block sizes chosen per region by collage error ---------------------- */
+/* ---- quadtree extension (FIC_MODE_GREY_QT, FIC_MODE_RGB_QT): block sizes chosen per region by collage error --- */
 
 /* EXTENSION the reference cannot read.  Levels b_max, b_max/2, ..., b_min (b_max in {8, 16}, b_min in {4, 8, 16},
  * b_min <= b_max); level L's codes are exactly what fic_encode_grey_u8(plane, W, H, B_L, wk_L) returns on this handle
@@ -270,6 +271,30 @@ int fic_quadtree_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *
  * fic_quadtree_stream_info. */
 int fic_decode_quadtree(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *plane_out,
                         float *avg_error, int *iterations);
+
+/* RGB quadtree (FIC_MODE_RGB_QT, EXTENSION): the grey rule above with the reference's RGB codes.  Level L's codes are
+ * exactly what fic_encode_rgb_planes(planes, W, H, B_L, wk_L) returns on this handle with its options.  The collage
+ * error sums over the three channels: E = sum over pixels and c in {R, G, B} of (decode_px(a, b_c, d_c) - s_c)^2, the
+ * code {c, qa, qbR, qbG, qbB} dequantised as the RGB decoder does (a = qa / 1e6f, bR = qbR / 1e5f, bG = qbG / 1e5f,
+ * bB = qbB: blue is unscaled, FC:446-450), d_c read from the source's RGB-decimated planes (scaleImageRGB's tap
+ * (p00 + p10 + 2 p01) / 4, FC:901-962).  A block above b_min splits iff (double)E > max_mse * (double)(3 * B_L^2), so
+ * max_mse is a mean squared error per channel sample, as for grey.
+ *
+ * Stream: header 4, W, H, 0, wk, b_max, b_min, n_leaves; the grey stream's split-flag bytes; then 20 bytes per leaf,
+ * {c, qa, qbR, qbG, qbB} as writeData writes that range's RGB code (FC:250-254), in the grey stream's order.  Size:
+ * 32 + pad4(NR_top) + 20 * n_leaves <= fic_quadtree_rgb_stream_bound.
+ *
+ * Pixels in and out: three W*H 8-bit planes R, G, B.  Decode: the constant-128 image in all three planes; each sweep
+ * RGB-decimates the last image and every leaf writes decode_px(a, b_c, d_c) per channel; S is the exact sum of squared
+ * changes over pixels and channels, avgError = (float)S / (float)(W*H).  The grey entries refuse an RGB stream and these
+ * refuse a grey one (FIC_E_STREAM); arguments, capacity, timings and FIC_E_STREAM otherwise as the grey entries. */
+size_t fic_quadtree_rgb_stream_bound(int W, int H, int b_max, int b_min);
+int fic_encode_quadtree_rgb(fic_handle *h, const uint8_t *planes, int W, int H, int b_max, int b_min, int wk,
+                            double max_mse, uint8_t *stream, size_t capacity, size_t *stream_bytes);
+int fic_quadtree_rgb_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *H, int *b_max, int *b_min, int *wk,
+                                 int64_t *n_leaves);
+int fic_decode_quadtree_rgb(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *planes_out,
+                            float *avg_error, int *iterations);
 
 /* ---- multi-GPU: the same encode over several GPUs of one node (SURVEY 8b, 8e) --- */
 

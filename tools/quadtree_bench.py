@@ -1,14 +1,17 @@
-"""Rate, quality and device time of the quadtree extension (FIC_MODE_GREY_QT) against the fixed block sizes.
+"""Rate, quality and device time of the quadtree extension (FIC_MODE_GREY_QT, with --rgb FIC_MODE_RGB_QT) against the
+fixed block sizes.
 
-    python tools/quadtree_bench.py OUT_DIR [--quick]
+    python tools/quadtree_bench.py OUT_DIR [--quick] [--rgb]
 
-Workloads: a structured synthetic 4096^2 image and LenaGrey 256^2, quadtrees (16, 8) and (16, 4) with the whole pool
-and with widthKernel 2 over a sweep of max_mse, and the fixed B = 16 / 8 / 4 encodes of the same images as baselines.
+Workloads: a structured synthetic 4096^2 image and LenaGrey 256^2 (--rgb: LenaColored 256^2 and a structured 2048^2 RGB
+image, three synth.structured planes of different seeds; 2048^2 because the RGB B = 16 full pool has no tensor-core path
+and every quadtree encode repeats it), quadtrees (16, 8) and (16, 4) with the whole pool and with widthKernel 2 over a
+sweep of max_mse, and the fixed B = 16 / 8 / 4 encodes of the same images as baselines.
 Per row: encode device ms (the call's total and its stages summed over levels), the quadtree kernels alone
 (k_qt_collage_sse, k_qt_decide, k_qt_scatter: torch.profiler, one profiled call of its own), stream bytes and bits per
-pixel, decode device ms, iterations, per-sweep kernel time, and PSNR against the source.  Writes OUT_DIR/quadtree_bench.json
-with the GPU's name and power limit read in the same run.  Exits 1 if a 256^2 stream does not decode through the CPU
-oracle to the GPU's pixels, iteration count and avgError.
+pixel, decode device ms, iterations, per-sweep kernel time, and PSNR against the source (RGB: over the 3*W*H samples).
+Writes OUT_DIR/quadtree_bench.json (--rgb: quadtree_rgb_bench.json) with the GPU's name and power limit read in the same
+run.  Exits 1 if a 256^2 stream does not decode through the CPU oracle to the GPU's pixels, iteration count and avgError.
 """
 from __future__ import annotations
 
@@ -24,6 +27,7 @@ sys.path.insert(0, ROOT)
 
 import fractal_image_compression_b200 as fic  # noqa: E402
 from oracle import quadtree as O  # noqa: E402
+from oracle import quadtree_rgb as O_rgb  # noqa: E402
 
 REPS = 5
 MSES = [0.0, 4.0, 16.0, 36.0, 64.0, 100.0, 200.0, float("inf")]
@@ -75,27 +79,36 @@ def best(fn, h):
 def main():
     out_dir = sys.argv[1]
     quick = "--quick" in sys.argv
+    rgb = "--rgb" in sys.argv
     os.makedirs(out_dir, exist_ok=True)
     import torch
 
     torch.cuda.init()
     h = fic.Handle(0)
-    lena = np.fromfile(os.path.join(ROOT, "tests", "golden", "lena_grey_256.u8"), np.uint8).reshape(256, 256)
-    images = {"lena256": lena}
-    if not quick:
-        images["structured4096"] = fic.synth.structured(4096, 4096, 1)
+    if rgb:
+        lena = np.fromfile(os.path.join(ROOT, "tests", "golden", "lena_colored_256.rgb"), np.uint8).reshape(256, 256, 3)
+        images = {"lena_colored256": lena.transpose(2, 0, 1).copy()}
+        if not quick:
+            images["structured_rgb2048"] = np.stack([fic.synth.structured(2048, 2048, 1 + k) for k in range(3)])
+        oracle_decode, code_bytes = O_rgb.decode_quadtree_rgb, 20
+    else:
+        lena = np.fromfile(os.path.join(ROOT, "tests", "golden", "lena_grey_256.u8"), np.uint8).reshape(256, 256)
+        images = {"lena256": lena}
+        if not quick:
+            images["structured4096"] = fic.synth.structured(4096, 4096, 1)
+        oracle_decode, code_bytes = O.decode_quadtree, 12
     res = {"device": gpu_info(), "reps": REPS, "fixed": [], "quadtree": []}
     failed = 0
     for name, plane in images.items():
-        H, W = plane.shape
+        H, W = plane.shape[-2:]
         for wk in (0, 2):
             for B in (16, 8, 4):
                 wkl = wk or 2 * (W // B) - 3
                 (info, q), t = best(lambda: h.encode_u8(plane, B, wkl), h)
-                (img, avg, it), td = best(lambda: h.decode_u8(q, W, H, B, wkl, False), h)
-                sw, nsw = kernel_us(lambda: h.decode_u8(q, W, H, B, wkl, False), ["k_decode_sweep"])
-                res["fixed"].append({"image": name, "B": B, "wk": wk, "encode": stages(t), "bytes": 20 + 12 * len(q),
-                                     "bpp": (20 + 12 * len(q)) * 8 / (W * H), "decode_ms": td.total_ms, "iterations": it,
+                (img, avg, it), td = best(lambda: h.decode_u8(q, W, H, B, wkl, rgb), h)
+                sw, nsw = kernel_us(lambda: h.decode_u8(q, W, H, B, wkl, rgb), ["k_decode_sweep"])
+                res["fixed"].append({"image": name, "B": B, "wk": wk, "encode": stages(t), "bytes": 20 + code_bytes * len(q),
+                                     "bpp": (20 + code_bytes * len(q)) * 8 / (W * H), "decode_ms": td.total_ms, "iterations": it,
                                      "sweep_us": sum(sw.values()) / max(sum(nsw.values()), 1), "psnr": psnr(img, plane)})
                 print(json.dumps(res["fixed"][-1]), flush=True)
             for b_max, b_min in ((16, 8), (16, 4)):
@@ -110,14 +123,14 @@ def main():
                            "avg_error": float(avg), "sweep_us": sw.get("k_decode_sweep_qt", 0.0) / max(nsw.get("k_decode_sweep_qt", 1), 1),
                            "psnr": psnr(img, plane)}
                     if W * H <= 256 * 256:
-                        oimg, oavg, oit = O.decode_quadtree(s)
+                        oimg, oavg, oit = oracle_decode(s)
                         row["oracle_roundtrip"] = bool((oimg == img).all() and oit == it and oavg.tobytes() == avg.tobytes())
                         failed += not row["oracle_roundtrip"]
                     res["quadtree"].append(row)
                     print(json.dumps(row), flush=True)
     h.close()
     res["oracle_roundtrip_failures"] = failed
-    with open(os.path.join(out_dir, "quadtree_bench.json"), "w") as f:
+    with open(os.path.join(out_dir, "quadtree_rgb_bench.json" if rgb else "quadtree_bench.json"), "w") as f:
         json.dump(res, f, indent=1)
     sys.exit(1 if failed else 0)
 
