@@ -337,6 +337,44 @@ class Handle:
         self._check(fn(self._h, _ptr(buf), len(buf), max_iters, _ptr(out), C.byref(avg), C.byref(it)))
         return out, np.float32(avg.value), it.value
 
+    def encode_quadtree_batch(self, planes: np.ndarray, b_max: int, b_min: int, wk: int, max_mse: float) -> list[bytes]:
+        """fic_encode_quadtree_batch: uint8 [n, H, W] grey planes (FIC_MODE_GREY_QT) or [n, 3, H, W] RGB planes
+        (FIC_MODE_RGB_QT); returns the n streams, each equal to encode_quadtree() of that image."""
+        a = np.ascontiguousarray(planes, dtype=np.uint8)
+        assert a.ndim in (3, 4) and (a.ndim == 3 or a.shape[1] == 3), "planes must be [n, H, W] or [n, 3, H, W]"
+        rgb = a.ndim == 4
+        n, H, W = a.shape[0], a.shape[-2], a.shape[-1]
+        bound = self._L.fic_quadtree_rgb_stream_bound if rgb else self._L.fic_quadtree_stream_bound
+        stride = bound(W, H, b_max, b_min)
+        buf = np.empty(max(n * stride, 1), np.uint8)
+        sizes = np.zeros(max(n, 1), np.uintp)
+        self._check(self._L.fic_encode_quadtree_batch(self._h, _lib.FIC_MODE_RGB_QT if rgb else _lib.FIC_MODE_GREY_QT, _ptr(a), n,
+                                                      W, H, b_max, b_min, wk, float(max_mse), _ptr(buf), stride, _ptr(sizes)))
+        return [buf[i * stride:i * stride + int(sizes[i])].tobytes() for i in range(n)]
+
+    def decode_quadtree_batch(self, streams, max_iters: int = 50):
+        """fic_decode_quadtree_batch: n quadtree streams of one mode and geometry -> (planes uint8 [n, H, W] or
+        [n, 3, H, W], avgError float32 [n], iterations int32 [n]).  The mode and shape come from stream 0's header."""
+        n = len(streams)
+        s0 = streams[0] if n else b""
+        mode, W, H, _, _, b_max, b_min = struct.unpack(">7i", s0[:28]) if len(s0) >= 32 else (0,) * 7
+        rgb = mode == _lib.FIC_MODE_RGB_QT
+        if not (0 < W <= 32768 and 0 < H <= 32768):
+            W = H = 0  # the library rejects the stream
+        bound = self._L.fic_quadtree_rgb_stream_bound if rgb else self._L.fic_quadtree_stream_bound
+        stride = max([bound(W, H, b_max, b_min) if W else 0] + [len(s) for s in streams])
+        buf = np.zeros(max(n * stride, 1), np.uint8)
+        for i, s in enumerate(streams):
+            buf[i * stride:i * stride + len(s)] = np.frombuffer(s, np.uint8)
+        nbytes = np.array([len(s) for s in streams] or [0], np.uintp)
+        out = np.empty((n, 3, H, W) if rgb else (n, H, W), np.uint8)
+        avg = np.zeros(max(n, 1), np.float32)
+        it = np.zeros(max(n, 1), np.int32)
+        self._check(self._L.fic_decode_quadtree_batch(self._h, mode if mode in (_lib.FIC_MODE_GREY_QT, _lib.FIC_MODE_RGB_QT) else
+                                                      _lib.FIC_MODE_GREY_QT, n, _ptr(buf), stride, _ptr(nbytes), max_iters,
+                                                      _ptr(out if out.size else np.empty(1, np.uint8)), _ptr(avg), _ptr(it)))
+        return out, avg[:n], it[:n]
+
     def collage(self, argb: np.ndarray, info: np.ndarray, B: int, wk: int, rgb: bool):
         """fic_collage; `info` is rewritten in place (window-local -> codebook index, FC:273)."""
         a = np.ascontiguousarray(argb, dtype=np.int32)

@@ -1084,59 +1084,93 @@ int fic_stream_read_codes(const uint8_t *stream, size_t nbytes, int32_t *qcodes)
 // One body per entry for both modes: the mode decides the channel count (the level encodes, the planes in and out) and,
 // inside qt_geom / qt_parse, the header value and the leaf size.
 
-// One upload, then every level's ordinary grey or RGB encode (the engine fic_encode_grey_u8 / fic_encode_rgb_planes would
-// pick, into that level's code table), one decimation of the source for the collage errors, and the stream body built on
-// the device (launch_qt_stream); the body comes down in one copy once the leaf count is known.
-static int encode_quadtree(fic_handle *h, int mode, const uint8_t *planes, int W, int H, int b_max, int b_min, int wk,
-                           double max_mse, uint8_t *stream, size_t capacity, size_t *stream_bytes)
+// Images go up and their streams come down in groups; a group is at most the smallest group any level's plan allows (so
+// every level's run fits its engine's bounds) and at most kDecodeBatchMax images (one grid row and one leaf start of
+// h_stage each).  Per group: one upload, then every level's ordinary grey or RGB batch run (the engine fic_encode_batch_u8
+// would pick, into that level's [n][NR_L] code table; the direct engine image by image), one decimation of the sources for
+// the collage errors, and the stream bodies built on the device (launch_qt_stream).  The leaf counts come down in one
+// small copy, then the bodies in one copy with the caller's stride as pitch.  A single image is the group of one.
+static int encode_quadtree(fic_handle *h, int mode, const uint8_t *planes, int n_images, int W, int H, int b_max, int b_min,
+                           int wk, double max_mse, uint8_t *streams, size_t stride, size_t *stream_bytes)
 {
-    if (!h) return FIC_E_ARG;
-    if (!planes || !stream_bytes) return set_err(h, FIC_E_ARG, "%s and stream_bytes must be non-NULL", mode == FIC_MODE_RGB_QT ? "planes" : "plane");
     if (max_mse != max_mse) return set_err(h, FIC_E_ARG, "max_mse is NaN");
     QtGeom q;
     const char *why = "";
     int rc = qt_geom(mode, W, H, b_max, b_min, wk, &q, &why);
     if (rc) return set_err(h, rc, "%s", why);
+    const Geom &fine = q.g[q.nl - 1];
+    const size_t C = (size_t)fine.C, S = (size_t)code_stride(fine), image_bytes = C * W * H, body = qt_body_bytes(q);
+    size_t bytes;
+    if (__builtin_mul_overflow((size_t)n_images, image_bytes, &bytes) || __builtin_mul_overflow((size_t)n_images, stride, &bytes))
+        return set_err(h, FIC_E_ARG, "n_images = %d images of %d x %d overflow a byte count", n_images, W, H);
     CU(cudaSetDevice(h->device));
     reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
-    const Geom &fine = q.g[q.nl - 1];
-    const size_t C = (size_t)fine.C, S = (size_t)code_stride(fine);
-    ENSURE(w.src, S_SRC, C * W * H);
-    ENSURE(w.dec, S_DEC, C * fine.sw * fine.sh);
-    ENSURE(w.info, S_INFO, sizeof(float) * S * fine.NR);
-    ENSURE(w.qt_codes, S_QT_CODES, sizeof(int32_t) * S * q.codes);
-    ENSURE(w.qt_err, S_QT_ERR, sizeof(uint32_t) * qt_err_words(q));
-    ENSURE(w.qt_stream, S_QT_STREAM, qt_stream_bound(mode, W, H, b_max, b_min) - kQtHeaderBytes);
+    EncodePlan plan[kQtMaxLevels];
+    int group = n_images < kDecodeBatchMax ? n_images : kDecodeBatchMax;
+    for (int L = 0; L < q.nl; L++) {
+        if ((rc = status_err(h, plan_encode(h->enc, q.g[L], 0, q.g[L].NR, n_images, false, s, &plan[L])))) return rc;
+        if (plan[L].group < group) group = plan[L].group;
+    }
+    ENSURE(w.src, S_SRC, image_bytes * group);
+    ENSURE(w.dec, S_DEC, C * fine.sw * fine.sh * group);
+    ENSURE(w.info, S_INFO, sizeof(float) * S * fine.NR * group);
+    ENSURE(w.qt_codes, S_QT_CODES, sizeof(int32_t) * S * q.codes * group);
+    ENSURE(w.qt_err, S_QT_ERR, sizeof(uint32_t) * qt_err_words(q, group));
+    ENSURE(w.qt_stream, S_QT_STREAM, body * group);
+    const uint32_t *starts = (const uint32_t *)h->h_stage;
+    int too_long = -1;  // the lowest image whose stream does not fit
     DrainOnExit drain(s);
     CU(cudaEventRecord(h->call_begin, s));
-    CU(cudaMemcpyAsync(w.src, planes, C * W * H, cudaMemcpyHostToDevice, s));
-    for (int L = 0; L < q.nl; L++) {
-        const Geom &g = q.g[L];
-        EncodePlan plan;
-        if ((rc = status_err(h, plan_encode(h->enc, g, 0, g.NR, 1, false, s, &plan)))) return rc;
-        if ((rc = status_err(h, run_encode(h->enc, w, g, plan, w.src, false, 0, g.NR, 1, w.info, w.qt_codes + S * q.first[L], &h->tm, s))))
-            return rc;
-        CU(cudaStreamSynchronize(s));  // the level's stage events, before the next level records them again
-        read_stages(h->enc, &h->tm, nullptr, nullptr);
+    for (int i0 = 0; i0 < n_images; i0 += group) {
+        const int gn = n_images - i0 < group ? n_images - i0 : group;
+        CU(cudaMemcpyAsync(w.src, planes + i0 * image_bytes, image_bytes * gn, cudaMemcpyHostToDevice, s));
+        for (int L = 0; L < q.nl; L++) {
+            const Geom &g = q.g[L];
+            const int per_run = plan[L].engine == FIC_ENGINE_DIRECT ? 1 : gn;
+            for (int i = 0; i < gn; i += per_run) {
+                rc = status_err(h, run_encode(h->enc, w, g, plan[L], w.src + i * image_bytes, false, 0, g.NR, per_run, w.info,
+                                              w.qt_codes + S * (q.first[L] * gn + i * g.NR), &h->tm, s));
+                if (rc) return rc;
+                CU(cudaStreamSynchronize(s));  // the run's stage events, before the next run records them again
+                read_stages(h->enc, &h->tm, nullptr, nullptr);
+            }
+        }
+        h->tm.launches += launch_decimate(w.src, w.dec, fine, s, gn);  // the fused engine leaves no decimated plane behind
+        h->tm.launches += launch_qt_stream(w, q, gn, max_mse, s);
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(h->h_acc, w.qt_err, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        if (gn > 1)  // every image's first leaf: the first of its warp totals after the group's scan
+            CU(cudaMemcpy2DAsync(h->h_stage, sizeof(uint32_t), w.qt_err + 1 + gn * q.flag_bytes, sizeof(uint32_t) * ((q.flag_bytes + 31) / 32),
+                                 sizeof(uint32_t), gn, cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
+        const uint32_t total = *(const uint32_t *)h->h_acc;
+        size_t longest = 0;
+        for (int i = 0; i < gn; i++) {
+            const int64_t leaves = (i + 1 < gn ? starts[i + 1] : total) - (gn > 1 ? starts[i] : 0);
+            const size_t need = kQtHeaderBytes + (size_t)q.flag_bytes + qt_leaf_bytes(q) * (size_t)leaves;
+            stream_bytes[i0 + i] = need;
+            if ((!streams || need > stride) && too_long < 0) too_long = i0 + i;
+            if (need > longest) longest = need;
+            if (too_long < 0) {
+                const int32_t hd[8] = {mode, W, H, 0, wk, b_max, b_min, (int32_t)leaves};
+                for (int k = 0; k < 8; k++) put_be32(streams + (i0 + i) * stride + 4 * k, hd[k]);
+            }
+        }
+        if (too_long >= 0) continue;
+        if (gn == 1) CU(cudaMemcpyAsync(streams + i0 * stride + kQtHeaderBytes, w.qt_stream, longest - kQtHeaderBytes, cudaMemcpyDeviceToHost, s));
+        else CU(cudaMemcpy2DAsync(streams + i0 * stride + kQtHeaderBytes, stride, w.qt_stream, body, longest - kQtHeaderBytes, gn,
+                                  cudaMemcpyDeviceToHost, s));
     }
-    h->tm.launches += launch_decimate(w.src, w.dec, fine, s);  // the fused engine leaves no decimated plane behind
-    h->tm.launches += launch_qt_stream(w, q, max_mse, s);
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(h->h_acc, w.qt_err, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    const int64_t leaves = *(const uint32_t *)h->h_acc;
-    const size_t need = kQtHeaderBytes + (size_t)q.flag_bytes + qt_leaf_bytes(q) * (size_t)leaves;
-    *stream_bytes = need;
-    if (!stream || capacity < need) return set_err(h, FIC_E_ARG, "the stream needs %zu bytes, capacity is %zu", need, capacity);
-    const int32_t hd[8] = {mode, W, H, 0, wk, b_max, b_min, (int32_t)leaves};
-    for (int k = 0; k < 8; k++) put_be32(stream + 4 * k, hd[k]);
-    CU(cudaMemcpyAsync(stream + kQtHeaderBytes, w.qt_stream, need - kQtHeaderBytes, cudaMemcpyDeviceToHost, s));
     CU(cudaEventRecord(h->call_end, s));
     CU(cudaStreamSynchronize(s));
     float ms = 0;
     h->tm.total_ms = cudaEventElapsedTime(&ms, h->call_begin, h->call_end) == cudaSuccess ? ms : 0.0f;  // the whole call
+    if (too_long >= 0) {
+        if (n_images == 1) return set_err(h, FIC_E_ARG, "the stream needs %zu bytes, capacity is %zu", stream_bytes[0], stride);
+        return set_err(h, FIC_E_ARG, "image %d: the stream needs %zu bytes, stride is %zu", too_long, stream_bytes[too_long], stride);
+    }
     return FIC_OK;
 }
 
@@ -1156,38 +1190,86 @@ static int quadtree_stream_info(int mode, const uint8_t *stream, size_t nbytes, 
     return FIC_OK;
 }
 
-static int decode_quadtree(fic_handle *h, int mode, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *planes_out,
-                           float *avg_error, int *iterations)
+// Image and plane workspace (img, dec, dec2) one decode group holds at most; a group is also at most kDecodeBatchMax
+// images (their state blocks come back through h_stage).
+constexpr size_t kQtDecodeGroupBytes = (size_t)256 << 20;
+
+// Every stream is parsed (the lowest bad image is named) and must share stream 0's geometry.  Per group of images: the
+// flag bytes and then the leaves of every image packed into one upload (a single image's body as it is), the first-leaf
+// tables (counted over the group) in another, then decode_quadtree_run.
+static int decode_quadtree(fic_handle *h, int mode, int n_images, const uint8_t *streams, size_t stride, const size_t *nbytes,
+                           int max_iters, uint8_t *planes_out, float *avg_error, int *iterations)
 {
-    if (!h) return FIC_E_ARG;
-    if (!stream || !planes_out) return set_err(h, FIC_E_ARG, "stream and %s must be non-NULL", mode == FIC_MODE_RGB_QT ? "planes_out" : "plane_out");
     if (max_iters < 1) return set_err(h, FIC_E_ARG, "max_iters must be >= 1");
+    const bool one = n_images == 1;
     QtGeom q;
     const char *why = "";
-    int rc = qt_parse(mode, stream, nbytes, &q, nullptr, false, &why);
-    if (rc) return set_err(h, rc, "%s", why);
-    std::vector<int32_t> base((size_t)q.g[0].NR);  // first leaf of every top block (the first pass gave their count)
-    qt_parse(mode, stream, nbytes, &q, base.data(), false, &why);
+    std::vector<int64_t> leaves((size_t)n_images);
+    for (int i = 0; i < n_images; i++) {
+        QtGeom qi;
+        const int rc = qt_parse(mode, streams + i * stride, nbytes[i], &qi, nullptr, false, &why);
+        if (rc) return one ? set_err(h, rc, "%s", why) : set_err(h, rc, "image %d: %s", i, why);
+        if (i == 0) q = qi;
+        else if (qi.g[0].W != q.g[0].W || qi.g[0].H != q.g[0].H || qi.g[0].B != q.g[0].B || qi.nl != q.nl || qi.wk != q.wk)
+            return set_err(h, FIC_E_STREAM, "image %d: W, H, b_max, b_min or wk differ from image 0's", i);
+        leaves[i] = qi.leaves;
+    }
+    const Geom &g = q.g[0];
+    const size_t C = (size_t)g.C, plane = (size_t)g.W * g.H, bmin = (size_t)q.g[q.nl - 1].B, leaf_bytes = qt_leaf_bytes(q);
+    const size_t cells = plane / (bmin * bmin), ntop = (size_t)g.NR, flags = (size_t)q.flag_bytes;
+    const size_t per_image = C * (plane + 2 * (size_t)g.sw * g.sh);
+    size_t bytes;
+    if (__builtin_mul_overflow((size_t)n_images, C * plane, &bytes))
+        return set_err(h, FIC_E_ARG, "n_images = %d images of %d x %d overflow a byte count", n_images, g.W, g.H);
+    size_t fit = kQtDecodeGroupBytes / per_image;
+    fit = fit < 1 ? 1 : (fit > (size_t)kDecodeBatchMax ? (size_t)kDecodeBatchMax : fit);
+    const int group = (size_t)n_images < fit ? n_images : (int)fit;
+    int64_t most = 0;  // the most leaves of a group
+    for (int i0 = 0; i0 < n_images; i0 += group) {
+        int64_t sum = 0;
+        for (int i = i0; i < n_images && i < i0 + group; i++) sum += leaves[i];
+        if (sum > most) most = sum;
+    }
     CU(cudaSetDevice(h->device));
     reset_timings(h);
     Work &w = h->w;
     cudaStream_t s = h->stream;
-    const Geom &g = q.g[0];
-    const size_t C = (size_t)g.C, plane = (size_t)g.W * g.H, bmin = (size_t)q.g[q.nl - 1].B;
-    const size_t cells = plane / (bmin * bmin), used = kQtHeaderBytes + (size_t)q.flag_bytes + qt_leaf_bytes(q) * (size_t)q.leaves;
-    ENSURE(w.img, S_IMG, C * plane);
-    ENSURE(w.dec, S_DEC, C * g.sw * g.sh);
-    ENSURE(w.dec2, S_DEC2, C * g.sw * g.sh);
-    ENSURE(w.state, S_STATE, sizeof(DecodeState));
-    ENSURE(w.qt_stream, S_QT_STREAM, used - kQtHeaderBytes);
-    ENSURE(w.qt_leaf, S_QT_LEAF, sizeof(int4) * (C == 3 ? 2 : 1) * q.leaves);  // k_qt_dequant's records
-    ENSURE(w.qt_map, S_QT_MAP, sizeof(int32_t) * (cells + base.size()));
+    ENSURE(w.img, S_IMG, C * plane * group);
+    ENSURE(w.dec, S_DEC, C * g.sw * g.sh * group);
+    ENSURE(w.dec2, S_DEC2, C * g.sw * g.sh * group);
+    ENSURE(w.state, S_STATE, sizeof(DecodeState) * group);
+    ENSURE(w.qt_stream, S_QT_STREAM, flags * group + leaf_bytes * most);
+    ENSURE(w.qt_leaf, S_QT_LEAF, sizeof(int4) * (C == 3 ? 2 : 1) * most);  // k_qt_dequant's records
+    ENSURE(w.qt_map, S_QT_MAP, sizeof(int32_t) * (cells + ntop) * group);
+    std::vector<int32_t> base(ntop * group);  // every image's first leaf of each top block, counted over its group
+    std::vector<uint8_t> pack(one ? 0 : flags * group + leaf_bytes * most);
     DrainOnExit drain(s);
     CU(cudaEventRecord(h->call_begin, s));
-    CU(cudaMemcpyAsync(w.qt_stream, stream + kQtHeaderBytes, used - kQtHeaderBytes, cudaMemcpyHostToDevice, s));
-    CU(cudaMemcpyAsync(w.qt_map + cells, base.data(), sizeof(int32_t) * base.size(), cudaMemcpyHostToDevice, s));
-    const Status st = decode_quadtree_run(w, q, max_iters, planes_out, avg_error, iterations, h->h_acc, h->call_begin, h->call_end, &h->tm, s);
-    return status_err(h, st, "a leaf indexes outside its level's domain pool");
+    for (int i0 = 0; i0 < n_images; i0 += group) {
+        const int gn = n_images - i0 < group ? n_images - i0 : group;
+        int64_t first = 0;
+        for (int i = 0; i < gn; i++) {
+            const uint8_t *si = streams + (i0 + i) * stride;
+            QtGeom qi;
+            qt_parse(mode, si, nbytes[i0 + i], &qi, base.data() + i * ntop, false, &why);
+            for (size_t t = 0; t < ntop; t++) base[i * ntop + t] += (int32_t)first;
+            if (!one) {
+                memcpy(pack.data() + i * flags, si + kQtHeaderBytes, flags);
+                memcpy(pack.data() + gn * flags + leaf_bytes * first, si + kQtHeaderBytes + flags, leaf_bytes * qi.leaves);
+            }
+            first += qi.leaves;
+        }
+        const uint8_t *body = one ? streams + kQtHeaderBytes : pack.data();
+        CU(cudaMemcpyAsync(w.qt_stream, body, flags * gn + leaf_bytes * first, cudaMemcpyHostToDevice, s));
+        CU(cudaMemcpyAsync(w.qt_map + cells * gn, base.data(), sizeof(int32_t) * ntop * gn, cudaMemcpyHostToDevice, s));
+        int bad = 0;
+        const Status st = decode_quadtree_run(w, q, gn, max_iters, planes_out + i0 * C * plane, avg_error ? avg_error + i0 : nullptr,
+                                              iterations ? iterations + i0 : nullptr, h->h_stage, h->call_begin, h->call_end, &h->tm, &bad, s);
+        if (st.rc == FIC_E_STREAM && !one)
+            return set_err(h, FIC_E_STREAM, "image %d: a leaf indexes outside its level's domain pool", i0 + bad);
+        if (st.rc) return status_err(h, st, "a leaf indexes outside its level's domain pool");
+    }
+    return FIC_OK;
 }
 
 size_t fic_quadtree_stream_bound(int W, int H, int b_max, int b_min) { return qt_stream_bound(FIC_MODE_GREY_QT, W, H, b_max, b_min); }
@@ -1195,7 +1277,9 @@ size_t fic_quadtree_stream_bound(int W, int H, int b_max, int b_min) { return qt
 int fic_encode_quadtree(fic_handle *h, const uint8_t *plane, int W, int H, int b_max, int b_min, int wk, double max_mse,
                         uint8_t *stream, size_t capacity, size_t *stream_bytes)
 {
-    return encode_quadtree(h, FIC_MODE_GREY_QT, plane, W, H, b_max, b_min, wk, max_mse, stream, capacity, stream_bytes);
+    if (!h) return FIC_E_ARG;
+    if (!plane || !stream_bytes) return set_err(h, FIC_E_ARG, "plane and stream_bytes must be non-NULL");
+    return encode_quadtree(h, FIC_MODE_GREY_QT, plane, 1, W, H, b_max, b_min, wk, max_mse, stream, capacity, stream_bytes);
 }
 
 int fic_quadtree_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *H, int *b_max, int *b_min, int *wk,
@@ -1207,7 +1291,9 @@ int fic_quadtree_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *
 int fic_decode_quadtree(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *plane_out,
                         float *avg_error, int *iterations)
 {
-    return decode_quadtree(h, FIC_MODE_GREY_QT, stream, nbytes, max_iters, plane_out, avg_error, iterations);
+    if (!h) return FIC_E_ARG;
+    if (!stream || !plane_out) return set_err(h, FIC_E_ARG, "stream and plane_out must be non-NULL");
+    return decode_quadtree(h, FIC_MODE_GREY_QT, 1, stream, 0, &nbytes, max_iters, plane_out, avg_error, iterations);
 }
 
 size_t fic_quadtree_rgb_stream_bound(int W, int H, int b_max, int b_min) { return qt_stream_bound(FIC_MODE_RGB_QT, W, H, b_max, b_min); }
@@ -1215,7 +1301,9 @@ size_t fic_quadtree_rgb_stream_bound(int W, int H, int b_max, int b_min) { retur
 int fic_encode_quadtree_rgb(fic_handle *h, const uint8_t *planes, int W, int H, int b_max, int b_min, int wk,
                             double max_mse, uint8_t *stream, size_t capacity, size_t *stream_bytes)
 {
-    return encode_quadtree(h, FIC_MODE_RGB_QT, planes, W, H, b_max, b_min, wk, max_mse, stream, capacity, stream_bytes);
+    if (!h) return FIC_E_ARG;
+    if (!planes || !stream_bytes) return set_err(h, FIC_E_ARG, "planes and stream_bytes must be non-NULL");
+    return encode_quadtree(h, FIC_MODE_RGB_QT, planes, 1, W, H, b_max, b_min, wk, max_mse, stream, capacity, stream_bytes);
 }
 
 int fic_quadtree_rgb_stream_info(const uint8_t *stream, size_t nbytes, int *W, int *H, int *b_max, int *b_min, int *wk,
@@ -1227,7 +1315,30 @@ int fic_quadtree_rgb_stream_info(const uint8_t *stream, size_t nbytes, int *W, i
 int fic_decode_quadtree_rgb(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *planes_out,
                             float *avg_error, int *iterations)
 {
-    return decode_quadtree(h, FIC_MODE_RGB_QT, stream, nbytes, max_iters, planes_out, avg_error, iterations);
+    if (!h) return FIC_E_ARG;
+    if (!stream || !planes_out) return set_err(h, FIC_E_ARG, "stream and planes_out must be non-NULL");
+    return decode_quadtree(h, FIC_MODE_RGB_QT, 1, stream, 0, &nbytes, max_iters, planes_out, avg_error, iterations);
+}
+
+int fic_encode_quadtree_batch(fic_handle *h, int mode, const uint8_t *planes, int n_images, int W, int H, int b_max, int b_min,
+                              int wk, double max_mse, uint8_t *streams, size_t stride, size_t *stream_bytes)
+{
+    if (!h) return FIC_E_ARG;
+    if (n_images < 1) return set_err(h, FIC_E_ARG, "n_images must be >= 1");
+    if (!planes || !streams || !stream_bytes) return set_err(h, FIC_E_ARG, "planes, streams and stream_bytes must be non-NULL");
+    return encode_quadtree(h, mode, planes, n_images, W, H, b_max, b_min, wk, max_mse, streams, stride, stream_bytes);
+}
+
+int fic_decode_quadtree_batch(fic_handle *h, int mode, int n_images, const uint8_t *streams, size_t stride, const size_t *nbytes,
+                              int max_iters, uint8_t *planes_out, float *avg_error, int *iterations)
+{
+    if (!h) return FIC_E_ARG;
+    if (mode != FIC_MODE_GREY_QT && mode != FIC_MODE_RGB_QT) return set_err(h, FIC_E_ARG, "mode must be FIC_MODE_GREY_QT or FIC_MODE_RGB_QT");
+    if (n_images < 1) return set_err(h, FIC_E_ARG, "n_images must be >= 1");
+    if (!streams || !nbytes || !planes_out) return set_err(h, FIC_E_ARG, "streams, nbytes and planes_out must be non-NULL");
+    size_t bytes;
+    if (__builtin_mul_overflow((size_t)n_images, stride, &bytes)) return set_err(h, FIC_E_ARG, "n_images * stride overflows");
+    return decode_quadtree(h, mode, n_images, streams, stride, nbytes, max_iters, planes_out, avg_error, iterations);
 }
 
 }  // extern "C"

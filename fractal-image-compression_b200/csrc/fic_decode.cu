@@ -959,18 +959,27 @@ __global__ void k_replay_walk(const int32_t *__restrict__ perr, int64_t count, c
 // One thread per top block: its leaves (stream at `stream`, leaves from flag_bytes on, big endian) dequantised with their
 // level's Geom as k_dequant does -- grey leaf[i] = {a, b, byte offset of the domain block in a decimated plane,
 // log2 B_L}; RGB leaf[2i] = {a, bR, bG, bB}, leaf[2i + 1] = {byte offset, log2 B_L, 0, 0} -- and every b_min x b_min cell
-// of a leaf pointed at it in map (cw = W / b_min cells per row).
-template <int C>
+// of a leaf pointed at it in map (cw = W / b_min cells per row).  BATCH: image blockIdx.y of gridDim.y, whose flag bytes
+// are the blockIdx.y-th flag_bytes of `stream`, whose leaves follow every image's flags (base counts over the group), with
+// its own first-leaf table, cell map and state block.
+template <int C, bool BATCH>
 __global__ void k_qt_dequant(QtGeom q, const uint8_t *__restrict__ stream, const int32_t *__restrict__ base,
                              int4 *__restrict__ leaf, int32_t *__restrict__ map, int lcell, DecodeState *st)
 {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= q.g[0].NR) return;
     const int cw = q.g[0].W >> lcell;
+    const uint8_t *leaves = stream + gridDim.y * q.flag_bytes;
+    if (BATCH) {
+        stream += blockIdx.y * q.flag_bytes;
+        base += blockIdx.y * q.g[0].NR;
+        map += (int64_t)blockIdx.y * cw * (q.g[0].H >> lcell);
+        st += blockIdx.y;
+    }
     int32_t i = base[t];
     qt_visit_leaves(q, t, stream[t], [&](int L, int64_t j) {
         const Geom &g = q.g[L];
-        const uint8_t *p = stream + q.flag_bytes + (C == 1 ? 12 : 20) * (int64_t)i;
+        const uint8_t *p = (BATCH ? leaves : stream + q.flag_bytes) + (C == 1 ? 12 : 20) * (int64_t)i;
         auto be = [](const uint8_t *b) { return (int32_t)(((uint32_t)b[0] << 24) | ((uint32_t)b[1] << 16) | ((uint32_t)b[2] << 8) | b[3]); };
         int64_t idx = code_pool_index(g, j, (float)be(p));
         if (idx < 0) {
@@ -999,12 +1008,22 @@ __global__ void k_qt_dequant(QtGeom q, const uint8_t *__restrict__ stream, const
 // b_min = 4 (QUAD); one lookup serves every channel -- at its own block size.  FIRST: the sweep from the constant-128
 // image reads neither image nor plane.  Every sweep folds itself: the last CTA turns the exact total S (over pixels and
 // channels) into avgError = (float)S / (float)(W*H), which needs no replay because the rule is stated on the exact sum.
-template <int C, bool FIRST, bool QUAD>
+// BATCH: image blockIdx.y of a group, gridDim.x CTAs per image -- its planes, its cell map and its state block; an image
+// that has converged returns at once.
+template <int C, bool FIRST, bool QUAD, bool BATCH>
 __global__ void __launch_bounds__(256)
 k_decode_sweep_qt(const uint8_t *__restrict__ dec_in, uint8_t *__restrict__ img, uint8_t *__restrict__ dec_out,
                   const int4 *__restrict__ leaf, const int32_t *__restrict__ map, Geom g, int lcell, SweepCtl ctl, int last)
 {
+    if (BATCH) ctl.st += blockIdx.y;
     if (sweep_done(ctl)) return;
+    if (BATCH) {
+        const int64_t i = blockIdx.y;
+        dec_in += i * C * (int64_t)g.sw * g.sh;
+        dec_out += i * C * (int64_t)g.sw * g.sh;
+        img += i * C * (int64_t)g.W * g.H;
+        map += i * (int64_t)(g.W >> lcell) * (g.H >> lcell);
+    }
     constexpr int LS = C == 1 ? 1 : 2;  // int4 records per leaf (k_qt_dequant)
     const uint32_t usw8 = (uint32_t)(g.W / 8), nstrips = usw8 * (uint32_t)(g.H / 2);
     const int cw = g.W >> lcell;
@@ -1126,8 +1145,9 @@ static Plan decode_plan(const Geom &g)
 // Launches the grid-stride kernel K over min(need, one wave) CTAs of 256 threads.  The sweeps are grid-stride over
 // exactly one wave of resident CTAs (SMs x occupancy of the kernel): a second, partly filled wave cost a third of the
 // sweep at 4096^2 (1184 CTAs on 740 slots, profiles/README.md).  The wave is measured once per kernel.
+// images > 1: that many images of a group along gridDim.y, each over min(need, one wave) CTAs.
 template <auto K, class... A>
-static void launch_wave(int64_t need, cudaStream_t s, A... args)
+static void launch_wave_images(int64_t need, unsigned images, cudaStream_t s, A... args)
 {
     static const int64_t wave = [] {
         int dev = 0, sms = 148, per_sm = 4;
@@ -1136,7 +1156,13 @@ static void launch_wave(int64_t need, cudaStream_t s, A... args)
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, K, 256, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
         return (int64_t)sms * per_sm;
     }();
-    K<<<(unsigned)(need < wave ? need : wave), 256, 0, s>>>(args...);
+    K<<<dim3((unsigned)(need < wave ? need : wave), images), 256, 0, s>>>(args...);
+}
+
+template <auto K, class... A>
+static void launch_wave(int64_t need, cudaStream_t s, A... args)
+{
+    launch_wave_images<K>(need, 1u, s, args...);
 }
 
 template <int C, int B, class... A>
@@ -1485,33 +1511,36 @@ Status decode_float_sum(const Work &w, const int32_t *terms, int64_t count, floa
     return Status();
 }
 
-template <int C, bool FIRST>
-static void launch_sweep_qt(int64_t need, bool quad, cudaStream_t s, const uint8_t *dec_in, uint8_t *img, uint8_t *dec_out,
-                            const int4 *leaf, const int32_t *map, Geom g, int lcell, SweepCtl ctl, int last)
+template <int C, bool FIRST, bool BATCH>
+static void launch_sweep_qt(int64_t need, bool quad, unsigned n, cudaStream_t s, const uint8_t *dec_in, uint8_t *img,
+                            uint8_t *dec_out, const int4 *leaf, const int32_t *map, Geom g, int lcell, SweepCtl ctl, int last)
 {
-    if (quad) launch_wave<k_decode_sweep_qt<C, FIRST, true>>(need, s, dec_in, img, dec_out, leaf, map, g, lcell, ctl, last);
-    else launch_wave<k_decode_sweep_qt<C, FIRST, false>>(need, s, dec_in, img, dec_out, leaf, map, g, lcell, ctl, last);
+    if (quad) launch_wave_images<k_decode_sweep_qt<C, FIRST, true, BATCH>>(need, n, s, dec_in, img, dec_out, leaf, map, g, lcell, ctl, last);
+    else launch_wave_images<k_decode_sweep_qt<C, FIRST, false, BATCH>>(need, n, s, dec_in, img, dec_out, leaf, map, g, lcell, ctl, last);
 }
 
-template <int C>
-static Status decode_quadtree_c(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
-                                int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, cudaStream_t s)
+// Sweeps go `batch` at a time behind the images' done flags; after each batch the host reads every state block of the
+// group in one copy and stops when all images are done or at max_iters.  n = 1 runs the single-image kernels.
+template <int C, bool BATCH>
+static Status decode_quadtree_c(const Work &w, const QtGeom &q, int n, int max_iters, uint8_t *planes_out, float *avg_error,
+                                int *iterations, void *h_stage, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm,
+                                int *bad_image, cudaStream_t s)
 {
     const Geom &g = q.g[0];
-    const DecodeState *hs = (const DecodeState *)h_scratch;
+    const DecodeState *hs = (const DecodeState *)h_stage;
     const size_t plane = (size_t)g.W * g.H;
     const float fwh = (float)(g.W * g.H);
     const int lcell = __builtin_ctz((unsigned)q.g[q.nl - 1].B);
-    const int32_t *base = w.qt_map + (plane >> (2 * lcell));
+    const int32_t *base = w.qt_map + n * (plane >> (2 * lcell));
     int launches = 0;
-    Status st;
-    DCU(cudaMemsetAsync(w.state, 0, sizeof(DecodeState), s));
-    k_qt_dequant<C><<<(unsigned)((g.NR + 127) / 128), 128, 0, s>>>(q, w.qt_stream, base, w.qt_leaf, w.qt_map, lcell, w.state);
+    DCU(cudaMemsetAsync(w.state, 0, sizeof(DecodeState) * n, s));
+    k_qt_dequant<C, BATCH><<<dim3((unsigned)((g.NR + 127) / 128), n), 128, 0, s>>>(q, w.qt_stream, base, w.qt_leaf, w.qt_map, lcell, w.state);
     launches++;
     const int64_t need = ((int64_t)(g.W / 8) * (g.H / 2) + 255) / 256;
-    const bool speculative_out = C * plane <= ((size_t)4 << 20);  // as decode_run: copy behind every batch of sweeps
-    // as decode_run: RGB decodes need more sweeps than grey (13-22 against 5-9 in the fixed decoder)
-    const int batch = (C == 3 && speculative_out) ? 16 : 8;
+    const bool small = C * plane <= ((size_t)4 << 20), speculative_out = small && C * plane * n <= ((size_t)4 << 20);
+    // as decode_run: copy behind every batch of sweeps when the output is small; RGB decodes need more sweeps than grey
+    // (13-22 against 5-9 in the fixed decoder)
+    const int batch = (C == 3 && small) ? 16 : 8;
     uint8_t *dcur = w.dec, *dnext = w.dec2;
     int it = 0;
     while (it < max_iters) {
@@ -1519,37 +1548,51 @@ static Status decode_quadtree_c(const Work &w, const QtGeom &q, int max_iters, u
         for (; it < batch_end; it++) {
             const SweepCtl ctl = {w.state, it, 1, fwh};
             const int last = it == max_iters - 1;
-            (it == 0 ? launch_sweep_qt<C, true> : launch_sweep_qt<C, false>)(need, lcell == 2, s, dcur, w.img, dnext, w.qt_leaf, w.qt_map, g, lcell, ctl, last);
+            (it == 0 ? launch_sweep_qt<C, true, BATCH> : launch_sweep_qt<C, false, BATCH>)(need, lcell == 2, (unsigned)n, s, dcur, w.img, dnext,
+                                                                                          w.qt_leaf, w.qt_map, g, lcell, ctl, last);
             launches++;
             uint8_t *t = dcur; dcur = dnext; dnext = t;
         }
-        DCU(cudaMemcpyAsync(h_scratch, w.state, sizeof(DecodeState), cudaMemcpyDeviceToHost, s));
+        DCU(cudaMemcpyAsync(h_stage, w.state, sizeof(DecodeState) * n, cudaMemcpyDeviceToHost, s));
         if (speculative_out) {
-            DCU(cudaMemcpyAsync(planes_out, w.img, C * plane, cudaMemcpyDeviceToHost, s));
+            DCU(cudaMemcpyAsync(planes_out, w.img, C * plane * n, cudaMemcpyDeviceToHost, s));
             DCU(cudaEventRecord(end, s));
         }
-        if ((st = sync_state(hs, s)).rc) return st;
-        if (hs->done) break;
+        DCU(cudaStreamSynchronize(s));
+        bool done = true;
+        for (int i = 0; i < n; i++) {
+            if (hs[i].bad_index) {
+                *bad_image = i;
+                return Status(FIC_E_STREAM);
+            }
+            done = done && hs[i].done;
+        }
+        if (done) break;
     }
     if (!speculative_out) {
-        DCU(cudaMemcpyAsync(planes_out, w.img, C * plane, cudaMemcpyDeviceToHost, s));
+        DCU(cudaMemcpyAsync(planes_out, w.img, C * plane * n, cudaMemcpyDeviceToHost, s));
         DCU(cudaEventRecord(end, s));
         DCU(cudaStreamSynchronize(s));
     }
     DCU(cudaGetLastError());
     float ms = 0;
     if (cudaEventElapsedTime(&ms, ev0, end) == cudaSuccess) tm->total_ms = ms;
-    tm->launches = launches;
-    if (avg_error) memcpy(avg_error, &hs->avg_bits, sizeof *avg_error);
-    if (iterations) *iterations = (int)hs->iters;
+    tm->launches += launches;
+    for (int i = 0; i < n; i++) {
+        if (avg_error) memcpy(avg_error + i, &hs[i].avg_bits, sizeof *avg_error);
+        if (iterations) iterations[i] = (int)hs[i].iters;
+    }
     return Status();
 }
 
-Status decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
-                                 int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm, cudaStream_t s)
+Status decode_quadtree_run(const Work &w, const QtGeom &q, int n, int max_iters, uint8_t *planes_out, float *avg_error,
+                           int *iterations, void *h_stage, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm,
+                           int *bad_image, cudaStream_t s)
 {
-    return (q.g[0].C == 3 ? decode_quadtree_c<3> : decode_quadtree_c<1>)(w, q, max_iters, planes_out, avg_error, iterations,
-                                                                         h_scratch, ev0, end, tm, s);
+    const bool rgb = q.g[0].C == 3;
+    const auto run = n == 1 ? (rgb ? decode_quadtree_c<3, false> : decode_quadtree_c<1, false>)
+                            : (rgb ? decode_quadtree_c<3, true> : decode_quadtree_c<1, true>);
+    return run(w, q, n, max_iters, planes_out, avg_error, iterations, h_stage, ev0, end, tm, bad_image, s);
 }
 
 }  // namespace fic

@@ -256,18 +256,27 @@ size_t qt_stream_bound(int mode, int W, int H, int b_max, int b_min);
 // NR_top entries): the first leaf of every top block.  check_leaves: also every leaf's domain index against its level's
 // pool.
 int qt_parse(int mode, const uint8_t *stream, size_t nbytes, QtGeom *q, int32_t *base, bool check_leaves, const char **why);
-// Words of Work::qt_err an encode needs.
-size_t qt_err_words(const QtGeom &q);
-// After every level's codes are in w.qt_codes and the source's decimated planes in w.dec: collage errors, split flags,
-// leaf scan and leaf scatter into w.qt_stream (flags at 0, leaves at flag_bytes); the leaf count lands in w.qt_err[0].
-int launch_qt_stream(const Work &w, const QtGeom &q, double max_mse, cudaStream_t s);
-// Iterative decode of the stream in w.qt_stream (the first-leaf table in w.qt_map after the cell map) into w.img (C planes),
-// copied to planes_out.  avgError = (float)S / (float)(W*H) of the exact sum S of squared changes over pixels and
-// channels; stops below 1 or after max_iters sweeps.  Workspace: img, dec, dec2 (C planes each), state, qt_leaf
-// (q.leaves records, two int4 each for RGB), qt_map.
-Status decode_quadtree_run(const Work &w, const QtGeom &q, int max_iters, uint8_t *planes_out, float *avg_error,
-                                 int *iterations, void *h_scratch, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm,
-                                 cudaStream_t s);
+// Words of Work::qt_err an encode of a group of n images needs.
+size_t qt_err_words(const QtGeom &q, int n);
+// Bytes of one image's stream body on the device (flags and the most leaves it can have): the stream bound less the header.
+size_t qt_body_bytes(const QtGeom &q);
+// A group of n images (planes [n][C][H][W] in w.src, decimated planes [n][C][sh][sw] in w.dec, every level's codes in
+// w.qt_codes level-major and image-major: level L of image i at first[L] * n + i * NR_L): collage errors, split flags,
+// leaf scan and leaf scatter into image i's body at w.qt_stream + i * qt_body_bytes (flags at 0, leaves at flag_bytes).
+// The group's leaf total lands in w.qt_err[0] and image i's first leaf (counted over the group) at
+// w.qt_err[1 + n * flag_bytes + i * ceil(flag_bytes / 32)].  n = 1 runs the single-image kernels.
+int launch_qt_stream(const Work &w, const QtGeom &q, int n, double max_mse, cudaStream_t s);
+// Iterative decode of n streams of one geometry into w.img (C planes per image), copied to planes_out [n][C][H][W].
+// w.qt_stream holds the n images' flag bytes back to back and then every leaf of the group, image after image; w.qt_map
+// holds n cell maps and then n first-leaf tables (NR_top entries each, counted over the group).  Each image's avgError =
+// (float)S / (float)(W*H) of the exact sum S of its squared changes over pixels and channels; an image stops below 1 and
+// stays frozen while the others sweep, all stop after max_iters sweeps.  avg_error and iterations ([n]) may be NULL.
+// h_stage: pinned, n * sizeof(DecodeState).  Workspace: img, dec, dec2 (C planes per image), state (n blocks), qt_leaf
+// (the group's leaves, two int4 each for RGB), qt_map.  On FIC_E_STREAM *bad_image is the lowest image with a leaf
+// outside its level's pool.  Adds its launches to tm; total_ms runs from ev0 to end.
+Status decode_quadtree_run(const Work &w, const QtGeom &q, int n, int max_iters, uint8_t *planes_out, float *avg_error,
+                           int *iterations, void *h_stage, cudaEvent_t ev0, cudaEvent_t end, fic_timings *tm,
+                           int *bad_image, cudaStream_t s);
 // Exclusive prefix sums of n counters in place (one block, the radix sort's row scan); *total = their sum.
 int launch_scan_u32(uint32_t *d, int64_t n, uint32_t *total, cudaStream_t s);
 

@@ -84,20 +84,31 @@ int qt_parse(int mode, const uint8_t *s, size_t nbytes, QtGeom *q, int32_t *base
 
 // ---- device: collage error, split flags, leaf scatter --------------------------------------------------------------------
 
-// qt_err layout: [0] leaf total, then the per-top-block in-warp prefixes (flag_bytes words), the per-warp totals, then the
-// collage errors of every level (level-major, QtGeom::first).
-static int64_t qt_warps(const QtGeom &q) { return (q.flag_bytes + 31) / 32; }
-static int64_t qt_err_at(const QtGeom &q) { return 1 + q.flag_bytes + qt_warps(q); }
-size_t qt_err_words(const QtGeom &q) { return (size_t)(qt_err_at(q) + q.codes); }
+// qt_err layout for a group of n images: [0] leaf total, then the per-top-block in-warp prefixes (n * flag_bytes words),
+// the per-warp totals (n * qt_warps), then the collage errors of every level (level-major, then image-major: level L of
+// image i at n * QtGeom::first[L] + i * NR_L).  An image's top blocks start a new warp, so its prefixes and warp totals
+// are its own; one scan over every warp total of the group gives each image's first leaf at its first warp.
+__host__ __device__ inline int64_t qt_warps(const QtGeom &q) { return (q.flag_bytes + 31) / 32; }
+static int64_t qt_err_at(const QtGeom &q, int n) { return 1 + n * (q.flag_bytes + qt_warps(q)); }
+size_t qt_err_words(const QtGeom &q, int n) { return (size_t)(qt_err_at(q, n) + n * q.codes); }
+__host__ __device__ inline int64_t qt_body_pitch(const QtGeom &q) { return q.flag_bytes + (q.g[0].C == 3 ? 20 : 12) * q.g[q.nl - 1].NR; }
 
 // E(j) = sum over range block j (and its C channels) of (decode_px(a, b_c, d_c) - s_c)^2: the code dequantised as the
 // decoder does (FC:372-374 grey, FC:446-450 RGB), the domain pixels d_c read from the source's decimated planes at the
 // code's codebook index (FC:853-893).  B threads per range block, one row each (B divides 32: a block's rows share a warp
-// and reduce with shuffles).  E < 2^32: at most 3 * 255^2 * 256.
-template <int C>
+// and reduce with shuffles).  E < 2^32: at most 3 * 255^2 * 256.  BATCH: image blockIdx.y of a group -- its planes, and
+// its rows of the level's [n][NR] code and error tables.
+template <int C, bool BATCH>
 __global__ void __launch_bounds__(256) k_qt_collage_sse(const uint8_t *__restrict__ src, const uint8_t *__restrict__ dec,
                                                         const int32_t *__restrict__ q, uint32_t *__restrict__ err, Geom g)
 {
+    if (BATCH) {
+        const int64_t i = blockIdx.y;
+        src += i * C * (int64_t)g.W * g.H;
+        dec += i * C * (int64_t)g.sw * g.sh;
+        q += i * (C == 1 ? 3 : 5) * g.NR;
+        err += i * g.NR;
+    }
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int B = g.B;
     const int64_t j = t / B;
@@ -132,27 +143,40 @@ struct QtSplit {
     double max_mse;
 };
 
-// A block above b_min is split iff (double)E > max_mse * (double)(C * B * B).
-template <int C>
+// Where range j of level L of the CTA's image sits in the level-major tables (BATCH: image blockIdx.y of gridDim.y).
+template <bool BATCH>
+__device__ __forceinline__ int64_t qt_at(const QtGeom &q, int L, int64_t j)
+{
+    return BATCH ? (int64_t)gridDim.y * q.first[L] + (int64_t)blockIdx.y * q.g[L].NR + j : q.first[L] + j;
+}
+
+// A block above b_min is split iff (double)E > max_mse * (double)(C * B * B).  BATCH: of the CTA's image.
+template <int C, bool BATCH>
 __device__ __forceinline__ bool qt_split(const QtSplit &p, int L, int64_t j)
 {
-    return L < p.q.nl - 1 && (double)p.err[p.q.first[L] + j] > __dmul_rn(p.max_mse, (double)(C * p.q.g[L].n));
+    return L < p.q.nl - 1 && (double)p.err[qt_at<BATCH>(p.q, L, j)] > __dmul_rn(p.max_mse, (double)(C * p.q.g[L].n));
 }
 
 // One thread per top block (and per padding byte of the flags): its flag byte into the stream, its leaf count's
-// exclusive prefix within the warp to pre[t], the warp's total to wsum[warp].
-template <int C>
+// exclusive prefix within the warp to pre[t], the warp's total to wsum[warp].  BATCH: image blockIdx.y, whose stream body
+// starts at flags + blockIdx.y * qt_body_pitch and whose prefixes and warp totals are its own (the qt_err layout).
+template <int C, bool BATCH>
 __global__ void __launch_bounds__(256) k_qt_decide(QtSplit p, uint8_t *__restrict__ flags, uint32_t *__restrict__ pre,
                                                    uint32_t *__restrict__ wsum)
 {
+    if (BATCH) {
+        flags += blockIdx.y * qt_body_pitch(p.q);
+        pre += blockIdx.y * p.q.flag_bytes;
+        wsum += blockIdx.y * qt_warps(p.q);
+    }
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
-    uint32_t f = 0, n = 0;
+    uint32_t n = 0, f = 0;
     if (t < p.q.g[0].NR) {
-        if (qt_split<C>(p, 0, t)) {
+        if (qt_split<C, BATCH>(p, 0, t)) {
             f = 1;
             for (int k = 0; k < 4; k++)
-                if (qt_split<C>(p, 1, qt_child(p.q, 0, t, k))) f |= 2u << k;
+                if (qt_split<C, BATCH>(p, 1, qt_child(p.q, 0, t, k))) f |= 2u << k;
         }
         n = (uint32_t)qt_leaf_count(f);
     }
@@ -171,8 +195,8 @@ __global__ void __launch_bounds__(256) k_qt_decide(QtSplit p, uint8_t *__restric
 __device__ __forceinline__ uint32_t bswap32(int32_t v) { return __byte_perm((uint32_t)v, 0u, 0x0123); }
 
 // One thread per top block: its leaves' codes (3 ints grey, 5 RGB), big endian (DataOutputStream.writeInt), at their
-// place in the stream.
-template <int C>
+// place in the stream.  BATCH: image blockIdx.y, its leaves after its own flag bytes, counted from its first leaf.
+template <int C, bool BATCH>
 __global__ void __launch_bounds__(256) k_qt_scatter(QtGeom q, const int32_t *__restrict__ codes, const uint8_t *__restrict__ flags,
                                                     const uint32_t *__restrict__ pre, const uint32_t *__restrict__ wsum,
                                                     uint32_t *__restrict__ leaves)
@@ -180,9 +204,18 @@ __global__ void __launch_bounds__(256) k_qt_scatter(QtGeom q, const int32_t *__r
     constexpr int S = C == 1 ? 3 : 5;
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= q.g[0].NR) return;
-    uint32_t *o = leaves + S * (int64_t)(wsum[t >> 5] + pre[t]);
+    uint32_t first = 0;
+    if (BATCH) {
+        const int64_t body = blockIdx.y * qt_body_pitch(q);
+        flags += body;
+        leaves += body / 4;
+        pre += blockIdx.y * q.flag_bytes;
+        wsum += blockIdx.y * qt_warps(q);
+        first = wsum[0];
+    }
+    uint32_t *o = leaves + S * (int64_t)(wsum[t >> 5] + pre[t] - first);
     qt_visit_leaves(q, t, flags[t], [&](int L, int64_t j) {
-        const int32_t *c = codes + S * (q.first[L] + j);
+        const int32_t *c = codes + S * qt_at<BATCH>(q, L, j);
         o[0] = bswap32(c[0]);
         o[1] = bswap32(c[1]);
         o[2] = bswap32(c[2]);
@@ -194,29 +227,33 @@ __global__ void __launch_bounds__(256) k_qt_scatter(QtGeom q, const int32_t *__r
     });
 }
 
-template <int C>
-static int launch_qt_stream_c(const Work &w, const QtGeom &q, double max_mse, cudaStream_t s)
+template <int C, bool BATCH>
+static int launch_qt_stream_c(const Work &w, const QtGeom &q, int n, double max_mse, cudaStream_t s)
 {
     constexpr int S = C == 1 ? 3 : 5;
-    uint32_t *total = w.qt_err, *pre = w.qt_err + 1, *wsum = pre + q.flag_bytes, *err = w.qt_err + qt_err_at(q);
+    uint32_t *total = w.qt_err, *pre = w.qt_err + 1, *wsum = pre + n * q.flag_bytes, *err = w.qt_err + qt_err_at(q, n);
     int launches = 0;
     for (int L = 0; L < q.nl; L++) {
         const Geom &g = q.g[L];
         const int64_t threads = g.NR * g.B;
-        k_qt_collage_sse<C><<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(w.src, w.dec, w.qt_codes + S * q.first[L], err + q.first[L], g);
+        k_qt_collage_sse<C, BATCH><<<dim3((unsigned)((threads + 255) / 256), n), 256, 0, s>>>(w.src, w.dec, w.qt_codes + S * n * q.first[L],
+                                                                                             err + n * q.first[L], g);
         launches++;
     }
     const QtSplit p = {q, err, max_mse};
-    k_qt_decide<C><<<(unsigned)((q.flag_bytes + 255) / 256), 256, 0, s>>>(p, w.qt_stream, pre, wsum);
-    launches += 1 + launch_scan_u32(wsum, qt_warps(q), total, s);
-    k_qt_scatter<C><<<(unsigned)((q.g[0].NR + 255) / 256), 256, 0, s>>>(q, w.qt_codes, w.qt_stream, pre, wsum,
-                                                                          (uint32_t *)(w.qt_stream + q.flag_bytes));
+    k_qt_decide<C, BATCH><<<dim3((unsigned)((q.flag_bytes + 255) / 256), n), 256, 0, s>>>(p, w.qt_stream, pre, wsum);
+    launches += 1 + launch_scan_u32(wsum, n * qt_warps(q), total, s);
+    k_qt_scatter<C, BATCH><<<dim3((unsigned)((q.g[0].NR + 255) / 256), n), 256, 0, s>>>(q, w.qt_codes, w.qt_stream, pre, wsum,
+                                                                                       (uint32_t *)(w.qt_stream + q.flag_bytes));
     return launches + 1;
 }
 
-int launch_qt_stream(const Work &w, const QtGeom &q, double max_mse, cudaStream_t s)
+int launch_qt_stream(const Work &w, const QtGeom &q, int n, double max_mse, cudaStream_t s)
 {
-    return q.g[0].C == 3 ? launch_qt_stream_c<3>(w, q, max_mse, s) : launch_qt_stream_c<1>(w, q, max_mse, s);
+    if (n == 1) return q.g[0].C == 3 ? launch_qt_stream_c<3, false>(w, q, 1, max_mse, s) : launch_qt_stream_c<1, false>(w, q, 1, max_mse, s);
+    return q.g[0].C == 3 ? launch_qt_stream_c<3, true>(w, q, n, max_mse, s) : launch_qt_stream_c<1, true>(w, q, n, max_mse, s);
 }
+
+size_t qt_body_bytes(const QtGeom &q) { return (size_t)qt_body_pitch(q); }
 
 }  // namespace fic

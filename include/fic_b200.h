@@ -296,6 +296,33 @@ int fic_quadtree_rgb_stream_info(const uint8_t *stream, size_t nbytes, int *W, i
 int fic_decode_quadtree_rgb(fic_handle *h, const uint8_t *stream, size_t nbytes, int max_iters, uint8_t *planes_out,
                             float *avg_error, int *iterations);
 
+/* Quadtree batches: n_images same-size images per call, mode FIC_MODE_GREY_QT or FIC_MODE_RGB_QT.  Planes in and out
+ * are [n][C][H][W] (C = 1 for FIC_MODE_GREY_QT: the red channel; 3 for FIC_MODE_RGB_QT).  Stream i sits at
+ * streams + i * stride: the encode writes its length to stream_bytes[i]; the decode reads nbytes[i] bytes.
+ *
+ * Image i's stream_bytes[i] and stream bytes equal what fic_encode_quadtree (grey) or fic_encode_quadtree_rgb (RGB)
+ * returns for that image alone on the same handle with the same options; image i's decoded planes, avgError bits and
+ * sweep count equal what fic_decode_quadtree[_rgb] gives for stream i (no carry-in, as the single decode).  The caller
+ * states the mode, so a grey caller's buffers are never written with three planes: the decode refuses any stream whose
+ * header is not `mode`.
+ *
+ * Encode: the images go up and their streams come down in groups, each level encoded as fic_encode_batch_u8 would
+ * (one fused launch or one tcgen05 group search per group and level; image by image on the direct engine), and the
+ * stream bodies built on the device for the whole group.  stride >= fic_quadtree[_rgb]_stream_bound(W, H, b_max, b_min)
+ * always suffices; if some stream is longer than stride, FIC_E_ARG with every image's size in stream_bytes.  Bytes of a
+ * slot past its stream's length are unspecified.  Decode: a group of images sweeps together, each image stopping when it
+ * converges; avg_error [n] and iterations [n] may be NULL.
+ *
+ * Besides the single entries' rejections: FIC_E_ARG for n_images < 1, NULL arrays, a byte count of the batch that
+ * overflows, or a NaN max_mse; FIC_E_STREAM for a stream whose header, flags or size is bad, whose W, H, b_max, b_min or
+ * wk differ from stream 0's, or with a leaf outside its level's pool (fic_last_error names the lowest such image).
+ * fic_get_timings reports the whole call: total_ms, launches, search_evals summed over levels and images, the finest
+ * level's engine, and on the encode the stage times summed over levels and groups. */
+int fic_encode_quadtree_batch(fic_handle *h, int mode, const uint8_t *planes, int n_images, int W, int H, int b_max,
+                              int b_min, int wk, double max_mse, uint8_t *streams, size_t stride, size_t *stream_bytes);
+int fic_decode_quadtree_batch(fic_handle *h, int mode, int n_images, const uint8_t *streams, size_t stride,
+                              const size_t *nbytes, int max_iters, uint8_t *planes_out, float *avg_error, int *iterations);
+
 /* ---- multi-GPU: the same encode over several GPUs of one node (SURVEY 8b, 8e) --- */
 
 /* Replaces the same reference loops (FC:119 + FC:125-159, FC:181 + FC:186-215) with the range-block rows sharded
