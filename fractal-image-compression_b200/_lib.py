@@ -38,7 +38,7 @@ ABI_SYMBOLS = [
     "fic_encode_batch", "fic_encode_batch_u8", "fic_decode_batch", "fic_decode_batch_u8",
     "fic_quadtree_stream_bound", "fic_encode_quadtree", "fic_quadtree_stream_info", "fic_decode_quadtree",
     "fic_quadtree_rgb_stream_bound", "fic_encode_quadtree_rgb", "fic_quadtree_rgb_stream_info", "fic_decode_quadtree_rgb",
-    "fic_encode_quadtree_batch", "fic_decode_quadtree_batch",
+    "fic_encode_quadtree_batch", "fic_decode_quadtree_batch", "fic_encode_quadtree_budget", "fic_encode_quadtree_budget_batch",
 ]
 
 
@@ -134,6 +134,9 @@ def load() -> C.CDLL:
         fn.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, f32p, C.POINTER(C.c_int)]
     L.fic_encode_quadtree_batch.argtypes = [vp, C.c_int, vp] + [C.c_int] * 6 + [C.c_double, vp, C.c_size_t, vp]
     L.fic_decode_quadtree_batch.argtypes = [vp, C.c_int, C.c_int, vp, C.c_size_t, vp, C.c_int, vp, vp, vp]
+    L.fic_encode_quadtree_budget.argtypes = [vp, C.c_int, vp] + [C.c_int] * 5 + [C.c_size_t, vp, C.c_size_t, C.POINTER(C.c_size_t),
+                                                                                 C.POINTER(C.c_double)]
+    L.fic_encode_quadtree_budget_batch.argtypes = [vp, C.c_int, vp] + [C.c_int] * 6 + [vp, vp, C.c_size_t, vp, vp]
     for name in ABI_SYMBOLS:
         fn = getattr(L, name)
         if fn.restype is C.c_int and name not in ("fic_version", "fic_last_error", "fic_stream_size", "fic_multi_last_error",

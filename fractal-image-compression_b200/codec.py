@@ -352,6 +352,40 @@ class Handle:
                                                       W, H, b_max, b_min, wk, float(max_mse), _ptr(buf), stride, _ptr(sizes)))
         return [buf[i * stride:i * stride + int(sizes[i])].tobytes() for i in range(n)]
 
+    def encode_quadtree_budget(self, planes: np.ndarray, b_max: int, b_min: int, wk: int, max_bytes: int) -> tuple[bytes, float]:
+        """fic_encode_quadtree_budget on a grey plane (uint8 [H, W], FIC_MODE_GREY_QT) or RGB planes (uint8 [3, H, W],
+        FIC_MODE_RGB_QT): (stream, m*), the stream encode_quadtree() writes at max_mse = m*, the smallest max_mse whose
+        stream has at most max_bytes bytes (-inf when the fully split tree fits)."""
+        a = np.ascontiguousarray(planes, dtype=np.uint8)
+        rgb = a.ndim == 3
+        assert not rgb or a.shape[0] == 3
+        H, W = a.shape[-2:]
+        bound = self._L.fic_quadtree_rgb_stream_bound if rgb else self._L.fic_quadtree_stream_bound
+        cap = min(int(max_bytes), bound(W, H, b_max, b_min))
+        buf = np.empty(max(cap, 1), np.uint8)
+        n, m = C.c_size_t(0), C.c_double(0.0)
+        self._check(self._L.fic_encode_quadtree_budget(self._h, _lib.FIC_MODE_RGB_QT if rgb else _lib.FIC_MODE_GREY_QT, _ptr(a), W, H,
+                                                       b_max, b_min, wk, int(max_bytes), _ptr(buf), cap, C.byref(n), C.byref(m)))
+        return buf[:n.value].tobytes(), m.value
+
+    def encode_quadtree_budget_batch(self, planes: np.ndarray, b_max: int, b_min: int, wk: int, max_bytes):
+        """fic_encode_quadtree_budget_batch: uint8 [n, H, W] grey planes or [n, 3, H, W] RGB planes, max_bytes an int
+        or one per image; returns (the n streams, m* float64 [n]), each image's equal to encode_quadtree_budget()."""
+        a = np.ascontiguousarray(planes, dtype=np.uint8)
+        assert a.ndim in (3, 4) and (a.ndim == 3 or a.shape[1] == 3), "planes must be [n, H, W] or [n, 3, H, W]"
+        rgb = a.ndim == 4
+        n, H, W = a.shape[0], a.shape[-2], a.shape[-1]
+        budgets = np.ascontiguousarray(np.broadcast_to(np.asarray(max_bytes, np.uintp), (n,)))
+        bound = self._L.fic_quadtree_rgb_stream_bound if rgb else self._L.fic_quadtree_stream_bound
+        stride = min(int(budgets.max()) if n else 0, bound(W, H, b_max, b_min))
+        buf = np.empty(max(n * stride, 1), np.uint8)
+        sizes = np.zeros(max(n, 1), np.uintp)
+        mse = np.zeros(max(n, 1), np.float64)
+        self._check(self._L.fic_encode_quadtree_budget_batch(self._h, _lib.FIC_MODE_RGB_QT if rgb else _lib.FIC_MODE_GREY_QT, _ptr(a),
+                                                             n, W, H, b_max, b_min, wk, _ptr(budgets if n else sizes), _ptr(buf),
+                                                             stride, _ptr(sizes), _ptr(mse)))
+        return [buf[i * stride:i * stride + int(sizes[i])].tobytes() for i in range(n)], mse[:n]
+
     def decode_quadtree_batch(self, streams, max_iters: int = 50):
         """fic_decode_quadtree_batch: n quadtree streams of one mode and geometry -> (planes uint8 [n, H, W] or
         [n, 3, H, W], avgError float32 [n], iterations int32 [n]).  The mode and shape come from stream 0's header."""

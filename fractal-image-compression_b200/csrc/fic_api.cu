@@ -185,7 +185,7 @@ void fic_destroy(fic_handle *h)
     Work &w = h->w;
     void *ptrs[] = {w.argb, w.src, w.dec, w.dsum, w.dsq, w.rsum, w.best, w.info, w.q, w.opA, w.opB,
                     w.img, w.dec2, w.dcode, w.perr, w.state, w.dec3, w.replay, w.qt_stream, w.qt_codes, w.qt_err,
-                    w.qt_leaf, w.qt_map};
+                    w.qt_leaf, w.qt_map, w.qt_keys};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (cudaEvent_t ev : {h->call_begin, h->call_end})
@@ -1084,20 +1084,44 @@ int fic_stream_read_codes(const uint8_t *stream, size_t nbytes, int32_t *qcodes)
 // One body per entry for both modes: the mode decides the channel count (the level encodes, the planes in and out) and,
 // inside qt_geom / qt_parse, the header value and the leaf size.
 
+// Budget form's side of h_stage: the first leaves take its first kDecodeBatchMax words, the allowed splits (int64) and the
+// qt_err head (the leaf total, a spare word and a double per image) follow.
+constexpr size_t kQtStageSplits = sizeof(uint32_t) * kDecodeBatchMax, kQtStageHead = kQtStageSplits + sizeof(int64_t) * kDecodeBatchMax;
+static_assert(kQtStageHead + sizeof(uint32_t) * (2 + 2 * kDecodeBatchMax) <= kStageBytes, "a group's budget words fit h_stage");
+
 // Images go up and their streams come down in groups; a group is at most the smallest group any level's plan allows (so
 // every level's run fits its engine's bounds) and at most kDecodeBatchMax images (one grid row and one leaf start of
 // h_stage each).  Per group: one upload, then every level's ordinary grey or RGB batch run (the engine fic_encode_batch_u8
 // would pick, into that level's [n][NR_L] code table; the direct engine image by image), one decimation of the sources for
 // the collage errors, and the stream bodies built on the device (launch_qt_stream).  The leaf counts come down in one
 // small copy, then the bodies in one copy with the caller's stride as pitch.  A single image is the group of one.
+// Budget form (max_bytes non-NULL, one per image): every image's allowed splits go up with its pixels, its max_mse is
+// chosen on the device (launch_qt_stream) and comes down with the leaf total into out_mse[i]; an infeasible budget fails
+// the call before any device work.
 static int encode_quadtree(fic_handle *h, int mode, const uint8_t *planes, int n_images, int W, int H, int b_max, int b_min,
-                           int wk, double max_mse, uint8_t *streams, size_t stride, size_t *stream_bytes)
+                           int wk, double max_mse, uint8_t *streams, size_t stride, size_t *stream_bytes,
+                           const size_t *max_bytes = nullptr, double *out_mse = nullptr)
 {
-    if (max_mse != max_mse) return set_err(h, FIC_E_ARG, "max_mse is NaN");
+    const bool budget = max_bytes != nullptr;
+    if (!budget && max_mse != max_mse) return set_err(h, FIC_E_ARG, "max_mse is NaN");
     QtGeom q;
     const char *why = "";
     int rc = qt_geom(mode, W, H, b_max, b_min, wk, &q, &why);
     if (rc) return set_err(h, rc, "%s", why);
+    if (budget) {
+        int low = -1;  // the lowest image whose budget is below the unsplit tree
+        for (int i = 0; i < n_images; i++)
+            if (qt_budget_splits(q, max_bytes[i]) < 0 && low < 0) low = i;
+        if (low >= 0) {
+            const size_t least = kQtHeaderBytes + (size_t)q.flag_bytes + qt_leaf_bytes(q) * (size_t)q.g[0].NR;
+            for (int i = 0; i < n_images; i++) {
+                stream_bytes[i] = least;
+                out_mse[i] = INFINITY;
+            }
+            if (n_images == 1) return set_err(h, FIC_E_ARG, "max_bytes = %zu is below the unsplit tree's %zu bytes", max_bytes[0], least);
+            return set_err(h, FIC_E_ARG, "image %d: max_bytes = %zu is below the unsplit tree's %zu bytes", low, max_bytes[low], least);
+        }
+    }
     const Geom &fine = q.g[q.nl - 1];
     const size_t C = (size_t)fine.C, S = (size_t)code_stride(fine), image_bytes = C * W * H, body = qt_body_bytes(q);
     size_t bytes;
@@ -1119,13 +1143,21 @@ static int encode_quadtree(fic_handle *h, int mode, const uint8_t *planes, int n
     ENSURE(w.qt_codes, S_QT_CODES, sizeof(int32_t) * S * q.codes * group);
     ENSURE(w.qt_err, S_QT_ERR, sizeof(uint32_t) * qt_err_words(q, group));
     ENSURE(w.qt_stream, S_QT_STREAM, body * group);
+    if (budget) ENSURE(w.qt_keys, S_QT_KEYS, (sizeof(int64_t) + sizeof(uint32_t) * qt_nodes(q)) * group);
     const uint32_t *starts = (const uint32_t *)h->h_stage;
+    // budget form: the allowed splits go up from, and the qt_err head comes down to, h_stage past the first leaves
+    int64_t *h_splits = (int64_t *)(h->h_stage + kQtStageSplits);
+    const uint32_t *head = budget ? (const uint32_t *)(h->h_stage + kQtStageHead) : (const uint32_t *)h->h_acc;
     int too_long = -1;  // the lowest image whose stream does not fit
     DrainOnExit drain(s);
     CU(cudaEventRecord(h->call_begin, s));
     for (int i0 = 0; i0 < n_images; i0 += group) {
         const int gn = n_images - i0 < group ? n_images - i0 : group;
         CU(cudaMemcpyAsync(w.src, planes + i0 * image_bytes, image_bytes * gn, cudaMemcpyHostToDevice, s));
+        if (budget) {
+            for (int i = 0; i < gn; i++) h_splits[i] = qt_budget_splits(q, max_bytes[i0 + i]);
+            CU(cudaMemcpyAsync(w.qt_keys, h_splits, sizeof(int64_t) * gn, cudaMemcpyHostToDevice, s));
+        }
         for (int L = 0; L < q.nl; L++) {
             const Geom &g = q.g[L];
             const int per_run = plan[L].engine == FIC_ENGINE_DIRECT ? 1 : gn;
@@ -1138,14 +1170,15 @@ static int encode_quadtree(fic_handle *h, int mode, const uint8_t *planes, int n
             }
         }
         h->tm.launches += launch_decimate(w.src, w.dec, fine, s, gn);  // the fused engine leaves no decimated plane behind
-        h->tm.launches += launch_qt_stream(w, q, gn, max_mse, s);
+        h->tm.launches += launch_qt_stream(w, q, gn, max_mse, budget, s);
         CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(h->h_acc, w.qt_err, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync((void *)head, w.qt_err, sizeof(uint32_t) * (budget ? qt_head_words(gn) : 1), cudaMemcpyDeviceToHost, s));
         if (gn > 1)  // every image's first leaf: the first of its warp totals after the group's scan
-            CU(cudaMemcpy2DAsync(h->h_stage, sizeof(uint32_t), w.qt_err + 1 + gn * q.flag_bytes, sizeof(uint32_t) * ((q.flag_bytes + 31) / 32),
+            CU(cudaMemcpy2DAsync(h->h_stage, sizeof(uint32_t), w.qt_err + qt_starts_at(q, gn), sizeof(uint32_t) * ((q.flag_bytes + 31) / 32),
                                  sizeof(uint32_t), gn, cudaMemcpyDeviceToHost, s));
         CU(cudaStreamSynchronize(s));
-        const uint32_t total = *(const uint32_t *)h->h_acc;
+        const uint32_t total = head[0];
+        if (budget) memcpy(out_mse + i0, head + 2, sizeof(double) * gn);
         size_t longest = 0;
         for (int i = 0; i < gn; i++) {
             const int64_t leaves = (i + 1 < gn ? starts[i + 1] : total) - (gn > 1 ? starts[i] : 0);
@@ -1327,6 +1360,25 @@ int fic_encode_quadtree_batch(fic_handle *h, int mode, const uint8_t *planes, in
     if (n_images < 1) return set_err(h, FIC_E_ARG, "n_images must be >= 1");
     if (!planes || !streams || !stream_bytes) return set_err(h, FIC_E_ARG, "planes, streams and stream_bytes must be non-NULL");
     return encode_quadtree(h, mode, planes, n_images, W, H, b_max, b_min, wk, max_mse, streams, stride, stream_bytes);
+}
+
+int fic_encode_quadtree_budget(fic_handle *h, int mode, const uint8_t *planes, int W, int H, int b_max, int b_min, int wk,
+                               size_t max_bytes, uint8_t *stream, size_t capacity, size_t *stream_bytes, double *max_mse)
+{
+    if (!h) return FIC_E_ARG;
+    if (!planes || !stream_bytes || !max_mse) return set_err(h, FIC_E_ARG, "planes, stream_bytes and max_mse must be non-NULL");
+    return encode_quadtree(h, mode, planes, 1, W, H, b_max, b_min, wk, 0.0, stream, capacity, stream_bytes, &max_bytes, max_mse);
+}
+
+int fic_encode_quadtree_budget_batch(fic_handle *h, int mode, const uint8_t *planes, int n_images, int W, int H, int b_max,
+                                     int b_min, int wk, const size_t *max_bytes, uint8_t *streams, size_t stride,
+                                     size_t *stream_bytes, double *max_mse)
+{
+    if (!h) return FIC_E_ARG;
+    if (n_images < 1) return set_err(h, FIC_E_ARG, "n_images must be >= 1");
+    if (!planes || !max_bytes || !streams || !stream_bytes || !max_mse)
+        return set_err(h, FIC_E_ARG, "planes, max_bytes, streams, stream_bytes and max_mse must be non-NULL");
+    return encode_quadtree(h, mode, planes, n_images, W, H, b_max, b_min, wk, 0.0, streams, stride, stream_bytes, max_bytes, max_mse);
 }
 
 int fic_decode_quadtree_batch(fic_handle *h, int mode, int n_images, const uint8_t *streams, size_t stride, const size_t *nbytes,

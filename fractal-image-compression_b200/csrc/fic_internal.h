@@ -81,11 +81,12 @@ struct Work {
     int4 *qt_leaf = nullptr;       // decode, per leaf: grey {a, b, domain byte offset, log2 blockgroesse}; RGB two records,
                                    // {a, bR, bG, bB} and {domain byte offset, log2 blockgroesse, 0, 0}
     int32_t *qt_map = nullptr;     // decode: leaf of every b_min x b_min cell, then the first leaf of every top block
+    int64_t *qt_keys = nullptr;    // budget encode: every image's allowed splits K, then its effective keys (qt_nodes each)
     size_t cap[24] = {0};
 };
 
 enum Slot { S_ARGB, S_SRC, S_DEC, S_DSUM, S_DSQ, S_RSUM, S_BEST, S_INFO, S_Q, S_OPA, S_OPB, S_IMG, S_DEC2, S_DCODE, S_PERR, S_STATE, S_DEC3, S_REPLAY, S_QT_STREAM, S_QT_CODES,
-            S_QT_ERR, S_QT_LEAF, S_QT_MAP };
+            S_QT_ERR, S_QT_LEAF, S_QT_MAP, S_QT_KEYS };
 
 // Grows workspace buffer p (its capacity is w.cap[slot]) to at least `bytes`; never shrinks it.
 template <typename T>
@@ -256,16 +257,27 @@ size_t qt_stream_bound(int mode, int W, int H, int b_max, int b_min);
 // NR_top entries): the first leaf of every top block.  check_leaves: also every leaf's domain index against its level's
 // pool.
 int qt_parse(int mode, const uint8_t *stream, size_t nbytes, QtGeom *q, int32_t *base, bool check_leaves, const char **why);
-// Words of Work::qt_err an encode of a group of n images needs.
+// Words of Work::qt_err an encode of a group of n images needs; its first qt_head_words(n): [0] the group's leaf total,
+// [2, 2 + 2n) every image's max_mse as a double (budget form); image i's first leaf sits at
+// w.qt_err[qt_starts_at(q, n) + i * ceil(flag_bytes / 32)].
 size_t qt_err_words(const QtGeom &q, int n);
+size_t qt_head_words(int n);
+size_t qt_starts_at(const QtGeom &q, int n);
+// Split-capable nodes of one image (blocks above b_min): NR_top, 5 NR_top when b_min is two levels down, 0 for one level.
+int64_t qt_nodes(const QtGeom &q);
+// Splits a stream of at most max_bytes can hold, K = (max_bytes - 32 - flag_bytes - leaf_bytes * NR_top) / (3 * leaf_bytes)
+// (capped at INT64_MAX), or -1 when max_bytes is below the unsplit tree's size.
+int64_t qt_budget_splits(const QtGeom &q, size_t max_bytes);
 // Bytes of one image's stream body on the device (flags and the most leaves it can have): the stream bound less the header.
 size_t qt_body_bytes(const QtGeom &q);
 // A group of n images (planes [n][C][H][W] in w.src, decimated planes [n][C][sh][sw] in w.dec, every level's codes in
 // w.qt_codes level-major and image-major: level L of image i at first[L] * n + i * NR_L): collage errors, split flags,
 // leaf scan and leaf scatter into image i's body at w.qt_stream + i * qt_body_bytes (flags at 0, leaves at flag_bytes).
-// The group's leaf total lands in w.qt_err[0] and image i's first leaf (counted over the group) at
-// w.qt_err[1 + n * flag_bytes + i * ceil(flag_bytes / 32)].  n = 1 runs the single-image kernels.
-int launch_qt_stream(const Work &w, const QtGeom &q, int n, double max_mse, cudaStream_t s);
+// The group's leaf total lands in w.qt_err[0] and image i's first leaf (counted over the group) as qt_err_words says.
+// n = 1 runs the single-image kernels.  budget: max_mse is ignored; image i's is the smallest double whose tree needs at
+// most w.qt_keys[i] splits (qt_budget_splits), found on the device from the collage errors (the keys after the n counts
+// in w.qt_keys, n * qt_nodes words) and left in the qt_err head.
+int launch_qt_stream(const Work &w, const QtGeom &q, int n, double max_mse, bool budget, cudaStream_t s);
 // Iterative decode of n streams of one geometry into w.img (C planes per image), copied to planes_out [n][C][H][W].
 // w.qt_stream holds the n images' flag bytes back to back and then every leaf of the group, image after image; w.qt_map
 // holds n cell maps and then n first-leaf tables (NR_top entries each, counted over the group).  Each image's avgError =

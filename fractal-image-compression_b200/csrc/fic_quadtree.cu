@@ -1,8 +1,10 @@
 // fic_quadtree.cu -- the quadtree extension (FIC_MODE_GREY_QT and FIC_MODE_RGB_QT, not in the reference): the stream's
 // geometry and parser, and the kernels that turn every level's codes into the stream body on the device -- the collage
-// error of each range block, the split flags of each top block, the leaf scan and the big-endian leaf scatter.  The
+// error of each range block, the split flags of each top block, the leaf scan and the big-endian leaf scatter; for an
+// encode to a byte budget, the keys and the per-image radix select that choose max_mse on the device.  The
 // per-level encodes are the library's ordinary grey or RGB encodes (fic_encode.cu); the decoder sweep lives with the
 // other sweeps in fic_decode.cu.  The kernels take the channel count C (1 grey, 3 RGB) as a template parameter.
+#include <math.h>
 #include <string.h>
 
 #include "fic_device.cuh"
@@ -84,13 +86,18 @@ int qt_parse(int mode, const uint8_t *s, size_t nbytes, QtGeom *q, int32_t *base
 
 // ---- device: collage error, split flags, leaf scatter --------------------------------------------------------------------
 
-// qt_err layout for a group of n images: [0] leaf total, then the per-top-block in-warp prefixes (n * flag_bytes words),
-// the per-warp totals (n * qt_warps), then the collage errors of every level (level-major, then image-major: level L of
-// image i at n * QtGeom::first[L] + i * NR_L).  An image's top blocks start a new warp, so its prefixes and warp totals
-// are its own; one scan over every warp total of the group gives each image's first leaf at its first warp.
+// qt_err layout for a group of n images: [0] leaf total, [1] unused, [2, 2 + 2n) the budget form's max_mse of every
+// image (doubles, so that they come down in the copy of the leaf total), then the per-top-block in-warp prefixes
+// (n * flag_bytes words), the per-warp totals (n * qt_warps), then the collage errors of every level (level-major, then
+// image-major: level L of image i at n * QtGeom::first[L] + i * NR_L).  An image's top blocks start a new warp, so its
+// prefixes and warp totals are its own; one scan over every warp total of the group gives each image's first leaf at its
+// first warp.
 __host__ __device__ inline int64_t qt_warps(const QtGeom &q) { return (q.flag_bytes + 31) / 32; }
-static int64_t qt_err_at(const QtGeom &q, int n) { return 1 + n * (q.flag_bytes + qt_warps(q)); }
+size_t qt_head_words(int n) { return 2 + 2 * (size_t)n; }
+size_t qt_starts_at(const QtGeom &q, int n) { return qt_head_words(n) + n * q.flag_bytes; }
+static int64_t qt_err_at(const QtGeom &q, int n) { return (int64_t)qt_starts_at(q, n) + n * qt_warps(q); }
 size_t qt_err_words(const QtGeom &q, int n) { return (size_t)(qt_err_at(q, n) + n * q.codes); }
+int64_t qt_nodes(const QtGeom &q) { return q.nl == 1 ? 0 : q.g[0].NR * (q.nl == 3 ? 5 : 1); }
 __host__ __device__ inline int64_t qt_body_pitch(const QtGeom &q) { return q.flag_bytes + (q.g[0].C == 3 ? 20 : 12) * q.g[q.nl - 1].NR; }
 
 // E(j) = sum over range block j (and its C channels) of (decode_px(a, b_c, d_c) - s_c)^2: the code dequantised as the
@@ -152,17 +159,18 @@ __device__ __forceinline__ int64_t qt_at(const QtGeom &q, int L, int64_t j)
 
 // A block above b_min is split iff (double)E > max_mse * (double)(C * B * B).  BATCH: of the CTA's image.
 template <int C, bool BATCH>
-__device__ __forceinline__ bool qt_split(const QtSplit &p, int L, int64_t j)
+__device__ __forceinline__ bool qt_split(const QtSplit &p, double max_mse, int L, int64_t j)
 {
-    return L < p.q.nl - 1 && (double)p.err[qt_at<BATCH>(p.q, L, j)] > __dmul_rn(p.max_mse, (double)(C * p.q.g[L].n));
+    return L < p.q.nl - 1 && (double)p.err[qt_at<BATCH>(p.q, L, j)] > __dmul_rn(max_mse, (double)(C * p.q.g[L].n));
 }
 
 // One thread per top block (and per padding byte of the flags): its flag byte into the stream, its leaf count's
 // exclusive prefix within the warp to pre[t], the warp's total to wsum[warp].  BATCH: image blockIdx.y, whose stream body
 // starts at flags + blockIdx.y * qt_body_pitch and whose prefixes and warp totals are its own (the qt_err layout).
-template <int C, bool BATCH>
+// BUDGET: the image's max_mse is thr[image] (k_qt_select's), not p.max_mse.
+template <int C, bool BATCH, bool BUDGET>
 __global__ void __launch_bounds__(256) k_qt_decide(QtSplit p, uint8_t *__restrict__ flags, uint32_t *__restrict__ pre,
-                                                   uint32_t *__restrict__ wsum)
+                                                   uint32_t *__restrict__ wsum, const double *__restrict__ thr)
 {
     if (BATCH) {
         flags += blockIdx.y * qt_body_pitch(p.q);
@@ -173,10 +181,11 @@ __global__ void __launch_bounds__(256) k_qt_decide(QtSplit p, uint8_t *__restric
     const int lane = threadIdx.x & 31;
     uint32_t n = 0, f = 0;
     if (t < p.q.g[0].NR) {
-        if (qt_split<C, BATCH>(p, 0, t)) {
+        const double m = BUDGET ? thr[BATCH ? blockIdx.y : 0] : p.max_mse;
+        if (qt_split<C, BATCH>(p, m, 0, t)) {
             f = 1;
             for (int k = 0; k < 4; k++)
-                if (qt_split<C, BATCH>(p, 1, qt_child(p.q, 0, t, k))) f |= 2u << k;
+                if (qt_split<C, BATCH>(p, m, 1, qt_child(p.q, 0, t, k))) f |= 2u << k;
         }
         n = (uint32_t)qt_leaf_count(f);
     }
@@ -227,11 +236,124 @@ __global__ void __launch_bounds__(256) k_qt_scatter(QtGeom q, const int32_t *__r
     });
 }
 
-template <int C, bool BATCH>
+// ---- device: the budget form's threshold ---------------------------------------------------------------------------------
+// With N0 = C * b_max^2 and N_L = N0 / s_L^2, s_L = b_max / B_L a power of two, fl(m * N_L) * s_L^2 == fl(m * N0) for every
+// double m (the scaling is exact; where fl(m * N_L) is subnormal or infinite both sides compare alike with the integer
+// keys), so a node of level L splits at m iff fl(m * N0) < E * s_L^2, its key.  A level-1 node splits only if its parent
+// does: its effective key is min(parent's key, own key), and the nodes that split at m are those with effective key >
+// fl(m * N0).  Keys are below 3 * 255^2 * 256 < 2^26.
+
+// One thread per top block: the effective keys of its split-capable nodes, the top block's at t, its four children's
+// (when b_min is two levels down) at NR_top + 4t + k.  Image blockIdx.y's keys at keys + blockIdx.y * qt_nodes.
+__global__ void __launch_bounds__(256) k_qt_keys(QtGeom q, const uint32_t *__restrict__ err, uint32_t *__restrict__ keys)
+{
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, ntop = q.g[0].NR;
+    if (t >= ntop) return;
+    keys += blockIdx.y * ntop * (q.nl == 3 ? 5 : 1);
+    const uint32_t k0 = err[qt_at<true>(q, 0, t)];
+    keys[t] = k0;
+    if (q.nl == 3)
+        for (int k = 0; k < 4; k++) keys[ntop + 4 * t + k] = min(k0, 4u * err[qt_at<true>(q, 1, qt_child(q, 0, t, k))]);
+}
+
+constexpr int kSelThreads = 1024, kSelDigit = 13, kSelBins = 1 << kSelDigit;
+
+// Of the keys whose digit above `shift` equals `prefix`: the histogram of their 13-bit digit at `shift`, then the digit d
+// holding the rank-r key counting from the largest (0-based), and r less the keys above d.  r must be below their count.
+__device__ void qt_select_digit(const uint32_t *__restrict__ keys, int64_t nk, int shift, uint32_t prefix, uint32_t *hist,
+                                uint32_t *part, uint32_t &digit, uint32_t &r)
+{
+    const int tid = threadIdx.x, lane = tid & 31;
+    for (int b = tid; b < kSelBins; b += kSelThreads) hist[b] = 0;
+    __syncthreads();
+    for (int64_t j0 = tid - lane; j0 < nk; j0 += kSelThreads) {  // warp-uniform trips
+        const int64_t j = j0 + lane;
+        const uint32_t k = j < nk ? keys[j] : 0u;
+        const bool in = j < nk && (k >> shift >> kSelDigit) == prefix;
+        const uint32_t bin = in ? (k >> shift) & (kSelBins - 1) : kSelBins;
+        const uint32_t peers = __match_any_sync(0xffffffffu, bin);  // flat images: many equal keys, one atomic
+        if (in && lane == __ffs(peers) - 1) atomicAdd(&hist[bin], __popc(peers));
+    }
+    __syncthreads();
+    // Thread tid owns the 8 bins below kSelBins - 8 * tid: a suffix count over threads finds the owner of rank r.
+    constexpr int per = kSelBins / kSelThreads;
+    const int top = kSelBins - 1 - per * tid;
+    uint32_t own = 0;
+    for (int b = 0; b < per; b++) own += hist[top - b];
+    uint32_t incl = own;
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += v;
+    }
+    if (lane == 31) part[tid >> 5] = incl;
+    __syncthreads();
+    uint32_t before = 0;  // keys in the bins of lower-numbered threads (larger digits)
+    for (int wi = 0; wi < (tid >> 5); wi++) before += part[wi];
+    before += incl - own;
+    const uint32_t want = r;
+    __syncthreads();
+    if (want >= before && want < before + own) {
+        uint32_t c = before;
+        for (int b = 0; b < per; b++) {
+            const uint32_t hb = hist[top - b];
+            if (want < c + hb) {
+                part[32] = (uint32_t)(top - b);
+                part[33] = want - c;
+                break;
+            }
+            c += hb;
+        }
+    }
+    __syncthreads();
+    digit = part[32];
+    r = part[33];
+    __syncthreads();
+}
+
+// One CTA per image of the group: the image's max_mse m* = the smallest double with fl(m* * N0) >= v, v the (K+1)-th
+// largest effective key (K = kq[image], the splits the budget allows), by a two-digit radix select over the keys; -inf
+// when there are at most K keys; +0.0 when v == 0.  Into thr[image].
+__global__ void __launch_bounds__(kSelThreads) k_qt_select(const uint32_t *__restrict__ keys, int64_t nk, const int64_t *__restrict__ kq,
+                                                           double N0, double *__restrict__ thr)
+{
+    __shared__ uint32_t hist[kSelBins], part[34];
+    const int i = blockIdx.x;
+    const int64_t K = kq[i];
+    if (K >= nk) {
+        if (threadIdx.x == 0) thr[i] = -INFINITY;
+        return;
+    }
+    keys += i * nk;
+    uint32_t hi, lo, r = (uint32_t)K;
+    qt_select_digit(keys, nk, kSelDigit, 0, hist, part, hi, r);
+    qt_select_digit(keys, nk, 0, hi, hist, part, lo, r);
+    if (threadIdx.x) return;
+    const double v = (double)(hi << kSelDigit | lo);
+    double m = 0.0;
+    if (v > 0) {  // v / N0 is exact for grey (N0 a power of two); RGB's N0 = 3 * 4^k may need a step of an ulp
+        m = __ddiv_rn(v, N0);  // positive: an ulp step is +-1 on its bits
+        while (__dmul_rn(m, N0) < v) m = __longlong_as_double(__double_as_longlong(m) + 1);
+        for (double d = __longlong_as_double(__double_as_longlong(m) - 1); __dmul_rn(d, N0) >= v;
+             d = __longlong_as_double(__double_as_longlong(m) - 1))
+            m = d;
+    }
+    thr[i] = m;
+}
+
+int64_t qt_budget_splits(const QtGeom &q, size_t max_bytes)
+{
+    const size_t leaf = qt_leaf_bytes(q), least = kQtHeaderBytes + (size_t)q.flag_bytes + leaf * (size_t)q.g[0].NR;
+    if (max_bytes < least) return -1;
+    const size_t k = (max_bytes - least) / (3 * leaf);
+    return k > (size_t)INT64_MAX ? INT64_MAX : (int64_t)k;
+}
+
+template <int C, bool BATCH, bool BUDGET>
 static int launch_qt_stream_c(const Work &w, const QtGeom &q, int n, double max_mse, cudaStream_t s)
 {
     constexpr int S = C == 1 ? 3 : 5;
-    uint32_t *total = w.qt_err, *pre = w.qt_err + 1, *wsum = pre + n * q.flag_bytes, *err = w.qt_err + qt_err_at(q, n);
+    uint32_t *total = w.qt_err, *pre = w.qt_err + qt_head_words(n), *wsum = pre + n * q.flag_bytes, *err = w.qt_err + qt_err_at(q, n);
+    double *thr = (double *)(w.qt_err + 2);
     int launches = 0;
     for (int L = 0; L < q.nl; L++) {
         const Geom &g = q.g[L];
@@ -240,18 +362,32 @@ static int launch_qt_stream_c(const Work &w, const QtGeom &q, int n, double max_
                                                                                              err + n * q.first[L], g);
         launches++;
     }
+    if (BUDGET) {
+        const int64_t nk = qt_nodes(q);
+        uint32_t *keys = (uint32_t *)(w.qt_keys + n);
+        if (nk) k_qt_keys<<<dim3((unsigned)((q.g[0].NR + 255) / 256), n), 256, 0, s>>>(q, err, keys);
+        k_qt_select<<<n, kSelThreads, 0, s>>>(keys, nk, w.qt_keys, (double)(C * q.g[0].n), thr);
+        launches += 1 + (nk > 0);
+    }
     const QtSplit p = {q, err, max_mse};
-    k_qt_decide<C, BATCH><<<dim3((unsigned)((q.flag_bytes + 255) / 256), n), 256, 0, s>>>(p, w.qt_stream, pre, wsum);
+    k_qt_decide<C, BATCH, BUDGET><<<dim3((unsigned)((q.flag_bytes + 255) / 256), n), 256, 0, s>>>(p, w.qt_stream, pre, wsum, thr);
     launches += 1 + launch_scan_u32(wsum, n * qt_warps(q), total, s);
     k_qt_scatter<C, BATCH><<<dim3((unsigned)((q.g[0].NR + 255) / 256), n), 256, 0, s>>>(q, w.qt_codes, w.qt_stream, pre, wsum,
                                                                                        (uint32_t *)(w.qt_stream + q.flag_bytes));
     return launches + 1;
 }
 
-int launch_qt_stream(const Work &w, const QtGeom &q, int n, double max_mse, cudaStream_t s)
+template <bool BUDGET>
+static int launch_qt_stream_b(const Work &w, const QtGeom &q, int n, double max_mse, cudaStream_t s)
 {
-    if (n == 1) return q.g[0].C == 3 ? launch_qt_stream_c<3, false>(w, q, 1, max_mse, s) : launch_qt_stream_c<1, false>(w, q, 1, max_mse, s);
-    return q.g[0].C == 3 ? launch_qt_stream_c<3, true>(w, q, n, max_mse, s) : launch_qt_stream_c<1, true>(w, q, n, max_mse, s);
+    if (n == 1)
+        return q.g[0].C == 3 ? launch_qt_stream_c<3, false, BUDGET>(w, q, 1, max_mse, s) : launch_qt_stream_c<1, false, BUDGET>(w, q, 1, max_mse, s);
+    return q.g[0].C == 3 ? launch_qt_stream_c<3, true, BUDGET>(w, q, n, max_mse, s) : launch_qt_stream_c<1, true, BUDGET>(w, q, n, max_mse, s);
+}
+
+int launch_qt_stream(const Work &w, const QtGeom &q, int n, double max_mse, bool budget, cudaStream_t s)
+{
+    return budget ? launch_qt_stream_b<true>(w, q, n, max_mse, s) : launch_qt_stream_b<false>(w, q, n, max_mse, s);
 }
 
 size_t qt_body_bytes(const QtGeom &q) { return (size_t)qt_body_pitch(q); }

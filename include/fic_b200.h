@@ -323,6 +323,33 @@ int fic_encode_quadtree_batch(fic_handle *h, int mode, const uint8_t *planes, in
 int fic_decode_quadtree_batch(fic_handle *h, int mode, int n_images, const uint8_t *streams, size_t stride,
                               const size_t *nbytes, int max_iters, uint8_t *planes_out, float *avg_error, int *iterations);
 
+/* Quadtree to a byte budget (EXTENSION): the finest tree of the max_mse family whose stream fits max_bytes, mode
+ * FIC_MODE_GREY_QT or FIC_MODE_RGB_QT, planes as in the entries above.  size(m), the size of the stream
+ * fic_encode_quadtree[_rgb] writes at max_mse = m, is non-increasing in m (the split rule (double)E > m * (double)N_L,
+ * N_L = C * B_L^2, is monotone in m).  The entry writes exactly the stream fic_encode_quadtree[_rgb] writes on this
+ * handle with the same options at max_mse = m*, and reports m* in *max_mse: the smallest double m with
+ * size(m) <= max_bytes; -inf when the fully split tree fits; +0.0 (never -0.0) when the answer lies at zero.
+ * Equivalently: the stream fits, and either m* = -inf or the stream at nextafter(m*, -inf) does not fit.  Blocks whose
+ * collage errors give the same threshold join or leave the tree together, so the stream may be well under the budget
+ * (a flat or tiled image has large groups of equal errors).
+ *
+ * m* is chosen on the device from the collage errors of the one encode: a node of level L splits at m iff
+ * fl(m * C * b_max^2) < E * (b_max / B_L)^2 (scaling by a power of two is exact), a level-1 node only if its parent does,
+ * so the tree that fits is a selection of the K + 1 largest such keys, K the splits the budget allows.
+ *
+ * max_bytes below the unsplit tree's size, 32 + pad4(NR_top) + leaf_bytes * NR_top (leaf_bytes 12 grey, 20 RGB), is
+ * FIC_E_ARG before any device work, with that size in *stream_bytes and +inf in *max_mse.  Capacity (stride in the
+ * batch) as the other encodes: the size needed is reported with FIC_E_ARG; min(max_bytes,
+ * fic_quadtree[_rgb]_stream_bound(W, H, b_max, b_min)) always suffices.  Batch: max_bytes[i] and max_mse[i] per image,
+ * image i's outputs equal the single entry's for that image; an infeasible budget anywhere fails the whole batch before
+ * device work, with the minimum size in every stream_bytes[i] (fic_last_error names the lowest such image).
+ * fic_get_timings as the quadtree encodes. */
+int fic_encode_quadtree_budget(fic_handle *h, int mode, const uint8_t *planes, int W, int H, int b_max, int b_min, int wk,
+                               size_t max_bytes, uint8_t *stream, size_t capacity, size_t *stream_bytes, double *max_mse);
+int fic_encode_quadtree_budget_batch(fic_handle *h, int mode, const uint8_t *planes, int n_images, int W, int H, int b_max,
+                                     int b_min, int wk, const size_t *max_bytes, uint8_t *streams, size_t stride,
+                                     size_t *stream_bytes, double *max_mse);
+
 /* ---- multi-GPU: the same encode over several GPUs of one node (SURVEY 8b, 8e) --- */
 
 /* Replaces the same reference loops (FC:119 + FC:125-159, FC:181 + FC:186-215) with the range-block rows sharded
